@@ -8,6 +8,7 @@ log_blowup 1): stage-1 `pcs.commit` (reference src/prover.rs:350) and stage-2 `p
 
   python bench.py [--gpus N] [--steps K] [--warmup W]       our CUDA path (one JSON line on rank 0)
   python bench.py --impl reference ...                      CPU restatement of the reference path
+  python bench.py ... --dump-outputs DIR                    also write the last timed step's outputs (see dump_commit)
 
 metric = LDE+Merkle Gelem/s (committed LDE elements sum(n*B*w) per second, whole job).
 `value`: inputs resident in HBM.  `e2e`: through the host-pointer C-ABI call (`msgpu_commit`) with
@@ -135,6 +136,39 @@ def merkle_bytes(stages, log_blowup):
         tot += sum(8 * (m.shape[0] << log_blowup) * m.shape[1] + 32 * (m.shape[0] << log_blowup) for m in st)
         tot += 96 * (nb - 1)
     return tot
+
+
+# ------------------------------------------------------------------------------------------------
+# --dump-outputs: what the timed path hands its caller, so that two builds can be compared output for output. Every value
+# is an exact integer stored as float64: a byte as it is, a 64-bit field element as [low 32 bits, high 32 bits].
+# ------------------------------------------------------------------------------------------------
+DUMP_ROWS = 4096  # rows kept of each tall LDE matrix: 43 columns x 4096 rows x 16 bytes = 2.8 MB in all
+
+
+def u64_halves(a):
+    a = np.asarray(a, dtype=np.uint64)
+    return np.stack([a & np.uint64(0xFFFFFFFF), a >> np.uint64(32)], axis=-1).astype(np.float64)
+
+
+def dump_commit(out_dir, pds):
+    """The ProverData of one step's commitments (stage s = 1, 2): stage{s}_root, the 32 root bytes, and for every committed
+    matrix i (LDE rows in bit-reversed order, as ProverData holds them) stage{s}_lde{i}, the rows listed in stage{s}_lde{i}_rows:
+    all rows of a matrix of at most DUMP_ROWS rows, else DUMP_ROWS rows drawn with the fixed seed (s, i)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for s, pd in enumerate(pds, 1):
+        np.save(os.path.join(out_dir, "stage%d_root.npy" % s), np.asarray(pd.root, dtype=np.float64))
+        for i in range(pd.num_matrices):
+            lde = pd.read_rows(i)
+            rows = np.arange(len(lde)) if len(lde) <= DUMP_ROWS else np.sort(
+                np.random.default_rng([s, i]).choice(len(lde), DUMP_ROWS, replace=False))
+            np.save(os.path.join(out_dir, "stage%d_lde%d.npy" % (s, i)), u64_halves(lde[rows]))
+            np.save(os.path.join(out_dir, "stage%d_lde%d_rows.npy" % (s, i)), rows.astype(np.float64))
+
+
+def dump_proof(out_dir, name, proof):
+    """Proof::to_bytes of a prove() leg's last timed call, one float64 per byte."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), np.frombuffer(proof, dtype=np.uint8).astype(np.float64))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -318,7 +352,8 @@ def prove_stage_bytes(log_rows, log_blowup):
 
 
 def gpu_prove_leg(args, ms, ctx, log_rows, steps, warmup, verify, peak=None):
-    """prove() end to end through the public API: HOST (pinned) traces and claims in, Proof::to_bytes out."""
+    """prove() end to end through the public API: HOST (pinned) traces and claims in, Proof::to_bytes out.
+    Returns (results, the proof of the last timed call)."""
     system = ms.System("u32_add", **prove_params(args))
     prover = ms.Prover(ctx, system)  # System::new: programs + preprocessed commitment (setup, untimed like Criterion's setup)
     byte, add, claims = u32_add_traces(log_rows)
@@ -364,10 +399,10 @@ def gpu_prove_leg(args, ms, ctx, log_rows, steps, warmup, verify, peak=None):
         out["verified"] = S.verify(list(claims), proof) == "Ok"
         S.close()
     prover.close()
-    return out
+    return out, proof
 
 
-def sharded_prove_leg(args, ms, msd, ctx, rank, world, steps=4):
+def sharded_prove_leg(args, ms, msd, ctx, rank, world, steps):
     """ONE proof over all ranks (BASELINE configs[3] shape, SURVEY 8e partitioning A): byte table + 7 U32-add circuits of
     2^18..2^22 rows, circuits -> ranks by height class; compared with the same proof on one GPU (rank 0)."""
     import hashlib
@@ -448,7 +483,7 @@ def rowshard_commit_leg(args, ms, msd, ctx, rs, rank, world, steps, warmup):
     return out["resident"], out["host"], roots, sum(b.nbytes for st in blocks for b in st)
 
 
-def rowshard_prove_leg(args, ms, msd, ctx, rank, world, kind, log_heights, steps=3):
+def rowshard_prove_leg(args, ms, msd, ctx, rank, world, kind, log_heights, steps):
     """ONE proof over the row shards of every matrix, all ranks (kind "u32_add": one circuit of 2^log_heights[0] rows; "multi:K":
     BASELINE configs[3] shape). Compared with the same proof on one GPU (rank 0): the bytes must be identical."""
     import hashlib
@@ -560,7 +595,13 @@ def main():
     ap.add_argument("--cpu-prove-log-rows", type=int, default=20, help="rows of the CPU prove() baseline (default: the GPU leg's)")
     ap.add_argument("--big-log-rows", type=int, default=22, help="second prove() leg, GPU and CPU (north_star: 2^22 rows); 0 = off")
     ap.add_argument("--no-prove", action="store_true", help="skip the prove() leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy "
+                    "(commitment roots, a seeded sample of the LDE rows, proof bytes)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path; it has no meaning with --impl reference")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -595,12 +636,15 @@ def main():
     resident_args = [[(t.data_ptr(), t.shape[0], t.shape[1]) for t in st] for st in resident]
     torch.cuda.synchronize()
 
-    def step_resident():
+    def step_resident(keep=None):
         roots = []
         for st in resident_args:
             root, pd = pcs.commit_dev(st)
             roots.append(bytes(root))
-            pd.free()
+            if keep is None:
+                pd.free()
+            else:
+                keep.append(pd)
         return roots
 
     def step_e2e_serial():
@@ -636,15 +680,16 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
-    def timed(fn, steps, profile=False):
+    def timed(fn, steps, profile=False, last=None):
+        """`last`, if given, runs in place of `fn` as the final timed step."""
         barrier()
         if profile:
             ctx.profile_begin()
         l0 = ctx.launches
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        for _ in range(steps):
-            out = fn()
+        for i in range(steps):
+            out = last() if last is not None and i == steps - 1 else fn()
         e1.record()
         torch.cuda.synchronize()
         ms_total = e0.elapsed_time(e1)
@@ -666,11 +711,17 @@ def main():
     t_s = time.perf_counter()
     while len(sampler.lines) < 1 and time.perf_counter() - t_s < 3.0:  # nvidia-smi needs ~0.5 s to print its first sample
         step_resident()
-    ms_res, launches, prof, _ = timed(step_resident, args.steps, profile=True)
+    kept = []  # ProverData of the last timed step, kept for --dump-outputs
+    ms_res, launches, prof, _ = timed(step_resident, args.steps, profile=True,
+                                      last=(lambda: step_resident(keep=kept)) if args.dump_outputs else None)
+    if kept:
+        if rank == 0:
+            dump_commit(args.dump_outputs, kept)
+        for pd in kept:
+            pd.free()
     ms_e2e, _, _, _ = timed(step_e2e, args.steps)
     e2e_drain()
-    ms_e2e_serial, _, _, _ = timed(step_e2e_serial, max(3, args.steps // 2))
-    ms_e2e_serial *= args.steps / max(3, args.steps // 2)
+    ms_e2e_serial, _, _, _ = timed(step_e2e_serial, args.steps)
     t_s = time.perf_counter()
     while len(sampler.lines) < 8 and time.perf_counter() - t_s < 2.0:  # same kernels, untimed: enough samples under load
         step_resident()
@@ -781,7 +832,9 @@ def main():
     prove = prove_big = None
     if not args.no_prove:
         barrier()
-        prove = gpu_prove_leg(args, ms, ctx, args.log_rows, steps=max(3, min(args.steps, 10)), warmup=2, verify=(rank == 0), peak=peak)
+        prove, proof = gpu_prove_leg(args, ms, ctx, args.log_rows, steps=args.steps, warmup=2, verify=(rank == 0), peak=peak)
+        if args.dump_outputs and rank == 0:
+            dump_proof(args.dump_outputs, "prove_proof", proof)
         if world > 1:
             prove["ms_max_over_ranks"] = msd.max_over_ranks(prove["ms"])
             prove["proofs_per_s_all_ranks"] = world * 1e3 / prove["ms_max_over_ranks"]
@@ -794,19 +847,21 @@ def main():
         barrier()
         # north_star: prove() at 2^22 rows against the host-core parallel CPU prover, both measured here
         if world == 1 and args.big_log_rows > args.log_rows:
-            prove_big = gpu_prove_leg(args, ms, ctx, args.big_log_rows, steps=3, warmup=1, verify=(rank == 0), peak=peak)
+            prove_big, proof = gpu_prove_leg(args, ms, ctx, args.big_log_rows, steps=args.steps, warmup=1, verify=(rank == 0), peak=peak)
+            if args.dump_outputs:
+                dump_proof(args.dump_outputs, "prove_big_proof", proof)
             if cpu is not None:
                 prove_big["cpu"] = cpu_prove_time(args, args.big_log_rows)
                 prove_big["identical_to_cpu_proof"] = prove_big["cpu"]["digest"] == prove_big["digest"]
                 prove_big["speedup_vs_cpu_port"] = prove_big["cpu"]["ms"] / prove_big["ms"]
         if world > 1:
-            prove["sharded"] = sharded_prove_leg(args, ms, msd, ctx, rank, world)
+            prove["sharded"] = sharded_prove_leg(args, ms, msd, ctx, rank, world, args.steps)
             # every matrix split by rows over all ranks: one tall circuit (2^log_rows and 2^big rows) and the 7-circuit system
-            prove["rowshard"] = rowshard_prove_leg(args, ms, msd, ctx, rank, world, "u32_add", [args.log_rows])
+            prove["rowshard"] = rowshard_prove_leg(args, ms, msd, ctx, rank, world, "u32_add", [args.log_rows], args.steps)
             if args.big_log_rows > args.log_rows:
-                prove_big = rowshard_prove_leg(args, ms, msd, ctx, rank, world, "u32_add", [args.big_log_rows])
+                prove_big = rowshard_prove_leg(args, ms, msd, ctx, rank, world, "u32_add", [args.big_log_rows], args.steps)
             lhs = [min(h, args.log_rows + 2) for h in (22, 21, 21, 20, 20, 19, 18)]
-            prove["rowshard_multi7"] = rowshard_prove_leg(args, ms, msd, ctx, rank, world, "multi:7", lhs)
+            prove["rowshard_multi7"] = rowshard_prove_leg(args, ms, msd, ctx, rank, world, "multi:7", lhs, args.steps)
 
     if rank == 0:
         if roofline is not None and prove is not None and prove.get("stage_roofline"):
