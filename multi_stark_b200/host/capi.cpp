@@ -201,20 +201,16 @@ int msh_rowshard_commit(msh_prover* p, const uint64_t* const* mats, const uint64
         auto* be = dynamic_cast<RowShardBackend*>(p->backend.get());
         if (!be) throw std::runtime_error("not a row-sharded prover");
         std::vector<RowBlocks> blocks;
-        struct Free {
-            RowShardBackend* b; std::vector<RowBlocks>& v; bool on;
-            ~Free() { if (on) for (auto& x : v) b->free_blocks(x); }
-        } fr{be, blocks, host != 0};
         for (uint64_t i = 0; i < n; i++) {
             if (host) {
                 blocks.push_back(be->upload_blocks(mats[i], (size_t)heights[i], (size_t)widths[i]));
-            } else {
+            } else {  // borrowed: the caller's device buffers
                 RowBlocks b;
                 b.height = (size_t)heights[i];
                 b.width = (size_t)widths[i];
                 b.whole = !be->shardable(b.height, b.width);
-                b.dev = (uint64_t*)mats[i];
-                blocks.push_back(b);
+                b.dev = mats[i];
+                blocks.push_back(std::move(b));
             }
         }
         Digest root{};
@@ -339,7 +335,7 @@ int msh_pcs_open(msgpu_ctx* ctx, msh_challenger* c, uint64_t n_rounds, msgpu_pda
         std::vector<OpenRound> rounds;
         size_t mi = 0, pi = 0;
         for (uint64_t r = 0; r < n_rounds; r++) {
-            handles.push_back(std::make_unique<GpuPcsHandle>(pds[r], /*owns=*/false));
+            handles.push_back(std::make_unique<GpuPcsHandle>(pds[r]));  // borrowed
             OpenRound rd;
             rd.data = handles.back().get();
             for (size_t m = 0; m < handles.back()->num_matrices(); m++) {

@@ -63,6 +63,15 @@ struct CommView {
     void sendrecv_dev(void* dev, size_t bytes, int src, int dst) const {
         if (c.sendrecv_dev(c.user, dev, bytes, src, dst) != 0) throw DistError("comm: device send/recv failed");
     }
+    void alltoall_dev(void* send, const uint64_t* send_bytes, void* recv, const uint64_t* recv_bytes) const {
+        if (!c.alltoall_dev) throw DistError("comm: the communicator has no device all-to-all");
+        if (c.alltoall_dev(c.user, send, send_bytes, recv, recv_bytes) != 0) throw DistError("comm: device all-to-all failed");
+    }
+    // recv holds world() chunks of `bytes` in rank order; chunk rank() is `send`
+    void allgather_dev(void* send, void* recv, uint64_t bytes) const {
+        if (!c.allgather_dev) throw DistError("comm: the communicator has no device all-gather");
+        if (bytes && c.allgather_dev(c.user, send, recv, bytes) != 0) throw DistError("comm: device all-gather failed");
+    }
     // all-gather of byte strings of different lengths
     std::vector<std::vector<u8>> allgather_var(const std::vector<u8>& mine) const {
         std::vector<uint64_t> sizes(world());
@@ -79,22 +88,130 @@ struct CommView {
     }
 };
 
+// MSH_TRACE=2: one line per protocol step and rank on stderr (a rank that stops printing is where a multi-GPU run hangs)
+inline void rs_trace(int rank, const char* what, size_t a = 0, size_t b = 0) {
+    static const bool on = getenv("MSH_TRACE") && atoi(getenv("MSH_TRACE")) >= 2;
+    if (on) {
+        fprintf(stderr, "[rs %d] %s %zu %zu\n", rank, what, a, b);
+        fflush(stderr);
+    }
+}
+
+// What the circuit-sharded and the row-sharded backends share: the communicator, and the claims (global, not sharded), which
+// ONE rank uploads, hashes and accumulates -- the others receive 32 + 16 bytes. Each backend picks claims_rank_ in commit_stage1.
+class ShardedBackend : public GpuBackend {
+  public:
+    bool observe_claims(Challenger& ch, const ClaimsView& claims) override {
+        if (!claims_on_device(claims)) return GpuBackend::observe_claims(ch, claims);  // small set: every rank runs the host loop
+        Digest d{};
+        if (comm_.rank() == claims_rank_ && !claims_transcript_digest(ch.input_buffer(), claims, d))
+            throw DistError("claims: internal error, device path refused");
+        comm_.bcast(d.data(), 32, claims_rank_);
+        ch.set_flushed(d);
+        return true;
+    }
+    Fp2 claims_accumulator(const ClaimsView& claims, Fp2 beta, Fp2 gamma) override {
+        if (!claims_on_device(claims)) return GpuBackend::claims_accumulator(claims, beta, gamma);
+        uint64_t out[2] = {0, 0};
+        if (comm_.rank() == claims_rank_) {
+            Fp2 a = GpuBackend::claims_accumulator(claims, beta, gamma);
+            out[0] = a.c[0].v;
+            out[1] = a.c[1].v;
+        }
+        comm_.bcast(out, 16, claims_rank_);
+        return Fp2(Fp(out[0]), Fp(out[1]));
+    }
+
+  protected:
+    ShardedBackend(msgpu_ctx* ctx, const SystemShape& shape, const msh_comm& comm) : GpuBackend(ctx, shape), comm_{comm} {}
+    CommView comm_;
+    int claims_rank_ = 0;
+};
+
+// What the two sharded open devices share: the FRI owner runs the commit phase alone, and every other rank replays the
+// transcript from ONE broadcast of (roots, PoW witnesses, folded vector): the number of rounds and every length are known from
+// the shapes alone.
+class ShardedOpenDevice : public OpenDevice {
+  public:
+    ~ShardedOpenDevice() override {
+        if (op_) msgpu_open_free(op_);
+    }
+    size_t current_len() override { return cur_len_; }
+    // FRI owner only
+    Digest commit_round() override {
+        Digest d{};
+        gpu_check(msgpu_fri_commit_round(op_, d.data()));
+        return d;
+    }
+    void fold(Fp2 beta) override {
+        uint64_t b[2] = {beta.c[0].v, beta.c[1].v};
+        gpu_check(msgpu_fri_fold(op_, b));
+        cur_len_ /= 2;
+    }
+    void commit_phase(Challenger& ch, size_t stop_len, size_t pow_bits, FriProof& proof) override {
+        size_t rounds = 0;
+        for (size_t l = cur_len_; l > stop_len; l >>= 1) rounds++;
+        const size_t final_len = cur_len_ >> rounds;
+        std::vector<u8> blob(rounds * 40 + final_len * 16);
+        rs_trace(comm_.rank(), "fri commit phase", rounds);
+        if (comm_.rank() == fri_owner_) {
+            owner_commit_phase(ch, stop_len, pow_bits, proof);
+            if (proof.commit_phase_commits.size() != rounds) throw DistError("fri: internal error, round count");
+            for (size_t k = 0; k < rounds; k++) {
+                memcpy(blob.data() + 40 * k, proof.commit_phase_commits[k].data(), 32);
+                memcpy(blob.data() + 40 * k + 32, &proof.commit_pow_witnesses[k].v, 8);
+            }
+            gpu_check(msgpu_fri_read_current(op_, (uint64_t*)(blob.data() + rounds * 40)));
+        }
+        comm_.bcast(blob.data(), blob.size(), fri_owner_);
+        if (comm_.rank() != fri_owner_) {
+            for (size_t k = 0; k < rounds; k++) {
+                Digest d;
+                Fp w;
+                memcpy(d.data(), blob.data() + 40 * k, 32);
+                memcpy(&w.v, blob.data() + 40 * k + 32, 8);
+                ch.observe(d);
+                proof.commit_phase_commits.push_back(d);
+                if (!ch.check_witness(pow_bits, w)) throw DistError("fri: the owner's proof-of-work witness does not verify");
+                proof.commit_pow_witnesses.push_back(w);
+                betas.push_back(ch.sample_ext());
+            }
+        }
+        cur_len_ = final_len;
+        folded_.resize(final_len);
+        const uint64_t* f = (const uint64_t*)(blob.data() + rounds * 40);
+        for (size_t i = 0; i < final_len; i++) { folded_[i].c[0].v = f[2 * i]; folded_[i].c[1].v = f[2 * i + 1]; }
+    }
+    std::vector<Fp2> read_current() override { return folded_; }
+
+  protected:
+    ShardedOpenDevice(msgpu_ctx* ctx, const CommView& comm, const std::vector<OpenRound>& rounds) : ctx_(ctx), comm_(comm), rounds_(rounds) {}
+    // the FRI owner's rounds (the host loop unless overridden)
+    virtual void owner_commit_phase(Challenger& ch, size_t stop_len, size_t pow_bits, FriProof& proof) {
+        OpenDevice::commit_phase(ch, stop_len, pow_bits, proof);
+    }
+    msgpu_ctx* ctx_;
+    CommView comm_;
+    std::vector<OpenRound> rounds_;
+    msgpu_open* op_ = nullptr;
+    int fri_owner_ = 0;
+    unsigned log_max_height_ = 0;
+    size_t cur_len_ = 0;
+    std::vector<Fp2> folded_;
+};
+
 // Pcs::ProverData of a sharded commitment.
 struct DistPcsHandle : PcsHandle {
     std::vector<std::pair<size_t, size_t>> shapes;  // every matrix of the commitment: (LDE height, width), commit order
     std::vector<int> owner;                         // rank holding matrix i
     std::vector<int> local_index;                   // index inside `local`, -1 if the matrix lives elsewhere
-    msgpu_pdata* local = nullptr;                   // this rank's matrices (rows, no tree); null if it has none
-    msgpu_pdata* tree = nullptr;                    // digest layers, on the tree owner only
+    PdataPtr local;                                 // this rank's matrices (rows, no tree); null if it has none
+    PdataPtr tree;                                  // digest layers, on the tree owner only
     int tree_owner = 0;
-    ~DistPcsHandle() override {
-        if (local) msgpu_pdata_free(local);
-        if (tree) msgpu_pdata_free(tree);
-    }
     size_t num_matrices() const override { return shapes.size(); }
     size_t matrix_height(size_t i) const override { return shapes[i].first; }
     size_t matrix_width(size_t i) const override { return shapes[i].second; }
-    size_t local_max_height() const { return local ? (size_t)msgpu_pdata_max_height(local) : 0; }
+    size_t local_max_height() const { return local ? (size_t)msgpu_pdata_max_height(local.get()) : 0; }
     std::vector<size_t> matrices_of(int rank) const {
         std::vector<size_t> v;
         for (size_t i = 0; i < owner.size(); i++)
@@ -123,17 +240,17 @@ struct DistMatrix {
     uint64_t* dev;  // on the owner
 };
 
-// Pcs::commit / commit_ldes over the ranks. Adopts `dev` buffers when inputs_are_ldes.
-// `prebuilt_local`: the local part already built from `mats` (msgpu_commit_upload with local_only = 1), adopted.
+// Pcs::commit / commit_ldes over the ranks. `ldes` (commit_ldes): this rank's LDE buffers in commit order, released to the
+// prover data once it has adopted them. `local`: the local part already built from `mats` (msgpu_commit_upload with
+// local_only = 1).
 inline std::shared_ptr<DistPcsHandle> dist_commit(msgpu_ctx* ctx, const CommView& comm, const std::vector<DistMatrix>& mats, uint32_t log_blowup,
-                                                  bool inputs_are_ldes, Digest& root, msgpu_pdata* prebuilt_local = nullptr,
-                                                  bool* ldes_adopted = nullptr) {
+                                                  Digest& root, PdataPtr local = nullptr, std::vector<DevBuf>* ldes = nullptr) {
     auto h = std::make_shared<DistPcsHandle>();
-    h->local = prebuilt_local;  // adopted first: released with the handle on every error path
+    h->local = std::move(local);
     std::vector<uint64_t*> ptrs;
     std::vector<uint64_t> hs, ws;
     for (auto& m : mats) {
-        h->shapes.push_back({inputs_are_ldes ? m.height : (m.height << log_blowup), m.width});
+        h->shapes.push_back({ldes ? m.height : (m.height << log_blowup), m.width});
         h->owner.push_back(m.owner);
         if (m.owner == comm.rank()) {
             h->local_index.push_back((int)ptrs.size());
@@ -147,56 +264,58 @@ inline std::shared_ptr<DistPcsHandle> dist_commit(msgpu_ctx* ctx, const CommView
     if (mats.empty()) throw DistError("commit: no matrices given");
     auto cls = class_owners(h->shapes, h->owner);
     h->tree_owner = cls.begin()->second;
-    if (!prebuilt_local && !ptrs.empty()) gpu_check(msgpu_commit_local_dev(ctx, ptrs.data(), hs.data(), ws.data(), ptrs.size(), log_blowup, inputs_are_ldes ? 1 : 0, &h->local));
-    // from here on the handle owns the LDE buffers it was given (released with it on every later error path): the caller
-    // must not free them again -- the arena knows blocks by address only, and a released address may already be live elsewhere
-    if (ldes_adopted) *ldes_adopted = inputs_are_ldes && h->local != nullptr;
+    if (!h->local && !ptrs.empty()) {
+        msgpu_pdata* pd = nullptr;
+        gpu_check(msgpu_commit_local_dev(ctx, ptrs.data(), hs.data(), ws.data(), ptrs.size(), log_blowup, ldes ? 1 : 0, &pd));
+        h->local.reset(pd);
+        // adopted only on success: from here on the handle releases them, and the caller must not -- the arena knows blocks by
+        // address only, and a released address may already be live elsewhere
+        if (ldes)
+            for (auto& b : *ldes) b.release();
+    }
     // class digests -> tree owner
     std::vector<uint64_t> class_h;
     std::vector<const uint8_t*> class_ptr;
-    std::vector<void*> received;
+    std::vector<DevBuf> received;
     auto local_class = [&](size_t height) -> uint8_t* {
-        for (uint64_t k = 0; h->local && k < msgpu_pdata_num_classes(h->local); k++) {
+        for (uint64_t k = 0; h->local && k < msgpu_pdata_num_classes(h->local.get()); k++) {
             uint64_t lh = 0;
             uint8_t* p = nullptr;
-            gpu_check(msgpu_pdata_class_digests(h->local, k, &lh, &p));
+            gpu_check(msgpu_pdata_class_digests(h->local.get(), k, &lh, &p));
             if (lh == height) return p;
         }
         throw DistError("commit: internal error, class digests missing");
     };
-    try {
-        for (auto& kv : cls) {
-            size_t height = kv.first;
-            int own = kv.second;
-            if (own == h->tree_owner) {
-                if (comm.rank() == own) { class_h.push_back(height); class_ptr.push_back(local_class(height)); }
-                continue;
-            }
-            if (comm.rank() == own) {
-                comm.sendrecv_dev(local_class(height), height * 32, own, h->tree_owner);
-            } else if (comm.rank() == h->tree_owner) {
-                void* buf = nullptr;
-                gpu_check(msgpu_malloc(ctx, height * 32, &buf));
-                received.push_back(buf);
-                comm.sendrecv_dev(buf, height * 32, own, h->tree_owner);
-                class_h.push_back(height);
-                class_ptr.push_back((const uint8_t*)buf);
-            }
+    for (auto& kv : cls) {
+        size_t height = kv.first;
+        int own = kv.second;
+        if (own == h->tree_owner) {
+            if (comm.rank() == own) { class_h.push_back(height); class_ptr.push_back(local_class(height)); }
+            continue;
         }
-        if (comm.rank() == h->tree_owner)
-            gpu_check(msgpu_tree_from_digests(ctx, class_h.size(), class_h.data(), class_ptr.data(), &h->tree, root.data()));
-    } catch (...) {
-        for (void* b : received) msgpu_free(ctx, b);
-        throw;
+        if (comm.rank() == own) {
+            comm.sendrecv_dev(local_class(height), height * 32, own, h->tree_owner);
+        } else if (comm.rank() == h->tree_owner) {
+            received.emplace_back(ctx, height * 32);
+            comm.sendrecv_dev(received.back().get(), height * 32, own, h->tree_owner);
+            class_h.push_back(height);
+            class_ptr.push_back((const uint8_t*)received.back().get());
+        }
     }
-    for (void* b : received) msgpu_free(ctx, b);
+    if (comm.rank() == h->tree_owner) {
+        msgpu_pdata* pd = nullptr;
+        gpu_check(msgpu_tree_from_digests(ctx, class_h.size(), class_h.data(), class_ptr.data(), &pd, root.data()));
+        h->tree.reset(pd);
+    }
+    received.clear();
     comm.bcast(root.data(), 32, h->tree_owner);
     return h;
 }
 
-class DistOpenDevice : public OpenDevice {
+class DistOpenDevice : public ShardedOpenDevice {
   public:
-    DistOpenDevice(msgpu_ctx* ctx, const CommView& comm, const std::vector<OpenRound>& rounds, uint32_t log_blowup) : ctx_(ctx), comm_(comm) {
+    DistOpenDevice(msgpu_ctx* ctx, const CommView& comm, const std::vector<OpenRound>& rounds, uint32_t log_blowup)
+        : ShardedOpenDevice(ctx, comm, rounds) {
         std::vector<const msgpu_pdata*> pds;
         std::vector<uint64_t> npts, pts;
         std::vector<std::pair<size_t, size_t>> all_shapes;
@@ -206,11 +325,10 @@ class DistOpenDevice : public OpenDevice {
             if (!h) throw DistError("open: prover data does not belong to the sharded backend");
             if (r.points.size() != h->shapes.size()) throw DistError("open: one point list per committed matrix expected");
             handles_.push_back(h);
-            points_.push_back(r.points);
             all_shapes.insert(all_shapes.end(), h->shapes.begin(), h->shapes.end());
             all_owner.insert(all_owner.end(), h->owner.begin(), h->owner.end());
             if (!h->local) continue;
-            pds.push_back(h->local);
+            pds.push_back(h->local.get());
             for (size_t m = 0; m < h->shapes.size(); m++) {
                 if (h->local_index[m] < 0) continue;
                 npts.push_back(r.points[m].size());
@@ -223,43 +341,33 @@ class DistOpenDevice : public OpenDevice {
         if (pts.empty()) pts.push_back(0);
         if (!pds.empty()) gpu_check(msgpu_open_begin(ctx_, pds.size(), pds.data(), npts.data(), pts.data(), log_blowup, &op_, &n_local_values_));
     }
-    ~DistOpenDevice() override {
-        if (op_) msgpu_open_free(op_);
-    }
 
     std::vector<OpenedValuesForRound> evaluate() override {
         // global flat layout (round, matrix, point, column); every rank fills the values of its matrices
+        std::vector<size_t> len;  // u64 of matrix (r, m), in that order
         size_t total = 0;
         for (size_t r = 0; r < handles_.size(); r++)
-            for (size_t m = 0; m < handles_[r]->shapes.size(); m++) total += points_[r][m].size() * handles_[r]->shapes[m].second;
-        std::vector<uint64_t> local(std::max<size_t>(2 * n_local_values_, 1)), mine(std::max<size_t>(2 * total, 1), 0);
-        if (op_) gpu_check(msgpu_open_values(op_, local.data()));
-        size_t lo = 0, go = 0;
-        for (size_t r = 0; r < handles_.size(); r++)
             for (size_t m = 0; m < handles_[r]->shapes.size(); m++) {
-                size_t n = 2 * points_[r][m].size() * handles_[r]->shapes[m].second;
-                if (handles_[r]->owner[m] == comm_.rank()) {
-                    memcpy(mine.data() + go, local.data() + lo, n * 8);
-                    lo += n;
-                }
-                go += n;
+                len.push_back(2 * rounds_[r].points[m].size() * handles_[r]->shapes[m].second);
+                total += len.back();
             }
+        std::vector<uint64_t> local(std::max<size_t>(2 * n_local_values_, 1)), mine(std::max<size_t>(total, 1), 0);
+        if (op_) gpu_check(msgpu_open_values(op_, local.data()));
+        size_t lo = 0, go = 0, i = 0;
+        for (size_t r = 0; r < handles_.size(); r++)
+            for (size_t m = 0; m < handles_[r]->shapes.size(); m++, go += len[i++])
+                if (handles_[r]->owner[m] == comm_.rank()) {
+                    memcpy(mine.data() + go, local.data() + lo, len[i] * 8);
+                    lo += len[i];
+                }
         std::vector<uint64_t> all(mine.size() * comm_.world());
         comm_.allgather(mine.data(), all.data(), mine.size() * 8);
-        std::vector<OpenedValuesForRound> out(handles_.size());
-        go = 0;
-        for (size_t r = 0; r < handles_.size(); r++) {
-            out[r].resize(handles_[r]->shapes.size());
-            for (size_t m = 0; m < handles_[r]->shapes.size(); m++) {
-                const uint64_t* src = all.data() + (size_t)handles_[r]->owner[m] * mine.size();
-                out[r][m].resize(points_[r][m].size());
-                for (auto& pv : out[r][m]) {
-                    pv.resize(handles_[r]->shapes[m].second);
-                    for (auto& v : pv) { v.c[0].v = src[go++]; v.c[1].v = src[go++]; }
-                }
-            }
-        }
-        return out;
+        // every matrix's values from its owner's share
+        go = i = 0;
+        for (size_t r = 0; r < handles_.size(); r++)
+            for (size_t m = 0; m < handles_[r]->shapes.size(); m++, go += len[i++])
+                memcpy(mine.data() + go, all.data() + (size_t)handles_[r]->owner[m] * mine.size() + go, len[i] * 8);
+        return decode_opened_values(rounds_, mine.data());
     }
 
     void reduce(Fp2 alpha, unsigned& log_max_height) override {
@@ -290,77 +398,27 @@ class DistOpenDevice : public OpenDevice {
         cur_len_ = size_t(1) << log_max_height_;
         log_max_height = log_max_height_;
     }
-    size_t current_len() override { return cur_len_; }
-    // FRI owner only (the default commit_phase loop runs there)
-    Digest commit_round() override {
-        Digest d{};
-        gpu_check(msgpu_fri_commit_round(op_, d.data()));
-        return d;
-    }
-    void fold(Fp2 beta) override {
-        uint64_t b[2] = {beta.c[0].v, beta.c[1].v};
-        gpu_check(msgpu_fri_fold(op_, b));
-        cur_len_ /= 2;
-    }
-    // The owner folds; every other rank replays the transcript from ONE broadcast of (roots, PoW witnesses, folded vector):
-    // the number of rounds and every length are known from the shapes alone.
-    void commit_phase(Challenger& ch, size_t stop_len, size_t pow_bits, FriProof& proof) override {
-        size_t rounds = 0;
-        for (size_t l = cur_len_; l > stop_len; l >>= 1) rounds++;
-        const size_t final_len = cur_len_ >> rounds;
-        std::vector<u8> blob(rounds * 40 + final_len * 16);
-        if (comm_.rank() == fri_owner_) {
-            OpenDevice::commit_phase(ch, stop_len, pow_bits, proof);
-            if (proof.commit_phase_commits.size() != rounds || cur_len_ != final_len) throw DistError("fri: internal error, round count");
-            for (size_t k = 0; k < rounds; k++) {
-                memcpy(blob.data() + 40 * k, proof.commit_phase_commits[k].data(), 32);
-                memcpy(blob.data() + 40 * k + 32, &proof.commit_pow_witnesses[k].v, 8);
-            }
-            gpu_check(msgpu_fri_read_current(op_, (uint64_t*)(blob.data() + rounds * 40)));
-        }
-        comm_.bcast(blob.data(), blob.size(), fri_owner_);
-        if (comm_.rank() != fri_owner_) {
-            for (size_t k = 0; k < rounds; k++) {
-                Digest d;
-                Fp w;
-                memcpy(d.data(), blob.data() + 40 * k, 32);
-                memcpy(&w.v, blob.data() + 40 * k + 32, 8);
-                ch.observe(d);
-                proof.commit_phase_commits.push_back(d);
-                if (!ch.check_witness(pow_bits, w)) throw DistError("fri: the owner's proof-of-work witness does not verify");
-                proof.commit_pow_witnesses.push_back(w);
-                betas.push_back(ch.sample_ext());
-            }
-            cur_len_ = final_len;
-        }
-        folded_.resize(final_len);
-        const uint64_t* f = (const uint64_t*)(blob.data() + rounds * 40);
-        for (size_t i = 0; i < final_len; i++) { folded_[i].c[0].v = f[2 * i]; folded_[i].c[1].v = f[2 * i + 1]; }
-    }
-    std::vector<Fp2> read_current() override { return folded_; }
-    std::vector<BatchOpening> open_round(size_t, const std::vector<size_t>&) override { throw DistError("open_round: use open_queries"); }
-    std::vector<BatchOpening> open_layer(size_t, const std::vector<size_t>&) override { throw DistError("open_layer: use open_queries"); }
 
     // What rank `rk` contributes to the query phase, in the order of its msgpu_open_batch_multi call.
     struct Piece {
         enum Kind { Rows, Path, Layer } kind;
         size_t round_or_layer;
         std::vector<size_t> mats;  // Rows: global matrix indices of the round held by the rank
-        size_t total_width, depth;
+        TreeShape shape;
     };
     std::vector<Piece> pieces_of(int rk, const std::vector<unsigned>& round_shifts, size_t n_layers) const {
         std::vector<Piece> v;
         for (size_t r = 0; r < handles_.size(); r++) {
             auto mine = handles_[r]->matrices_of(rk);
             if (!mine.empty()) {
-                size_t tw = 0;
-                for (size_t m : mine) tw += handles_[r]->shapes[m].second;
-                v.push_back(Piece{Piece::Rows, r, mine, tw, 0});
+                TreeShape s;
+                for (size_t m : mine) s.widths.push_back(handles_[r]->shapes[m].second);
+                v.push_back(Piece{Piece::Rows, r, mine, s});
             }
-            if (handles_[r]->tree_owner == rk) v.push_back(Piece{Piece::Path, r, {}, 0, (size_t)(log_max_height_ - round_shifts[r])});
+            if (handles_[r]->tree_owner == rk) v.push_back(Piece{Piece::Path, r, {}, TreeShape{{}, (size_t)(log_max_height_ - round_shifts[r])}});
         }
         if (rk == fri_owner_)
-            for (size_t k = 0; k < n_layers; k++) v.push_back(Piece{Piece::Layer, k, {}, 4, (size_t)(log_max_height_ - k - 1)});
+            for (size_t k = 0; k < n_layers; k++) v.push_back(Piece{Piece::Layer, k, {}, TreeShape{{4}, (size_t)(log_max_height_ - k - 1)}});
         return v;
     }
 
@@ -377,30 +435,21 @@ class DistOpenDevice : public OpenDevice {
         // this rank's share in one launch
         std::vector<const msgpu_pdata*> trees;
         std::vector<uint32_t> shifts;
-        size_t open_total = 0, proof_total = 0;
+        std::vector<TreeShape> shapes;
         for (auto& pc : pieces_of(comm_.rank(), round_shifts, n_layers)) {
             if (pc.kind == Piece::Rows) {
-                trees.push_back(handles_[pc.round_or_layer]->local);
+                trees.push_back(handles_[pc.round_or_layer]->local.get());
                 shifts.push_back((uint32_t)(log_max_height_ - log2_strict(handles_[pc.round_or_layer]->local_max_height())));
             } else if (pc.kind == Piece::Path) {
-                trees.push_back(handles_[pc.round_or_layer]->tree);
+                trees.push_back(handles_[pc.round_or_layer]->tree.get());
                 shifts.push_back(round_shifts[pc.round_or_layer]);
             } else {
-                const msgpu_pdata* pd = msgpu_fri_layer_pdata(op_, pc.round_or_layer);
-                if (!pd) throw DistError("open: no such commit-phase layer");
-                trees.push_back(pd);
+                trees.push_back(fri_layer(op_, pc.round_or_layer));
                 shifts.push_back((uint32_t)(pc.round_or_layer + 1));
             }
-            open_total += n * pc.total_width;
-            proof_total += n * pc.depth * 32;
+            shapes.push_back(pc.shape);
         }
-        std::vector<uint64_t> idx(indices.begin(), indices.end()), opened(std::max<size_t>(open_total, 1));
-        std::vector<uint8_t> proofs(std::max<size_t>(proof_total, 1));
-        if (!trees.empty())
-            gpu_check(msgpu_open_batch_multi(ctx_, trees.data(), shifts.data(), trees.size(), idx.data(), n, opened.data(), proofs.data()));
-        std::vector<u8> blob(open_total * 8 + proof_total);
-        if (open_total) memcpy(blob.data(), opened.data(), open_total * 8);
-        if (proof_total) memcpy(blob.data() + open_total * 8, proofs.data(), proof_total);
+        std::vector<u8> blob = open_batch_multi(ctx_, trees, shifts, shapes, indices);
         lapq("local_open");
         std::vector<std::vector<u8>> all = comm_.allgather_var(blob);
         lapq("allgather");
@@ -411,66 +460,45 @@ class DistOpenDevice : public OpenDevice {
             for (size_t q = 0; q < n; q++) rounds_out[r][q].opened_values.resize(handles_[r]->shapes.size());
         for (int rk = 0; rk < comm_.world(); rk++) {
             auto pcs = pieces_of(rk, round_shifts, n_layers);
-            size_t ot = 0, pt = 0;
-            for (auto& pc : pcs) { ot += n * pc.total_width; pt += n * pc.depth * 32; }
-            if (all[rk].size() != ot * 8 + pt) throw DistError("open: a rank sent a query share of unexpected size");
-            const u8* ob = all[rk].data();
-            const u8* pb = all[rk].data() + ot * 8;
-            for (auto& pc : pcs) {
+            shapes.clear();
+            for (auto& pc : pcs) shapes.push_back(pc.shape);
+            if (all[rk].size() != batch_bytes(shapes, n)) throw DistError("open: a rank sent a query share of unexpected size");
+            auto got = decode_batch_openings(shapes, n, all[rk]);
+            for (size_t i = 0; i < pcs.size(); i++)
                 for (size_t q = 0; q < n; q++) {
-                    BatchOpening& bo = pc.kind == Piece::Layer ? layers_out[pc.round_or_layer][q] : rounds_out[pc.round_or_layer][q];
-                    if (pc.kind == Piece::Rows) {
-                        for (size_t m : pc.mats) {
-                            std::vector<Fp> row(handles_[pc.round_or_layer]->shapes[m].second);
-                            memcpy(row.data(), ob, row.size() * 8);
-                            ob += row.size() * 8;
-                            bo.opened_values[m] = std::move(row);
-                        }
-                    } else if (pc.kind == Piece::Layer) {
-                        std::vector<Fp> row(4);
-                        memcpy(row.data(), ob, 32);
-                        ob += 32;
-                        bo.opened_values.push_back(std::move(row));
+                    const Piece& pc = pcs[i];
+                    if (pc.kind == Piece::Layer) {
+                        layers_out[pc.round_or_layer][q] = std::move(got[i][q]);
+                        continue;
                     }
-                    if (pc.depth) {
-                        bo.opening_proof.resize(pc.depth);
-                        for (size_t l = 0; l < pc.depth; l++, pb += 32) memcpy(bo.opening_proof[l].data(), pb, 32);
-                    }
+                    BatchOpening& bo = rounds_out[pc.round_or_layer][q];
+                    for (size_t j = 0; j < pc.mats.size(); j++) bo.opened_values[pc.mats[j]] = std::move(got[i][q].opened_values[j]);
+                    if (pc.kind == Piece::Path) bo.opening_proof = std::move(got[i][q].opening_proof);
                 }
-            }
         }
         lapq("assemble");
     }
 
   private:
-    msgpu_ctx* ctx_;
-    CommView comm_;
-    msgpu_open* op_ = nullptr;
     uint64_t n_local_values_ = 0;
     std::vector<DistPcsHandle*> handles_;
-    std::vector<std::vector<std::vector<Fp2>>> points_;
     std::map<size_t, int, std::greater<size_t>> classes_;
-    int fri_owner_ = 0;
-    unsigned log_max_height_ = 0;
-    size_t cur_len_ = 0;
-    std::vector<Fp2> folded_;
 };
 
-class DistGpuBackend : public GpuBackend {
+class DistGpuBackend : public ShardedBackend {
   public:
     // owner[ci] = rank that holds circuit ci
     DistGpuBackend(msgpu_ctx* ctx, const SystemShape& shape, const msh_comm& comm, const std::vector<int>& owner)
-        : GpuBackend(ctx, shape), comm_{comm}, owner_(owner) {
+        : ShardedBackend(ctx, shape, comm), owner_(owner) {
         if (owner_.size() != shape.circuits.size()) throw DistError("sharded prover: one owner per circuit expected");
         for (int o : owner_)
             if (o < 0 || o >= comm_.world()) throw DistError("sharded prover: owner rank out of range");
     }
-    ~DistGpuBackend() override { DistGpuBackend::end_proof(); }
 
     // System::new: the preprocessed commitment over every circuit that has a preprocessed trace (src/system.rs:180-196)
     PcsHandlePtr commit(const std::vector<const Matrix*>& evals, Digest& root) override {
         std::vector<DistMatrix> mats;
-        std::vector<uint64_t*> up;
+        std::vector<DevBuf> up;
         size_t k = 0;
         for (size_t ci = 0; ci < shape_.circuits.size(); ci++) {
             if (!shape_.circuits[ci].has_preprocessed) continue;
@@ -478,20 +506,12 @@ class DistGpuBackend : public GpuBackend {
             const Matrix* m = evals[k++];
             DistMatrix dm{m->height(), m->width, owner_[ci], nullptr};
             if (owner_[ci] == comm_.rank()) {
-                dm.dev = upload((const uint64_t*)m->values.data(), m->values.size());
-                up.push_back(dm.dev);
+                up.push_back(upload((const uint64_t*)m->values.data(), m->values.size()));
+                dm.dev = up.back().get();
             }
             mats.push_back(dm);
         }
-        PcsHandlePtr h;
-        try {
-            h = dist_commit(ctx_, comm_, mats, (uint32_t)shape_.log_blowup(), false, root);
-        } catch (...) {
-            for (auto* d : up) msgpu_free(ctx_, d);
-            throw;
-        }
-        for (auto* d : up) msgpu_free(ctx_, d);
-        return h;
+        return dist_commit(ctx_, comm_, mats, (uint32_t)shape_.log_blowup(), root);
     }
 
     PcsHandlePtr commit_stage1(const std::vector<size_t>& circuits, const std::vector<MatrixView>& traces, Digest& root) override {
@@ -512,8 +532,8 @@ class DistGpuBackend : public GpuBackend {
             ws.push_back(m.width);
             local_pos.push_back(p);
         }
-        // The claims (global, not sharded) are uploaded, hashed and accumulated by ONE rank, the one with the least trace
-        // data; the others receive 32 + 16 bytes. (Every rank doing it put N copies of the claims on the host's PCIe.)
+        // The claims are handled by the rank with the least trace data. (Every rank doing it put N copies of the claims on the
+        // host's PCIe.)
         {
             std::vector<uint64_t> load(comm_.world(), 0);
             for (auto& m : mats) load[m.owner] += (uint64_t)m.height * m.width;
@@ -522,88 +542,57 @@ class DistGpuBackend : public GpuBackend {
                 if (load[r] <= load[claims_rank_]) claims_rank_ = r;
             if (comm_.rank() != claims_rank_) announced_ = ClaimsView();
         }
-        trace_dev_.assign(circuits.size(), nullptr);
-        msgpu_pdata* local = nullptr;
+        trace_dev_.resize(circuits.size());
+        PdataPtr local;
         if (!ptrs.empty()) {
             // this rank's traces cross PCIe on the copy stream while the earlier ones are extended; the claims follow them
             msgpu_upload* up = nullptr;
             gpu_check(msgpu_upload_begin(ctx_, ptrs.data(), hs.data(), ws.data(), ptrs.size(), &up));
-            try {
-                prefetch_announced_claims();
-            } catch (...) {
-                msgpu_upload_free(up);
-                throw;
-            }
+            std::unique_ptr<msgpu_upload, void (*)(msgpu_upload*)> pending(up, msgpu_upload_free);
+            prefetch_announced_claims();
             std::vector<uint64_t*> kept(ptrs.size(), nullptr);
-            gpu_check(msgpu_commit_upload(up, (uint32_t)shape_.log_blowup(), 1, kept.data(), 1, &local, nullptr));
+            msgpu_pdata* pd = nullptr;
+            // takes the upload on every path; the kept inputs are ours only on success
+            gpu_check(msgpu_commit_upload(pending.release(), (uint32_t)shape_.log_blowup(), 1, kept.data(), 1, &pd, nullptr));
+            local.reset(pd);
             for (size_t k = 0; k < kept.size(); k++) {
-                trace_dev_[local_pos[k]] = kept[k];
+                trace_dev_[local_pos[k]] = DevBuf(ctx_, kept[k]);
                 mats[local_pos[k]].dev = kept[k];
             }
         } else {
             prefetch_announced_claims();
         }
-        return dist_commit(ctx_, comm_, mats, (uint32_t)shape_.log_blowup(), false, root, local);
-    }
-
-    bool observe_claims(Challenger& ch, const ClaimsView& claims) override {
-        if (!claims_on_device(claims)) return GpuBackend::observe_claims(ch, claims);  // small set: every rank runs the host loop
-        Digest d{};
-        if (comm_.rank() == claims_rank_ && !claims_transcript_digest(ch.input_buffer(), claims, d))
-            throw DistError("claims: internal error, device path refused");
-        comm_.bcast(d.data(), 32, claims_rank_);
-        ch.set_flushed(d);
-        return true;
-    }
-    Fp2 claims_accumulator(const ClaimsView& claims, Fp2 beta, Fp2 gamma) override {
-        if (!claims_on_device(claims)) return GpuBackend::claims_accumulator(claims, beta, gamma);
-        uint64_t out[2] = {0, 0};
-        if (comm_.rank() == claims_rank_) {
-            Fp2 a = GpuBackend::claims_accumulator(claims, beta, gamma);
-            out[0] = a.c[0].v;
-            out[1] = a.c[1].v;
-        }
-        comm_.bcast(out, 16, claims_rank_);
-        return Fp2(Fp(out[0]), Fp(out[1]));
+        return dist_commit(ctx_, comm_, mats, (uint32_t)shape_.log_blowup(), root, std::move(local));
     }
 
     PcsHandlePtr commit_stage2(Fp2 beta, Fp2 gamma, Fp2 acc, std::vector<Fp2>& intermediate, Digest& root) override {
         uint64_t b[2] = {beta.c[0].v, beta.c[1].v}, g[2] = {gamma.c[0].v, gamma.c[1].v};
         std::vector<DistMatrix> mats;
         std::vector<uint64_t> sums(2 * active_.size(), 0);
-        std::vector<uint64_t*> s2;
-        PcsHandlePtr h;
-        try {
-            for (size_t p = 0; p < active_.size(); p++) {
-                const Circuit& c = shape_.circuits[active_[p]];
-                uint64_t rows = trace_rows_[p];
-                DistMatrix dm{rows, c.stage_2_width, owner_[active_[p]], nullptr};
-                if (dm.owner == comm_.rank()) {
-                    void* out = nullptr;
-                    gpu_check(msgpu_malloc(ctx_, std::max<uint64_t>(rows * c.stage_2_width * 8, 8), &out));
-                    s2.push_back((uint64_t*)out);
-                    dm.dev = (uint64_t*)out;
-                    gpu_check(msgpu_stage2_trace(ctx_, programs_[active_[p]], pre_dev_[active_[p]], trace_dev_[p], rows, b, g, dm.dev, &sums[2 * p]));
-                }
-                mats.push_back(dm);
+        std::vector<DevBuf> s2;  // scratch
+        for (size_t p = 0; p < active_.size(); p++) {
+            const Circuit& c = shape_.circuits[active_[p]];
+            uint64_t rows = trace_rows_[p];
+            DistMatrix dm{rows, c.stage_2_width, owner_[active_[p]], nullptr};
+            if (dm.owner == comm_.rank()) {
+                s2.emplace_back(ctx_, rows * c.stage_2_width * 8);
+                dm.dev = s2.back().get();
+                gpu_check(msgpu_stage2_trace(ctx_, programs_[active_[p]], pre_dev_[active_[p]].get(), trace_dev_[p].get(), rows, b, g, dm.dev,
+                                             &sums[2 * p]));
             }
-            // chain the per-circuit sums of all ranks (src/lookup.rs:530-543 runs this chain serially over the circuits)
-            std::vector<uint64_t> all(sums.size() * comm_.world());
-            comm_.allgather(sums.data(), all.data(), sums.size() * 8);
-            intermediate.clear();
-            for (size_t p = 0; p < active_.size(); p++) {
-                const uint64_t* s = all.data() + (size_t)owner_[active_[p]] * sums.size() + 2 * p;
-                acc += Fp2(Fp(s[0]), Fp(s[1]));
-                intermediate.push_back(acc);
-            }
-            h = dist_commit(ctx_, comm_, mats, (uint32_t)shape_.log_blowup(), false, root);
-        } catch (...) {
-            for (auto* d : s2) msgpu_free(ctx_, d);
-            throw;
+            mats.push_back(dm);
         }
-        for (auto* d : s2) msgpu_free(ctx_, d);
-        for (auto* d : trace_dev_)
-            if (d) msgpu_free(ctx_, d);
+        // chain the per-circuit sums of all ranks (src/lookup.rs:530-543 runs this chain serially over the circuits)
+        std::vector<uint64_t> all(sums.size() * comm_.world());
+        comm_.allgather(sums.data(), all.data(), sums.size() * 8);
+        intermediate.clear();
+        for (size_t p = 0; p < active_.size(); p++) {
+            const uint64_t* s = all.data() + (size_t)owner_[active_[p]] * sums.size() + 2 * p;
+            acc += Fp2(Fp(s[0]), Fp(s[1]));
+            intermediate.push_back(acc);
+        }
+        auto h = dist_commit(ctx_, comm_, mats, (uint32_t)shape_.log_blowup(), root);
+        s2.clear();
         trace_dev_.clear();
         return h;
     }
@@ -617,51 +606,33 @@ class DistGpuBackend : public GpuBackend {
         uint64_t a[2] = {alpha.c[0].v, alpha.c[1].v};
         uint32_t lb = (uint32_t)shape_.log_blowup();
         std::vector<DistMatrix> mats;
-        std::vector<uint64_t*> ldes;
-        bool adopted = false;
-        try {
-            for (auto& j : jobs) {
-                DistMatrix dm{(size_t)1 << (j.log_degree + lb), (size_t)2 << j.log_quotient_degree, owner_[j.circuit], nullptr};
-                if (dm.owner == comm_.rank()) {
-                    uint64_t pub[8];
-                    for (int k = 0; k < 8; k++) pub[k] = j.publics[k].v;
-                    const msgpu_pdata* ppd = nullptr;
-                    uint64_t pidx = 0;
-                    if (j.preprocessed_idx >= 0 && hp) {
-                        ppd = hp->local;
-                        pidx = (uint64_t)hp->local_index[j.preprocessed_idx];
-                    }
-                    gpu_check(msgpu_quotient(ctx_, programs_[j.circuit], ppd, pidx, h1->local, (uint64_t)h1->local_index[j.pos], h2->local,
-                                             (uint64_t)h2->local_index[j.pos], j.log_degree, j.log_quotient_degree, lb, pub, a, &dm.dev, nullptr));
-                    ldes.push_back(dm.dev);
+        std::vector<DevBuf> ldes;
+        for (auto& j : jobs) {
+            DistMatrix dm{(size_t)1 << (j.log_degree + lb), (size_t)2 << j.log_quotient_degree, owner_[j.circuit], nullptr};
+            if (dm.owner == comm_.rank()) {
+                uint64_t pub[8];
+                for (int k = 0; k < 8; k++) pub[k] = j.publics[k].v;
+                const msgpu_pdata* ppd = nullptr;
+                uint64_t pidx = 0;
+                if (j.preprocessed_idx >= 0 && hp) {
+                    ppd = hp->local.get();
+                    pidx = (uint64_t)hp->local_index[j.preprocessed_idx];
                 }
-                mats.push_back(dm);
+                gpu_check(msgpu_quotient(ctx_, programs_[j.circuit], ppd, pidx, h1->local.get(), (uint64_t)h1->local_index[j.pos], h2->local.get(),
+                                         (uint64_t)h2->local_index[j.pos], j.log_degree, j.log_quotient_degree, lb, pub, a, &dm.dev, nullptr));
+                ldes.emplace_back(ctx_, dm.dev);
             }
-            return dist_commit(ctx_, comm_, mats, lb, true, root, nullptr, &adopted);  // adopts the LDE buffers
-        } catch (...) {
-            if (!adopted)  // ownership was never transferred: the buffers are still ours
-                for (auto* d : ldes) msgpu_free(ctx_, d);
-            throw;
+            mats.push_back(dm);
         }
+        return dist_commit(ctx_, comm_, mats, lb, root, nullptr, &ldes);
     }
 
     std::unique_ptr<OpenDevice> open_begin(const std::vector<OpenRound>& rounds) override {
         return std::make_unique<DistOpenDevice>(ctx_, comm_, rounds, (uint32_t)shape_.log_blowup());
     }
 
-    void end_proof() override {
-        drop_claims();
-        for (auto* d : trace_dev_)
-            if (d) msgpu_free(ctx_, d);
-        trace_dev_.clear();
-        trace_rows_.clear();
-        active_.clear();
-    }
-
   private:
-    CommView comm_;
     std::vector<int> owner_;
-    int claims_rank_ = 0;
 };
 
 }  // namespace msh

@@ -5,6 +5,7 @@
 #include "prover.hpp"
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include "program.hpp"
 #include "../../include/msgpu.h"
 
@@ -17,68 +18,198 @@ inline void gpu_check(int code) {
     if (code != 0) throw GpuError(std::string("libmsgpu: ") + msgpu_last_error());
 }
 
+// A device buffer from the context's arena, released with it. Move-only. The adopting constructor takes over a buffer the
+// library handed out (the kept inputs of msgpu_commit_upload, the LDE of msgpu_quotient / msgpu_quotient_finish); release()
+// gives one up to a call that adopts it, once that call has succeeded.
+class DevBuf {
+  public:
+    DevBuf() = default;
+    DevBuf(msgpu_ctx* ctx, size_t bytes) : ctx_(ctx) {
+        void* p = nullptr;
+        gpu_check(msgpu_malloc(ctx_, std::max<size_t>(bytes, 8), &p));
+        p_ = (uint64_t*)p;
+    }
+    DevBuf(msgpu_ctx* ctx, uint64_t* adopted) : ctx_(ctx), p_(adopted) {}
+    DevBuf(DevBuf&& o) noexcept : ctx_(o.ctx_), p_(o.release()) {}
+    DevBuf& operator=(DevBuf&& o) noexcept {
+        if (this != &o) {
+            reset();
+            ctx_ = o.ctx_;
+            p_ = o.release();
+        }
+        return *this;
+    }
+    ~DevBuf() { reset(); }
+    void reset() {
+        if (p_) msgpu_free(ctx_, p_);
+        p_ = nullptr;
+    }
+    uint64_t* release() {
+        uint64_t* p = p_;
+        p_ = nullptr;
+        return p;
+    }
+    uint64_t* get() const { return p_; }
+
+  private:
+    msgpu_ctx* ctx_ = nullptr;
+    uint64_t* p_ = nullptr;
+};
+
+inline std::vector<uint64_t*> raw_ptrs(const std::vector<DevBuf>& v) {
+    std::vector<uint64_t*> out;
+    for (auto& b : v) out.push_back(b.get());
+    return out;
+}
+
+struct PdataFree {
+    void operator()(msgpu_pdata* pd) const { msgpu_pdata_free(pd); }
+};
+using PdataPtr = std::unique_ptr<msgpu_pdata, PdataFree>;
+
 struct GpuPcsHandle : PcsHandle {
-    msgpu_pdata* pd = nullptr;
+    PdataPtr owned;  // empty when the handle borrows the caller's prover data (msh_pcs_open)
+    const msgpu_pdata* pd = nullptr;
     std::vector<std::pair<size_t, size_t>> shapes;
-    bool owns = true;
-    explicit GpuPcsHandle(msgpu_pdata* p, bool owns_ = true) : pd(p), owns(owns_) {
+    explicit GpuPcsHandle(const msgpu_pdata* p) : pd(p) {
         for (uint64_t i = 0; i < msgpu_pdata_num_matrices(pd); i++) {
             uint64_t r = 0, c = 0;
             gpu_check(msgpu_pdata_matrix(pd, i, nullptr, &r, &c));
             shapes.push_back({(size_t)r, (size_t)c});
         }
     }
-    ~GpuPcsHandle() override {
-        if (owns) msgpu_pdata_free(pd);
-    }
+    explicit GpuPcsHandle(PdataPtr p) : GpuPcsHandle(p.get()) { owned = std::move(p); }
     size_t num_matrices() const override { return shapes.size(); }
     size_t matrix_height(size_t i) const override { return shapes[i].first; }
     size_t matrix_width(size_t i) const override { return shapes[i].second; }
 };
 
-inline std::vector<BatchOpening> gpu_open_batch(msgpu_ctx* ctx, const msgpu_pdata* pd, const std::vector<size_t>& indices) {
-    size_t nm = msgpu_pdata_num_matrices(pd), tw = 0, maxh = 0;
-    std::vector<size_t> widths;
-    for (size_t i = 0; i < nm; i++) {
-        uint64_t r = 0, c = 0;
-        gpu_check(msgpu_pdata_matrix(pd, i, nullptr, &r, &c));
-        widths.push_back((size_t)c);
-        tw += (size_t)c;
-        maxh = std::max(maxh, (size_t)r);
-    }
-    size_t depth = log2_strict(maxh), n = indices.size();
-    std::vector<uint64_t> idx(indices.begin(), indices.end()), opened(std::max<size_t>(n * tw, 1));
-    std::vector<uint8_t> proofs(std::max<size_t>(n * depth * 32, 1));
-    gpu_check(msgpu_open_batch(ctx, pd, idx.data(), n, opened.data(), proofs.data()));
-    std::vector<BatchOpening> out(n);
-    for (size_t q = 0; q < n; q++) {
-        size_t o = q * tw;
-        for (size_t m = 0; m < nm; m++) {
-            std::vector<Fp> row(widths[m]);
-            for (size_t c = 0; c < widths[m]; c++) row[c].v = opened[o++];
-            out[q].opened_values.push_back(std::move(row));
+// msgpu_open_values output -- (round, matrix, point, column), 2 u64 per value -- as [round][matrix][point][column]
+inline std::vector<OpenedValuesForRound> decode_opened_values(const std::vector<OpenRound>& rounds, const uint64_t* flat) {
+    std::vector<OpenedValuesForRound> out(rounds.size());
+    size_t o = 0;
+    for (size_t r = 0; r < rounds.size(); r++) {
+        out[r].resize(rounds[r].points.size());
+        for (size_t m = 0; m < rounds[r].points.size(); m++) {
+            out[r][m].resize(rounds[r].points[m].size());
+            for (auto& pv : out[r][m]) {
+                pv.resize(rounds[r].data->matrix_width(m));
+                for (auto& v : pv) { v.c[0].v = flat[o++]; v.c[1].v = flat[o++]; }
+            }
         }
-        out[q].opening_proof.resize(depth);
-        for (size_t l = 0; l < depth; l++) memcpy(out[q].opening_proof[l].data(), proofs.data() + (q * depth + l) * 32, 32);
     }
     return out;
 }
 
+// One tree of an msgpu_open_batch[_multi] result: the widths of its matrices and the sibling digests per query.
+struct TreeShape {
+    std::vector<size_t> widths;
+    size_t depth = 0;
+};
+inline TreeShape tree_shape(const msgpu_pdata* pd) {
+    TreeShape s;
+    size_t maxh = 0;
+    for (uint64_t i = 0; i < msgpu_pdata_num_matrices(pd); i++) {
+        uint64_t r = 0, c = 0;
+        gpu_check(msgpu_pdata_matrix(pd, i, nullptr, &r, &c));
+        s.widths.push_back((size_t)c);
+        maxh = std::max(maxh, (size_t)r);
+    }
+    s.depth = log2_strict(maxh);
+    return s;
+}
+// An msgpu_open_batch_multi result for n queries in one buffer: every tree's rows (8 bytes a value), then every tree's paths
+inline size_t batch_row_bytes(const std::vector<TreeShape>& trees, size_t n) {
+    size_t b = 0;
+    for (auto& t : trees)
+        for (size_t w : t.widths) b += n * w * 8;
+    return b;
+}
+inline size_t batch_bytes(const std::vector<TreeShape>& trees, size_t n) {
+    size_t b = batch_row_bytes(trees, n);
+    for (auto& t : trees) b += n * t.depth * 32;
+    return b;
+}
+// tree t opened at indices[q] >> shifts[t]
+inline std::vector<u8> open_batch_multi(msgpu_ctx* ctx, const std::vector<const msgpu_pdata*>& trees, const std::vector<uint32_t>& shifts,
+                                        const std::vector<TreeShape>& shapes, const std::vector<size_t>& indices) {
+    const size_t n = indices.size(), rb = batch_row_bytes(shapes, n), total = batch_bytes(shapes, n);
+    std::vector<u8> out(std::max<size_t>(total, 8));
+    if (!trees.empty()) {
+        std::vector<uint64_t> idx(indices.begin(), indices.end());
+        gpu_check(msgpu_open_batch_multi(ctx, trees.data(), shifts.data(), trees.size(), idx.data(), n, (uint64_t*)out.data(), out.data() + rb));
+    }
+    out.resize(total);
+    return out;
+}
+// [tree][query] from such a buffer
+inline std::vector<std::vector<BatchOpening>> decode_batch_openings(const std::vector<TreeShape>& shapes, size_t n, const std::vector<u8>& buf) {
+    if (buf.size() != batch_bytes(shapes, n)) throw GpuError("open: internal error, batch opening size");
+    const u8* ro = buf.data();
+    const u8* po = buf.data() + batch_row_bytes(shapes, n);
+    std::vector<std::vector<BatchOpening>> out(shapes.size(), std::vector<BatchOpening>(n));
+    for (size_t t = 0; t < shapes.size(); t++)
+        for (auto& bo : out[t]) {
+            for (size_t w : shapes[t].widths) {
+                std::vector<Fp> row(w);
+                if (w) memcpy(row.data(), ro, w * 8);
+                ro += w * 8;
+                bo.opened_values.push_back(std::move(row));
+            }
+            bo.opening_proof.resize(shapes[t].depth);
+            for (auto& sib : bo.opening_proof) {
+                memcpy(sib.data(), po, 32);
+                po += 32;
+            }
+        }
+    return out;
+}
+
+inline const msgpu_pdata* fri_layer(msgpu_open* op, size_t k) {
+    const msgpu_pdata* pd = msgpu_fri_layer_pdata(op, k);
+    if (!pd) throw GpuError("open: no such commit-phase layer");
+    return pd;
+}
+
+// p3-fri `commit_phase` with the transcript on the device (no root read-back per round); the host challenger replays the rounds
+// afterwards and every beta is compared. Returns false, having done nothing, where that path does not apply: a proof of work to
+// grind, a challenger buffer the device transcript does not take (empty or over 960 bytes), more than 64 rounds or none.
+inline bool fri_commit_phase_on_device(msgpu_open* op, size_t cur_len, Challenger& ch, size_t stop_len, size_t pow_bits, FriProof& proof,
+                                       std::vector<Fp2>& betas) {
+    const std::vector<u8>& buf = ch.input_buffer();
+    size_t rounds = 0;
+    for (size_t l = cur_len; l > stop_len; l >>= 1) rounds++;
+    if (pow_bits != 0 || buf.empty() || buf.size() > 960 || rounds == 0 || rounds > 64) return false;
+    uint8_t roots[64 * 32];
+    uint64_t bt[64 * 2], n = 0;
+    gpu_check(msgpu_fri_commit_phase(op, buf.data(), buf.size(), stop_len, 64, roots, bt, &n));
+    for (uint64_t k = 0; k < n; k++) {
+        Digest commit;
+        memcpy(commit.data(), roots + 32 * k, 32);
+        ch.observe(commit);
+        proof.commit_phase_commits.push_back(commit);
+        proof.commit_pow_witnesses.push_back(ch.grind(0));
+        Fp2 beta = ch.sample_ext();
+        if (beta.c[0].v != bt[2 * k] || beta.c[1].v != bt[2 * k + 1])
+            throw GpuError("fri: the device transcript and the host challenger disagree on a folding challenge");
+        betas.push_back(beta);
+    }
+    return true;
+}
+
 class GpuOpenDevice : public OpenDevice {
   public:
-    GpuOpenDevice(msgpu_ctx* ctx, const std::vector<OpenRound>& rounds, uint32_t log_blowup) : ctx_(ctx) {
+    GpuOpenDevice(msgpu_ctx* ctx, const std::vector<OpenRound>& rounds, uint32_t log_blowup) : ctx_(ctx), rounds_(rounds) {
         std::vector<uint64_t> npts, pts;
         for (auto& r : rounds) {
             auto* h = dynamic_cast<GpuPcsHandle*>(r.data);
             if (!h) throw GpuError("open: prover data does not belong to the GPU backend");
             pds_.push_back(h->pd);
-            shapes_.push_back(h->shapes);
             if (r.points.size() != h->shapes.size()) throw GpuError("open: one point list per committed matrix expected");
             for (auto& mp : r.points) {
                 npts.push_back(mp.size());
                 for (auto& z : mp) { pts.push_back(z.c[0].v); pts.push_back(z.c[1].v); }
             }
-            points_.push_back(r.points);
         }
         if (pts.empty()) pts.push_back(0);
         gpu_check(msgpu_open_begin(ctx_, pds_.size(), pds_.data(), npts.data(), pts.data(), log_blowup, &op_, &n_values_));
@@ -88,19 +219,7 @@ class GpuOpenDevice : public OpenDevice {
     std::vector<OpenedValuesForRound> evaluate() override {
         std::vector<uint64_t> flat(std::max<size_t>(2 * n_values_, 1));
         gpu_check(msgpu_open_values(op_, flat.data()));
-        std::vector<OpenedValuesForRound> out(pds_.size());
-        size_t o = 0;
-        for (size_t r = 0; r < pds_.size(); r++) {
-            out[r].resize(shapes_[r].size());
-            for (size_t m = 0; m < shapes_[r].size(); m++) {
-                out[r][m].resize(points_[r][m].size());
-                for (auto& pv : out[r][m]) {
-                    pv.resize(shapes_[r][m].second);
-                    for (auto& v : pv) { v.c[0].v = flat[o++]; v.c[1].v = flat[o++]; }
-                }
-            }
-        }
-        return out;
+        return decode_opened_values(rounds_, flat.data());
     }
     void reduce(Fp2 alpha, unsigned& log_max_height) override {
         uint64_t a[2] = {alpha.c[0].v, alpha.c[1].v}, n = 0;
@@ -122,29 +241,8 @@ class GpuOpenDevice : public OpenDevice {
         uint64_t b[2] = {beta.c[0].v, beta.c[1].v};
         gpu_check(msgpu_fri_fold(op_, b));
     }
-    // p3-fri `commit_phase` with the transcript on the device (no root read-back per round) when there is no proof of work
-    // to grind; the host challenger replays the rounds afterwards and every beta is compared.
     void commit_phase(Challenger& ch, size_t stop_len, size_t pow_bits, FriProof& proof) override {
-        const std::vector<u8>& buf = ch.input_buffer();
-        static const bool host_loop = getenv("MSGPU_FRI_HOST_LOOP") != nullptr;
-        if (pow_bits != 0 || buf.empty() || buf.size() > 960 || host_loop || current_len() <= stop_len) {
-            OpenDevice::commit_phase(ch, stop_len, pow_bits, proof);
-            return;
-        }
-        uint8_t roots[64 * 32];
-        uint64_t bt[64 * 2], n = 0;
-        gpu_check(msgpu_fri_commit_phase(op_, buf.data(), buf.size(), stop_len, 64, roots, bt, &n));
-        for (uint64_t k = 0; k < n; k++) {
-            Digest commit;
-            memcpy(commit.data(), roots + 32 * k, 32);
-            ch.observe(commit);
-            proof.commit_phase_commits.push_back(commit);
-            proof.commit_pow_witnesses.push_back(ch.grind(0));
-            Fp2 beta = ch.sample_ext();
-            if (beta.c[0].v != bt[2 * k] || beta.c[1].v != bt[2 * k + 1])
-                throw GpuError("fri: the device transcript and the host challenger disagree on a folding challenge");
-            betas.push_back(beta);
-        }
+        if (!fri_commit_phase_on_device(op_, current_len(), ch, stop_len, pow_bits, proof, betas)) OpenDevice::commit_phase(ch, stop_len, pow_bits, proof);
     }
     std::vector<Fp2> read_current() override {
         size_t len = current_len();
@@ -154,69 +252,30 @@ class GpuOpenDevice : public OpenDevice {
         for (size_t i = 0; i < len; i++) { out[i].c[0].v = flat[2 * i]; out[i].c[1].v = flat[2 * i + 1]; }
         return out;
     }
-    std::vector<BatchOpening> open_round(size_t r, const std::vector<size_t>& indices) override {
-        return gpu_open_batch(ctx_, pds_[r], indices);
-    }
-    std::vector<BatchOpening> open_layer(size_t k, const std::vector<size_t>& pair_indices) override {
-        const msgpu_pdata* pd = msgpu_fri_layer_pdata(op_, k);
-        if (!pd) throw GpuError("open: no such commit-phase layer");
-        return gpu_open_batch(ctx_, pd, pair_indices);
-    }
 
+    // every round and every commit-phase layer in one launch
     void open_queries(const std::vector<size_t>& indices, const std::vector<unsigned>& round_shifts, size_t n_layers,
                       std::vector<std::vector<BatchOpening>>& rounds_out, std::vector<std::vector<BatchOpening>>& layers_out) override {
         std::vector<const msgpu_pdata*> trees(pds_.begin(), pds_.end());
         std::vector<uint32_t> shifts(round_shifts.begin(), round_shifts.end());
         for (size_t k = 0; k < n_layers; k++) {
-            const msgpu_pdata* pd = msgpu_fri_layer_pdata(op_, k);
-            if (!pd) throw GpuError("open: no such commit-phase layer");
-            trees.push_back(pd);
+            trees.push_back(fri_layer(op_, k));
             shifts.push_back((uint32_t)(k + 1));
         }
-        size_t n = indices.size(), open_total = 0, proof_total = 0;
-        std::vector<std::vector<size_t>> widths(trees.size());
-        std::vector<size_t> depth(trees.size()), tw(trees.size());
-        for (size_t t = 0; t < trees.size(); t++) {
-            size_t nm = msgpu_pdata_num_matrices(trees[t]), maxh = 0;
-            for (size_t i = 0; i < nm; i++) {
-                uint64_t r = 0, c = 0;
-                gpu_check(msgpu_pdata_matrix(trees[t], i, nullptr, &r, &c));
-                widths[t].push_back((size_t)c);
-                tw[t] += (size_t)c;
-                maxh = std::max(maxh, (size_t)r);
-            }
-            depth[t] = log2_strict(maxh);
-            open_total += n * tw[t];
-            proof_total += n * depth[t] * 32;
-        }
-        std::vector<uint64_t> idx(indices.begin(), indices.end()), opened(std::max<size_t>(open_total, 1));
-        std::vector<uint8_t> proofs(std::max<size_t>(proof_total, 1));
-        gpu_check(msgpu_open_batch_multi(ctx_, trees.data(), shifts.data(), trees.size(), idx.data(), n, opened.data(), proofs.data()));
-        rounds_out.assign(round_shifts.size(), {});
-        layers_out.assign(n_layers, {});
-        size_t oo = 0, po = 0;
-        for (size_t t = 0; t < trees.size(); t++) {
-            std::vector<BatchOpening>& out = t < round_shifts.size() ? rounds_out[t] : layers_out[t - round_shifts.size()];
-            out.resize(n);
-            for (size_t q = 0; q < n; q++) {
-                for (size_t m = 0; m < widths[t].size(); m++) {
-                    std::vector<Fp> row(widths[t][m]);
-                    for (auto& v : row) v.v = opened[oo++];
-                    out[q].opened_values.push_back(std::move(row));
-                }
-                out[q].opening_proof.resize(depth[t]);
-                for (size_t l = 0; l < depth[t]; l++, po += 32) memcpy(out[q].opening_proof[l].data(), proofs.data() + po, 32);
-            }
-        }
+        std::vector<TreeShape> shapes;
+        for (auto* t : trees) shapes.push_back(tree_shape(t));
+        auto all = decode_batch_openings(shapes, indices.size(), open_batch_multi(ctx_, trees, shifts, shapes, indices));
+        auto split = all.begin() + (ptrdiff_t)round_shifts.size();
+        rounds_out.assign(std::make_move_iterator(all.begin()), std::make_move_iterator(split));
+        layers_out.assign(std::make_move_iterator(split), std::make_move_iterator(all.end()));
     }
 
   private:
     msgpu_ctx* ctx_;
     msgpu_open* op_ = nullptr;
     uint64_t n_values_ = 0;
+    std::vector<OpenRound> rounds_;
     std::vector<const msgpu_pdata*> pds_;
-    std::vector<std::vector<std::pair<size_t, size_t>>> shapes_;
-    std::vector<std::vector<std::vector<Fp2>>> points_;
 };
 
 class GpuBackend : public ProverBackend {
@@ -229,18 +288,15 @@ class GpuBackend : public ProverBackend {
             gpu_check(msgpu_program_create(ctx_, &d.desc, &p));
             programs_.push_back(p);
             // the preprocessed trace in natural order stays on the device for the stage-2 construction
-            uint64_t* dp = nullptr;
             if (c.has_preprocessed && !c.preprocessed.values.empty())
-                dp = upload((const uint64_t*)c.preprocessed.values.data(), c.preprocessed.values.size());
-            pre_dev_.push_back(dp);
+                pre_dev_.push_back(upload((const uint64_t*)c.preprocessed.values.data(), c.preprocessed.values.size()));
+            else
+                pre_dev_.emplace_back();
         }
     }
     ~GpuBackend() override {
         end_proof();
-        if (injected_) msgpu_pdata_free(injected_);
         for (auto* p : programs_) msgpu_program_free(p);
-        for (auto* d : pre_dev_)
-            if (d) msgpu_free(ctx_, d);
     }
 
     PcsHandlePtr commit(const std::vector<const Matrix*>& evals, Digest& root) override {
@@ -249,24 +305,19 @@ class GpuBackend : public ProverBackend {
         for (auto* m : evals) { ptrs.push_back((const uint64_t*)m->values.data()); hs.push_back(m->height()); ws.push_back(m->width); }
         msgpu_pdata* pd = nullptr;
         gpu_check(msgpu_commit(ctx_, ptrs.data(), hs.data(), ws.data(), evals.size(), (uint32_t)shape_.log_blowup(), &pd, root.data()));
-        return std::make_shared<GpuPcsHandle>(pd);
+        return std::make_shared<GpuPcsHandle>(PdataPtr(pd));
     }
 
     // The next proof's stage-1 commitment was made elsewhere (one wide matrix committed by column blocks over several GPUs and
     // assembled with msgpu_pdata_from_parts): adopt it instead of uploading and committing the traces. Only for systems whose
     // stage-2 construction does not read the main traces (no lookups): they are not on this device.
-    void inject_stage1(msgpu_pdata* pd) {
-        if (injected_) msgpu_pdata_free(injected_);
-        injected_ = pd;
-    }
+    void inject_stage1(msgpu_pdata* pd) { injected_.reset(pd); }
 
     PcsHandlePtr commit_stage1(const std::vector<size_t>& circuits, const std::vector<MatrixView>& traces, Digest& root) override {
         end_proof();
         active_ = circuits;
         if (injected_) {
-            msgpu_pdata* pd = injected_;
-            injected_ = nullptr;
-            auto h = std::make_shared<GpuPcsHandle>(pd);  // owns it from here
+            auto h = std::make_shared<GpuPcsHandle>(std::move(injected_));
             if (h->num_matrices() != traces.size()) throw GpuError("injected stage-1 commitment: matrix count does not match the active circuits");
             for (size_t i = 0; i < traces.size(); i++) {
                 if (h->matrix_height(i) != (traces[i].height() << shape_.log_blowup()) || h->matrix_width(i) != traces[i].width)
@@ -275,9 +326,9 @@ class GpuBackend : public ProverBackend {
                     throw GpuError("injected stage-1 commitment: a circuit with lookups needs its main trace on the device");
                 trace_rows_.push_back(traces[i].height());
             }
-            trace_dev_.assign(traces.size(), nullptr);
+            trace_dev_.resize(traces.size());
             announced_ = ClaimsView();
-            gpu_check(msgpu_pdata_root(pd, root.data()));
+            gpu_check(msgpu_pdata_root(h->pd, root.data()));
             return h;
         }
         std::vector<const uint64_t*> ptrs;
@@ -291,20 +342,15 @@ class GpuBackend : public ProverBackend {
         // uploads on the copy stream (trace i + 1 crosses PCIe while trace i is extended), the claims queued right behind them
         msgpu_upload* up = nullptr;
         gpu_check(msgpu_upload_begin(ctx_, ptrs.data(), hs.data(), ws.data(), traces.size(), &up));
-        try {
-            prefetch_announced_claims();
-        } catch (...) {
-            msgpu_upload_free(up);
-            throw;
-        }
-        trace_dev_.assign(traces.size(), nullptr);
+        std::unique_ptr<msgpu_upload, void (*)(msgpu_upload*)> pending(up, msgpu_upload_free);
+        prefetch_announced_claims();
+        std::vector<uint64_t*> kept(traces.size(), nullptr);
         msgpu_pdata* pd = nullptr;
-        int rc = msgpu_commit_upload(up, (uint32_t)shape_.log_blowup(), 1, trace_dev_.data(), 0, &pd, root.data());
-        if (rc != 0) {
-            trace_dev_.clear();  // the library released the buffers
-            gpu_check(rc);
-        }
-        return std::make_shared<GpuPcsHandle>(pd);
+        // takes the upload on every path; the kept inputs are ours only on success
+        gpu_check(msgpu_commit_upload(pending.release(), (uint32_t)shape_.log_blowup(), 1, kept.data(), 0, &pd, root.data()));
+        PdataPtr owned(pd);
+        for (auto* k : kept) trace_dev_.emplace_back(ctx_, k);
+        return std::make_shared<GpuPcsHandle>(std::move(owned));
     }
 
     void announce_claims(const ClaimsView& claims) override { announced_ = claims; }
@@ -349,34 +395,25 @@ class GpuBackend : public ProverBackend {
 
     PcsHandlePtr commit_stage2(Fp2 beta, Fp2 gamma, Fp2 acc, std::vector<Fp2>& intermediate, Digest& root) override {
         uint64_t b[2] = {beta.c[0].v, beta.c[1].v}, g[2] = {gamma.c[0].v, gamma.c[1].v};
-        std::vector<uint64_t*> s2;
+        std::vector<DevBuf> s2;  // scratch, released when this returns or throws
         std::vector<uint64_t> hs, ws;
         intermediate.clear();
-        struct FreeAll {  // the stage-2 traces are scratch: released on every path, including a throwing msgpu_stage2_trace
-            msgpu_ctx* ctx;
-            std::vector<uint64_t*>& v;
-            ~FreeAll() { for (auto* d : v) msgpu_free(ctx, d); }
-        } guard{ctx_, s2};
         for (size_t p = 0; p < active_.size(); p++) {
             const Circuit& c = shape_.circuits[active_[p]];
             uint64_t rows = trace_rows_[p];
-            void* out = nullptr;
-            gpu_check(msgpu_malloc(ctx_, std::max<uint64_t>(rows * c.stage_2_width * 8, 8), &out));
-            s2.push_back((uint64_t*)out);
+            s2.emplace_back(ctx_, rows * c.stage_2_width * 8);
             uint64_t local[2] = {0, 0};
-            gpu_check(msgpu_stage2_trace(ctx_, programs_[active_[p]], pre_dev_[active_[p]], trace_dev_[p], rows, b, g, (uint64_t*)out, local));
+            gpu_check(msgpu_stage2_trace(ctx_, programs_[active_[p]], pre_dev_[active_[p]].get(), trace_dev_[p].get(), rows, b, g, s2.back().get(), local));
             acc += Fp2(Fp(local[0]), Fp(local[1]));
             intermediate.push_back(acc);
             hs.push_back(rows);
             ws.push_back(c.stage_2_width);
         }
         msgpu_pdata* pd = nullptr;
-        gpu_check(msgpu_commit_dev(ctx_, (const uint64_t* const*)s2.data(), hs.data(), ws.data(), s2.size(), (uint32_t)shape_.log_blowup(), &pd,
-                                   root.data()));
-        // the natural-order traces are not needed any more
-        for (auto* d : trace_dev_) msgpu_free(ctx_, d);
-        trace_dev_.clear();
-        return std::make_shared<GpuPcsHandle>(pd);
+        gpu_check(msgpu_commit_dev(ctx_, raw_ptrs(s2).data(), hs.data(), ws.data(), s2.size(), (uint32_t)shape_.log_blowup(), &pd, root.data()));
+        PdataPtr owned(pd);
+        trace_dev_.clear();  // the natural-order traces are not needed any more
+        return std::make_shared<GpuPcsHandle>(std::move(owned));
     }
 
     PcsHandlePtr commit_quotient(const std::vector<QuotientJob>& jobs, PcsHandle* pre, PcsHandle* s1, PcsHandle* s2, Fp2 alpha,
@@ -385,28 +422,24 @@ class GpuBackend : public ProverBackend {
         auto* h2 = dynamic_cast<GpuPcsHandle*>(s2);
         auto* hp = pre ? dynamic_cast<GpuPcsHandle*>(pre) : nullptr;
         uint64_t a[2] = {alpha.c[0].v, alpha.c[1].v};
-        std::vector<uint64_t*> ldes;
+        std::vector<DevBuf> ldes;
         std::vector<uint64_t> hs, ws;
         uint32_t lb = (uint32_t)shape_.log_blowup();
-        try {
-            for (auto& j : jobs) {
-                uint64_t pub[8];
-                for (int k = 0; k < 8; k++) pub[k] = j.publics[k].v;
-                uint64_t* lde = nullptr;
-                gpu_check(msgpu_quotient(ctx_, programs_[j.circuit], j.preprocessed_idx >= 0 && hp ? hp->pd : nullptr,
-                                         j.preprocessed_idx >= 0 ? (uint64_t)j.preprocessed_idx : 0, h1->pd, j.pos, h2->pd, j.pos,
-                                         j.log_degree, j.log_quotient_degree, lb, pub, a, &lde, nullptr));
-                ldes.push_back(lde);
-                hs.push_back((uint64_t)1 << (j.log_degree + lb));
-                ws.push_back((uint64_t)2 << j.log_quotient_degree);
-            }
-            msgpu_pdata* pd = nullptr;
-            gpu_check(msgpu_commit_ldes_dev(ctx_, ldes.data(), hs.data(), ws.data(), ldes.size(), 1, &pd, root.data()));
-            return std::make_shared<GpuPcsHandle>(pd);
-        } catch (...) {
-            for (auto* d : ldes) msgpu_free(ctx_, d);
-            throw;
+        for (auto& j : jobs) {
+            uint64_t pub[8];
+            for (int k = 0; k < 8; k++) pub[k] = j.publics[k].v;
+            uint64_t* lde = nullptr;
+            gpu_check(msgpu_quotient(ctx_, programs_[j.circuit], j.preprocessed_idx >= 0 && hp ? hp->pd : nullptr,
+                                     j.preprocessed_idx >= 0 ? (uint64_t)j.preprocessed_idx : 0, h1->pd, j.pos, h2->pd, j.pos, j.log_degree,
+                                     j.log_quotient_degree, lb, pub, a, &lde, nullptr));
+            ldes.emplace_back(ctx_, lde);
+            hs.push_back((uint64_t)1 << (j.log_degree + lb));
+            ws.push_back((uint64_t)2 << j.log_quotient_degree);
         }
+        msgpu_pdata* pd = nullptr;
+        gpu_check(msgpu_commit_ldes_dev(ctx_, raw_ptrs(ldes).data(), hs.data(), ws.data(), ldes.size(), 1, &pd, root.data()));
+        for (auto& l : ldes) l.release();  // adopted by the prover data
+        return std::make_shared<GpuPcsHandle>(PdataPtr(pd));
     }
 
     std::unique_ptr<OpenDevice> open_begin(const std::vector<OpenRound>& rounds) override {
@@ -415,7 +448,6 @@ class GpuBackend : public ProverBackend {
 
     void end_proof() override {
         drop_claims();
-        for (auto* d : trace_dev_) msgpu_free(ctx_, d);
         trace_dev_.clear();
         trace_rows_.clear();
         active_.clear();
@@ -448,17 +480,10 @@ class GpuBackend : public ProverBackend {
         return true;
     }
     // H2D copy + check that every value is canonical (the ABI's precondition, verified on the device)
-    uint64_t* upload(const uint64_t* src, size_t n) {
-        void* d = nullptr;
-        gpu_check(msgpu_malloc(ctx_, std::max<size_t>(n * 8, 8), &d));
-        if (n) {
-            int rc = msgpu_upload_canonical(ctx_, d, src, n);
-            if (rc != 0) {
-                msgpu_free(ctx_, d);
-                gpu_check(rc);
-            }
-        }
-        return (uint64_t*)d;
+    DevBuf upload(const uint64_t* src, size_t n) {
+        DevBuf d(ctx_, n * 8);
+        if (n) gpu_check(msgpu_upload_canonical(ctx_, d.get(), src, n));
+        return d;
     }
     void drop_claims() {
         if (claims_dev_) msgpu_claims_free(claims_dev_);
@@ -477,7 +502,7 @@ class GpuBackend : public ProverBackend {
         prefetched_n_ = cl.size();
         prefetched_len_ = len;
     }
-    msgpu_pdata* injected_ = nullptr;
+    PdataPtr injected_;
     ClaimsView announced_;
     const void* prefetched_from_ = nullptr;
     size_t prefetched_n_ = 0, prefetched_len_ = 0;
@@ -485,9 +510,9 @@ class GpuBackend : public ProverBackend {
     msgpu_claims* claims_dev_ = nullptr;
     const SystemShape& shape_;
     std::vector<msgpu_program*> programs_;
-    std::vector<uint64_t*> pre_dev_;
+    std::vector<DevBuf> pre_dev_;
     std::vector<size_t> active_;
-    std::vector<uint64_t*> trace_dev_;
+    std::vector<DevBuf> trace_dev_;
     std::vector<uint64_t> trace_rows_;
 };
 

@@ -69,26 +69,11 @@ struct OpenDevice {
             fold(beta);
         }
     }
-    // Mmcs::open_batch of round `r` at every index (already reduced to the round's height)
-    virtual std::vector<BatchOpening> open_round(size_t r, const std::vector<size_t>& indices) = 0;
-    // Mmcs::open_batch of commit-phase layer `k` at every pair index: opened row = 2 extension values
-    virtual std::vector<BatchOpening> open_layer(size_t k, const std::vector<size_t>& pair_indices) = 0;
-    // The whole query phase at once: round r is opened at indices[q] >> round_shifts[r], layer k at indices[q] >> (k + 1).
-    // rounds_out[r][q], layers_out[k][q]. A device backend overrides this with a single launch.
+    // The whole query phase (Mmcs::open_batch of every round and commit-phase layer): round r is opened at
+    // indices[q] >> round_shifts[r], layer k at the pair index indices[q] >> (k + 1) (opened row = 2 extension values).
+    // rounds_out[r][q], layers_out[k][q].
     virtual void open_queries(const std::vector<size_t>& indices, const std::vector<unsigned>& round_shifts, size_t n_layers,
-                              std::vector<std::vector<BatchOpening>>& rounds_out, std::vector<std::vector<BatchOpening>>& layers_out) {
-        rounds_out.clear();
-        layers_out.clear();
-        std::vector<size_t> reduced(indices.size());
-        for (size_t r = 0; r < round_shifts.size(); r++) {
-            for (size_t q = 0; q < indices.size(); q++) reduced[q] = indices[q] >> round_shifts[r];
-            rounds_out.push_back(open_round(r, reduced));
-        }
-        for (size_t k = 0; k < n_layers; k++) {
-            for (size_t q = 0; q < indices.size(); q++) reduced[q] = indices[q] >> (k + 1);
-            layers_out.push_back(open_layer(k, reduced));
-        }
-    }
+                              std::vector<std::vector<BatchOpening>>& rounds_out, std::vector<std::vector<BatchOpening>>& layers_out) = 0;
 };
 
 inline unsigned log2_exact(size_t n) { return log2_strict(n); }

@@ -33,10 +33,6 @@
 
 namespace msh {
 
-struct RowShardError : std::runtime_error {
-    using std::runtime_error::runtime_error;
-};
-
 // A block of the symmetric peer heap: the same (segment, offset) on every rank.
 struct SymBlock {
     uint32_t seg = 0;
@@ -46,22 +42,16 @@ struct SymBlock {
 
 // Pcs::ProverData of a row-sharded commitment.
 struct RowShardHandle : PcsHandle {
-    msgpu_ctx* ctx = nullptr;
     int n_shards = 1, shard = 0;
     std::vector<std::pair<size_t, size_t>> shapes;  // (GLOBAL LDE height, width), commit order
     std::vector<uint64_t*> views;                   // this rank's rows of matrix i: shapes[i].first / n_shards rows
     std::vector<bool> whole;                        // views[i] points into the WHOLE LDE (every rank has every row)
-    std::vector<uint64_t*> owned;                   // device buffers behind the views (shard buffers or whole LDEs)
+    std::vector<DevBuf> owned;                      // device buffers behind the views (shard buffers or whole LDEs)
     // (pointer, width) of the column blocks a view is still to be assembled from (peer memory: the shard is written by the
     // pass that hashes it); empty once the commitment is built
     std::vector<std::vector<std::pair<const uint64_t*, uint64_t>>> pending;
-    msgpu_pdata* local = nullptr;                   // MMCS over the views: leaf digests + subtree of this rank's rows
-    msgpu_pdata* top = nullptr;                     // the top log2(n_shards) levels over the subtree roots
-    ~RowShardHandle() override {
-        if (local) msgpu_pdata_free(local);
-        if (top) msgpu_pdata_free(top);
-        for (auto* p : owned) msgpu_free(ctx, p);
-    }
+    PdataPtr local;                                 // MMCS over the views: leaf digests + subtree of this rank's rows
+    PdataPtr top;                                   // the top log2(n_shards) levels over the subtree roots
     size_t num_matrices() const override { return shapes.size(); }
     size_t matrix_height(size_t i) const override { return shapes[i].first; }
     size_t matrix_width(size_t i) const override { return shapes[i].second; }
@@ -69,27 +59,6 @@ struct RowShardHandle : PcsHandle {
     // rows of shard `e` of matrix i when the whole LDE is here
     uint64_t* whole_rows_of(size_t i, int e) const { return views[i] + ((ptrdiff_t)e - shard) * (ptrdiff_t)(shard_rows(i) * shapes[i].second); }
 };
-
-struct RowShardComm : CommView {
-    void alltoall_dev(void* send, const uint64_t* send_bytes, void* recv, const uint64_t* recv_bytes) const {
-        if (!c.alltoall_dev) throw RowShardError("comm: the communicator has no device all-to-all");
-        if (c.alltoall_dev(c.user, send, send_bytes, recv, recv_bytes) != 0) throw RowShardError("comm: device all-to-all failed");
-    }
-    // recv holds world() chunks of `bytes` in rank order; chunk rank() is `send`
-    void allgather_dev(void* send, void* recv, uint64_t bytes) const {
-        if (!c.allgather_dev) throw RowShardError("comm: the communicator has no device all-gather");
-        if (bytes && c.allgather_dev(c.user, send, recv, bytes) != 0) throw RowShardError("comm: device all-gather failed");
-    }
-};
-
-// MSH_TRACE=2: one line per protocol step and rank on stderr (a rank that stops printing is where a multi-GPU run hangs)
-inline void rs_trace(int rank, const char* what, size_t a = 0, size_t b = 0) {
-    static const bool on = getenv("MSH_TRACE") && atoi(getenv("MSH_TRACE")) >= 2;
-    if (on) {
-        fprintf(stderr, "[rs %d] %s %zu %zu\n", rank, what, a, b);
-        fflush(stderr);
-    }
-}
 
 inline unsigned rs_rev_bits(unsigned x, unsigned bits) {
     unsigned r = 0;
@@ -102,17 +71,18 @@ inline unsigned rs_rev_bits(unsigned x, unsigned bits) {
 struct RowBlocks {
     size_t height = 0, width = 0;  // of the whole matrix
     bool whole = false;
-    uint64_t* dev = nullptr;       // this rank's block (height / N rows) or the whole matrix
+    DevBuf own;                    // the buffer behind `dev`, empty when it is the caller's (msh_rowshard_commit)
+    const uint64_t* dev = nullptr; // this rank's block (height / N rows) or the whole matrix
 };
 
 class RowShardOpenDevice;
 
-class RowShardBackend : public GpuBackend {
+class RowShardBackend : public ShardedBackend {
   public:
-    RowShardBackend(msgpu_ctx* ctx, const SystemShape& shape, const msh_comm& comm) : GpuBackend(ctx, shape), comm_{{comm}} {
+    RowShardBackend(msgpu_ctx* ctx, const SystemShape& shape, const msh_comm& comm) : ShardedBackend(ctx, shape, comm) {
         const int n = comm_.world();
-        if (n < 1 || (n & (n - 1))) throw RowShardError("row-sharded prover: the number of ranks must be a power of two");
-        if (n > 16) throw RowShardError("row-sharded prover: at most 16 ranks");
+        if (n < 1 || (n & (n - 1))) throw DistError("row-sharded prover: the number of ranks must be a power of two");
+        if (n > 16) throw DistError("row-sharded prover: at most 16 ranks");
         for (auto& c : shape_.circuits)  // a wrap-around next-row read inside a lookup would need a one-row halo between the blocks
             for (size_t i = 0; i < c.graph.lookup_prefix_len; i++)
                 if (c.graph.nodes[i].op == Op::Var && c.graph.nodes[i].col.offset == RowOffset::Next) lookup_next_ = true;
@@ -127,14 +97,10 @@ class RowShardBackend : public GpuBackend {
     uint64_t peer_bytes() const { return peer_bytes_; }
     // matrices that take the peer-memory path: split by columns for the NTT, and tall enough for a two-pass transform
     bool peer_path(size_t height, size_t width) const { return peers_ && shardable(height, width); }
-    void free_blocks(RowBlocks& b) {
-        if (b.dev) msgpu_free(ctx_, b.dev);
-        b.dev = nullptr;
-    }
 
     int world() const { return comm_.world(); }
     int rank() const { return comm_.rank(); }
-    const RowShardComm& comm() const { return comm_; }
+    const CommView& comm() const { return comm_; }
     msgpu_ctx* ctx() const { return ctx_; }
 
     // wide and tall enough to be split by columns for the NTT and by rows afterwards
@@ -147,24 +113,19 @@ class RowShardBackend : public GpuBackend {
 
     // ---- commitments ---------------------------------------------------------------------------------------------------
     // rows of this rank's shard of the LDE of `m` (shardable: column-sharded NTT between two all-to-alls; otherwise the whole LDE
-    // on every rank). Returns the buffer to own and the view of this rank's rows.
-    void lde_shard(const RowBlocks& m, uint64_t** owned, uint64_t** view, bool* whole) {
+    // on every rank). Returns the buffer to own; *view = this rank's rows.
+    DevBuf lde_shard(const RowBlocks& m, uint64_t** view, bool* whole) {
         const int N = world(), d = rank();
         const uint32_t lb = (uint32_t)shape_.log_blowup();
         const size_t n = m.height, w = m.width, H = n << lb, Ls = H / (size_t)N;
-        if (H < (size_t)N) throw RowShardError("row-sharded prover: a committed matrix has fewer LDE rows than there are ranks");
-        if (!m.whole && !shardable(n, w)) throw RowShardError("row-sharded prover: internal error, row blocks of an unshardable matrix");
+        if (H < (size_t)N) throw DistError("row-sharded prover: a committed matrix has fewer LDE rows than there are ranks");
+        if (!m.whole && !shardable(n, w)) throw DistError("row-sharded prover: internal error, row blocks of an unshardable matrix");
         if (m.whole) {
-            void* lde = nullptr;
-            gpu_check(msgpu_malloc(ctx_, std::max<size_t>(H * w * 8, 8), &lde));
-            if (w) {
-                int rc = msgpu_coset_lde_batch_bitrev_dev(ctx_, m.dev, n, w, lb, GL_GENERATOR, (uint64_t*)lde);
-                if (rc != 0) { msgpu_free(ctx_, lde); gpu_check(rc); }
-            }
-            *owned = (uint64_t*)lde;
-            *view = (uint64_t*)lde + (size_t)d * Ls * w;
+            DevBuf lde(ctx_, H * w * 8);
+            if (w) gpu_check(msgpu_coset_lde_batch_bitrev_dev(ctx_, m.dev, n, w, lb, GL_GENERATOR, lde.get()));
+            *view = lde.get() + (size_t)d * Ls * w;
             *whole = true;
-            return;
+            return lde;
         }
         // column blocks: the first w % N ranks get one more column
         std::vector<uint64_t> c0(N), c1(N), wd(N);
@@ -173,26 +134,25 @@ class RowShardBackend : public GpuBackend {
             for (int e = 0; e < N; e++) { c0[e] = c; c += base + ((size_t)e < rem ? 1 : 0); c1[e] = c; wd[e] = c1[e] - c0[e]; }
         }
         const size_t nb = n / (size_t)N;  // rows of a natural-order block
-        DevPtr packed(ctx_, nb * w * 8), colblock(ctx_, n * wd[d] * 8);
-        gpu_check(msgpu_pack_column_blocks_dev(ctx_, m.dev, nb, w, N, c0.data(), c1.data(), packed.u()));
+        DevBuf packed(ctx_, nb * w * 8), colblock(ctx_, n * wd[d] * 8);
+        gpu_check(msgpu_pack_column_blocks_dev(ctx_, m.dev, nb, w, N, c0.data(), c1.data(), packed.get()));
         std::vector<uint64_t> sb(N), rb(N);
         for (int e = 0; e < N; e++) { sb[e] = nb * wd[e] * 8; rb[e] = nb * wd[d] * 8; }
-        comm_.alltoall_dev(packed.p, sb.data(), colblock.p, rb.data());  // pieces arrive in rank order = natural row order
+        comm_.alltoall_dev(packed.get(), sb.data(), colblock.get(), rb.data());  // pieces arrive in rank order = natural row order
         packed.reset();
-        DevPtr lde(ctx_, H * wd[d] * 8);
-        gpu_check(msgpu_coset_lde_batch_bitrev_dev(ctx_, colblock.u(), n, wd[d], lb, GL_GENERATOR, lde.u()));
+        DevBuf lde(ctx_, H * wd[d] * 8);
+        gpu_check(msgpu_coset_lde_batch_bitrev_dev(ctx_, colblock.get(), n, wd[d], lb, GL_GENERATOR, lde.get()));
         colblock.reset();
         // rows [e Ls, (e + 1) Ls) of my columns are contiguous: chunk e goes to rank e
-        DevPtr chunks(ctx_, Ls * w * 8);
+        DevBuf chunks(ctx_, Ls * w * 8);
         for (int e = 0; e < N; e++) { sb[e] = Ls * wd[d] * 8; rb[e] = Ls * wd[e] * 8; }
-        comm_.alltoall_dev(lde.p, sb.data(), chunks.p, rb.data());
+        comm_.alltoall_dev(lde.get(), sb.data(), chunks.get(), rb.data());
         lde.reset();
-        void* shard = nullptr;
-        gpu_check(msgpu_malloc(ctx_, Ls * w * 8, &shard));
-        int rc = msgpu_interleave_column_blocks_dev(ctx_, chunks.u(), Ls, N, wd.data(), (uint64_t*)shard);
-        if (rc != 0) { msgpu_free(ctx_, shard); gpu_check(rc); }
-        *owned = *view = (uint64_t*)shard;
+        DevBuf shard(ctx_, Ls * w * 8);
+        gpu_check(msgpu_interleave_column_blocks_dev(ctx_, chunks.get(), Ls, N, wd.data(), shard.get()));
+        *view = shard.get();
         *whole = false;
+        return shard;
     }
 
     // MMCS over the shards: local subtree + replicated top
@@ -201,13 +161,15 @@ class RowShardBackend : public GpuBackend {
         std::vector<uint64_t*> ptrs;
         std::vector<uint64_t> hs, ws;
         for (size_t i = 0; i < h->shapes.size(); i++) {
-            if (h->shapes[i].first < (size_t)N) throw RowShardError("row-sharded prover: a committed matrix has fewer LDE rows than there are ranks");
+            if (h->shapes[i].first < (size_t)N) throw DistError("row-sharded prover: a committed matrix has fewer LDE rows than there are ranks");
             ptrs.push_back(h->views[i]);
             hs.push_back(h->shard_rows(i));
             ws.push_back(h->shapes[i].second);
         }
+        msgpu_pdata* pd = nullptr;
         if (N == 1) {
-            gpu_check(msgpu_commit_ldes_dev(ctx_, ptrs.data(), hs.data(), ws.data(), ptrs.size(), 0, &h->local, root.data()));
+            gpu_check(msgpu_commit_ldes_dev(ctx_, ptrs.data(), hs.data(), ws.data(), ptrs.size(), 0, &pd, root.data()));
+            h->local.reset(pd);
             return h;
         }
         // views that are still column blocks in the peers' windows are assembled by the leaf-hash pass itself
@@ -228,11 +190,12 @@ class RowShardBackend : public GpuBackend {
         // leaf digests + subtree, stream-ordered (no read-back); the 32-byte subtree roots are all-gathered on the device and the
         // top levels built from them: ONE host synchronisation per commitment, for the root the transcript needs
         gpu_check(msgpu_commit_ldes_blocks_dev(ctx_, ptrs.data(), hs.data(), ws.data(), ptrs.size(), n_blocks, n_blocks ? bptr.data() : nullptr,
-                                               n_blocks ? bwid.data() : nullptr, 0, &h->local, nullptr));
+                                               n_blocks ? bwid.data() : nullptr, 0, &pd, nullptr));
+        h->local.reset(pd);
         h->pending.clear();
         uint8_t* dg = nullptr;
         uint64_t nd = 0;
-        gpu_check(msgpu_pdata_digests(h->local, &dg, &nd));
+        gpu_check(msgpu_pdata_digests(h->local.get(), &dg, &nd));
         uint64_t hh = (uint64_t)N;
         if (peers_) {
             // every rank stores its root into slot `rank` of every peer's ring entry; the flag barrier publishes them
@@ -240,21 +203,22 @@ class RowShardBackend : public GpuBackend {
             gpu_check(msgpu_peers_put_root(peers_, dg + (nd - 1) * 32, &gathered));
             gpu_check(msgpu_peers_barrier(peers_));
             const uint8_t* pp = gathered;
-            gpu_check(msgpu_tree_from_digests(ctx_, 1, &hh, &pp, &h->top, root.data()));
+            gpu_check(msgpu_tree_from_digests(ctx_, 1, &hh, &pp, &pd, root.data()));
+            h->top.reset(pd);
             gpu_check(msgpu_peers_check(peers_));  // a barrier of this commitment timed out: fail here, not with a wrong root
             rs_trace(rank(), "root");
             return h;
         }
-        DevPtr d_roots(ctx_, 32 * (size_t)N);
-        comm_.allgather_dev(dg + (nd - 1) * 32, d_roots.p, 32);
-        const uint8_t* pp = (const uint8_t*)d_roots.p;
-        gpu_check(msgpu_tree_from_digests(ctx_, 1, &hh, &pp, &h->top, root.data()));
+        DevBuf d_roots(ctx_, 32 * (size_t)N);
+        comm_.allgather_dev(dg + (nd - 1) * 32, d_roots.get(), 32);
+        const uint8_t* pp = (const uint8_t*)d_roots.get();
+        gpu_check(msgpu_tree_from_digests(ctx_, 1, &hh, &pp, &pd, root.data()));
+        h->top.reset(pd);
         return h;
     }
 
     std::shared_ptr<RowShardHandle> commit_blocks(const std::vector<RowBlocks>& mats, Digest& root) {
         auto h = std::make_shared<RowShardHandle>();
-        h->ctx = ctx_;
         h->n_shards = world();
         h->shard = rank();
         const uint32_t lb = (uint32_t)shape_.log_blowup();
@@ -293,29 +257,26 @@ class RowShardBackend : public GpuBackend {
         if (any_peer) gpu_check(msgpu_peers_barrier(peers_));  // every rank's column block of every LDE is complete
         for (size_t i = 0; i < mats.size(); i++) {
             const RowBlocks& m = mats[i];
-            uint64_t *owned = nullptr, *view = nullptr;
+            uint64_t* view = nullptr;
             bool whole = false;
             if (col[i].live) {
                 // my row shard from every rank's column block: remote loads of whole lines
                 const size_t Ls = (m.height << lb) / N;
-                void* shard = nullptr;
-                gpu_check(msgpu_malloc(ctx_, Ls * m.width * 8, &shard));
-                owned = view = (uint64_t*)shard;
-                h->owned.push_back(owned);
+                h->owned.emplace_back(ctx_, Ls * m.width * 8);
+                view = h->owned.back().get();
                 // ... inside the pass that hashes them (commit_shards): block e = rank e's columns of my rows
                 std::vector<std::pair<const uint64_t*, uint64_t>> blocks;
                 const size_t base = m.width / N, rem = m.width % N;
                 for (size_t e = 0; e < N; e++) {
                     const size_t wde = base + (e < rem ? 1 : 0);
                     const uint64_t* p = (const uint64_t*)msgpu_peers_ptr(peers_, lde[i].seg, lde[i].off, (int32_t)e);
-                    if (!p) throw RowShardError("peer heap: internal error, unmapped block");
+                    if (!p) throw DistError("peer heap: internal error, unmapped block");
                     blocks.push_back({p + d * Ls * wde, wde});
                 }
                 h->pending.resize(i + 1);
                 h->pending[i] = std::move(blocks);
             } else {
-                lde_shard(m, &owned, &view, &whole);
-                h->owned.push_back(owned);
+                h->owned.push_back(lde_shard(m, &view, &whole));
             }
             h->views.push_back(view);
             h->whole.push_back(whole);
@@ -333,14 +294,14 @@ class RowShardBackend : public GpuBackend {
         b.width = width;
         b.whole = !shardable(height, width);
         const size_t rows = b.whole ? height : height / (size_t)world(), row0 = b.whole ? 0 : rows * (size_t)rank();
-        b.dev = upload(host + row0 * width, rows * width);
+        b.own = upload(host + row0 * width, rows * width);
+        b.dev = b.own.get();
         return b;
     }
 
     // System::new: the preprocessed commitment (src/system.rs:180-196)
     PcsHandlePtr commit(const std::vector<const Matrix*>& evals, Digest& root) override {
         std::vector<RowBlocks> mats;
-        struct Free { RowShardBackend* be; std::vector<RowBlocks>& v; ~Free() { for (auto& b : v) be->free_blocks(b); } } fr{this, mats};
         for (auto* m : evals) mats.push_back(upload_blocks((const uint64_t*)m->values.data(), m->height(), m->width));
         return commit_blocks(mats, root);
     }
@@ -348,46 +309,24 @@ class RowShardBackend : public GpuBackend {
     PcsHandlePtr commit_stage1(const std::vector<size_t>& circuits, const std::vector<MatrixView>& traces, Digest& root) override {
         end_proof();
         active_ = circuits;
-        claims_rank_ = world() - 1;  // the claims are uploaded, hashed and accumulated by ONE rank (not the FRI owner)
+        claims_rank_ = world() - 1;  // not the FRI owner
         if (rank() != claims_rank_) announced_ = ClaimsView();
         for (size_t p = 0; p < circuits.size(); p++) {
             const MatrixView& m = traces[p];
-            if (!m.data) throw RowShardError("row-sharded prover: every rank needs (read access to) every trace");
+            if (!m.data) throw DistError("row-sharded prover: every rank needs (read access to) every trace");
             trace_rows_.push_back(m.height());
             if (lookup_next_ && shardable(m.height(), m.width))
-                throw RowShardError("row-sharded prover: lookups that read the next row are not supported on row blocks");
+                throw DistError("row-sharded prover: lookups that read the next row are not supported on row blocks");
             main_.push_back(upload_blocks((const uint64_t*)m.data, m.height(), m.width));
         }
         prefetch_announced_claims();
         return commit_blocks(main_, root);
     }
 
-    bool observe_claims(Challenger& ch, const ClaimsView& claims) override {
-        if (!claims_on_device(claims)) return GpuBackend::observe_claims(ch, claims);
-        Digest d{};
-        if (rank() == claims_rank_ && !claims_transcript_digest(ch.input_buffer(), claims, d))
-            throw RowShardError("claims: internal error, device path refused");
-        comm_.bcast(d.data(), 32, claims_rank_);
-        ch.set_flushed(d);
-        return true;
-    }
-    Fp2 claims_accumulator(const ClaimsView& claims, Fp2 beta, Fp2 gamma) override {
-        if (!claims_on_device(claims)) return GpuBackend::claims_accumulator(claims, beta, gamma);
-        uint64_t out[2] = {0, 0};
-        if (rank() == claims_rank_) {
-            Fp2 a = GpuBackend::claims_accumulator(claims, beta, gamma);
-            out[0] = a.c[0].v;
-            out[1] = a.c[1].v;
-        }
-        comm_.bcast(out, 16, claims_rank_);
-        return Fp2(Fp(out[0]), Fp(out[1]));
-    }
-
     PcsHandlePtr commit_stage2(Fp2 beta, Fp2 gamma, Fp2 acc, std::vector<Fp2>& intermediate, Digest& root) override {
         const int N = world(), d = rank();
         uint64_t b[2] = {beta.c[0].v, beta.c[1].v}, g[2] = {gamma.c[0].v, gamma.c[1].v};
         std::vector<RowBlocks> s2;
-        struct Free { RowShardBackend* be; std::vector<RowBlocks>& v; ~Free() { for (auto& x : v) be->free_blocks(x); } } fr{this, s2};
         std::vector<uint64_t> sums(2 * active_.size(), 0);
         for (size_t p = 0; p < active_.size(); p++) {
             const Circuit& c = shape_.circuits[active_[p]];
@@ -397,12 +336,12 @@ class RowShardBackend : public GpuBackend {
             out.height = mt.height;
             out.width = c.stage_2_width;
             out.whole = mt.whole;
-            void* buf = nullptr;
-            gpu_check(msgpu_malloc(ctx_, std::max<size_t>(rows * c.stage_2_width * 8, 8), &buf));
-            out.dev = (uint64_t*)buf;
-            s2.push_back(out);
-            const uint64_t* pre = pre_dev_[active_[p]] ? pre_dev_[active_[p]] + row0 * c.preprocessed_width : nullptr;
-            gpu_check(msgpu_stage2_trace(ctx_, programs_[active_[p]], pre, mt.dev, rows, b, g, out.dev, &sums[2 * p]));
+            out.own = DevBuf(ctx_, rows * c.stage_2_width * 8);
+            out.dev = out.own.get();
+            uint64_t* dst = out.own.get();
+            s2.push_back(std::move(out));
+            const uint64_t* pre = pre_dev_[active_[p]].get() ? pre_dev_[active_[p]].get() + row0 * c.preprocessed_width : nullptr;
+            gpu_check(msgpu_stage2_trace(ctx_, programs_[active_[p]], pre, mt.dev, rows, b, g, dst, &sums[2 * p]));
         }
         // the ranks' totals: offsets of the row blocks' running sums, and the circuits' totals for the accumulator chain
         std::vector<uint64_t> all(sums.size() * (size_t)N);
@@ -422,7 +361,7 @@ class RowShardBackend : public GpuBackend {
                 }
                 if (!offset.is_zero()) {
                     uint64_t o2[2] = {offset.c[0].v, offset.c[1].v};
-                    gpu_check(msgpu_ext_add_scalar_dev(ctx_, s2[p].dev, (s2[p].height / (size_t)N) * (c.stage_2_width / 2), o2));
+                    gpu_check(msgpu_ext_add_scalar_dev(ctx_, s2[p].own.get(), (s2[p].height / (size_t)N) * (c.stage_2_width / 2), o2));
                 }
             }
             acc += total;
@@ -432,15 +371,13 @@ class RowShardBackend : public GpuBackend {
         for (size_t p = 0; p < s2.size(); p++) {
             if (s2[p].whole || shardable(s2[p].height, s2[p].width)) continue;
             const size_t nb = s2[p].height / (size_t)N, w = s2[p].width;
-            void* full = nullptr;
-            gpu_check(msgpu_malloc(ctx_, s2[p].height * w * 8, &full));
-            comm_.allgather_dev(s2[p].dev, full, nb * w * 8);
-            free_blocks(s2[p]);
-            s2[p].dev = (uint64_t*)full;
+            DevBuf full(ctx_, s2[p].height * w * 8);
+            comm_.allgather_dev(s2[p].own.get(), full.get(), nb * w * 8);
+            s2[p].own = std::move(full);
+            s2[p].dev = s2[p].own.get();
             s2[p].whole = true;
         }
         auto h = commit_blocks(s2, root);
-        for (auto& m : main_) free_blocks(m);
         main_.clear();
         return h;
     }
@@ -450,12 +387,11 @@ class RowShardBackend : public GpuBackend {
         auto* h1 = dynamic_cast<RowShardHandle*>(s1);
         auto* h2 = dynamic_cast<RowShardHandle*>(s2);
         auto* hp = pre ? dynamic_cast<RowShardHandle*>(pre) : nullptr;
-        if (!h1 || !h2 || (pre && !hp)) throw RowShardError("quotient: prover data does not belong to the row-sharded backend");
+        if (!h1 || !h2 || (pre && !hp)) throw DistError("quotient: prover data does not belong to the row-sharded backend");
         const int N = world(), d = rank();
         const uint32_t lb = (uint32_t)shape_.log_blowup();
         uint64_t a[2] = {alpha.c[0].v, alpha.c[1].v};
         auto h = std::make_shared<RowShardHandle>();
-        h->ctx = ctx_;
         h->n_shards = N;
         h->shard = d;
         for (auto& j : jobs) {
@@ -482,7 +418,7 @@ class RowShardBackend : public GpuBackend {
                     lo[k] = std::min<size_t>(lo[k], nd.col.index);
                     hi[k] = std::max<size_t>(hi[k], (size_t)nd.col.index + 1);
                 }
-            std::vector<DevPtr> halos;
+            std::vector<DevBuf> halos;
             size_t next_row0 = row0;
             const size_t dn = (size_t)d < Np ? next_of((size_t)d) : (size_t)d;
             if ((size_t)d < Np) next_row0 = dn * Ls;
@@ -490,7 +426,7 @@ class RowShardBackend : public GpuBackend {
                 if (k == 0 && !has_pre) continue;
                 RowShardHandle* sh = src[k].h;
                 const size_t i = src[k].idx, w = sh->shapes[i].second;
-                if (sh->shapes[i].first != H) throw RowShardError("quotient: the circuit's committed matrices differ in height");
+                if (sh->shapes[i].first != H) throw DistError("quotient: the circuit's committed matrices differ in height");
                 cur[k] = sh->views[i];
                 nxt[k] = sh->views[i];  // never read when the source has no next-row reference
                 nw[k] = (uint32_t)w;
@@ -506,37 +442,37 @@ class RowShardBackend : public GpuBackend {
                     // next rows they are (a permutation of the ranks: one all-to-all call)
                     const size_t wc = hi[k] - lo[k], rows = std::min(Ls, nq), bytes = rows * wc * 8;
                     std::vector<uint64_t> sb(N, 0), rb(N, 0);
-                    DevPtr packed(ctx_, bytes);
+                    DevBuf packed(ctx_, bytes);
                     bool need = false;
                     if ((size_t)d < Np && dn != (size_t)d) {
                         for (size_t e = 0; e < Np; e++)
                             if (next_of(e) == (size_t)d && e != (size_t)d) sb[e] = bytes;
-                        gpu_check(msgpu_extract_columns_dev(ctx_, sh->views[i], rows, w, lo[k], hi[k], packed.u()));
+                        gpu_check(msgpu_extract_columns_dev(ctx_, sh->views[i], rows, w, lo[k], hi[k], packed.get()));
                         rb[dn] = bytes;
                         need = true;
                     }
                     halos.emplace_back(ctx_, need ? bytes : 8);
                     rs_trace(rank(), "halo a2a", (size_t)k, bytes);
-                    comm_.alltoall_dev(packed.p, sb.data(), halos.back().p, rb.data());
+                    comm_.alltoall_dev(packed.get(), sb.data(), halos.back().get(), rb.data());
                     if (need) {
-                        nxt[k] = halos.back().u();
+                        nxt[k] = halos.back().get();
                         nw[k] = (uint32_t)wc;
                         nc0[k] = (uint32_t)lo[k];
                     }
                 }
             }
             // quotient evaluations of the local rows (stored order) -> all ranks -> the 2q-column quotient LDE on every rank
-            DevPtr mine(ctx_, std::max<size_t>(Ls * 16, 16)), all(ctx_, (size_t)N * Ls * 16);
+            DevBuf mine(ctx_, std::max<size_t>(Ls * 16, 16)), all(ctx_, (size_t)N * Ls * 16);
             uint64_t pub[8];
             for (int k = 0; k < 8; k++) pub[k] = j.publics[k].v;
             gpu_check(msgpu_quotient_values_shard(ctx_, programs_[j.circuit], cur, nxt, nw, nc0, row0, n_local, next_row0, j.log_degree,
-                                                  j.log_quotient_degree, pub, a, mine.u()));
+                                                  j.log_quotient_degree, pub, a, mine.get()));
             halos.clear();
             rs_trace(rank(), "quotient values allgather", Ls * 16);
-            comm_.allgather_dev(mine.p, all.p, Ls * 16);  // the first nq rows of the result are the quotient domain
+            comm_.allgather_dev(mine.get(), all.get(), Ls * 16);  // the first nq rows of the result are the quotient domain
             uint64_t* lde = nullptr;
-            gpu_check(msgpu_quotient_finish(ctx_, all.u(), j.log_degree, j.log_quotient_degree, lb, &lde));
-            h->owned.push_back(lde);
+            gpu_check(msgpu_quotient_finish(ctx_, all.get(), j.log_degree, j.log_quotient_degree, lb, &lde));
+            h->owned.emplace_back(ctx_, lde);
             h->views.push_back(lde + (size_t)d * Ls * (2 * q));
             h->whole.push_back(true);
             h->shapes.push_back({H, 2 * q});
@@ -547,24 +483,9 @@ class RowShardBackend : public GpuBackend {
     std::unique_ptr<OpenDevice> open_begin(const std::vector<OpenRound>& rounds) override;
 
     void end_proof() override {
-        drop_claims();
-        for (auto& m : main_) free_blocks(m);
+        GpuBackend::end_proof();
         main_.clear();
-        trace_rows_.clear();
-        active_.clear();
     }
-
-    // RAII device buffer over the C ABI
-    struct DevPtr {
-        msgpu_ctx* c;
-        void* p = nullptr;
-        DevPtr(msgpu_ctx* c_, size_t bytes) : c(c_) { gpu_check(msgpu_malloc(c, std::max<size_t>(bytes, 8), &p)); }
-        DevPtr(DevPtr&& o) noexcept : c(o.c), p(o.p) { o.p = nullptr; }
-        DevPtr(const DevPtr&) = delete;
-        ~DevPtr() { reset(); }
-        void reset() { if (p) msgpu_free(c, p); p = nullptr; }
-        uint64_t* u() const { return (uint64_t*)p; }
-    };
 
     // ---- the symmetric peer heap -----------------------------------------------------------------------------------------
     // Every rank makes the same calls with the same sizes, so the deterministic allocator returns the same (segment, offset)
@@ -575,7 +496,7 @@ class RowShardBackend : public GpuBackend {
         if (rc == 1) {
             sym_grow(bytes);
             rc = msgpu_peers_alloc(peers_, bytes, &b.seg, &b.off);
-            if (rc == 1) throw RowShardError("peer heap: internal error, a fresh window cannot hold the block it was made for");
+            if (rc == 1) throw DistError("peer heap: internal error, a fresh window cannot hold the block it was made for");
         }
         gpu_check(rc);
         b.live = true;
@@ -609,7 +530,7 @@ class RowShardBackend : public GpuBackend {
         return ok;
     }
     void sym_grow(size_t need) {
-        if (!sym_grow_try(need)) throw RowShardError(std::string("peer heap: a window could not be created or mapped on every rank: ") + msgpu_last_error());
+        if (!sym_grow_try(need)) throw DistError(std::string("peer heap: a window could not be created or mapped on every rank: ") + msgpu_last_error());
     }
     void init_peers() {
         gpu_check(msgpu_peers_create(ctx_, comm_.rank(), comm_.world(), &peers_));
@@ -621,16 +542,14 @@ class RowShardBackend : public GpuBackend {
     }
     msgpu_peers* peers_ = nullptr;
     uint64_t peer_bytes_ = 0;
-    RowShardComm comm_;
     std::vector<RowBlocks> main_;  // the natural-order traces (row blocks or whole), kept for the stage-2 construction
-    int claims_rank_ = 0;
     bool lookup_next_ = false;
 };
 
 // Pcs::open over the row shards.
-class RowShardOpenDevice : public OpenDevice {
+class RowShardOpenDevice : public ShardedOpenDevice {
   public:
-    RowShardOpenDevice(RowShardBackend& be, const std::vector<OpenRound>& rounds, uint32_t log_blowup) : be_(be), ctx_(be.ctx()), comm_(be.comm()) {
+    RowShardOpenDevice(RowShardBackend& be, const std::vector<OpenRound>& rounds, uint32_t log_blowup) : ShardedOpenDevice(be.ctx(), be.comm(), rounds) {
         const int N = comm_.world(), d = comm_.rank();
         std::vector<const msgpu_pdata*> pds;
         std::vector<uint32_t> modes;
@@ -638,11 +557,10 @@ class RowShardOpenDevice : public OpenDevice {
         size_t max_h = 0;
         for (auto& r : rounds) {
             auto* h = dynamic_cast<RowShardHandle*>(r.data);
-            if (!h) throw RowShardError("open: prover data does not belong to the row-sharded backend");
-            if (r.points.size() != h->shapes.size()) throw RowShardError("open: one point list per committed matrix expected");
+            if (!h) throw DistError("open: prover data does not belong to the row-sharded backend");
+            if (r.points.size() != h->shapes.size()) throw DistError("open: one point list per committed matrix expected");
             handles_.push_back(h);
-            points_.push_back(r.points);
-            pds.push_back(h->local);
+            pds.push_back(h->local.get());
             modes.push_back(1);
             for (size_t m = 0; m < h->shapes.size(); m++) {
                 max_h = std::max(max_h, h->shapes[m].first);
@@ -667,26 +585,11 @@ class RowShardOpenDevice : public OpenDevice {
         }
         gpu_check(msgpu_open_finish_values(op_, mine.data()));
     }
-    ~RowShardOpenDevice() override {
-        if (op_) msgpu_open_free(op_);
-    }
 
     std::vector<OpenedValuesForRound> evaluate() override {
         std::vector<uint64_t> flat(std::max<size_t>(2 * n_values_, 1));
         gpu_check(msgpu_open_values(op_, flat.data()));
-        std::vector<OpenedValuesForRound> out(handles_.size());
-        size_t o = 0;
-        for (size_t r = 0; r < handles_.size(); r++) {
-            out[r].resize(handles_[r]->shapes.size());
-            for (size_t m = 0; m < handles_[r]->shapes.size(); m++) {
-                out[r][m].resize(points_[r][m].size());
-                for (auto& pv : out[r][m]) {
-                    pv.resize(handles_[r]->shapes[m].second);
-                    for (auto& v : pv) { v.c[0].v = flat[o++]; v.c[1].v = flat[o++]; }
-                }
-            }
-        }
-        return out;
+        return decode_opened_values(rounds_, flat.data());
     }
 
     void reduce(Fp2 alpha, unsigned& log_max_height) override {
@@ -705,10 +608,10 @@ class RowShardOpenDevice : public OpenDevice {
             if (d == fri_owner_) {
                 for (int e = 0; e < N; e++)
                     if (e != fri_owner_) rb[e] = Ls * 16;
-                RowShardBackend::DevPtr tmp(ctx_, (uint64_t)(N - 1) * Ls * 16);
-                comm_.alltoall_dev(p, sb.data(), tmp.p, rb.data());
+                DevBuf tmp(ctx_, (uint64_t)(N - 1) * Ls * 16);
+                comm_.alltoall_dev(p, sb.data(), tmp.get(), rb.data());
                 // chunks arrive in rank order; the owner is rank 0, so they are the rows from Ls on
-                gpu_check(msgpu_ext_add_dev(ctx_, p + 2 * Ls, tmp.u(), (uint64_t)(N - 1) * Ls));
+                gpu_check(msgpu_ext_add_dev(ctx_, p + 2 * Ls, tmp.get(), (uint64_t)(N - 1) * Ls));
                 gpu_check(msgpu_sync(ctx_));
             } else {
                 sb[fri_owner_] = Ls * 16;
@@ -718,79 +621,13 @@ class RowShardOpenDevice : public OpenDevice {
         cur_len_ = size_t(1) << log_max_height_;
         log_max_height = log_max_height_;
     }
-    size_t current_len() override { return cur_len_; }
-    Digest commit_round() override { throw RowShardError("commit_round: the commit phase runs as a whole"); }
-    void fold(Fp2) override { throw RowShardError("fold: the commit phase runs as a whole"); }
-
-    // The owner folds (transcript on the device when there is no proof of work); every other rank replays the transcript from
-    // ONE broadcast of (roots, PoW witnesses, folded vector).
-    void commit_phase(Challenger& ch, size_t stop_len, size_t pow_bits, FriProof& proof) override {
-        size_t rounds = 0;
-        for (size_t l = cur_len_; l > stop_len; l >>= 1) rounds++;
-        const size_t final_len = cur_len_ >> rounds;
-        std::vector<u8> blob(rounds * 40 + final_len * 16);
-        rs_trace(comm_.rank(), "fri commit phase", rounds);
-        if (comm_.rank() == fri_owner_) {
-            const std::vector<u8>& buf = ch.input_buffer();
-            if (pow_bits == 0 && !buf.empty() && buf.size() <= 960 && rounds <= 64) {
-                uint8_t roots[64 * 32];
-                uint64_t bt[64 * 2], n = 0;
-                gpu_check(msgpu_fri_commit_phase(op_, buf.data(), buf.size(), stop_len, 64, roots, bt, &n));
-                for (uint64_t k = 0; k < n; k++) {
-                    Digest commit;
-                    memcpy(commit.data(), roots + 32 * k, 32);
-                    ch.observe(commit);
-                    proof.commit_phase_commits.push_back(commit);
-                    proof.commit_pow_witnesses.push_back(ch.grind(0));
-                    Fp2 beta = ch.sample_ext();
-                    if (beta.c[0].v != bt[2 * k] || beta.c[1].v != bt[2 * k + 1])
-                        throw RowShardError("fri: the device transcript and the host challenger disagree on a folding challenge");
-                    betas.push_back(beta);
-                }
-            } else {
-                while (cur_len_ > stop_len) {
-                    Digest commit{};
-                    gpu_check(msgpu_fri_commit_round(op_, commit.data()));
-                    ch.observe(commit);
-                    proof.commit_phase_commits.push_back(commit);
-                    proof.commit_pow_witnesses.push_back(ch.grind(pow_bits));
-                    Fp2 beta = ch.sample_ext();
-                    betas.push_back(beta);
-                    uint64_t b2[2] = {beta.c[0].v, beta.c[1].v};
-                    gpu_check(msgpu_fri_fold(op_, b2));
-                    cur_len_ /= 2;
-                }
-            }
-            if (proof.commit_phase_commits.size() != rounds) throw RowShardError("fri: internal error, round count");
-            for (size_t k = 0; k < rounds; k++) {
-                memcpy(blob.data() + 40 * k, proof.commit_phase_commits[k].data(), 32);
-                memcpy(blob.data() + 40 * k + 32, &proof.commit_pow_witnesses[k].v, 8);
-            }
-            gpu_check(msgpu_fri_read_current(op_, (uint64_t*)(blob.data() + rounds * 40)));
-        }
-        comm_.bcast(blob.data(), blob.size(), fri_owner_);
-        if (comm_.rank() != fri_owner_) {
-            for (size_t k = 0; k < rounds; k++) {
-                Digest dg;
-                Fp w;
-                memcpy(dg.data(), blob.data() + 40 * k, 32);
-                memcpy(&w.v, blob.data() + 40 * k + 32, 8);
-                ch.observe(dg);
-                proof.commit_phase_commits.push_back(dg);
-                if (!ch.check_witness(pow_bits, w)) throw RowShardError("fri: the owner's proof-of-work witness does not verify");
-                proof.commit_pow_witnesses.push_back(w);
-                betas.push_back(ch.sample_ext());
-            }
-        }
-        cur_len_ = final_len;
-        folded_.resize(final_len);
-        const uint64_t* f = (const uint64_t*)(blob.data() + rounds * 40);
-        for (size_t i = 0; i < final_len; i++) { folded_[i].c[0].v = f[2 * i]; folded_[i].c[1].v = f[2 * i + 1]; }
+  protected:
+    // the device transcript when there is no proof of work, otherwise the host loop
+    void owner_commit_phase(Challenger& ch, size_t stop_len, size_t pow_bits, FriProof& proof) override {
+        if (!fri_commit_phase_on_device(op_, cur_len_, ch, stop_len, pow_bits, proof, betas)) OpenDevice::commit_phase(ch, stop_len, pow_bits, proof);
     }
-    std::vector<Fp2> read_current() override { return folded_; }
-    std::vector<BatchOpening> open_round(size_t, const std::vector<size_t>&) override { throw RowShardError("open_round: use open_queries"); }
-    std::vector<BatchOpening> open_layer(size_t, const std::vector<size_t>&) override { throw RowShardError("open_layer: use open_queries"); }
 
+  public:
     // Rows and the lower log2(H / N) siblings of a query come from the rank that holds the row, the top log2 N siblings from the
     // top tree (on every rank); the FRI layers from the owner. One all-gather of every rank's share.
     void open_queries(const std::vector<size_t>& indices, const std::vector<unsigned>& round_shifts, size_t n_layers,
@@ -820,7 +657,7 @@ class RowShardOpenDevice : public OpenDevice {
             if (mine.empty()) continue;
             std::vector<uint64_t> opened(mine.size() * std::max<size_t>(tw[r], 1));
             std::vector<uint8_t> paths(std::max<size_t>(mine.size() * lo_depth[r] * 32, 1));
-            gpu_check(msgpu_open_batch(ctx_, handles_[r]->local, mine.data(), mine.size(), opened.data(), paths.data()));
+            gpu_check(msgpu_open_batch(ctx_, handles_[r]->local.get(), mine.data(), mine.size(), opened.data(), paths.data()));
             const size_t ob = mine.size() * tw[r] * 8, pb = mine.size() * lo_depth[r] * 32;
             const size_t at = blob.size();
             blob.resize(at + ob + pb);
@@ -831,7 +668,7 @@ class RowShardOpenDevice : public OpenDevice {
         std::vector<size_t> share(N, 0);
         for (size_t r = 0; r < R; r++)
             for (size_t q = 0; q < n; q++) share[holder[r][q]] += tw[r] * 8 + lo_depth[r] * 32;
-        if (share[d] != blob.size()) throw RowShardError("open: internal error, query share size");
+        if (share[d] != blob.size()) throw DistError("open: internal error, query share size");
         size_t mx = 8;
         for (size_t sz : share) mx = std::max(mx, sz);
         std::vector<u8> sendbuf(mx, 0), recvbuf(mx * (size_t)N);
@@ -840,25 +677,21 @@ class RowShardOpenDevice : public OpenDevice {
         std::vector<std::vector<u8>> all(N);
         for (int e = 0; e < N; e++) all[e].assign(recvbuf.begin() + (size_t)e * mx, recvbuf.begin() + (size_t)e * mx + share[e]);
         // the commit-phase layers live on the FRI owner: one broadcast of their openings
-        std::vector<u8> layer_blob;
+        layers_out.clear();
         if (n_layers) {
-            size_t open_total = n_layers * n * 4, proof_total = 0;
-            for (size_t k = 0; k < n_layers; k++) proof_total += n * (log_max_height_ - k - 1) * 32;
-            layer_blob.resize(open_total * 8 + proof_total);
-            if (d == fri_owner_) {
-                std::vector<const msgpu_pdata*> trees;
-                std::vector<uint32_t> shifts;
-                for (size_t k = 0; k < n_layers; k++) {
-                    const msgpu_pdata* pd = msgpu_fri_layer_pdata(op_, k);
-                    if (!pd) throw RowShardError("open: no such commit-phase layer");
-                    trees.push_back(pd);
+            std::vector<const msgpu_pdata*> trees;
+            std::vector<uint32_t> shifts;
+            std::vector<TreeShape> shapes;
+            for (size_t k = 0; k < n_layers; k++) {
+                if (d == fri_owner_) {
+                    trees.push_back(fri_layer(op_, k));
                     shifts.push_back((uint32_t)(k + 1));
                 }
-                std::vector<uint64_t> idx(indices.begin(), indices.end());
-                gpu_check(msgpu_open_batch_multi(ctx_, trees.data(), shifts.data(), trees.size(), idx.data(), n, (uint64_t*)layer_blob.data(),
-                                                 layer_blob.data() + open_total * 8));
+                shapes.push_back(TreeShape{{4}, (size_t)(log_max_height_ - k - 1)});
             }
+            std::vector<u8> layer_blob = d == fri_owner_ ? open_batch_multi(ctx_, trees, shifts, shapes, indices) : std::vector<u8>(batch_bytes(shapes, n));
             comm_.bcast(layer_blob.data(), layer_blob.size(), fri_owner_);
+            layers_out = decode_batch_openings(shapes, n, layer_blob);
         }
         // the top siblings of every (round, query): the top tree's leaf is the holder's subtree root
         std::vector<std::vector<uint8_t>> top_paths(R);
@@ -866,10 +699,9 @@ class RowShardOpenDevice : public OpenDevice {
             std::vector<uint64_t> tidx(holder[r].begin(), holder[r].end());
             top_paths[r].resize(n * log_n_shards * 32);
             uint64_t dummy = 0;
-            gpu_check(msgpu_open_batch(ctx_, handles_[r]->top, tidx.data(), n, &dummy, top_paths[r].data()));
+            gpu_check(msgpu_open_batch(ctx_, handles_[r]->top.get(), tidx.data(), n, &dummy, top_paths[r].data()));
         }
         rounds_out.assign(R, std::vector<BatchOpening>(n));
-        layers_out.assign(n_layers, std::vector<BatchOpening>(n));
         std::vector<size_t> cursor(N, 0);
         for (size_t r = 0; r < R; r++) {
             // the holders' shares list their queries in query order: walk them with one cursor per rank
@@ -880,7 +712,7 @@ class RowShardOpenDevice : public OpenDevice {
                 const u8* base = all[e].data() + cursor[e];
                 const u8* rowp = base + seen[e] * tw[r] * 8;
                 const u8* pathp = base + cnt[e] * tw[r] * 8 + seen[e] * lo_depth[r] * 32;
-                if (cursor[e] + cnt[e] * (tw[r] * 8 + lo_depth[r] * 32) > all[e].size()) throw RowShardError("open: a rank sent a query share of unexpected size");
+                if (cursor[e] + cnt[e] * (tw[r] * 8 + lo_depth[r] * 32) > all[e].size()) throw DistError("open: a rank sent a query share of unexpected size");
                 BatchOpening& bo = rounds_out[r][q];
                 for (auto& s : handles_[r]->shapes) {
                     std::vector<Fp> row(s.second);
@@ -896,36 +728,11 @@ class RowShardOpenDevice : public OpenDevice {
             }
             for (int e = 0; e < N; e++) cursor[e] += cnt[e] * (tw[r] * 8 + lo_depth[r] * 32);
         }
-        if (n_layers) {
-            const u8* ob = layer_blob.data();
-            const u8* pb = ob + n_layers * n * 32;
-            for (size_t k = 0; k < n_layers; k++) {
-                const size_t depth = log_max_height_ - k - 1;
-                for (size_t q = 0; q < n; q++) {
-                    BatchOpening& bo = layers_out[k][q];
-                    std::vector<Fp> row(4);
-                    memcpy(row.data(), ob, 32);
-                    ob += 32;
-                    bo.opened_values.push_back(std::move(row));
-                    bo.opening_proof.resize(depth);
-                    for (size_t l = 0; l < depth; l++, pb += 32) memcpy(bo.opening_proof[l].data(), pb, 32);
-                }
-            }
-        }
     }
 
   private:
-    RowShardBackend& be_;
-    msgpu_ctx* ctx_;
-    const RowShardComm& comm_;
-    msgpu_open* op_ = nullptr;
     uint64_t n_values_ = 0;
     std::vector<RowShardHandle*> handles_;
-    std::vector<std::vector<std::vector<Fp2>>> points_;
-    const int fri_owner_ = 0;
-    unsigned log_max_height_ = 0;
-    size_t cur_len_ = 0;
-    std::vector<Fp2> folded_;
 };
 
 inline std::unique_ptr<OpenDevice> RowShardBackend::open_begin(const std::vector<OpenRound>& rounds) {

@@ -201,22 +201,38 @@ class CpuOpenDevice : public OpenDevice {
 
     std::vector<Fp2> read_current() override { return cur_; }
 
-    std::vector<msh::BatchOpening> open_round(size_t r, const std::vector<size_t>& indices) override {
-        auto* pd = dynamic_cast<CpuPcsData*>(rounds_[r].data);
-        std::vector<msh::BatchOpening> out;
-        for (size_t i : indices) out.push_back(to_host_opening(open_batch(pd->tree, i)));
-        return out;
-    }
-    std::vector<msh::BatchOpening> open_layer(size_t k, const std::vector<size_t>& pair_indices) override {
-        std::vector<msh::BatchOpening> out;
-        for (size_t i : pair_indices) out.push_back(to_host_opening(open_batch(layers_.at(k)->tree, i)));
-        return out;
+    void open_queries(const std::vector<size_t>& indices, const std::vector<unsigned>& round_shifts, size_t n_layers,
+                      std::vector<std::vector<msh::BatchOpening>>& rounds_out, std::vector<std::vector<msh::BatchOpening>>& layers_out) override {
+        rounds_out.clear();
+        layers_out.clear();
+        std::vector<size_t> reduced(indices.size());
+        for (size_t r = 0; r < round_shifts.size(); r++) {
+            for (size_t q = 0; q < indices.size(); q++) reduced[q] = indices[q] >> round_shifts[r];
+            rounds_out.push_back(open_round(r, reduced));
+        }
+        for (size_t k = 0; k < n_layers; k++) {
+            for (size_t q = 0; q < indices.size(); q++) reduced[q] = indices[q] >> (k + 1);
+            layers_out.push_back(open_layer(k, reduced));
+        }
     }
 
     // test hook: FRI input k (tallest first)
     const std::vector<std::vector<Fp2>>& inputs() const { return inputs_; }
 
   private:
+    // Mmcs::open_batch of round `r` at every index (already reduced to the round's height)
+    std::vector<msh::BatchOpening> open_round(size_t r, const std::vector<size_t>& indices) {
+        auto* pd = dynamic_cast<CpuPcsData*>(rounds_[r].data);
+        std::vector<msh::BatchOpening> out;
+        for (size_t i : indices) out.push_back(to_host_opening(open_batch(pd->tree, i)));
+        return out;
+    }
+    // Mmcs::open_batch of commit-phase layer `k` at every pair index
+    std::vector<msh::BatchOpening> open_layer(size_t k, const std::vector<size_t>& pair_indices) {
+        std::vector<msh::BatchOpening> out;
+        for (size_t i : pair_indices) out.push_back(to_host_opening(open_batch(layers_.at(k)->tree, i)));
+        return out;
+    }
     // 1 / (z - x), x = GENERATOR * w_H^{rev(i)} (p3 `compute_inverse_denominators`), cached per (z, log H)
     const std::vector<Fp2>& inverse_denominators(const Fp2& z, unsigned lh) {
         for (auto& e : invden_)

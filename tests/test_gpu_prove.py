@@ -145,6 +145,10 @@ def test_invalid_witness_is_an_error_not_a_crash(gpu):
     bad[3, 0] = P  # not canonical
     with pytest.raises(ms.MsgpuError):
         prover.prove([bad], [])
+    # the refused proofs left no per-proof state behind: the same prover still proves the valid trace, byte for byte
+    fresh = ms.Prover(ctx, system)
+    assert prover.prove([tr], []) == fresh.prove([tr], [])
+    fresh.close()
     prover.close()
 
 
