@@ -137,6 +137,7 @@ class MsgpuError(RuntimeError):
     def __init__(self, code, message):
         super().__init__("msgpu error %d: %s" % (code, message))
         self.code = code
+        self.message = message
 
 
 def lib_path():
@@ -166,6 +167,12 @@ def lib():
 def check(code):
     if code != 0:
         raise MsgpuError(code, (lib().msgpu_last_error() or b"").decode("utf-8", "replace"))
+
+
+def host_error(code, extra=""):
+    """MsgpuError(code) carrying libmshost.so's last error message, followed by `extra` (a communicator's errors) if given."""
+    message = (host_lib().msh_last_error() or b"").decode("utf-8", "replace")
+    return MsgpuError(code, message + " " + extra if extra else message)
 
 
 # ---- libmshost.so: host-side protocol layer (system assembly, workloads, prove driver) ---------------

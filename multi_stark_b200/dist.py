@@ -4,15 +4,20 @@ The commitment path shards by independent units -- whole proofs, or the circuit 
 so there is NO data-path collective: every rank runs the full single-GPU pipeline on its own units. Ranks exchange only
 what the protocol makes public anyway (32-byte commitments / proof digests) and the timing needed for an honest aggregate
 (max over ranks). The reference has no multi-process story at all (SURVEY section 2: rayon inside one process)."""
+import contextlib
+import ctypes as _C
 import hashlib
 import os
 import sys
 import time
 
+import numpy as np
 import torch
 import torch.distributed as dist
 
-from ._ffi import check
+from ._ffi import check, host_error, host_lib
+from .pcs import ProverData
+from .system import ProverBase
 
 
 def world():
@@ -105,8 +110,6 @@ def prove_sharded(units, prove_fn):
 # ------------------------------------------------------------------------------------------------------------------
 # One proof over several GPUs: the collectives the sharded prover (host/dist_backend.hpp) calls back into.
 # ------------------------------------------------------------------------------------------------------------------
-import ctypes as _C  # noqa: E402
-
 _ALLGATHER = _C.CFUNCTYPE(_C.c_int, _C.c_void_p, _C.c_void_p, _C.c_void_p, _C.c_uint64)
 _BCAST = _C.CFUNCTYPE(_C.c_int, _C.c_void_p, _C.c_void_p, _C.c_uint64, _C.c_int32)
 _SENDRECV = _C.CFUNCTYPE(_C.c_int, _C.c_void_p, _C.c_void_p, _C.c_uint64, _C.c_int32, _C.c_int32)
@@ -131,20 +134,20 @@ class _DevView:
 class TorchComm:
     """Collectives over the default torch.distributed group. Host buffers travel as CPU tensors over gloo, or staged through
     the device over NCCL; device buffers travel device-to-device over NCCL (NVLink), or staged through pinned host memory
-    over gloo (the single-GPU tests run two ranks on one device that way)."""
+    over gloo (the single-GPU tests run two ranks on one device that way). Each collective raises on failure; `struct` holds
+    them as the C callbacks of `msh_comm`, which report a failure as 1 and its exception in `errors`."""
 
     def __init__(self, ctx, group=None):
-        import torch.distributed as dist
         self.ctx = ctx
-        self.dist = dist
         self.group = group
         self.nccl = dist.get_backend(group) == "nccl"
         self.rank, self.world = dist.get_rank(group), dist.get_world_size(group)
         self.bytes_dev = 0   # device bytes sent or received by this rank (reported by bench / tools)
         self.bytes_host = 0
         self.errors = []
-        self.seconds = {}    # wall time spent inside the callbacks, by kind
+        self.seconds = {}    # wall time spent inside the collectives, by kind
         self._stage = None
+        self._seq = 0
         self.trace = bool(os.environ.get("MSH_TRACE"))
         self.trace2 = int(os.environ.get("MSH_TRACE") or 0) >= 2
         if self.nccl:
@@ -153,20 +156,37 @@ class TorchComm:
             cur = torch.cuda.current_stream().cuda_stream
             if int(ctx.stream or 0) != int(cur):
                 raise ValueError("TorchComm: create the GpuContext on torch's current stream (GpuContext(dev, stream=torch.cuda.current_stream().cuda_stream))")
-        self._cb = (_ALLGATHER(self._allgather), _BCAST(self._bcast), _SENDRECV(self._sendrecv), _ALLTOALL(self._alltoall_cb),
-                    _ALLGATHER_DEV(self._allgather_dev_cb))  # keep the thunks alive
+        self._cb = (self._callback(_ALLGATHER, self.allgather_host), self._callback(_BCAST, self.bcast_host),
+                    self._callback(_SENDRECV, self.sendrecv_dev), self._callback(_ALLTOALL, self.all_to_all_dev),
+                    self._callback(_ALLGATHER_DEV, self.allgather_dev))  # keep the thunks alive
         # peer memory (csrc/peer.cu): NCCL ranks of one node, one GPU each; MSGPU_P2P=0 keeps every exchange on the collectives
         self.peer_memory = int(self.nccl and self.world > 1 and os.environ.get("MSGPU_P2P", "1") != "0"
                                and torch.cuda.device_count() >= self.world)
         self.struct = MshComm(None, self.rank, self.world, *self._cb, self.peer_memory)
 
-    # ---- host buffers
-    def _host_tensor(self, ptr, nbytes):
-        return torch.frombuffer((_C.c_uint8 * nbytes).from_address(ptr), dtype=torch.uint8)
+    def _callback(self, cfunctype, collective):
+        """`collective` as an msh_comm callback (its first argument, `user`, is unused)"""
+        def cb(user, *args):
+            if self.trace2:
+                print("[comm %d] %s%r" % (self.rank, collective.__name__, args), file=sys.stderr, flush=True)
+            try:
+                collective(*args)
+                return 0
+            except Exception as e:  # never unwind into C++
+                self.errors.append(repr(e))
+                return 1
+        return cfunctype(cb)
 
-    def _t2(self, what, n=0):
-        if self.trace2:
-            print("[comm %d] %s %d" % (self.rank, what, n), file=sys.stderr, flush=True)
+    @contextlib.contextmanager
+    def _timed(self, kind):
+        t0 = time.perf_counter()
+        try:
+            yield
+        finally:
+            self.seconds[kind] = self.seconds.get(kind, 0.0) + time.perf_counter() - t0
+
+    def _global(self, r):
+        return dist.get_global_rank(self.group, r) if self.group is not None else r
 
     def _same_call(self, kind):
         """gloo only: the staged device exchanges below move data pairwise, so a rank that SKIPPED one (a rank-dependent branch
@@ -174,20 +194,16 @@ class TorchComm:
         number, kind) first; a mismatch fails the call on every rank."""
         if self.nccl:
             return
-        self._seq = getattr(self, "_seq", 0) + 1
+        self._seq += 1
         mine = torch.tensor([self._seq, kind], dtype=torch.int64)
         allv = torch.empty(2 * self.world, dtype=torch.int64)
-        self.dist.all_gather_into_tensor(allv, mine, group=self.group)
+        dist.all_gather_into_tensor(allv, mine, group=self.group)
         if any(allv[2 * r] != self._seq or allv[2 * r + 1] != kind for r in range(self.world)):
             raise RuntimeError("ranks disagree on the sequence of device collectives: %s" % allv.tolist())
 
-    def _allgather(self, user, send, recv, nbytes):
-        self._t2("allgather_host", nbytes)
-        t0 = time.perf_counter()
-        try:
-            return self._allgather_impl(send, recv, nbytes)
-        finally:
-            self.seconds["allgather"] = self.seconds.get("allgather", 0.0) + time.perf_counter() - t0
+    # ---- host buffers
+    def _host_tensor(self, ptr, nbytes):
+        return torch.frombuffer((_C.c_uint8 * nbytes).from_address(ptr), dtype=torch.uint8)
 
     def _staging(self, nbytes):
         """persistent pinned-host and device staging buffers (grow-only): a fresh pageable tensor per call costs ms"""
@@ -197,8 +213,9 @@ class TorchComm:
             self._stage = (torch.empty(cap, dtype=torch.uint8).pin_memory(), torch.empty(cap, dtype=torch.uint8, device=dev))
         return self._stage
 
-    def _allgather_impl(self, send, recv, nbytes):
-        try:
+    def allgather_host(self, send, recv, nbytes):
+        """Host all-gather of equal chunks: recv = world chunks of nbytes in rank order."""
+        with self._timed("allgather"):
             nbytes = int(nbytes)
             s = self._host_tensor(send, nbytes)
             r = self._host_tensor(recv, nbytes * self.world)
@@ -210,7 +227,7 @@ class TorchComm:
                 _C.memmove(pin.data_ptr(), send, nbytes)  # (torch's CPU copy_ spins up its thread pool: ms for 1 MB)
                 dev[total:total + nbytes].copy_(pin[:nbytes], non_blocking=True)
                 tr.append(time.perf_counter())
-                self.dist.all_gather_into_tensor(dev[:total], dev[total:total + nbytes], group=self.group)
+                dist.all_gather_into_tensor(dev[:total], dev[total:total + nbytes], group=self.group)
                 tr.append(time.perf_counter())
                 pin[:total].copy_(dev[:total], non_blocking=True)
                 torch.cuda.current_stream().synchronize()
@@ -221,17 +238,12 @@ class TorchComm:
                     print("[comm] rank %d allgather %d B: staging %.3f, h2d %.3f, nccl call %.3f, d2h+sync %.3f, copy out %.3f ms" % (
                         (self.rank, nbytes) + tuple((b - a) * 1e3 for a, b in zip(tr, tr[1:]))), file=sys.stderr, flush=True)
             else:
-                self.dist.all_gather_into_tensor(r, s.clone(), group=self.group)
+                dist.all_gather_into_tensor(r, s.clone(), group=self.group)
             self.bytes_host += nbytes * self.world
-            return 0
-        except Exception as e:  # never unwind into C++
-            self.errors.append(repr(e))
-            return 1
 
-    def _bcast(self, user, buf, nbytes, root):
-        self._t2("bcast_host", nbytes)
-        t0 = time.perf_counter()
-        try:
+    def bcast_host(self, buf, nbytes, root):
+        """Host broadcast of nbytes from rank `root`."""
+        with self._timed("bcast"):
             nbytes = int(nbytes)
             t = self._host_tensor(buf, nbytes)
             if self.nccl:
@@ -239,136 +251,95 @@ class TorchComm:
                 if self.rank == root:
                     _C.memmove(pin.data_ptr(), buf, nbytes)
                     dev[:nbytes].copy_(pin[:nbytes], non_blocking=True)
-                self.dist.broadcast(dev[:nbytes], src=self._global(root), group=self.group)
+                dist.broadcast(dev[:nbytes], src=self._global(root), group=self.group)
                 if self.rank != root:
                     pin[:nbytes].copy_(dev[:nbytes], non_blocking=True)
                     torch.cuda.current_stream().synchronize()
                     _C.memmove(buf, pin.data_ptr(), nbytes)
             else:
-                self.dist.broadcast(t, src=self._global(root), group=self.group)
+                dist.broadcast(t, src=self._global(root), group=self.group)
             self.bytes_host += nbytes
-            return 0
-        except Exception as e:
-            self.errors.append(repr(e))
-            return 1
-        finally:
-            self.seconds["bcast"] = self.seconds.get("bcast", 0.0) + time.perf_counter() - t0
-
-    def _global(self, r):
-        return self.dist.get_global_rank(self.group, r) if self.group is not None else r
 
     # ---- device buffers
-    def _sendrecv(self, user, dev, nbytes, src, dst):
-        t0 = time.perf_counter()
-        try:
-            return self._sendrecv_impl(dev, nbytes, src, dst)
-        finally:
-            self.seconds["sendrecv"] = self.seconds.get("sendrecv", 0.0) + time.perf_counter() - t0
+    def _d2h(self, dev, nbytes):
+        """gloo staging: nbytes of device memory in a new host tensor"""
+        host = torch.empty(nbytes, dtype=torch.uint8)
+        if nbytes:
+            check(self.ctx.L.msgpu_memcpy_d2h(self.ctx.h, _C.c_void_p(host.data_ptr()), _C.c_void_p(dev), nbytes))
+        return host
 
-    def _sendrecv_impl(self, dev, nbytes, src, dst):
-        try:
+    def _h2d(self, dev, host):
+        """gloo staging: a host tensor back to device memory"""
+        if host.numel():
+            check(self.ctx.L.msgpu_memcpy_h2d(self.ctx.h, _C.c_void_p(dev), _C.c_void_p(host.data_ptr()), host.numel()))
+
+    def sendrecv_dev(self, dev, nbytes, src, dst):
+        """Device point-to-point: rank `src` sends nbytes at `dev`, rank `dst` receives them at its `dev`."""
+        with self._timed("sendrecv"):
             nbytes = int(nbytes)
             self.bytes_dev += nbytes
             if self.nccl:
                 t = torch.as_tensor(_DevView(dev, nbytes), device=torch.device("cuda", torch.cuda.current_device()))
                 if self.rank == src:
-                    self.dist.send(t, dst=self._global(dst), group=self.group)
+                    dist.send(t, dst=self._global(dst), group=self.group)
                 else:
-                    self.dist.recv(t, src=self._global(src), group=self.group)
+                    dist.recv(t, src=self._global(src), group=self.group)
                 torch.cuda.current_stream().synchronize()
-                return 0
-            # gloo: stage through host memory
-            host = torch.empty(nbytes, dtype=torch.uint8)
-            if self.rank == src:
-                check(self.ctx.L.msgpu_memcpy_d2h(self.ctx.h, _C.c_void_p(host.data_ptr()), _C.c_void_p(dev), nbytes))
-                self.dist.send(host, dst=self._global(dst), group=self.group)
+            elif self.rank == src:
+                dist.send(self._d2h(dev, nbytes), dst=self._global(dst), group=self.group)
             else:
-                self.dist.recv(host, src=self._global(src), group=self.group)
-                check(self.ctx.L.msgpu_memcpy_h2d(self.ctx.h, _C.c_void_p(dev), _C.c_void_p(host.data_ptr()), nbytes))
-            return 0
-        except Exception as e:
-            self.errors.append(repr(e))
-            return 1
+                host = torch.empty(nbytes, dtype=torch.uint8)
+                dist.recv(host, src=self._global(src), group=self.group)
+                self._h2d(dev, host)
 
+    def all_to_all_dev(self, send_ptr, send_counts, recv_ptr, recv_counts):
+        """Device all-to-all with per-peer byte counts (chunks in rank order in both buffers)."""
+        with self._timed("all_to_all"):
+            self._same_call(1)
+            send_counts = [int(send_counts[k]) for k in range(self.world)]
+            recv_counts = [int(recv_counts[k]) for k in range(self.world)]
+            self.bytes_dev += sum(send_counts) - send_counts[self.rank] + sum(recv_counts) - recv_counts[self.rank]
+            if self.nccl:
+                dev = torch.device("cuda", torch.cuda.current_device())
+                empty = torch.empty(0, dtype=torch.uint8, device=dev)
+                s = torch.as_tensor(_DevView(send_ptr, sum(send_counts)), device=dev) if sum(send_counts) else empty
+                r = torch.as_tensor(_DevView(recv_ptr, sum(recv_counts)), device=dev) if sum(recv_counts) else empty
+                # stream-ordered on the context's stream (checked in __init__): later kernels see the data, no host wait needed
+                dist.all_to_all_single(r, s, output_split_sizes=recv_counts, input_split_sizes=send_counts, group=self.group)
+                return
+            # gloo: staged through the host, pairwise
+            so = [sum(send_counts[:k]) for k in range(self.world)]
+            ro = [sum(recv_counts[:k]) for k in range(self.world)]
+            host_s = self._d2h(send_ptr, sum(send_counts))
+            host_r = torch.empty(sum(recv_counts), dtype=torch.uint8)
+            reqs = []
+            for k in range(self.world):
+                if k == self.rank:
+                    host_r[ro[k]:ro[k] + recv_counts[k]] = host_s[so[k]:so[k] + send_counts[k]]
+                    continue
+                if send_counts[k]:
+                    reqs.append(dist.isend(host_s[so[k]:so[k] + send_counts[k]], dst=self._global(k), group=self.group))
+                if recv_counts[k]:
+                    reqs.append(dist.irecv(host_r[ro[k]:ro[k] + recv_counts[k]], src=self._global(k), group=self.group))
+            for q in reqs:
+                q.wait()
+            self._h2d(recv_ptr, host_r)
 
-def _all_to_all_dev(self, send_ptr, send_counts, recv_ptr, recv_counts):
-    """Device all-to-all with per-peer byte counts (chunks in rank order in both buffers)."""
-    self._t2("alltoall_dev", sum(send_counts))
-    self._same_call(1)
-    t0 = time.perf_counter()
-    self.bytes_dev += sum(send_counts) - send_counts[self.rank] + sum(recv_counts) - recv_counts[self.rank]
-    if self.nccl:
-        dev = torch.device("cuda", torch.cuda.current_device())
-        empty = torch.empty(0, dtype=torch.uint8, device=dev)
-        s = torch.as_tensor(_DevView(send_ptr, sum(send_counts)), device=dev) if sum(send_counts) else empty
-        r = torch.as_tensor(_DevView(recv_ptr, sum(recv_counts)), device=dev) if sum(recv_counts) else empty
-        # stream-ordered on the context's stream (checked in __init__): later kernels see the data, no host wait needed
-        self.dist.all_to_all_single(r, s, output_split_sizes=list(recv_counts), input_split_sizes=list(send_counts), group=self.group)
-    else:  # gloo: staged through the host, pairwise
-        so = [sum(send_counts[:k]) for k in range(self.world)]
-        ro = [sum(recv_counts[:k]) for k in range(self.world)]
-        host_s = torch.empty(max(sum(send_counts), 1), dtype=torch.uint8)
-        host_r = torch.empty(max(sum(recv_counts), 1), dtype=torch.uint8)
-        if sum(send_counts):
-            check(self.ctx.L.msgpu_memcpy_d2h(self.ctx.h, _C.c_void_p(host_s.data_ptr()), _C.c_void_p(send_ptr), sum(send_counts)))
-        reqs = []
-        for k in range(self.world):
-            if k == self.rank:
-                host_r[ro[k]:ro[k] + recv_counts[k]] = host_s[so[k]:so[k] + send_counts[k]]
-                continue
-            if send_counts[k]:
-                reqs.append(self.dist.isend(host_s[so[k]:so[k] + send_counts[k]], dst=self._global(k), group=self.group))
-            if recv_counts[k]:
-                reqs.append(self.dist.irecv(host_r[ro[k]:ro[k] + recv_counts[k]], src=self._global(k), group=self.group))
-        for q in reqs:
-            q.wait()
-        if sum(recv_counts):
-            check(self.ctx.L.msgpu_memcpy_h2d(self.ctx.h, _C.c_void_p(recv_ptr), _C.c_void_p(host_r.data_ptr()), sum(recv_counts)))
-    self.seconds["all_to_all"] = self.seconds.get("all_to_all", 0.0) + time.perf_counter() - t0
-
-
-TorchComm.all_to_all_dev = _all_to_all_dev
-
-
-def _alltoall_cb(self, user, send, send_bytes, recv, recv_bytes):
-    try:
-        self.all_to_all_dev(int(send or 0), [int(send_bytes[k]) for k in range(self.world)], int(recv or 0),
-                            [int(recv_bytes[k]) for k in range(self.world)])
-        return 0
-    except Exception as e:  # never unwind into C++
-        self.errors.append(repr(e))
-        return 1
-
-
-def _allgather_dev_cb(self, user, send, recv, nbytes):
-    """Device all-gather of equal chunks: recv = world chunks of nbytes in rank order."""
-    self._t2("allgather_dev", nbytes)
-    t0 = time.perf_counter()
-    try:
-        self._same_call(2)
-        nbytes = int(nbytes)
-        self.bytes_dev += nbytes * (self.world - 1) * 2
-        if self.nccl:
-            dev = torch.device("cuda", torch.cuda.current_device())
-            s = torch.as_tensor(_DevView(send, nbytes), device=dev)
-            r = torch.as_tensor(_DevView(recv, nbytes * self.world), device=dev)
-            self.dist.all_gather_into_tensor(r, s, group=self.group)  # stream-ordered, as the all-to-all
-        else:  # gloo: staged through the host
-            hs = torch.empty(nbytes, dtype=torch.uint8)
-            hr = torch.empty(nbytes * self.world, dtype=torch.uint8)
-            check(self.ctx.L.msgpu_memcpy_d2h(self.ctx.h, _C.c_void_p(hs.data_ptr()), _C.c_void_p(send), nbytes))
-            self.dist.all_gather_into_tensor(hr, hs, group=self.group)
-            check(self.ctx.L.msgpu_memcpy_h2d(self.ctx.h, _C.c_void_p(recv), _C.c_void_p(hr.data_ptr()), nbytes * self.world))
-        return 0
-    except Exception as e:
-        self.errors.append(repr(e))
-        return 1
-    finally:
-        self.seconds["allgather_dev"] = self.seconds.get("allgather_dev", 0.0) + time.perf_counter() - t0
-
-
-TorchComm._alltoall_cb = _alltoall_cb
-TorchComm._allgather_dev_cb = _allgather_dev_cb
+    def allgather_dev(self, send, recv, nbytes):
+        """Device all-gather of equal chunks: recv = world chunks of nbytes in rank order."""
+        with self._timed("allgather_dev"):
+            self._same_call(2)
+            nbytes = int(nbytes)
+            self.bytes_dev += nbytes * (self.world - 1) * 2
+            if self.nccl:
+                dev = torch.device("cuda", torch.cuda.current_device())
+                s = torch.as_tensor(_DevView(send, nbytes), device=dev)
+                r = torch.as_tensor(_DevView(recv, nbytes * self.world), device=dev)
+                dist.all_gather_into_tensor(r, s, group=self.group)  # stream-ordered, as the all-to-all
+            else:  # gloo: staged through the host
+                host = torch.empty(nbytes * self.world, dtype=torch.uint8)
+                dist.all_gather_into_tensor(host, self._d2h(send, nbytes), group=self.group)
+                self._h2d(recv, host)
 
 
 def assign_owners(heights, world_size):
@@ -391,85 +362,53 @@ def assign_owners(heights, world_size):
     return owner
 
 
-class DistProver:
+class _ShardedProver(ProverBase):
+    """A prover whose backend calls back into a TorchComm; its errors carry the communicator's. No __del__: the teardown
+    unmaps peer memory, so these provers are freed by an explicit close()."""
+
+    def __init__(self, ctx, system, group, create, *args):
+        self.comm = TorchComm(ctx, group)
+        super().__init__(ctx, system, create, _C.byref(self.comm.struct), *args)
+
+    def _error(self, code):
+        return host_error(code, "; ".join(self.comm.errors))
+
+    @property
+    def bytes_dev(self):
+        """device bytes this rank exchanged so far"""
+        return self.comm.bytes_dev
+
+
+class DistProver(_ShardedProver):
     """`System::prove_multiple_claims` (src/prover.rs:289-603) as ONE proof over the ranks of a torch.distributed group: each
     rank owns whole circuits (`owner[i]`), builds and commits their traces and answers their openings; the proof bytes are
     identical on every rank and identical to the single-GPU proof."""
 
     def __init__(self, ctx, system, owner, group=None):
-        from . import _ffi
-        self.H = _ffi.host_lib()
-        self.ctx, self.system = ctx, system
-        self.comm = TorchComm(ctx, group)
         self.owner = [int(o) for o in owner]
         if len(self.owner) != system.num_circuits:
             raise ValueError("one owner per circuit expected")
-        arr = (_C.c_int32 * len(self.owner))(*self.owner)
-        self.h = self.H.msh_dist_prover_create(system.h, ctx.h, _C.byref(self.comm.struct), arr)
-        if not self.h:
-            raise _ffi.MsgpuError(-3, (self.H.msh_last_error() or b"").decode() + " " + "; ".join(self.comm.errors))
-        self.last_stage_ms = None
-
-    def preprocessed_commit(self):
-        import numpy as np
-        out = np.zeros(32, dtype=np.uint8)
-        return bytes(out) if self.H.msh_prover_preprocessed_commit(self.h, out.ctypes.data_as(_C.c_void_p)) else None
+        super().__init__(ctx, system, group, host_lib().msh_dist_prover_create, (_C.c_int32 * len(self.owner))(*self.owner))
 
     def prove(self, traces, heights, claims):
         """traces[i]: (h x main_width) uint64 array for the circuits this rank owns, None otherwise; heights[i]: trace rows of
-        EVERY circuit (0 = inactive); claims: (n, len) uint64 array, the same on every rank. Returns `Proof::to_bytes`."""
-        import numpy as np
-        from . import _ffi
-        from .system import STAGE_NAMES
-        n = self.system.num_circuits
+        EVERY circuit (0 = inactive); claims: as Prover.prove takes them, the same on every rank. Returns `Proof::to_bytes`."""
         mats = [None if t is None else np.ascontiguousarray(t, dtype=np.uint64) for t in traces]
-        for i in range(n):
+        for i in range(self.system.num_circuits):
             if self.owner[i] == self.comm.rank and heights[i] and (mats[i] is None or mats[i].shape[0] != heights[i]):
                 raise ValueError("the trace of circuit %d (owned by this rank) is missing or has the wrong height" % i)
-        ptrs = (_C.c_void_p * n)(*[m.ctypes.data if (m is not None and m.size and self.owner[i] == self.comm.rank) else None
-                                   for i, m in enumerate(mats)])
-        hs = (_C.c_uint64 * n)(*[int(h) for h in heights])
-        cl = np.ascontiguousarray(claims, dtype=np.uint64)
-        if cl.ndim != 2:
-            raise ValueError("claims: an (n, len) array is expected")
-        flat = cl.reshape(-1) if cl.size else np.zeros(1, dtype=np.uint64)
-        out, ln = _C.c_void_p(), _C.c_uint64()
-        ms = (_C.c_double * 6)()
-        rc = self.H.msh_prove(self.h, ptrs, hs, flat.ctypes.data_as(_ffi.c_u64p), None, cl.shape[1], cl.shape[0],
-                              _C.byref(out), _C.byref(ln), ms)
-        if rc != 0:
-            raise _ffi.MsgpuError(rc, (self.H.msh_last_error() or b"").decode() + " " + "; ".join(self.comm.errors))
-        data = _C.string_at(out.value, ln.value)
-        self.H.msh_bytes_free(out)
-        self.last_stage_ms = dict(zip(STAGE_NAMES, ms))
-        return data
-
-    def close(self):
-        if getattr(self, "h", None):
-            self.H.msh_prover_free(self.h)
-            self.h = None
+        return self._prove([m.ctypes.data if (m is not None and m.size and self.owner[i] == self.comm.rank) else None
+                            for i, m in enumerate(mats)], heights, claims)
 
 
-class RowShardProver:
+class RowShardProver(_ShardedProver):
     """`System::prove_multiple_claims` as ONE proof over the ROW SHARDS of every committed matrix (host/rowshard_backend.hpp):
     rank d of N holds rows [d H / N, (d + 1) H / N) of every LDE, so a single tall circuit is proved by all GPUs. Every rank
     passes ALL traces (it reads only its row block of the tall ones); the proof bytes are identical on every rank and identical
     to the single-GPU proof."""
 
     def __init__(self, ctx, system, group=None):
-        from . import _ffi
-        self.H = _ffi.host_lib()
-        self.ctx, self.system = ctx, system
-        self.comm = TorchComm(ctx, group)
-        self.h = self.H.msh_rowshard_prover_create(system.h, ctx.h, _C.byref(self.comm.struct))
-        if not self.h:
-            raise _ffi.MsgpuError(-3, (self.H.msh_last_error() or b"").decode() + " " + "; ".join(self.comm.errors))
-        self.last_stage_ms = None
-
-    def preprocessed_commit(self):
-        import numpy as np
-        out = np.zeros(32, dtype=np.uint8)
-        return bytes(out) if self.H.msh_prover_preprocessed_commit(self.h, out.ctypes.data_as(_C.c_void_p)) else None
+        super().__init__(ctx, system, group, host_lib().msh_rowshard_prover_create)
 
     def shardable(self, height, width):
         """the backend's rule (RowShardBackend::shardable): such a trace is read as natural-order row blocks"""
@@ -495,7 +434,6 @@ class RowShardProver:
     def commit(self, mats, heights, widths, host):
         """`Pcs::commit` over the row shards alone. host=False: mats[i] = DEVICE pointer of this rank's natural-order row block
         (block_rows(heights[i], widths[i])); host=True: mats[i] = numpy array holding the rows this rank reads. Returns the root."""
-        import numpy as np
         n = len(mats)
         if host:
             keep = [np.ascontiguousarray(m, dtype=np.uint64) for m in mats]
@@ -507,51 +445,24 @@ class RowShardProver:
         ws = (_C.c_uint64 * n)(*[int(w) for w in widths])
         root = np.zeros(32, dtype=np.uint8)
         if self.H.msh_rowshard_commit(self.h, ptrs, hs, ws, n, 1 if host else 0, root.ctypes.data_as(_C.c_void_p)) != 0:
-            from . import _ffi
-            raise _ffi.MsgpuError(-1, (self.H.msh_last_error() or b"").decode() + " " + "; ".join(self.comm.errors))
+            raise self._error(-1)
         return bytes(root)
 
     def prove(self, traces, claims, heights=None):
-        """traces[i]: (h x main_width) uint64 array of circuit i on EVERY rank (h = 0: inactive); claims: (n, len) uint64 array,
-        the same on every rank. With `heights` (trace rows of every circuit) traces[i] may instead hold only the rows this rank
-        reads -- block_rows(heights[i], width) -- so that no rank needs the whole of a tall trace in host memory.
+        """traces[i]: (h x main_width) uint64 array of circuit i on EVERY rank (h = 0: inactive); claims: as Prover.prove takes
+        them, the same on every rank. With `heights` (trace rows of every circuit) traces[i] may instead hold only the rows this
+        rank reads -- block_rows(heights[i], width) -- so that no rank needs the whole of a tall trace in host memory.
         Returns `Proof::to_bytes`."""
-        import numpy as np
-        from . import _ffi
-        from .system import STAGE_NAMES
-        n = self.system.num_circuits
         mats = [np.ascontiguousarray(t, dtype=np.uint64) for t in traces]
         if heights is None:
-            ptrs = (_C.c_void_p * n)(*[m.ctypes.data if m.size else None for m in mats])
-            hs = (_C.c_uint64 * n)(*[int(m.shape[0]) for m in mats])
-        else:
-            plist = []
-            for m, h in zip(mats, heights):
-                row0, rows = self.block_rows(int(h), m.shape[1])
-                if m.shape[0] != rows:
-                    raise ValueError("a trace given as a row block must hold exactly the rows this rank reads")
-                plist.append(m.ctypes.data - row0 * m.shape[1] * 8 if m.size else None)  # the library touches [row0, row0 + rows) only
-            ptrs = (_C.c_void_p * n)(*plist)
-            hs = (_C.c_uint64 * n)(*[int(h) for h in heights])
-        cl = np.ascontiguousarray(claims, dtype=np.uint64) if len(claims) else np.zeros((0, 1), dtype=np.uint64)
-        if cl.ndim != 2:
-            raise ValueError("claims: an (n, len) array is expected")
-        flat = cl.reshape(-1) if cl.size else np.zeros(1, dtype=np.uint64)
-        out, ln = _C.c_void_p(), _C.c_uint64()
-        ms = (_C.c_double * 6)()
-        rc = self.H.msh_prove(self.h, ptrs, hs, flat.ctypes.data_as(_ffi.c_u64p), None, cl.shape[1], cl.shape[0],
-                              _C.byref(out), _C.byref(ln), ms)
-        if rc != 0:
-            raise _ffi.MsgpuError(rc, (self.H.msh_last_error() or b"").decode() + " " + "; ".join(self.comm.errors))
-        data = _C.string_at(out.value, ln.value)
-        self.H.msh_bytes_free(out)
-        self.last_stage_ms = dict(zip(STAGE_NAMES, ms))
-        return data
-
-    def close(self):
-        if getattr(self, "h", None):
-            self.H.msh_prover_free(self.h)
-            self.h = None
+            return self._prove([m.ctypes.data if m.size else None for m in mats], [m.shape[0] for m in mats], claims)
+        ptrs = []
+        for m, h in zip(mats, heights):
+            row0, rows = self.block_rows(int(h), m.shape[1])
+            if m.shape[0] != rows:
+                raise ValueError("a trace given as a row block must hold exactly the rows this rank reads")
+            ptrs.append(m.ctypes.data - row0 * m.shape[1] * 8 if m.size else None)  # the library touches [row0, row0 + rows) only
+        return self._prove(ptrs, heights, claims)
 
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -580,7 +491,6 @@ class WideCommit:
         """Mmcs::open_batch: (rows [n, width], sibling paths [n, log2(H), 32]) -- the same on every rank. The row and the
         lower log2(H / N) siblings come from the rank that holds the row, the top log2(N) siblings from the top tree
         (which every rank holds)."""
-        import numpy as np
         n, world = len(indices), self.comm.world
         shard = self.lde_height // world
         lo_depth, top_depth, width = shard.bit_length() - 1, world.bit_length() - 1, sum(self.widths)
@@ -597,8 +507,7 @@ class WideCommit:
         # every rank contributes the openings of the rows it holds (zeros elsewhere); pick each index from its owner
         blob = np.concatenate([rows.view(np.uint8).ravel(), low.ravel()])
         gathered = np.zeros(blob.size * world, dtype=np.uint8)
-        if self.comm.struct.allgather_host(None, blob.ctypes.data, gathered.ctypes.data, blob.size) != 0:
-            raise RuntimeError("allgather failed: %s" % self.comm.errors)
+        self.comm.allgather_host(blob.ctypes.data, gathered.ctypes.data, blob.size)
         gathered = gathered.reshape(world, -1)
         all_rows = gathered[:, :rows.nbytes].copy().view(np.uint64).reshape(world, n, width)
         all_low = gathered[:, rows.nbytes:].reshape(world, n, lo_depth, 32)
@@ -630,8 +539,6 @@ def commit_wide_sharded(ctx, comm, block, width, log_blowup, timings=None, keep_
     column-local), ONE all-to-all that turns column blocks into row shards (the block's rows [d * H / N, (d+1) * H / N) are
     contiguous and go to rank d), leaf hashing of the shard's full rows + its Merkle subtree, then the N subtree roots are
     all-gathered and the top log2(N) levels built on every rank. Root and openings are bit-identical to a single-GPU commit."""
-    import numpy as np
-    from .pcs import ProverData
     L = ctx.L
     world, rank = comm.world, comm.rank
     if world & (world - 1):
@@ -680,8 +587,7 @@ def commit_wide_sharded(ctx, comm, block, width, log_blowup, timings=None, keep_
     top, root = None, bytes(sub_root)
     if world > 1:
         roots = np.zeros(32 * world, dtype=np.uint8)
-        if comm.struct.allgather_host(None, sub_root.ctypes.data, roots.ctypes.data, 32) != 0:
-            raise RuntimeError("allgather failed: %s" % comm.errors)
+        comm.allgather_host(sub_root.ctypes.data, roots.ctypes.data, 32)
         d_roots = ctx.upload(roots)
         th = _C.c_void_p()
         r32 = np.zeros(32, dtype=np.uint8)
@@ -705,7 +611,6 @@ def prove_wide_sharded(ctx, comm, prover, block, width, log_blowup, claims=None,
     by all ranks (commit_wide_sharded); rank 0 then gathers the LDE blocks and the shards' digest layers over NVLink,
     assembles ordinary prover data (msgpu_pdata_from_parts) and runs the remaining stages alone. Returns the proof bytes on
     rank 0 (None elsewhere); they equal the single-GPU proof byte for byte. `prover` is a `Prover` on rank 0, None elsewhere."""
-    import numpy as np
     L = ctx.L
     t = [time.perf_counter()]
     root, wc = commit_wide_sharded(ctx, comm, block, width, log_blowup, timings=timings, keep_block=True)
@@ -715,17 +620,17 @@ def prove_wide_sharded(ctx, comm, prover, block, width, log_blowup, claims=None,
     dg, nd = _C.c_void_p(), _C.c_uint64()
     check(L.msgpu_pdata_digests(wc.local.h, _C.byref(dg), _C.byref(nd)))
     nd = int(nd.value)
-    proof = None
     if rank == 0:
-        blocks, parts = [wc.lde_block], [dg.value]
-        for r in range(1, world):
-            blocks.append(ctx.malloc(H * widths[r] * 8))
-            parts.append(ctx.malloc(nd * 32))
-        for r in range(1, world):
-            for ptr, nbytes in ((blocks[r], H * widths[r] * 8), (parts[r], nd * 32)):
-                if comm.struct.sendrecv_dev(None, ptr, nbytes, r, 0) != 0:
-                    raise RuntimeError("gather failed: %s" % comm.errors)
-        t.append(time.perf_counter())
+        blocks = [wc.lde_block] + [ctx.malloc(H * widths[r] * 8) for r in range(1, world)]
+        parts = [dg.value] + [ctx.malloc(nd * 32) for r in range(1, world)]
+        gathers = [(r, blocks[r], parts[r]) for r in range(1, world)]
+    else:
+        gathers = [(rank, wc.lde_block, dg.value)]
+    for r, block_ptr, part_ptr in gathers:  # rank r's LDE block and digest layer -> rank 0
+        comm.sendrecv_dev(block_ptr, H * widths[r] * 8, r, 0)
+        comm.sendrecv_dev(part_ptr, nd * 32, r, 0)
+    t.append(time.perf_counter())
+    if rank == 0:
         pd, r32 = _C.c_void_p(), np.zeros(32, dtype=np.uint8)
         ba = (_C.c_void_p * world)(*blocks)
         wa = (_C.c_uint64 * world)(*widths)
@@ -737,23 +642,14 @@ def prove_wide_sharded(ctx, comm, prover, block, width, log_blowup, claims=None,
         if bytes(r32) != root:
             L.msgpu_pdata_free(pd)
             raise RuntimeError("assembled commitment differs from the sharded one")
-        ctx.free(wc.lde_block)
-        wc.lde_block = None
-        wc.free()  # the row shard and its subtree are not needed any more: the assembled prover data serves the openings
-        t.append(time.perf_counter())
-        proof = prover.prove_precommitted(pd, [H >> log_blowup], claims)
-        t.append(time.perf_counter())
-        names = ["commit_sharded", "gather", "assemble", "prove_rest"]
-    else:
-        for ptr, nbytes in ((wc.lde_block, H * widths[rank] * 8), (dg.value, nd * 32)):
-            if comm.struct.sendrecv_dev(None, ptr, nbytes, rank, 0) != 0:
-                raise RuntimeError("gather failed: %s" % comm.errors)
-        t.append(time.perf_counter())
-        ctx.free(wc.lde_block)
-        wc.lde_block = None
-        wc.free()
-        names = ["commit_sharded", "gather"]
+    ctx.free(wc.lde_block)
+    wc.lde_block = None
+    wc.free()  # the row shard and its subtree are not needed any more: on rank 0 the assembled prover data serves the openings
+    t.append(time.perf_counter())
+    proof = prover.prove_precommitted(pd, [H >> log_blowup], claims) if rank == 0 else None
+    t.append(time.perf_counter())
     if timings is not None:
+        names = ["commit_sharded", "gather"] + (["assemble", "prove_rest"] if rank == 0 else [])
         for k, name in enumerate(names):
             timings[name] = (t[k + 1] - t[k]) * 1e3
     return proof

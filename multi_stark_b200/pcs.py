@@ -416,7 +416,7 @@ def pcs_open(ctx, rounds, challenger):
     rc = H.msh_pcs_open(ctx.h, challenger.h, n, pds, npts_a.ctypes.data_as(_ffi.c_u64p), pts_a.ctypes.data_as(_ffi.c_u64p),
                         C.byref(out), C.byref(ln), ms5)
     if rc != 0:
-        raise _ffi.MsgpuError(rc, (H.msh_last_error() or b"").decode())
+        raise _ffi.host_error(rc)
     data = C.string_at(out.value, ln.value)
     H.msh_bytes_free(out)
     return data, dict(zip(["evaluate", "reduce", "commit_phase", "final_poly", "queries"], ms5))

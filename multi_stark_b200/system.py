@@ -88,7 +88,7 @@ class System:
                                                           C.cast(hs, C.c_void_p), log_blowup, log_final_poly_len, max_log_arity,
                                                           num_queries, commit_pow_bits, query_pow_bits)
         if not self.h:
-            raise ValueError((self.H.msh_last_error() or b"").decode())
+            raise ValueError(_ffi.host_error(-1).message)
         self.num_circuits = int(self.H.msh_system_num_circuits(self.h))
         self.circuits = []
         for i in range(self.num_circuits):
@@ -256,60 +256,86 @@ def shifted_quotient_slices(ctx, m, q):
 STAGE_NAMES = ["stark/stage1_commit", "stark/claims", "stark/stage2_commit", "stark/quotient", "stark/fri_open", "stark/prove"]
 
 
-class Prover:
-    """`System::prove_multiple_claims` (src/prover.rs:289-603) on the device: the host runs the Fiat-Shamir transcript
-    (host/prover.hpp, host/pcs.hpp); every matrix stays in HBM between the LDE, Merkle, quotient and opening stages."""
+def _claims_args(claims):
+    """`claims` as msh_prove takes them: (flat uint64 buffer, offsets pointer or None, stride, n_claims). A 2-D uint64
+    C-contiguous array is passed without a copy and without offsets (4M claims through the offsets form = 8 ms of numpy in the
+    timed prove()); other 2-D arrays are converted once; a sequence of 1-D claims goes through offsets; None = no claims."""
+    if isinstance(claims, np.ndarray) and claims.ndim == 2:
+        flat = claims.reshape(-1) if (claims.dtype == np.uint64 and claims.flags.c_contiguous) else \
+            np.ascontiguousarray(claims, dtype=np.uint64).ravel()
+        (n_claims, stride), offs_p = claims.shape, None
+    else:
+        claims = [] if claims is None else claims
+        n_claims, stride = len(claims), 0
+        offs = np.zeros(n_claims + 1, dtype=np.uint64)
+        for i, c in enumerate(claims):
+            offs[i + 1] = offs[i] + len(c)
+        flat = np.concatenate([np.asarray(c, dtype=np.uint64).ravel() for c in claims]) if n_claims else offs[:0]
+        offs_p = offs.ctypes.data_as(_ffi.c_u64p)  # the pointer keeps `offs` alive
+    if flat.size == 0:
+        flat = np.zeros(1, dtype=np.uint64)
+    return flat, offs_p, stride, n_claims
 
-    def __init__(self, ctx, system):
+
+class ProverBase:
+    """What the single-GPU and the sharded provers share: an `msh_prover` made by `create(system.h, ctx.h, *args)`, its
+    verifier key, and the one msh_prove call."""
+
+    def __init__(self, ctx, system, create, *args):
         self.H = _ffi.host_lib()
         self.ctx = ctx
         self.system = system
-        self.h = self.H.msh_prover_create(system.h, ctx.h)
-        if not self.h:
-            raise _ffi.MsgpuError(-3, (self.H.msh_last_error() or b"").decode())
         self.last_stage_ms = None
+        self.h = create(system.h, ctx.h, *args)
+        if not self.h:
+            raise self._error(-3)
+
+    def _error(self, code):
+        return _ffi.host_error(code)
 
     def preprocessed_commit(self):
         out = np.zeros(32, dtype=np.uint8)
         return bytes(out) if self.H.msh_prover_preprocessed_commit(self.h, out.ctypes.data_as(C.c_void_p)) else None
 
-    def prove(self, traces, claims):
-        """traces: one (h x main_width) uint64 array per circuit (h = 0 deactivates the circuit);
-        claims: sequence of 1-D uint64 arrays. Returns `Proof::to_bytes`."""
-        mats = [np.ascontiguousarray(t, dtype=np.uint64) for t in traces]
-        n = len(mats)
-        if n != self.system.num_circuits:
-            raise _ffi.MsgpuError(-1, "expected one trace per circuit")
-        for m, info in zip(mats, self.system.circuits):
-            if m.ndim != 2 or (m.shape[0] and m.shape[1] != info["main_width"]):
-                raise _ffi.MsgpuError(-1, "trace width does not match the circuit")
-        ptrs = (C.c_void_p * n)(*[m.ctypes.data if m.size else None for m in mats])
-        hs = (C.c_uint64 * n)(*[m.shape[0] for m in mats])
-        stride, offs_p = 0, None
-        if isinstance(claims, np.ndarray) and claims.ndim == 2:  # one call shape: no offsets array (4M claims = 8 ms of numpy)
-            flat = claims.reshape(-1) if (claims.dtype == np.uint64 and claims.flags.c_contiguous) else \
-                np.ascontiguousarray(claims, dtype=np.uint64).ravel()
-            n_claims, stride = claims.shape
-        else:
-            n_claims = len(claims)
-            offs = np.zeros(n_claims + 1, dtype=np.uint64)
-            for i, c in enumerate(claims):
-                offs[i + 1] = offs[i] + len(c)
-            flat = (np.concatenate([np.asarray(c, dtype=np.uint64).ravel() for c in claims]) if n_claims
-                    else np.zeros(0, dtype=np.uint64))
-            offs_p = offs.ctypes.data_as(_ffi.c_u64p)
-        if flat.size == 0:
-            flat = np.zeros(1, dtype=np.uint64)
+    def _prove(self, trace_ptrs, heights, claims):
+        """msh_prove: trace_ptrs[i] = host pointer of circuit i's rows (None: no rows on this rank), heights[i] = its trace rows.
+        Returns `Proof::to_bytes` and sets last_stage_ms."""
+        n = self.system.num_circuits
+        flat, offs_p, stride, n_claims = _claims_args(claims)
         out, ln = C.c_void_p(), C.c_uint64()
         ms = (C.c_double * 6)()
-        rc = self.H.msh_prove(self.h, ptrs, hs, flat.ctypes.data_as(_ffi.c_u64p), offs_p, stride, n_claims,
-                              C.byref(out), C.byref(ln), ms)
+        rc = self.H.msh_prove(self.h, (C.c_void_p * n)(*trace_ptrs), (C.c_uint64 * n)(*[int(h) for h in heights]),
+                              flat.ctypes.data_as(_ffi.c_u64p), offs_p, stride, n_claims, C.byref(out), C.byref(ln), ms)
         if rc != 0:
-            raise _ffi.MsgpuError(rc, (self.H.msh_last_error() or b"").decode())
+            raise self._error(rc)
         data = C.string_at(out.value, ln.value)
         self.H.msh_bytes_free(out)
         self.last_stage_ms = dict(zip(STAGE_NAMES, ms))
         return data
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.H.msh_prover_free(self.h)
+            self.h = None
+
+
+class Prover(ProverBase):
+    """`System::prove_multiple_claims` (src/prover.rs:289-603) on the device: the host runs the Fiat-Shamir transcript
+    (host/prover.hpp, host/pcs.hpp); every matrix stays in HBM between the LDE, Merkle, quotient and opening stages."""
+
+    def __init__(self, ctx, system):
+        super().__init__(ctx, system, _ffi.host_lib().msh_prover_create)
+
+    def prove(self, traces, claims):
+        """traces: one (h x main_width) uint64 array per circuit (h = 0 deactivates the circuit);
+        claims: (n, len) uint64 array or sequence of 1-D uint64 arrays. Returns `Proof::to_bytes`."""
+        mats = [np.ascontiguousarray(t, dtype=np.uint64) for t in traces]
+        if len(mats) != self.system.num_circuits:
+            raise _ffi.MsgpuError(-1, "expected one trace per circuit")
+        for m, info in zip(mats, self.system.circuits):
+            if m.ndim != 2 or (m.shape[0] and m.shape[1] != info["main_width"]):
+                raise _ffi.MsgpuError(-1, "trace width does not match the circuit")
+        return self._prove([m.ctypes.data if m.size else None for m in mats], [m.shape[0] for m in mats], claims)
 
     def last_transcript(self):
         """Test hook: (challenges [(c0, c1)...] = beta, gamma, alpha, zeta, alpha_pcs, FRI betas; query indices) of the last
@@ -325,30 +351,11 @@ class Prover:
         """prove() whose stage-1 commitment was made elsewhere (`msgpu_pdata_from_parts`: one wide matrix committed by column
         blocks over several GPUs). `stage1_pdata`: raw msgpu_pdata handle, adopted; heights[i]: trace rows of circuit i. Only
         for lookup-free circuits (the stage-2 construction of a circuit with lookups reads its main trace)."""
-        n = self.system.num_circuits
-        if len(heights) != n:
+        if len(heights) != self.system.num_circuits:
             raise _ffi.MsgpuError(-1, "expected one height per circuit")
         if self.H.msh_prover_inject_stage1(self.h, stage1_pdata) != 0:
-            raise _ffi.MsgpuError(-1, (self.H.msh_last_error() or b"").decode())
-        ptrs = (C.c_void_p * n)(*([None] * n))
-        hs = (C.c_uint64 * n)(*[int(h) for h in heights])
-        cl = np.zeros((0, 1), dtype=np.uint64) if claims is None or len(claims) == 0 else np.ascontiguousarray(claims, dtype=np.uint64)
-        flat = cl.reshape(-1) if cl.size else np.zeros(1, dtype=np.uint64)
-        out, ln = C.c_void_p(), C.c_uint64()
-        ms = (C.c_double * 6)()
-        rc = self.H.msh_prove(self.h, ptrs, hs, flat.ctypes.data_as(_ffi.c_u64p), None, cl.shape[1], cl.shape[0],
-                              C.byref(out), C.byref(ln), ms)
-        if rc != 0:
-            raise _ffi.MsgpuError(rc, (self.H.msh_last_error() or b"").decode())
-        data = C.string_at(out.value, ln.value)
-        self.H.msh_bytes_free(out)
-        self.last_stage_ms = dict(zip(STAGE_NAMES, ms))
-        return data
-
-    def close(self):
-        if getattr(self, "h", None):
-            self.H.msh_prover_free(self.h)
-            self.h = None
+            raise self._error(-1)
+        return self._prove([None] * len(heights), heights, claims)
 
     def __del__(self):
         try:

@@ -77,7 +77,7 @@ def main():
     with open("%s.rank%d.proof" % (out_prefix, rank), "wb") as f:
         f.write(proof)
     info = {"rank": rank, "owner": owner, "heights": heights, "ms": times, "stages": prover.last_stage_ms,
-            "bytes_dev": getattr(prover, "bytes_dev", prover.comm.bytes_dev) // reps, "bytes_host": prover.comm.bytes_host // reps, "launches": ctx.launches,
+            "bytes_dev": prover.bytes_dev // reps, "bytes_host": prover.comm.bytes_host // reps, "launches": ctx.launches,
             "comm_ms_per_proof": {k: v * 1e3 for k, v in prover.comm.seconds.items()},
             "pre_commit": (prover.preprocessed_commit() or b"").hex()}
     if rank == 0 and os.environ.get("DIST_SINGLE", "1") == "1" and block_heights is None:
