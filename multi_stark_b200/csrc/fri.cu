@@ -80,15 +80,18 @@ struct BaryParams {
     u32 w, c0, wc;  // this launch covers columns [c0, c0 + wc)
     u32 rows_per_step, tile_rows;
 };
+// Offset (in u64) of the inverse-denominator tile behind the [tile_rows][wc] matrix tile. It is read and written as
+// ulonglong2, so it is rounded up to 16 bytes: tile_rows * wc is odd for some chunk widths (19, 129, ...).
+__host__ __device__ __forceinline__ size_t bary_dd_offset(u32 tile_rows, u32 wc) { return ((size_t)tile_rows * wc + 1) & ~(size_t)1; }
 // Tiles of tile_rows rows are staged through shared memory with back-to-back coalesced loads (enough bytes in flight to
 // keep HBM busy), then thread (column c, row lane) accumulates its rows of the tile.
 template <int NPTS>
 __global__ void __launch_bounds__(256) k_bary_partial(BaryParams p) {
-    extern __shared__ u64 sm_b[];
+    extern __shared__ __align__(16) u64 sm_b[];
     const u32 t = threadIdx.x;
     const u32 TR = p.tile_rows, wc = p.wc;
-    u64* tile = sm_b;                                                       // [TR][wc]
-    ulonglong2* dd = reinterpret_cast<ulonglong2*>(sm_b + (size_t)TR * wc);  // [TR][NPTS]
+    u64* tile = sm_b;                                                             // [TR][wc]
+    ulonglong2* dd = reinterpret_cast<ulonglong2*>(sm_b + bary_dd_offset(TR, wc));  // [TR][NPTS]
     const u32 active = p.rows_per_step * wc;
     const u32 c = t % wc, lane_row = t / wc;
     gl::Acc160 acc[2 * NPTS];
@@ -183,6 +186,16 @@ struct ReduceParams {
     u32 w, npts, tile_rows;
 };
 constexpr int kRedThreads = 128;
+constexpr size_t kRedMaxSmem = 200 * 1024;
+// rows per tile: the largest power of two <= 128 whose tile fits 64 KB; at least 4 so that the lanes sharing a row
+// (128 / tile_rows <= 32) sit in one warp
+static u32 reduce_tile_rows(u64 w) {
+    u32 tr = 128;
+    while (tr > 4 && (size_t)tr * (w | 1) * 8 > 64 * 1024) tr >>= 1;
+    return tr;
+}
+// the tile plus the w alpha powers; within kRedMaxSmem up to 4266 columns (4 * 4267 + 2 * 4266 = 25,600 u64)
+static size_t reduce_smem(u64 w) { return ((size_t)reduce_tile_rows(w) * (w | 1) + 2 * w) * 8; }
 // A tile of tile_rows rows (power of two <= 128) is staged in shared memory; 128 / tile_rows lanes share a row, each
 // accumulating the columns c = lane (mod lanes) lazily; the lanes' partial dot products are combined with shuffles.
 __global__ void __launch_bounds__(kRedThreads) k_reduce_openings(ReduceParams p) {
@@ -564,8 +577,10 @@ static void evaluate_all(Ctx& c, msgpu_open* op) {
                     u64* d_partial = (u64*)c.alloc((size_t)ctas * bp.wc * (npts + 1) * 16);
                     partials.push_back(d_partial);
                     bp.partial = d_partial;
+                    // at most 46,448 bytes when the dd tile is padded (wc = 19, tile_rows = 215, 4 points) and 49,152 without
+                    // (wc = 16, tile_rows = 256, 4 points): both within the default dynamic shared memory limit
                     size_t smem = std::max((size_t)bp.rows_per_step * bp.wc * (npts + 1) * 16,
-                                           (size_t)bp.tile_rows * (bp.wc * 8 + npts * 16));
+                                           (bary_dd_offset(bp.tile_rows, bp.wc) + (size_t)bp.tile_rows * npts * 2) * 8);
                     {
                         KLaunch kl(c, "k_bary_partial");
                         switch (npts) {
@@ -596,6 +611,11 @@ static void evaluate_all(Ctx& c, msgpu_open* op) {
 
 static void reduce_all(Ctx& c, msgpu_open* op, msh::Fp2 alpha) {
     StageScope ss(c, "open");
+    // checked before anything is allocated or copied, so that a refused opening leaves nothing behind
+    for (auto& round : op->rounds)
+        for (auto& m : round)
+            MSG_REQUIRE(m.points.empty() || m.rows == 0 || reduce_smem(m.width) <= kRedMaxSmem,
+                        "open: matrix too wide for the reduced-openings kernel (more than 4266 columns)");
     size_t max_w = 1;
     for (auto& round : op->rounds)
         for (auto& m : round) max_w = std::max<size_t>(max_w, m.width);
@@ -609,7 +629,7 @@ static void reduce_all(Ctx& c, msgpu_open* op, msh::Fp2 alpha) {
     u64* ro[33] = {nullptr};
     u64 ro_len[33] = {0};
     u64 num_reduced[33] = {0};
-    ensure_max_smem(k_reduce_openings, 200 * 1024);
+    ensure_max_smem(k_reduce_openings, (int)kRedMaxSmem);
     for (auto& round : op->rounds)
         for (auto& m : round) {
             u32 lh = m.log_h;
@@ -646,13 +666,9 @@ static void reduce_all(Ctx& c, msgpu_open* op, msh::Fp2 alpha) {
                     rp.yred[k][0] = yred.c[0].v; rp.yred[k][1] = yred.c[1].v;
                     num_reduced[lh] += m.width;
                 }
-                // rows per tile: the largest power of two <= 128 whose tile fits 64 KB; at least 4 so that the lanes sharing
-                // a row (128 / tile_rows <= 32) sit in one warp
-                u32 tr = 128;
-                while (tr > 4 && (size_t)tr * (m.width | 1) * 8 > 64 * 1024) tr >>= 1;
+                const u32 tr = reduce_tile_rows(m.width);
                 rp.tile_rows = tr;
-                size_t smem = ((size_t)tr * (m.width | 1) + 2 * m.width) * 8;
-                MSG_REQUIRE(smem <= 200 * 1024, "open: matrix too wide for the reduced-openings kernel (more than ~5000 columns)");
+                const size_t smem = reduce_smem(m.width);
                 {
                     KLaunch kl(c, "k_reduce_openings");
                     k_reduce_openings<<<(unsigned)((m.rows + tr - 1) / tr), kRedThreads, smem, c.stream>>>(rp);
@@ -758,6 +774,7 @@ static void open_begin_impl(msgpu_ctx* h, uint64_t n_rounds, const msgpu_pdata* 
     op->fri_owner = fri_owner != 0;
     size_t mi = 0, pi = 0;
     u64 total = 0;
+    const msh::Fp gen_inv = msh::Fp(msh::GL_GENERATOR).inverse();
     for (u64 r = 0; r < n_rounds; r++) {
         MSG_REQUIRE(pds[r], "open_begin: null prover data");
         const u32 mode = modes ? modes[r] : 0;
@@ -773,6 +790,10 @@ static void open_begin_impl(msgpu_ctx* h, uint64_t n_rounds, const msgpu_pdata* 
             u64 np = n_points[mi++];
             for (u64 k = 0; k < np; k++, pi++) {
                 MSG_REQUIRE(points[2 * pi] < GLD_P && points[2 * pi + 1] < GLD_P, "open_begin: point is not canonical");
+                // 1 / (z - x) has no value at a point x of the LDE coset GENERATOR * H; k_inv_denoms inverts in batches, so
+                // such a z would silently zero every inverse of its batch. Only a base-field z can lie on the coset.
+                MSG_REQUIRE(points[2 * pi + 1] != 0 || (msh::Fp(points[2 * pi]) * gen_inv).exp_power_of_2(m.log_h) != msh::Fp::one(),
+                            "open_begin: point lies on the committed LDE coset");
                 m.points.push_back(msh::Fp2(msh::Fp(points[2 * pi]), msh::Fp(points[2 * pi + 1])));
             }
             total += np * pm.width;
