@@ -215,6 +215,8 @@ typedef struct msgpu_graph_desc {
     uint32_t lookup_prefix_len;     /* nodes[..lookup_prefix_len] cover the lookup expressions */
     uint32_t pre_width, main_width, stage2_width;
 } msgpu_graph_desc;
+/* Refuses (MSGPU_ERR_INVALID) a lookup prefix that reads a stage-2 column or a public value: lookup values are computed in
+ * stage 1, before either exists. */
 int msgpu_program_create(msgpu_ctx* ctx, const msgpu_graph_desc* desc, msgpu_program** out);
 void msgpu_program_free(msgpu_program* prog);
 
@@ -223,12 +225,14 @@ void msgpu_program_free(msgpu_program* prog);
  * + `LookupValues::stage_2_traces` (src/lookup.rs:472-555: messages beta + fingerprint(gamma, args), batch
  * inverse, exclusive running sum of multiplicity / message in (row, lookup) order, starting at zero).
  * main_dev: rows x main_width; pre_dev: rows x pre_width or NULL. stage2_out_dev: rows x stage2_width
- * (device, written). local_sum receives the circuit's total (2 u64), to be added to the running accumulator. */
+ * (device, written). local_sum receives the circuit's total (2 u64), to be added to the running accumulator.
+ * MSGPU_ERR_INVALID if a message is zero (it has no inverse). */
 int msgpu_stage2_trace(msgpu_ctx* ctx, const msgpu_program* prog, const uint64_t* pre_dev, const uint64_t* main_dev,
                        uint64_t rows, const uint64_t* beta2, const uint64_t* gamma2, uint64_t* stage2_out_dev,
                        uint64_t* local_sum2);
 /* Sum over claims of 1 / (beta + fingerprint(gamma, claim)) (src/prover.rs:381-387). `claims` is a HOST array of
- * n_claims x claim_len values (all claims of one length per call). out2 += is NOT applied: out2 receives the sum. */
+ * n_claims x claim_len values (all claims of one length per call). out2 += is NOT applied: out2 receives the sum.
+ * MSGPU_ERR_INVALID if some beta + fingerprint is zero. */
 int msgpu_claims_accumulator(msgpu_ctx* ctx, const uint64_t* claims, uint64_t n_claims, uint64_t claim_len,
                              const uint64_t* beta2, const uint64_t* gamma2, uint64_t* out2);
 

@@ -312,7 +312,7 @@ __global__ void __launch_bounds__(128) k_lookup_messages(MsgParams p) {
     cx.rows[0][1] = p.pre + rn * p.wpre;
     cx.rows[1][0] = p.main + r * p.wmain;
     cx.rows[1][1] = p.main + rn * p.wmain;
-    cx.rows[2][0] = cx.rows[2][1] = nullptr;  // lookup expressions cannot read stage 2 (src/graph.rs:343-346)
+    cx.rows[2][0] = cx.rows[2][1] = nullptr;  // lookup expressions cannot read stage 2 or publics (refused by program_create)
     cx.publics = nullptr;
     cx.first = r == 0;
     cx.last = r + 1 == p.rows;
@@ -353,8 +353,10 @@ __device__ __forceinline__ gl::e2 block_sum(gl::e2 v, gl::e2* sm) {
     return r;
 }
 
-// msgs[i] <- mults[i] / msgs[i] (Montgomery batches of 8 per thread); block_sums[b] = sum of the block's terms
-__global__ void __launch_bounds__(kScanThreads) k_terms_and_block_sums(u64* msgs, const u64* mults, u64 total, u64* block_sums) {
+// msgs[i] <- mults[i] / msgs[i] (Montgomery batches of 8 per thread); block_sums[b] = sum of the block's terms. A zero message
+// (the batch product is zero only then: 7 is a non-residue, so only 0 has norm 0) sets *zero_msg instead of a silent 0 inverse.
+__global__ void __launch_bounds__(kScanThreads) k_terms_and_block_sums(u64* msgs, const u64* mults, u64 total, u64* block_sums,
+                                                                       u64* zero_msg) {
     __shared__ gl::e2 sm[kScanThreads / 32];
     u64 i0 = ((u64)blockIdx.x * kScanThreads + threadIdx.x) * kScanPerThread;
     // prefix products in registers (fully unrolled, constant indices: a dynamically indexed array would live in local memory,
@@ -367,6 +369,7 @@ __global__ void __launch_bounds__(kScanThreads) k_terms_and_block_sums(u64* msgs
         pref[k] = acc;
         if (k < cnt) acc = gl::e2_mul(acc, gl::e2_make(msgs[2 * (i0 + k)], msgs[2 * (i0 + k) + 1]));
     }
+    if (cnt && acc.a == 0 && acc.b == 0) *zero_msg = 1;
     gl::e2 inv = cnt ? e2_inverse(acc) : acc;
     gl::e2 sum = gl::e2_make(0, 0);
 #pragma unroll
@@ -446,9 +449,9 @@ __global__ void __launch_bounds__(kScanThreads) k_scan_write(const u64* terms, u
     }
 }
 
-// partial[b] = sum over the block's claims of 1 / (beta + fingerprint(gamma, claim))
+// partial[b] = sum over the block's claims of 1 / (beta + fingerprint(gamma, claim)); a zero message sets *zero_msg
 __global__ void __launch_bounds__(kScanThreads) k_claims(const u64* claims, u64 n_claims, u32 len, gl::e2 beta, gl::e2 gamma,
-                                                         u64* partial) {
+                                                         u64* partial, u64* zero_msg) {
     __shared__ gl::e2 sm[kScanThreads / 32];
     u64 i0 = ((u64)blockIdx.x * kScanThreads + threadIdx.x) * kScanPerThread;
     // fully unrolled, constant indices: the batch of 8 stays in registers
@@ -470,6 +473,7 @@ __global__ void __launch_bounds__(kScanThreads) k_claims(const u64* claims, u64 
             acc = gl::e2_mul(acc, v[k]);
         }
     }
+    if (cnt && acc.a == 0 && acc.b == 0) *zero_msg = 1;
     gl::e2 inv = cnt ? e2_inverse(acc) : acc;
     gl::e2 sum = gl::e2_make(0, 0);
 #pragma unroll
@@ -498,6 +502,11 @@ static T* upload_vec(Ctx& c, msgpu_program* prog, const std::vector<T>& v) {
 static msgpu_program* program_create(Ctx& c, const msgpu_graph_desc& g) {
     MSG_REQUIRE(g.lookup_prefix_len <= g.n_nodes, "program: lookup prefix longer than the node vector");
     MSG_REQUIRE(g.stage2_width == 2 * std::max<u32>(g.n_lookups, 1), "program: stage-2 width must be 2 * max(lookups, 1)");
+    // k_lookup_messages has no stage-2 rows and no publics: lookup values are computed before either exists
+    for (u32 i = 0; i < g.lookup_prefix_len; i++) {
+        MSG_REQUIRE(g.op[i] != OP_PUBLIC, "program: lookup expression reads a public value");
+        MSG_REQUIRE(g.op[i] != OP_VAR || (g.a[i] & 3) != 2, "program: lookup expression reads a stage-2 column");
+    }
     std::vector<u32> pin_lk, pin_all;
     u32 n_args = g.n_lookups ? g.lookup_arg_off[g.n_lookups] : 0;
     for (u32 j = 0; j < g.n_lookups; j++) pin_lk.push_back(g.lookup_mult[j]);
@@ -666,16 +675,18 @@ static void claims_sum(Ctx& c, const u64* d_claims, u64 n_claims, u64 claim_len,
     out2[0] = out2[1] = 0;
     if (n_claims == 0) return;
     u64 nblocks = (n_claims + kScanPerBlock - 1) / kScanPerBlock;
-    DevBuf part(c, nblocks * 16);
+    DevBuf part(c, nblocks * 16 + 8);  // the block partials, then the zero-message flag
+    MSG_CUDA(cudaMemsetAsync(part.u() + 2 * nblocks, 0, 8, c.stream));
     {
         KLaunch kl(c, "k_claims");
         k_claims<<<(unsigned)nblocks, kScanThreads, 0, c.stream>>>(d_claims, n_claims, (u32)claim_len, gl::e2{beta2[0], beta2[1]},
-                                                                   gl::e2{gamma2[0], gamma2[1]}, part.u());
+                                                                   gl::e2{gamma2[0], gamma2[1]}, part.u(), part.u() + 2 * nblocks);
     }
     MSG_CUDA(cudaGetLastError());
-    std::vector<u64> hp(nblocks * 2);
-    MSG_CUDA(cudaMemcpyAsync(hp.data(), part.p, nblocks * 16, cudaMemcpyDeviceToHost, c.stream));
+    std::vector<u64> hp(nblocks * 2 + 1);
+    MSG_CUDA(cudaMemcpyAsync(hp.data(), part.p, nblocks * 16 + 8, cudaMemcpyDeviceToHost, c.stream));
     c.sync();
+    MSG_REQUIRE(hp[2 * nblocks] == 0, "claims: a logUp message beta + fingerprint(gamma, claim) is zero");
     msh::Fp2 acc;
     for (u64 b = 0; b < nblocks; b++) acc += msh::Fp2(msh::Fp(hp[2 * b]), msh::Fp(hp[2 * b + 1]));
     out2[0] = acc.c[0].v;
@@ -715,7 +726,10 @@ int msgpu_stage2_trace(msgpu_ctx* h, const msgpu_program* prog, const uint64_t* 
         }
         u64 total = rows * L;
         u64 nblocks = (total + kScanPerBlock - 1) / kScanPerBlock;
-        DevBuf msgs(c, total * 16), mults(c, total * 8), bsums(c, (nblocks + 1) * 16);
+        // bsums: the block sums, the total, then the zero-message flag
+        DevBuf msgs(c, total * 16), mults(c, total * 8), bsums(c, (nblocks + 1) * 16 + 8);
+        u64* zero_msg = bsums.u() + 2 * (nblocks + 1);
+        MSG_CUDA(cudaMemsetAsync(zero_msg, 0, 8, c.stream));
         MsgParams mp{};
         mp.prog = prog->d_prefix;
         mp.n_instr = prog->n_prefix;
@@ -742,7 +756,7 @@ int msgpu_stage2_trace(msgpu_ctx* h, const msgpu_program* prog, const uint64_t* 
         MSG_CUDA(cudaGetLastError());
         {
             KLaunch kl(c, "k_terms_and_block_sums");
-            k_terms_and_block_sums<<<(unsigned)nblocks, kScanThreads, 0, c.stream>>>(msgs.u(), mults.u(), total, bsums.u());
+            k_terms_and_block_sums<<<(unsigned)nblocks, kScanThreads, 0, c.stream>>>(msgs.u(), mults.u(), total, bsums.u(), zero_msg);
         }
         MSG_CUDA(cudaGetLastError());
         {
@@ -755,8 +769,12 @@ int msgpu_stage2_trace(msgpu_ctx* h, const msgpu_program* prog, const uint64_t* 
             k_scan_write<<<(unsigned)nblocks, kScanThreads, 0, c.stream>>>(msgs.u(), total, bsums.u(), (u64*)stage2_out_dev);
         }
         MSG_CUDA(cudaGetLastError());
-        MSG_CUDA(cudaMemcpyAsync(local_sum2, bsums.u() + 2 * nblocks, 16, cudaMemcpyDeviceToHost, c.stream));
+        u64 tail[3];  // total, zero-message flag
+        MSG_CUDA(cudaMemcpyAsync(tail, bsums.u() + 2 * nblocks, 24, cudaMemcpyDeviceToHost, c.stream));
         c.sync();
+        MSG_REQUIRE(tail[2] == 0, "stage2_trace: a logUp message beta + fingerprint(gamma, args) is zero");
+        local_sum2[0] = tail[0];
+        local_sum2[1] = tail[1];
     });
 }
 

@@ -289,7 +289,10 @@ class Interner {
         return intern(n);
     }
 
-    u32 compile_expr(const Expr& e, const CircuitSpec& spec, bool allow_stage2) { return compile_node(e.node(), spec, allow_stage2); }
+    // allow_public = false: a lookup expression, evaluated in stage 1 before beta and gamma (publics 0..3) are drawn
+    u32 compile_expr(const Expr& e, const CircuitSpec& spec, bool allow_stage2, bool allow_public = true) {
+        return compile_node(e.node(), spec, allow_stage2, allow_public);
+    }
 
     std::vector<u32> expand_ext(const ExtExpr& e, const CircuitSpec& spec, const ExtensionParams& params, size_t constraint) {
         return expand_node(e.node(), spec, params, constraint);
@@ -307,7 +310,7 @@ class Interner {
         }
         return 0;
     }
-    u32 compile_node(const ExprNode& e, const CircuitSpec& spec, bool allow_stage2) {
+    u32 compile_node(const ExprNode& e, const CircuitSpec& spec, bool allow_stage2, bool allow_public) {
         switch (e.op) {
             case Op::Const: return constant(e.c);
             case Op::Var: {
@@ -325,15 +328,16 @@ class Interner {
                 return intern(n);
             }
             case Op::Public: {
+                if (!allow_public) throw CompileError("PublicInLookup");
                 if (e.pub >= spec.num_publics) throw CompileError("PublicOutOfRange");
                 Node n; n.op = Op::Public; n.a = e.pub;
                 return intern(n);
             }
             case Op::IsFirstRow: case Op::IsLastRow: case Op::IsTransition: { Node n; n.op = e.op; return intern(n); }
-            case Op::Add: { u32 a = compile_node(*e.a, spec, allow_stage2); u32 b = compile_node(*e.b, spec, allow_stage2); return add(a, b); }
-            case Op::Sub: { u32 a = compile_node(*e.a, spec, allow_stage2); u32 b = compile_node(*e.b, spec, allow_stage2); return sub(a, b); }
-            case Op::Mul: { u32 a = compile_node(*e.a, spec, allow_stage2); u32 b = compile_node(*e.b, spec, allow_stage2); return mul(a, b); }
-            case Op::Neg: { u32 a = compile_node(*e.a, spec, allow_stage2); return neg(a); }
+            case Op::Add: { u32 a = compile_node(*e.a, spec, allow_stage2, allow_public); u32 b = compile_node(*e.b, spec, allow_stage2, allow_public); return add(a, b); }
+            case Op::Sub: { u32 a = compile_node(*e.a, spec, allow_stage2, allow_public); u32 b = compile_node(*e.b, spec, allow_stage2, allow_public); return sub(a, b); }
+            case Op::Mul: { u32 a = compile_node(*e.a, spec, allow_stage2, allow_public); u32 b = compile_node(*e.b, spec, allow_stage2, allow_public); return mul(a, b); }
+            case Op::Neg: { u32 a = compile_node(*e.a, spec, allow_stage2, allow_public); return neg(a); }
         }
         throw CompileError("bad expression");
     }
@@ -420,8 +424,8 @@ inline ConstraintGraph compile(const CircuitSpec& spec, const ExtensionParams& p
     ConstraintGraph g;
     for (auto& l : spec.lookups) {
         Lookup<u32> cl;
-        cl.multiplicity = in.compile_expr(l.multiplicity, spec, false);
-        for (auto& a : l.args) cl.args.push_back(in.compile_expr(a, spec, false));
+        cl.multiplicity = in.compile_expr(l.multiplicity, spec, false, false);
+        for (auto& a : l.args) cl.args.push_back(in.compile_expr(a, spec, false, false));
         g.lookups.push_back(std::move(cl));
     }
     g.lookup_prefix_len = in.nodes.size();

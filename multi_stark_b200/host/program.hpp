@@ -97,6 +97,11 @@ inline ConstraintGraph graph_from_desc(const msgpu_graph_desc& d) {
         g.max_constraint_degree = std::max(g.max_constraint_degree, g.degrees[d.zeros[k]]);
     }
     if (d.lookup_prefix_len > d.n_nodes) fail("lookup prefix longer than the node vector");
+    // lookup values are computed in stage 1, before the stage-2 trace and beta, gamma (publics 0..3) exist (src/graph.rs:343-346)
+    for (uint32_t i = 0; i < d.lookup_prefix_len; i++) {
+        if (g.nodes[i].op == Op::Public) fail("lookup expression reads a public value");
+        if (g.nodes[i].op == Op::Var && g.nodes[i].col.source == Source::Stage2) fail("lookup expression reads a stage-2 column");
+    }
     for (uint32_t j = 0; j < d.n_lookups; j++) {
         Lookup<u32> l;
         l.multiplicity = d.lookup_mult[j];

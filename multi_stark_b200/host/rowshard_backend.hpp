@@ -83,9 +83,18 @@ class RowShardBackend : public ShardedBackend {
         const int n = comm_.world();
         if (n < 1 || (n & (n - 1))) throw DistError("row-sharded prover: the number of ranks must be a power of two");
         if (n > 16) throw DistError("row-sharded prover: at most 16 ranks");
-        for (auto& c : shape_.circuits)  // a wrap-around next-row read inside a lookup would need a one-row halo between the blocks
-            for (size_t i = 0; i < c.graph.lookup_prefix_len; i++)
-                if (c.graph.nodes[i].op == Op::Var && c.graph.nodes[i].col.offset == RowOffset::Next) lookup_next_ = true;
+        // msgpu_stage2_trace evaluates the lookups of a row block as if the block were the whole trace: a next-row read would need
+        // a one-row halo between the blocks, and the selectors would mark the block's first and last rows, not the trace's
+        for (auto& c : shape_.circuits) {
+            std::string& r = lookup_block_reads_.emplace_back();
+            for (size_t i = 0; i < c.graph.lookup_prefix_len && r.empty(); i++) {
+                const Node& nd = c.graph.nodes[i];
+                if (nd.op == Op::Var && nd.col.offset == RowOffset::Next) r = "the next row";
+                else if (nd.op == Op::IsFirstRow) r = "is_first_row";
+                else if (nd.op == Op::IsLastRow) r = "is_last_row";
+                else if (nd.op == Op::IsTransition) r = "is_transition";
+            }
+        }
         if (comm.peer_memory && n > 1) init_peers();
     }
     ~RowShardBackend() override {
@@ -315,8 +324,9 @@ class RowShardBackend : public ShardedBackend {
             const MatrixView& m = traces[p];
             if (!m.data) throw DistError("row-sharded prover: every rank needs (read access to) every trace");
             trace_rows_.push_back(m.height());
-            if (lookup_next_ && shardable(m.height(), m.width))
-                throw DistError("row-sharded prover: lookups that read the next row are not supported on row blocks");
+            const std::string& reads = lookup_block_reads_[circuits[p]];
+            if (!reads.empty() && shardable(m.height(), m.width))
+                throw DistError("row-sharded prover: lookups that read " + reads + " are not supported on row blocks");
             main_.push_back(upload_blocks((const uint64_t*)m.data, m.height(), m.width));
         }
         prefetch_announced_claims();
@@ -543,7 +553,7 @@ class RowShardBackend : public ShardedBackend {
     msgpu_peers* peers_ = nullptr;
     uint64_t peer_bytes_ = 0;
     std::vector<RowBlocks> main_;  // the natural-order traces (row blocks or whole), kept for the stage-2 construction
-    bool lookup_next_ = false;
+    std::vector<std::string> lookup_block_reads_;  // per circuit: what its lookups read that a row block cannot evaluate ("" = nothing)
 };
 
 // Pcs::open over the row shards.
