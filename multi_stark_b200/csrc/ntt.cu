@@ -14,6 +14,9 @@
 //           multiplications by compile-time constants with zero limbs and free sign flips, followed by ONE
 //           general multiplication per element by w_T^{off * r} (Cooley-Tukey / Gentleman-Sande with the
 //           twiddles pulled out of the butterflies): 15 general multiplications per 16 elements instead of 32.
+//           The twiddles of the round over bits [2, 6) are 64th roots of unity, powers of two as well (2^39 = w_64), so they
+//           are shifts too: a 10-bit tile pays ONE general twiddle multiplication per element, in the round over the top
+//           bits. DIT tiles run the DIF rounds in mirror order (radix-4 / 16 / 16 from the low bits up) for the same reason.
 //   The first round loads straight from global memory into registers and the last round stores straight
 //   from registers to global memory (with the inter-pass twiddle folded in), so a tile touches shared
 //   memory only between rounds. Thread -> (column, row group) is fixed for the whole kernel: no integer
@@ -61,9 +64,10 @@ using gl::gf::add;
 using gl::gf::mul;
 using gl::gf::sub;
 
-// two_adic_generator(k) = 2^root_exp(k) for k <= 4 (checked against the host field in tests); inverse = 2^(192 - e)
+// two_adic_generator(k) = 2^root_exp(k) for k <= 6 (checked against the host field when a context starts, and in tests);
+// inverse = 2^(192 - e). two_adic_generator(7) is not a power of two.
 __host__ __device__ constexpr int root_exp(int logr, bool inv) {
-    int e = logr == 1 ? 96 : logr == 2 ? 48 : logr == 3 ? 120 : logr == 4 ? 156 : 0;
+    int e = logr == 1 ? 96 : logr == 2 ? 48 : logr == 3 ? 120 : logr == 4 ? 156 : logr == 5 ? 78 : logr == 6 ? 39 : 0;
     return inv ? (192 - e) % 192 : e;
 }
 
@@ -73,6 +77,14 @@ __device__ __forceinline__ u64 sub_mul_pow2(u64 u, u64 x, int e) {
     if (e == 96) return sub(x, u);
     if (e < 96) return gl::gf::mul_pow2(sub(u, x), e);
     return gl::gf::mul_pow2(sub(x, u), e - 96);
+}
+// x * 2^e for canonical x, e in [0, 192) known at compile time after unrolling: 2^96 = -1, and -x = p - x costs no reduction
+// because mul_pow2 takes any u64
+__device__ __forceinline__ u64 mul_pow2_any(u64 x, int e) {
+    if (e == 0) return x;
+    if (e == 96) return sub(0, x);
+    if (e < 96) return gl::gf::mul_pow2(x, e);
+    return gl::gf::mul_pow2(GLD_P - x, e - 96);
 }
 
 // size-2^RB DFT in registers, natural order in, bit-reversed order out (decimation in frequency)
@@ -137,7 +149,9 @@ __host__ __device__ constexpr int rev_small(int x, int bits) {
     return r;
 }
 
-// Round sizes of a tb-bit tile: 4, 4, rest.
+// Round sizes of a tb-bit DIF tile from the top bits down: 4, 4, rest. A DIT tile runs the same rounds in mirror order from
+// the low bits up (rest, 4, 4), so both run the same (size, bit offset) rounds with the same twiddles -- except at tb = 7,
+// where DIT keeps 4, 3: its mirror 3, 4 would pay the general (order-128) twiddles on 15 of 16 elements instead of 7 of 8.
 __host__ __device__ constexpr int round_bits(int tb, int k) {
     int r1 = tb < 4 ? tb : 4, rem = tb - r1;
     int r2 = rem < 4 ? rem : 4;
@@ -146,6 +160,12 @@ __host__ __device__ constexpr int round_bits(int tb, int k) {
 
 // One round of RB bits at bit offset S0 of a TB-bit tile. Slot m of item (blk, off) is tile row
 // (blk << (S0 + RB)) + off + (m << S0). DIF: DFT then slot m *= w^{off * rev(m)}; DIT: the mirror image.
+// w = w_{2^(S0+RB)}: when S0 + RB <= 6 it is a power of two (the radix-16 round over bits [2, 6) of a 10-bit tile, [1, 5) of a
+// 9-bit one), and the twiddles are shifts by compile-time amounts, one unrolled body per value of off (off < 2^S0 <= 4). off
+// is taken from the HIGH bits of the item index so that it is warp-uniform (8 thread rows of a warp share it whenever a value
+// of off has >= 8 items): 256 threads, 64 items, off = trow >> 4. The half-warp's 4 rows then differ in two adjacent row bits
+// above bit 1 (bits 6-7 at TB = 10, 5-6 at TB = 9), which sw2() maps one-to-one onto the bank group: no conflict
+// (tools/smem_banks.py counts every round).
 // ld(row0, mm) / st(row0, mm, value) move the element of tile row row0 | mm of this thread's column (registers <-> global or
 // shared memory); mm = m << S0 is a compile-time constant after unrolling.
 // post (the LAST round only): table of the pass's output multipliers (inter-pass twiddles), indexed by tile row, or null.
@@ -158,8 +178,24 @@ __device__ __forceinline__ void tile_round(const u64* __restrict__ tw, u32 trow,
     constexpr int R = 1 << RB;
     constexpr u32 items = 1u << (TB - RB);
     constexpr bool kEarlyPost = R <= 4;
+    constexpr int kBlkBits = TB - RB - S0;
+    constexpr bool kShiftTw = S0 > 0 && S0 + RB <= 6;
+    auto twiddle = [&](u64(&v)[R], u32 off) {
+        if constexpr (kShiftTw) {
+#pragma unroll
+            for (int o = 1; o < (1 << S0); o++) {
+                if (off == (u32)o) {
+#pragma unroll
+                    for (int m = 1; m < R; m++) v[m] = mul_pow2_any(v[m], (root_exp(S0 + RB, INV) * o * rev_small(m, RB)) % 192);
+                }
+            }
+        } else if constexpr (S0 > 0) {
+#pragma unroll
+            for (int m = 1; m < R; m++) v[m] = mul(v[m], __ldg(tw + ((off * (u32)rev_small(m, RB)) << (kTwLog - S0 - RB))));
+        }
+    };
     for (u32 g = trow; g < items; g += nrows_thr) {
-        const u32 off = g & ((1u << S0) - 1), blk = g >> S0;
+        const u32 off = S0 > 0 ? g >> kBlkBits : 0u, blk = S0 > 0 ? g & ((1u << kBlkBits) - 1) : g;
         const u32 row0 = (blk << (S0 + RB)) + off;
         u64 v[R], pt[R];
         if (kEarlyPost && post_tab) {
@@ -169,19 +205,11 @@ __device__ __forceinline__ void tile_round(const u64* __restrict__ tw, u32 trow,
 #pragma unroll
         for (int m = 0; m < R; m++) v[m] = ld(row0, (u32)m << S0);
         if (DIT) {
-            if (S0 > 0) {
-#pragma unroll
-                for (int m = 1; m < R; m++)
-                    v[m] = mul(v[m], __ldg(tw + ((off * (u32)rev_small(m, RB)) << (kTwLog - S0 - RB))));
-            }
+            twiddle(v, off);
             dit_regs<RB, INV>(v);
         } else {
             dif_regs<RB, INV>(v);
-            if (S0 > 0) {
-#pragma unroll
-                for (int m = 1; m < R; m++)
-                    v[m] = mul(v[m], __ldg(tw + ((off * (u32)rev_small(m, RB)) << (kTwLog - S0 - RB))));
-            }
+            twiddle(v, off);
         }
         if (post_tab) {
             if (!kEarlyPost) {
@@ -220,19 +248,20 @@ __device__ __forceinline__ void tile_pass(u64* tile, const u64* __restrict__ tw,
             tile_round<TB, B2, 0, INV, false>(tw, trow, nrows_thr, sld, gst, post);
         }
     } else {
-        // round 0 works on the low bits
+        // the DIF rounds in mirror order: round 0 works on the low bits
         if constexpr (B1 == 0) {
             tile_round<TB, B0, 0, INV, true>(tw, trow, nrows_thr, gld, gst, post);
         } else if constexpr (B2 == 0) {
-            tile_round<TB, B0, 0, INV, true>(tw, trow, nrows_thr, gld, sst);
+            constexpr int D0 = TB == 7 ? B0 : B1, D1 = TB - D0;
+            tile_round<TB, D0, 0, INV, true>(tw, trow, nrows_thr, gld, sst);
             __syncthreads();
-            tile_round<TB, B1, B0, INV, true>(tw, trow, nrows_thr, sld, gst, post);
+            tile_round<TB, D1, D0, INV, true>(tw, trow, nrows_thr, sld, gst, post);
         } else {
-            tile_round<TB, B0, 0, INV, true>(tw, trow, nrows_thr, gld, sst);
+            tile_round<TB, B2, 0, INV, true>(tw, trow, nrows_thr, gld, sst);
             __syncthreads();
-            tile_round<TB, B1, B0, INV, true>(tw, trow, nrows_thr, sld, sst);
+            tile_round<TB, B1, B2, INV, true>(tw, trow, nrows_thr, sld, sst);
             __syncthreads();
-            tile_round<TB, B2, B0 + B1, INV, true>(tw, trow, nrows_thr, sld, gst, post);
+            tile_round<TB, B0, B1 + B2, INV, true>(tw, trow, nrows_thr, sld, gst, post);
         }
     }
 }
@@ -762,7 +791,7 @@ const gl::PowTable* Ctx::lde_coeff_tables(u32 log_n, u32 added_bits) {
 
 void ctx_init_tables(Ctx& c) {
     // the register DFTs hard-code two_adic_generator(k) = 2^root_exp(k): verify against the host field
-    for (int k = 1; k <= 4; k++) {
+    for (int k = 1; k <= 6; k++) {
         int e = root_exp(k, false);
         msh::Fp want = msh::two_adic_generator(k), got = msh::Fp(2).pow((msh::u64)e);
         if (want != got) throw Error(-3, "ntt: two-adic generator is not the expected power of two");
