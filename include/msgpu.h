@@ -397,6 +397,9 @@ int msgpu_blake3_hash(msgpu_ctx* ctx, const uint8_t* data, uint64_t len, uint8_t
 int msgpu_measure_int_peak(msgpu_ctx* ctx, double* out3);
 
 /* ---- test hooks --------------------------------------------------------------------------------- */
+/* Bytes of the context's device memory arena in use (live msgpu_malloc blocks and everything the context's handles hold). A
+ * call that leaves nothing behind, refused or complete with every handle freed, leaves this unchanged. */
+int msgpu_arena_in_use(msgpu_ctx* ctx, uint64_t* bytes);
 /* The selector tables of the quotient kernel: `trace_domain.selectors_on_coset(quotient_domain)` (src/prover.rs:775; p3's
  * UNNORMALISED Lagrange selectors, pinned in the reference by src/lookup.rs:697-756) at the points
  * x_i = GENERATOR * w_{n q}^i, i < n * q, in natural order. HOST outputs of n * q values each. */

@@ -111,6 +111,7 @@ SIGNATURES = {
     "msgpu_host_register": (C.c_int, [C.c_void_p, C.c_size_t]),
     "msgpu_host_unregister": (C.c_int, [C.c_void_p]),
     "msgpu_ctx_set_option": (C.c_int, [C.c_void_p, C.c_int, C.c_uint64]),
+    "msgpu_arena_in_use": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint64)]),
     "msgpu_selectors_on_coset": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "msgpu_commit_ldes_blocks_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p,
                                                C.c_int, C.c_void_p, C.c_void_p]),

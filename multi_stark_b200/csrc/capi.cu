@@ -112,6 +112,19 @@ void Ctx::arena_destroy() {
     arena = Arena();
 }
 
+Ctx::~Ctx() {
+    cudaSetDevice(device);
+    if (stream) cudaStreamSynchronize(stream);
+    for (auto& t : tw_full) t.reset();
+    ntt_tables.clear();
+    pow_cache.clear();
+    coset_cache.clear();
+    sel_cache.clear();
+    arena_destroy();
+    if (copy_stream) cudaStreamDestroy(copy_stream);
+    if (own_stream) cudaStreamDestroy(stream);
+}
+
 void b3_compress_raw_dev(Ctx& c, const u32* st, const u32* msg, u32* out);
 
 static void check_shape(u64 rows, u64 cols) {
@@ -131,40 +144,31 @@ static void host_transform(Ctx& c, const u64* in, u64 rows, u64 cols, u64 out_ro
     c.sync();
 }
 
-static msgpu_pdata* commit_impl(Ctx& c, const u64* const* mats, const u64* heights, const u64* widths, u64 n,
-                                u32 log_blowup, bool host_inputs, bool do_lde) {
+static std::unique_ptr<msgpu_pdata> commit_impl(Ctx& c, const u64* const* mats, const u64* heights, const u64* widths, u64 n,
+                                                u32 log_blowup, bool host_inputs, bool do_lde) {
     MSG_REQUIRE(n > 0, "commit: no matrices given");
-    msgpu_pdata* pd = new msgpu_pdata();
-    pd->ctx = &c;
-    try {
-        for (u64 i = 0; i < n; i++) {
-            check_shape(heights[i], widths[i]);
-            u64 h = heights[i], w = widths[i];
-            u64 out_h = do_lde ? (h << log_blowup) : h;
-            msgpu_pdata::Mat m{nullptr, out_h, w, true};
-            m.ptr = (u64*)c.alloc(out_h * w * 8);
-            pd->mats.push_back(m);
-            if (w == 0) continue;
-            if (!do_lde) {
-                MSG_CUDA(cudaMemcpyAsync(m.ptr, mats[i], h * w * 8, host_inputs ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice,
-                                         c.stream));
-                continue;
-            }
-            StageScope stage_scope(c, "lde");
-            DevBuf tmp(c, h * w * 8);
-            if (host_inputs) {
-                MSG_CUDA(cudaMemcpyAsync(tmp.p, mats[i], h * w * 8, cudaMemcpyHostToDevice, c.stream));
-                if (c.canonicalize_inputs) canonicalize(c, tmp.u(), h * w);
-                ntt_coset_lde(c, tmp.u(), m.ptr, tmp.u(), h, w, log_blowup, msh::GL_GENERATOR);
-            } else {
-                ntt_coset_lde(c, mats[i], m.ptr, tmp.u(), h, w, log_blowup, msh::GL_GENERATOR);
-            }
+    auto pd = std::make_unique<msgpu_pdata>();
+    for (u64 i = 0; i < n; i++) {
+        check_shape(heights[i], widths[i]);
+        u64 h = heights[i], w = widths[i];
+        pd->mats.push_back(msgpu_pdata::Mat::alloc(c, do_lde ? (h << log_blowup) : h, w));
+        u64* out = pd->mats.back().ptr;
+        if (w == 0) continue;
+        if (!do_lde) {
+            MSG_CUDA(cudaMemcpyAsync(out, mats[i], h * w * 8, host_inputs ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, c.stream));
+            continue;
         }
-        mmcs_build(c, pd);
-    } catch (...) {
-        pdata_destroy(pd);
-        throw;
+        StageScope stage_scope(c, "lde");
+        DevBuf tmp(c, h * w * 8);
+        if (host_inputs) {
+            MSG_CUDA(cudaMemcpyAsync(tmp.p, mats[i], h * w * 8, cudaMemcpyHostToDevice, c.stream));
+            if (c.canonicalize_inputs) canonicalize(c, tmp.u(), h * w);
+            ntt_coset_lde(c, tmp.u(), out, tmp.u(), h, w, log_blowup, msh::GL_GENERATOR);
+        } else {
+            ntt_coset_lde(c, mats[i], out, tmp.u(), h, w, log_blowup, msh::GL_GENERATOR);
+        }
     }
+    mmcs_build(c, pd.get());
     return pd;
 }
 
@@ -181,37 +185,23 @@ int msgpu_ctx_create(int device, void* stream, msgpu_ctx** out) {
         MSG_CUDA(cudaGetDeviceCount(&count));
         MSG_REQUIRE(device >= 0 && device < count, "ctx_create: no such CUDA device (libmsgpu has no CPU fallback)");
         MSG_CUDA(cudaSetDevice(device));
-        msgpu_ctx* h = new msgpu_ctx();
+        auto h = std::make_unique<msgpu_ctx>();
         h->c.device = device;
-        try {
-            if (stream) {
-                h->c.stream = (cudaStream_t)stream;
-            } else {
-                MSG_CUDA(cudaStreamCreateWithFlags(&h->c.stream, cudaStreamNonBlocking));
-                h->c.own_stream = true;
-            }
-            cudaDeviceProp prop;
-            MSG_CUDA(cudaGetDeviceProperties(&prop, device));
-            h->c.sm_count = prop.multiProcessorCount;
-            ctx_init_tables(h->c);
-        } catch (...) {
-            delete h;
-            throw;
+        if (stream) {
+            h->c.stream = (cudaStream_t)stream;
+        } else {
+            MSG_CUDA(cudaStreamCreateWithFlags(&h->c.stream, cudaStreamNonBlocking));
+            h->c.own_stream = true;
         }
-        *out = h;
+        cudaDeviceProp prop;
+        MSG_CUDA(cudaGetDeviceProperties(&prop, device));
+        h->c.sm_count = prop.multiProcessorCount;
+        ctx_init_tables(h->c);
+        *out = h.release();
     });
 }
 
-void msgpu_ctx_destroy(msgpu_ctx* h) {
-    if (!h) return;
-    cudaSetDevice(h->c.device);
-    cudaStreamSynchronize(h->c.stream);
-    for (void* p : h->c.owned) cudaFree(p);
-    h->c.arena_destroy();
-    if (h->c.copy_stream) cudaStreamDestroy(h->c.copy_stream);
-    if (h->c.own_stream) cudaStreamDestroy(h->c.stream);
-    delete h;
-}
+void msgpu_ctx_destroy(msgpu_ctx* h) { delete h; }
 
 const char* msgpu_last_error(void) { return g_last_error.c_str(); }
 int msgpu_sync(msgpu_ctx* h) {
@@ -225,6 +215,12 @@ int msgpu_malloc(msgpu_ctx* h, size_t bytes, void** dptr) {
 }
 int msgpu_free(msgpu_ctx* h, void* dptr) {
     return guard([&] { MSG_REQUIRE(h->c.free(dptr), "free: not a live block of this context"); });
+}
+int msgpu_arena_in_use(msgpu_ctx* h, uint64_t* bytes) {
+    return guard([&] {
+        MSG_REQUIRE(h && bytes, "arena_in_use: null argument");
+        *bytes = h->c.arena.in_use;
+    });
 }
 int msgpu_memcpy_h2d(msgpu_ctx* h, void* dst, const void* src, size_t bytes) {
     return guard([&] {
@@ -431,122 +427,93 @@ int msgpu_lde_from_shifted_coefficients_dev(msgpu_ctx* h, const uint64_t* in, ui
 int msgpu_commit(msgpu_ctx* h, const uint64_t* const* mats, const uint64_t* heights, const uint64_t* widths,
                  uint64_t n_mats, uint32_t log_blowup, msgpu_pdata** out, uint8_t* root32) {
     return guard([&] {
-        msgpu_pdata* pd = commit_impl(h->c, (const u64* const*)mats, (const u64*)heights, (const u64*)widths, n_mats,
-                                      log_blowup, true, true);
+        auto pd = commit_impl(h->c, (const u64* const*)mats, (const u64*)heights, (const u64*)widths, n_mats, log_blowup, true, true);
         memcpy(root32, pd->root, 32);
-        *out = pd;
+        *out = pd.release();
     });
 }
 // ---- pipelined host commit: uploads on the copy stream, LDEs on the main stream --------------------------------------------
 struct msgpu_upload {
     Ctx* ctx;
     struct Item {
-        u64* dev;
+        DevBuf dev;
         u64 height, width;
-        cudaEvent_t ready;
+        Event ready;  // the copy into `dev` has finished
     };
     std::vector<Item> items;
 };
-static void upload_destroy(msgpu_upload* up, bool free_buffers) {
-    if (!up) return;
-    for (auto& it : up->items) {
-        if (it.ready) {
-            cudaEventSynchronize(it.ready);  // a copy must not outlive its block
-            cudaEventDestroy(it.ready);
-        }
-        if (free_buffers && it.dev) up->ctx->free(it.dev);
-    }
-    delete up;
-}
 int msgpu_upload_begin(msgpu_ctx* h, const uint64_t* const* mats, const uint64_t* heights, const uint64_t* widths, uint64_t n_mats,
                        msgpu_upload** out) {
     return guard([&] {
         Ctx& c = h->c;
         MSG_REQUIRE(out && mats && heights && widths && n_mats > 0, "upload_begin: null or empty argument");
         if (!c.copy_stream) MSG_CUDA(cudaStreamCreateWithFlags(&c.copy_stream, cudaStreamNonBlocking));
-        msgpu_upload* up = new msgpu_upload();
+        auto up = std::make_unique<msgpu_upload>();
         up->ctx = &c;
-        try {
-            // the blocks may just have been freed by work still running on the main stream: the copies start behind it
-            cudaEvent_t e0;
-            MSG_CUDA(cudaEventCreateWithFlags(&e0, cudaEventDisableTiming));
-            MSG_CUDA(cudaEventRecord(e0, c.stream));
-            MSG_CUDA(cudaStreamWaitEvent(c.copy_stream, e0, 0));
-            cudaEventDestroy(e0);
-            for (u64 i = 0; i < n_mats; i++) {
-                check_shape(heights[i], widths[i]);
-                msgpu_upload::Item it{nullptr, heights[i], widths[i], nullptr};
-                const u64 bytes = heights[i] * widths[i] * 8;
-                it.dev = (u64*)c.alloc(bytes);
-                up->items.push_back(it);
-                MSG_CUDA(cudaEventCreateWithFlags(&up->items.back().ready, cudaEventDisableTiming));
-                if (bytes) {
-                    MSG_REQUIRE(mats[i], "upload_begin: null matrix");
-                    MSG_CUDA(cudaMemcpyAsync(it.dev, mats[i], bytes, cudaMemcpyHostToDevice, c.copy_stream));
-                }
-                MSG_CUDA(cudaEventRecord(up->items.back().ready, c.copy_stream));
+        up->items.reserve(n_mats);
+        // the blocks may just have been freed by work still running on the main stream: the copies start behind it
+        cudaEvent_t e0;
+        MSG_CUDA(cudaEventCreateWithFlags(&e0, cudaEventDisableTiming));
+        MSG_CUDA(cudaEventRecord(e0, c.stream));
+        MSG_CUDA(cudaStreamWaitEvent(c.copy_stream, e0, 0));
+        cudaEventDestroy(e0);
+        for (u64 i = 0; i < n_mats; i++) {
+            check_shape(heights[i], widths[i]);
+            const u64 bytes = heights[i] * widths[i] * 8;
+            up->items.push_back(msgpu_upload::Item{DevBuf(c, bytes), heights[i], widths[i], Event()});
+            auto& it = up->items.back();
+            if (bytes) {
+                MSG_REQUIRE(mats[i], "upload_begin: null matrix");
+                MSG_CUDA(cudaMemcpyAsync(it.dev.p, mats[i], bytes, cudaMemcpyHostToDevice, c.copy_stream));
             }
-        } catch (...) {
-            upload_destroy(up, true);
-            throw;
+            it.ready.record(c.copy_stream);
         }
-        *out = up;
+        *out = up.release();
     });
 }
-void msgpu_upload_free(msgpu_upload* up) { upload_destroy(up, true); }
+void msgpu_upload_free(msgpu_upload* up) { delete up; }
 int msgpu_commit_upload(msgpu_upload* up, uint32_t log_blowup, int verify_canonical, uint64_t** kept_inputs, int local_only,
                         msgpu_pdata** out, uint8_t* root32) {
     return guard([&] {
         MSG_REQUIRE(up && out && (root32 || local_only), "commit_upload: null argument");
+        std::unique_ptr<msgpu_upload> consumed(up);
         Ctx& c = *up->ctx;
-        msgpu_pdata* pd = new msgpu_pdata();
-        pd->ctx = &c;
+        auto pd = std::make_unique<msgpu_pdata>();
         DevBuf flag(c, 4);
-        try {
-            MSG_CUDA(cudaMemsetAsync(flag.p, 0, 4, c.stream));
-            for (auto& it : up->items) {
-                // matrix i is extended while matrices i + 1 ... are still arriving
-                MSG_CUDA(cudaStreamWaitEvent(c.stream, it.ready, 0));
-                const u64 out_h = it.height << log_blowup;
-                msgpu_pdata::Mat m{(u64*)c.alloc(out_h * it.width * 8), out_h, it.width, true};
-                pd->mats.push_back(m);
-                if (it.width == 0) continue;
-                if (c.canonicalize_inputs) canonicalize(c, it.dev, it.height * it.width);
-                else if (verify_canonical) check_canonical(c, it.dev, it.height * it.width, (u32*)flag.p);
-                StageScope stage_scope(c, "lde");
-                DevBuf tmp(c, it.height * it.width * 8);
-                ntt_coset_lde(c, it.dev, m.ptr, tmp.u(), it.height, it.width, log_blowup, msh::GL_GENERATOR);
-            }
-            u32 bad = 0;
-            MSG_CUDA(cudaMemcpyAsync(&bad, flag.p, 4, cudaMemcpyDeviceToHost, c.stream));
-            if (local_only) {
-                mmcs_build_local(c, pd);  // leaf digests per height class only (sharded commitments)
-                c.sync();
-            } else {
-                mmcs_build(c, pd);  // synchronises
-            }
-            MSG_REQUIRE(bad == 0, "commit_upload: value is not a canonical field element (>= p)");
-        } catch (...) {
-            pdata_destroy(pd);
-            upload_destroy(up, true);
-            throw;
+        MSG_CUDA(cudaMemsetAsync(flag.p, 0, 4, c.stream));
+        for (auto& it : up->items) {
+            // matrix i is extended while matrices i + 1 ... are still arriving
+            MSG_CUDA(cudaStreamWaitEvent(c.stream, it.ready.e, 0));
+            pd->mats.push_back(msgpu_pdata::Mat::alloc(c, it.height << log_blowup, it.width));
+            if (it.width == 0) continue;
+            if (c.canonicalize_inputs) canonicalize(c, it.dev.u(), it.height * it.width);
+            else if (verify_canonical) check_canonical(c, it.dev.u(), it.height * it.width, (u32*)flag.p);
+            StageScope stage_scope(c, "lde");
+            DevBuf tmp(c, it.height * it.width * 8);
+            ntt_coset_lde(c, it.dev.u(), pd->mats.back().ptr, tmp.u(), it.height, it.width, log_blowup, msh::GL_GENERATOR);
         }
-        for (size_t i = 0; i < up->items.size(); i++) {
-            if (kept_inputs) kept_inputs[i] = (uint64_t*)up->items[i].dev;
+        u32 bad = 0;
+        MSG_CUDA(cudaMemcpyAsync(&bad, flag.p, 4, cudaMemcpyDeviceToHost, c.stream));
+        if (local_only) {
+            mmcs_build_local(c, pd.get());  // leaf digests per height class only (sharded commitments)
+            c.sync();
+        } else {
+            mmcs_build(c, pd.get());  // synchronises
         }
-        upload_destroy(up, kept_inputs == nullptr);
+        MSG_REQUIRE(bad == 0, "commit_upload: value is not a canonical field element (>= p)");
+        if (kept_inputs)
+            for (size_t i = 0; i < up->items.size(); i++) kept_inputs[i] = (uint64_t*)up->items[i].dev.release();
         if (root32) memcpy(root32, pd->root, 32);
-        *out = pd;
+        *out = pd.release();
     });
 }
 
 int msgpu_commit_dev(msgpu_ctx* h, const uint64_t* const* mats, const uint64_t* heights, const uint64_t* widths,
                      uint64_t n_mats, uint32_t log_blowup, msgpu_pdata** out, uint8_t* root32) {
     return guard([&] {
-        msgpu_pdata* pd = commit_impl(h->c, (const u64* const*)mats, (const u64*)heights, (const u64*)widths, n_mats,
-                                      log_blowup, false, true);
+        auto pd = commit_impl(h->c, (const u64* const*)mats, (const u64*)heights, (const u64*)widths, n_mats, log_blowup, false, true);
         memcpy(root32, pd->root, 32);
-        *out = pd;
+        *out = pd.release();
     });
 }
 // ---- sharded commitments: one MMCS whose matrices live on several GPUs --------------------------------------------------
@@ -555,33 +522,27 @@ int msgpu_commit_local_dev(msgpu_ctx* h, uint64_t* const* mats, const uint64_t* 
     return guard([&] {
         Ctx& c = h->c;
         MSG_REQUIRE(n_mats > 0 && out, "commit_local: no matrices given");
-        msgpu_pdata* pd = new msgpu_pdata();
-        pd->ctx = &c;
-        try {
-            for (u64 i = 0; i < n_mats; i++) {
-                check_shape(heights[i], widths[i]);
-                if (inputs_are_ldes) {  // adopted (buffers from msgpu_malloc), as msgpu_commit_ldes_dev with take_ownership = 1
-                    pd->mats.push_back(msgpu_pdata::Mat{(u64*)mats[i], heights[i], widths[i], false});
-                    continue;
-                }
-                u64 hh = heights[i], w = widths[i], out_h = hh << log_blowup;
-                msgpu_pdata::Mat m{(u64*)c.alloc(out_h * w * 8), out_h, w, true};
-                pd->mats.push_back(m);
-                if (w == 0) continue;
-                StageScope stage_scope(c, "lde");
-                DevBuf tmp(c, hh * w * 8);
-                ntt_coset_lde(c, (const u64*)mats[i], m.ptr, tmp.u(), hh, w, log_blowup, msh::GL_GENERATOR);
+        auto pd = std::make_unique<msgpu_pdata>();
+        for (u64 i = 0; i < n_mats; i++) {
+            check_shape(heights[i], widths[i]);
+            if (inputs_are_ldes) {  // adopted (buffers from msgpu_malloc), as msgpu_commit_ldes_dev with take_ownership = 1
+                pd->mats.push_back(msgpu_pdata::Mat{(u64*)mats[i], heights[i], widths[i]});
+                continue;
             }
-            mmcs_build_local(c, pd);
-        } catch (...) {
-            pdata_destroy(pd);
-            throw;
+            u64 hh = heights[i], w = widths[i];
+            pd->mats.push_back(msgpu_pdata::Mat::alloc(c, hh << log_blowup, w));
+            if (w == 0) continue;
+            StageScope stage_scope(c, "lde");
+            DevBuf tmp(c, hh * w * 8);
+            ntt_coset_lde(c, (const u64*)mats[i], pd->mats.back().ptr, tmp.u(), hh, w, log_blowup, msh::GL_GENERATOR);
         }
-        for (auto& m : pd->mats) m.owned = true;
+        mmcs_build_local(c, pd.get());
         // The class digests are handed to the caller's transport next (an NCCL send ordered against ITS stream, not this
         // context's): they must be complete when this call returns, as in the local_only branch of msgpu_commit_upload.
         c.sync();
-        *out = pd;
+        if (inputs_are_ldes)
+            for (auto& m : pd->mats) m.own = DevBuf(c, (void*)m.ptr);
+        *out = pd.release();
     });
 }
 uint64_t msgpu_pdata_num_classes(const msgpu_pdata* pd) { return pd->class_leaves.size(); }
@@ -589,7 +550,7 @@ int msgpu_pdata_class_digests(const msgpu_pdata* pd, uint64_t k, uint64_t* lde_h
     return guard([&] {
         MSG_REQUIRE(k < pd->class_leaves.size(), "class_digests: no such height class");
         if (lde_height) *lde_height = pd->class_leaves[k].first;
-        if (dev_ptr) *dev_ptr = pd->class_leaves[k].second;
+        if (dev_ptr) *dev_ptr = pd->class_leaves[k].second.bytes();
     });
 }
 int msgpu_tree_from_digests(msgpu_ctx* h, uint64_t n_classes, const uint64_t* lde_heights, const uint8_t* const* digests_dev,
@@ -600,16 +561,10 @@ int msgpu_tree_from_digests(msgpu_ctx* h, uint64_t n_classes, const uint64_t* ld
         std::vector<std::pair<u64, const uint8_t*>> classes;
         for (u64 k = 0; k < n_classes; k++) classes.push_back({lde_heights[k], digests_dev[k]});
         std::sort(classes.begin(), classes.end(), [](auto& a, auto& b) { return a.first > b.first; });
-        msgpu_pdata* pd = new msgpu_pdata();
-        pd->ctx = &c;
-        try {
-            mmcs_build_from_classes(c, pd, classes);
-        } catch (...) {
-            pdata_destroy(pd);
-            throw;
-        }
+        auto pd = std::make_unique<msgpu_pdata>();
+        mmcs_build_from_classes(c, pd.get(), classes);
         memcpy(root32, pd->root, 32);
-        *out = pd;
+        *out = pd.release();
     });
 }
 uint64_t msgpu_pdata_max_height(const msgpu_pdata* pd) { return pd->max_height; }
@@ -622,7 +577,7 @@ int msgpu_pdata_root(const msgpu_pdata* pd, uint8_t* root32) {
 int msgpu_pdata_digests(const msgpu_pdata* pd, uint8_t** dev_ptr, uint64_t* n_digests) {
     return guard([&] {
         MSG_REQUIRE(pd && pd->digests && dev_ptr && n_digests, "pdata_digests: prover data without a tree");
-        *dev_ptr = pd->digests;
+        *dev_ptr = pd->digests.bytes();
         *n_digests = 2 * pd->max_height - 1;
     });
 }
@@ -651,26 +606,19 @@ int msgpu_pdata_from_parts(msgpu_ctx* h, uint64_t n_blocks, const uint64_t* cons
         std::vector<u64> ws;
         for (u64 b = 0; b < n_blocks; b++) { bl.push_back((const u64*)blocks[b]); ws.push_back(widths[b]); }
         std::vector<const uint8_t*> parts(part_digests, part_digests + n_parts);
-        msgpu_pdata* pd = new msgpu_pdata();
-        pd->ctx = &c;
-        try {
-            mmcs_from_parts(c, pd, bl, ws, lde_height, parts);
-        } catch (...) {
-            pdata_destroy(pd);
-            throw;
-        }
+        auto pd = std::make_unique<msgpu_pdata>();
+        mmcs_from_parts(c, pd.get(), bl, ws, lde_height, parts);
         memcpy(root32, pd->root, 32);
-        *out = pd;
+        *out = pd.release();
     });
 }
 
 int msgpu_mmcs_commit(msgpu_ctx* h, const uint64_t* const* mats, const uint64_t* heights, const uint64_t* widths,
                       uint64_t n_mats, msgpu_pdata** out, uint8_t* root32) {
     return guard([&] {
-        msgpu_pdata* pd =
-            commit_impl(h->c, (const u64* const*)mats, (const u64*)heights, (const u64*)widths, n_mats, 0, true, false);
+        auto pd = commit_impl(h->c, (const u64* const*)mats, (const u64*)heights, (const u64*)widths, n_mats, 0, true, false);
         memcpy(root32, pd->root, 32);
-        *out = pd;
+        *out = pd.release();
     });
 }
 int msgpu_commit_ldes_dev(msgpu_ctx* h, uint64_t* const* ldes, const uint64_t* heights, const uint64_t* widths,
@@ -688,39 +636,28 @@ int msgpu_commit_ldes_blocks_dev(msgpu_ctx* h, uint64_t* const* ldes, const uint
         Ctx& c = h->c;
         MSG_REQUIRE(n_mats > 0, "commit_ldes: no matrices given");
         MSG_REQUIRE(n_blocks <= 16 && (n_blocks == 0 || (block_ptrs && block_widths)), "commit_ldes: bad column-block list");
-        msgpu_pdata* pd = new msgpu_pdata();
-        pd->ctx = &c;
-        try {
-            for (u64 i = 0; i < n_mats; i++) {
-                check_shape(heights[i], widths[i]);
-                pd->mats.push_back(msgpu_pdata::Mat{(u64*)ldes[i], heights[i], widths[i], false});
-                if (n_blocks == 0 || !block_ptrs[i * n_blocks]) continue;
-                for (u64 b = 0; b < n_blocks; b++) {
-                    MSG_REQUIRE(block_ptrs[i * n_blocks + b] || block_widths[i * n_blocks + b] == 0, "commit_ldes: null column block");
-                    pd->mats.back().blocks.push_back({(const u64*)block_ptrs[i * n_blocks + b], block_widths[i * n_blocks + b]});
-                }
+        auto pd = std::make_unique<msgpu_pdata>();
+        for (u64 i = 0; i < n_mats; i++) {
+            check_shape(heights[i], widths[i]);
+            pd->mats.push_back(msgpu_pdata::Mat{(u64*)ldes[i], heights[i], widths[i]});
+            if (n_blocks == 0 || !block_ptrs[i * n_blocks]) continue;
+            for (u64 b = 0; b < n_blocks; b++) {
+                MSG_REQUIRE(block_ptrs[i * n_blocks + b] || block_widths[i * n_blocks + b] == 0, "commit_ldes: null column block");
+                pd->mats.back().blocks.push_back({(const u64*)block_ptrs[i * n_blocks + b], block_widths[i * n_blocks + b]});
             }
-            // root32 == NULL: stream-ordered, no read-back (the root is the last digest of msgpu_pdata_digests): a row shard's
-            // subtree root goes straight into a device all-gather
-            if (root32) mmcs_build(c, pd);
-            else mmcs_build_async(c, pd);
-        } catch (...) {
-            pdata_destroy(pd);
-            throw;
         }
+        // root32 == NULL: stream-ordered, no read-back (the root is the last digest of msgpu_pdata_digests): a row shard's
+        // subtree root goes straight into a device all-gather
+        if (root32) mmcs_build(c, pd.get());
+        else mmcs_build_async(c, pd.get());
         if (take_ownership)
-            for (auto& m : pd->mats) m.owned = true;
+            for (auto& m : pd->mats) m.own = DevBuf(c, (void*)m.ptr);
         if (root32) memcpy(root32, pd->root, 32);
-        *out = pd;
+        *out = pd.release();
     });
 }
 
-void msgpu_pdata_free(msgpu_pdata* pd) {
-    try {
-        pdata_destroy(pd);
-    } catch (...) {
-    }
-}
+void msgpu_pdata_free(msgpu_pdata* pd) { delete pd; }
 uint64_t msgpu_pdata_num_matrices(const msgpu_pdata* pd) { return pd->mats.size(); }
 int msgpu_pdata_matrix(const msgpu_pdata* pd, uint64_t idx, uint64_t** dev_ptr, uint64_t* rows, uint64_t* cols) {
     return guard([&] {
@@ -747,7 +684,7 @@ uint64_t msgpu_pdata_layer_len(const msgpu_pdata* pd, uint64_t layer) {
 int msgpu_pdata_read_layer(msgpu_ctx* h, const msgpu_pdata* pd, uint64_t layer, uint8_t* out) {
     return guard([&] {
         MSG_REQUIRE(layer < pd->layer_len.size(), "pdata_read_layer: layer out of range");
-        MSG_CUDA(cudaMemcpyAsync(out, pd->digests + pd->layer_off[layer] * 32, pd->layer_len[layer] * 32,
+        MSG_CUDA(cudaMemcpyAsync(out, pd->digests.bytes() + pd->layer_off[layer] * 32, pd->layer_len[layer] * 32,
                                  cudaMemcpyDeviceToHost, h->c.stream));
         h->c.sync();
     });

@@ -26,16 +26,4 @@ static int guard(F&& f) {
         return MSGPU_ERR_INTERNAL;
     }
 }
-
-struct DevBuf {  // RAII stream-ordered buffer
-    Ctx& c;
-    void* p = nullptr;
-    DevBuf(Ctx& c_, size_t bytes) : c(c_) { p = c.alloc(bytes); }
-    DevBuf(const DevBuf&) = delete;
-    ~DevBuf() {
-        if (p) c.free(p);
-    }
-    u64* u() const { return (u64*)p; }
-    void* release() { void* r = p; p = nullptr; return r; }
-};
 }  // namespace msg

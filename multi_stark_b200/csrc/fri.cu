@@ -431,7 +431,7 @@ struct msgpu_open {
     struct InvDen {
         msh::Fp2 z;
         u32 log_h;
-        u64* ptr;
+        msg::DevBuf buf;
         u64 row0 = 0, len = 0;
     };
     // sharded evaluation: the barycentric sums of the local rows, to be summed over the ranks before the values exist
@@ -448,15 +448,17 @@ struct msgpu_open {
     struct Input {
         u64* ptr;
         u64 len;
+        msg::DevBuf own;  // empty once the commit phase has taken the input over (input 0: `cur_own`) or rolled it in
     };
     std::vector<Input> inputs;  // tallest first
     size_t next_input = 0;
     u64* cur = nullptr;
     u64 cur_len = 0;
-    bool cur_committed = false;
-    std::vector<msgpu_pdata*> layers;
-    msgpu_pdata* pending = nullptr;  // layer over `cur` built ahead by the fused fold (owns cur); adopted by the next commit_round
-    bool pending_has_chal = false;   // the fused fold that built `pending` also ran the transcript step for its root
+    msg::DevBuf cur_own;         // holds `cur` until it is committed (then its layer holds it) or built ahead into `pending`
+    bool cur_committed = false;  // the protocol: a vector is committed before it is folded, and folded before the next commit
+    std::vector<std::unique_ptr<msgpu_pdata>> layers;
+    std::unique_ptr<msgpu_pdata> pending;  // layer over `cur` built ahead by the fused fold; adopted by the next commit_round
+    bool pending_has_chal = false;         // the fused fold that built `pending` also ran the transcript step for its root
 };
 
 namespace msg {
@@ -470,21 +472,20 @@ static gl::PowTable lde_x_table(Ctx& c, u32 log_h) {
 static u64* find_invden(msgpu_open* op, const msh::Fp2& z, const msgpu_open::Mat& m) {
     for (auto& d : op->invdens) {
         if (!(d.z == z)) continue;
-        if (!op->sharded && d.log_h >= m.log_h) return d.ptr;
-        if (op->sharded && d.log_h == m.log_h && d.row0 == m.row0 && d.len == m.rows) return d.ptr;
+        if (!op->sharded && d.log_h >= m.log_h) return d.buf.u();
+        if (op->sharded && d.log_h == m.log_h && d.row0 == m.row0 && d.len == m.rows) return d.buf.u();
     }
     throw Error(-3, "open: missing inverse denominators");
 }
 
-static void open_destroy(msgpu_open* op) {
-    if (!op) return;
-    Ctx& c = *op->ctx;
-    for (auto& d : op->invdens) c.free(d.ptr);
-    for (size_t k = op->next_input; k < op->inputs.size(); k++) c.free(op->inputs[k].ptr);
-    if (op->pending) pdata_destroy(op->pending);  // owns cur
-    else if (op->cur && !op->cur_committed) c.free(op->cur);
-    for (auto* pd : op->layers) pdata_destroy(pd);
-    delete op;
+// The tallest input is the first vector of the commit phase; the shorter ones are rolled into the folds of their height.
+static void start_commit_phase(msgpu_open* op) {
+    std::sort(op->inputs.begin(), op->inputs.end(), [](const msgpu_open::Input& a, const msgpu_open::Input& b) { return a.len > b.len; });
+    op->cur = op->inputs[0].ptr;
+    op->cur_len = op->inputs[0].len;
+    op->cur_own = std::move(op->inputs[0].own);
+    op->next_input = 1;
+    op->cur_committed = false;
 }
 
 // values from the barycentric sums (S1, S2 per column and point): y = (z * S2 - S1) * (z^h - g^h) / (h * g^h), g = GENERATOR
@@ -524,22 +525,18 @@ static void evaluate_all(Ctx& c, msgpu_open* op) {
                     if (!op->sharded) { d.log_h = std::max(d.log_h, m.log_h); d.len = 1ull << d.log_h; found = true; }
                     else if (d.log_h == m.log_h && d.row0 == m.row0 && d.len == m.rows) found = true;
                 }
-                if (!found) op->invdens.push_back(msgpu_open::InvDen{z, m.log_h, nullptr, m.row0, m.rows});
+                if (!found) op->invdens.push_back(msgpu_open::InvDen{z, m.log_h, DevBuf(), m.row0, m.rows});
             }
         }
     for (auto& d : op->invdens) {
-        d.ptr = (u64*)c.alloc(d.len * 16);
+        d.buf = DevBuf(c, d.len * 16);
         u64 threads = (d.len + kInvPerThread - 1) / kInvPerThread;
-        {
-            KLaunch kl(c, "k_inv_denoms");
-            k_inv_denoms<<<(unsigned)((threads + 255) / 256), 256, 0, c.stream>>>(d.ptr, d.log_h, gl::e2{d.z.c[0].v, d.z.c[1].v},
-                                                                                lde_x_table(c, d.log_h), d.row0, d.len);
-        }
-        MSG_CUDA(cudaGetLastError());
+        launch(c, "k_inv_denoms", k_inv_denoms, (unsigned)((threads + 255) / 256), 256, 0, d.buf.u(), d.log_h, gl::e2{d.z.c[0].v, d.z.c[1].v},
+               lde_x_table(c, d.log_h), d.row0, d.len);
     }
     // 2. barycentric sums per matrix (all of its points in one pass over the low coset = the first height >> log_blowup stored
     //    rows; a shard contributes the part of them it holds)
-    std::vector<u64*> partials;
+    std::vector<DevBuf> partials;
     size_t sums_total = 0;
     for (auto& round : op->rounds)
         for (auto& m : round)
@@ -574,29 +571,20 @@ static void evaluate_all(Ctx& c, msgpu_open* op) {
                     bp.tile_rows = (u32)std::min<u64>(256, std::max<u64>(8, 4096 / bp.wc));
                     u64 want = (h + bp.tile_rows - 1) / bp.tile_rows;
                     u32 ctas = (u32)std::min<u64>(want, (u64)c.sm_count * 6);
-                    u64* d_partial = (u64*)c.alloc((size_t)ctas * bp.wc * (npts + 1) * 16);
-                    partials.push_back(d_partial);
-                    bp.partial = d_partial;
+                    partials.emplace_back(c, (size_t)ctas * bp.wc * (npts + 1) * 16);
+                    bp.partial = partials.back().u();
                     // at most 46,448 bytes when the dd tile is padded (wc = 19, tile_rows = 215, 4 points) and 49,152 without
                     // (wc = 16, tile_rows = 256, 4 points): both within the default dynamic shared memory limit
                     size_t smem = std::max((size_t)bp.rows_per_step * bp.wc * (npts + 1) * 16,
                                            (bary_dd_offset(bp.tile_rows, bp.wc) + (size_t)bp.tile_rows * npts * 2) * 8);
-                    {
-                        KLaunch kl(c, "k_bary_partial");
-                        switch (npts) {
-                            case 1: k_bary_partial<1><<<ctas, 256, smem, c.stream>>>(bp); break;
-                            case 2: k_bary_partial<2><<<ctas, 256, smem, c.stream>>>(bp); break;
-                            case 3: k_bary_partial<3><<<ctas, 256, smem, c.stream>>>(bp); break;
-                            default: k_bary_partial<4><<<ctas, 256, smem, c.stream>>>(bp); break;
-                        }
+                    switch (npts) {
+                        case 1: launch(c, "k_bary_partial", k_bary_partial<1>, ctas, 256, smem, bp); break;
+                        case 2: launch(c, "k_bary_partial", k_bary_partial<2>, ctas, 256, smem, bp); break;
+                        case 3: launch(c, "k_bary_partial", k_bary_partial<3>, ctas, 256, smem, bp); break;
+                        default: launch(c, "k_bary_partial", k_bary_partial<4>, ctas, 256, smem, bp); break;
                     }
-                    MSG_CUDA(cudaGetLastError());
-                    {
-                        const u32 n = bp.wc * (npts + 1);
-                        KLaunch kl(c, "k_bary_sum");
-                        k_bary_sum<<<(n * 32 + 127) / 128, 128, 0, c.stream>>>(d_partial, ctas, n, d_sums.u() + my_off);
-                    }
-                    MSG_CUDA(cudaGetLastError());
+                    const u32 n = bp.wc * (npts + 1);
+                    launch(c, "k_bary_sum", k_bary_sum, (n * 32 + 127) / 128, 128, 0, bp.partial, ctas, n, d_sums.u() + my_off);
                 }
             }
         }
@@ -604,7 +592,6 @@ static void evaluate_all(Ctx& c, msgpu_open* op) {
     if (sums_total) MSG_CUDA(cudaMemcpyAsync(op->raw_sums.data(), d_sums.p, sums_total * 8, cudaMemcpyDeviceToHost, c.stream));  // ONE read-back
     c.sync();
     op->raw_sums.resize(sums_total);
-    for (u64* pp : partials) c.free(pp);
     // sharded: the sums of all ranks are added first (msgpu_open_sums / msgpu_open_finish_values)
     if (!op->sharded) finish_values(op, op->raw_sums.data());
 }
@@ -626,7 +613,7 @@ static void reduce_all(Ctx& c, msgpu_open* op, msh::Fp2 alpha) {
     for (size_t i = 0; i < max_w; i++) { apow_flat[2 * i] = apow[i].c[0].v; apow_flat[2 * i + 1] = apow[i].c[1].v; }
     DevBuf d_apow(c, apow_flat.size() * 8);
     MSG_CUDA(cudaMemcpyAsync(d_apow.p, apow_flat.data(), apow_flat.size() * 8, cudaMemcpyHostToDevice, c.stream));
-    u64* ro[33] = {nullptr};
+    DevBuf ro[33];
     u64 ro_len[33] = {0};
     u64 num_reduced[33] = {0};
     ensure_max_smem(k_reduce_openings, (int)kRedMaxSmem);
@@ -638,8 +625,8 @@ static void reduce_all(Ctx& c, msgpu_open* op, msh::Fp2 alpha) {
             const bool full = !op->sharded || op->fri_owner;
             if (!ro[lh] && (full || m.rows)) {  // p3 creates the height's vector for every matrix of every round, opened or not
                 ro_len[lh] = full ? m.height : m.rows;
-                ro[lh] = (u64*)c.alloc(ro_len[lh] * 16);
-                MSG_CUDA(cudaMemsetAsync(ro[lh], 0, ro_len[lh] * 16, c.stream));
+                ro[lh] = DevBuf(c, ro_len[lh] * 16);
+                MSG_CUDA(cudaMemsetAsync(ro[lh].p, 0, ro_len[lh] * 16, c.stream));
             }
             if (m.points.empty()) continue;
             if (m.rows == 0) {  // lives elsewhere: only the alpha-power counter of its height advances
@@ -652,7 +639,7 @@ static void reduce_all(Ctx& c, msgpu_open* op, msh::Fp2 alpha) {
                 ReduceParams rp{};
                 rp.M = m.ptr;
                 rp.apow = d_apow.u();
-                rp.ro = ro[lh];
+                rp.ro = ro[lh].u();
                 rp.H = m.rows;
                 rp.ro_off = full ? m.row0 : 0;
                 rp.w = (u32)m.width;
@@ -668,22 +655,14 @@ static void reduce_all(Ctx& c, msgpu_open* op, msh::Fp2 alpha) {
                 }
                 const u32 tr = reduce_tile_rows(m.width);
                 rp.tile_rows = tr;
-                const size_t smem = reduce_smem(m.width);
-                {
-                    KLaunch kl(c, "k_reduce_openings");
-                    k_reduce_openings<<<(unsigned)((m.rows + tr - 1) / tr), kRedThreads, smem, c.stream>>>(rp);
-                }
-                MSG_CUDA(cudaGetLastError());
+                launch(c, "k_reduce_openings", k_reduce_openings, (unsigned)((m.rows + tr - 1) / tr), kRedThreads, reduce_smem(m.width), rp);
             }
         }
     for (int lh = 32; lh >= 0; lh--)
-        if (ro[lh]) op->inputs.push_back(msgpu_open::Input{ro[lh], ro_len[lh]});
+        if (ro[lh]) op->inputs.push_back(msgpu_open::Input{ro[lh].u(), ro_len[lh], std::move(ro[lh])});
     c.sync();  // apow_flat (pageable) must outlive its copy
     MSG_REQUIRE(!op->inputs.empty(), "open: nothing to open");
-    op->cur = op->inputs[0].ptr;
-    op->cur_len = op->inputs[0].len;
-    op->next_input = 1;
-    op->cur_committed = false;
+    start_commit_phase(op);
 }
 
 
@@ -700,27 +679,21 @@ static void fri_fold_impl(msgpu_open* op, const msh::Fp2* beta, const FriChal* c
     if (beta) { hb = beta->halve(); bsq = beta->square(); }
     const u64* roll = nullptr;
     if (op->next_input < op->inputs.size() && op->inputs[op->next_input].len == half) roll = op->inputs[op->next_input].ptr;
-    u64* out = (u64*)c.alloc(half * 16);
+    DevBuf out_buf(c, half * 16);
+    u64* out = out_buf.u();
     gl::PowTable tab = c.pow_table(msh::two_adic_generator(log_half + 1).inverse().v, 1, log_half + 1).view();
     if (fuse_commit && half >= 2 && half <= kFusedFoldMax) {
         // fold + Merkle commitment of the folded vector (rows of 2 extension elements) in one launch
-        msgpu_pdata* pd = new msgpu_pdata();
-        pd->ctx = &c;
+        auto pd = std::make_unique<msgpu_pdata>();
         const u64 rows = half / 2;
-        try {
-            mmcs_layout_layers(c, pd, rows);
-        } catch (...) {
-            delete pd;
-            c.free(out);
-            throw;
-        }
-        pd->mats.push_back(msgpu_pdata::Mat{out, rows, 4, true});
+        mmcs_layout_layers(c, pd.get(), rows);
+        pd->mats.push_back(msgpu_pdata::Mat{out, rows, 4, std::move(out_buf)});
         pd->total_width = 4;
         FoldCommitParams fp{};
         fp.in = op->cur;
         fp.out = out;
         fp.roll = roll;
-        fp.digests = (uint4*)pd->digests;
+        fp.digests = (uint4*)pd->digests.p;
         fp.n_layers = (u32)pd->layer_off.size();
         for (size_t l = 0; l < pd->layer_off.size(); l++) fp.layer_off[l] = pd->layer_off[l];
         fp.half_beta = gl::e2{hb.c[0].v, hb.c[1].v};
@@ -733,22 +706,17 @@ static void fri_fold_impl(msgpu_open* op, const msh::Fp2* beta, const FriChal* c
         fp.chal_next = next_chal;
         fp.root_out = next_root_out;
         ensure_max_smem(k_fri_fold_commit, (int)(kFusedFoldMax / 2 * 48));
-        {
-            KLaunch kl(c, "k_fri_fold_commit");
-            k_fri_fold_commit<<<1, 256, (size_t)rows * 48, c.stream>>>(fp);
-        }
-        MSG_CUDA(cudaGetLastError());
-        if (!chal) MSG_CUDA(cudaMemcpyAsync(pd->root, pd->digests + pd->layer_off.back() * 32, 32, cudaMemcpyDeviceToHost, c.stream));
-        op->pending = pd;
+        launch(c, "k_fri_fold_commit", k_fri_fold_commit, 1, 256, (size_t)rows * 48, fp);
+        if (!chal) MSG_CUDA(cudaMemcpyAsync(pd->root, pd->digests.bytes() + pd->layer_off.back() * 32, 32, cudaMemcpyDeviceToHost, c.stream));
+        op->pending = std::move(pd);
         op->pending_has_chal = next_chal != nullptr;
     } else {
-        KLaunch kl(c, "k_fri_fold");
-        k_fri_fold<<<(unsigned)((half + 255) / 256), 256, 0, c.stream>>>(op->cur, out, half, log_half, gl::e2{hb.c[0].v, hb.c[1].v}, tab,
-                                                                         roll, gl::e2{bsq.c[0].v, bsq.c[1].v}, chal);
+        launch(c, "k_fri_fold", k_fri_fold, (unsigned)((half + 255) / 256), 256, 0, op->cur, out, half, log_half,
+               gl::e2{hb.c[0].v, hb.c[1].v}, tab, roll, gl::e2{bsq.c[0].v, bsq.c[1].v}, chal);
+        op->cur_own = std::move(out_buf);
     }
-    MSG_CUDA(cudaGetLastError());
     if (roll) {
-        c.free(op->inputs[op->next_input].ptr);
+        op->inputs[op->next_input].own.reset();
         op->next_input++;
     }
     op->cur = out;
@@ -765,9 +733,7 @@ static void open_begin_impl(msgpu_ctx* h, uint64_t n_rounds, const msgpu_pdata* 
                             msgpu_open** out, uint64_t* n_values) {
     Ctx& c = h->c;
     MSG_REQUIRE(pds && out && n_values, "open_begin: null argument");
-    auto op = std::unique_ptr<msgpu_open, void (*)(msgpu_open*)>(new msgpu_open(), [](msgpu_open* o) {
-        try { open_destroy(o); } catch (...) {}
-    });
+    auto op = std::make_unique<msgpu_open>();
     op->ctx = &c;
     op->log_blowup = log_blowup;
     op->sharded = modes != nullptr;
@@ -845,16 +811,15 @@ int msgpu_open_finish_values(msgpu_open* op, const uint64_t* total_sums) {
 int msgpu_pdata_placeholder(msgpu_ctx* h, uint64_t n_mats, const uint64_t* heights, const uint64_t* widths, msgpu_pdata** out) {
     return guard([&] {
         MSG_REQUIRE(out && n_mats > 0 && heights && widths, "pdata_placeholder: bad argument");
-        msgpu_pdata* pd = new msgpu_pdata();
-        pd->ctx = &h->c;
+        auto pd = std::make_unique<msgpu_pdata>();
         for (u64 i = 0; i < n_mats; i++) {
-            if (!is_pow2(heights[i])) { delete pd; throw Error(-1, "pdata_placeholder: heights must be powers of two"); }
-            pd->mats.push_back(msgpu_pdata::Mat{nullptr, heights[i], widths[i], false});
+            MSG_REQUIRE(is_pow2(heights[i]), "pdata_placeholder: heights must be powers of two");
+            pd->mats.push_back(msgpu_pdata::Mat{nullptr, heights[i], widths[i]});
             pd->total_width += widths[i];
             pd->max_height = std::max<u64>(pd->max_height, heights[i]);
         }
         memset(pd->root, 0, 32);
-        *out = pd;
+        *out = pd.release();
     });
 }
 // dst[i] += src[i] / v[i] += c over n extension elements (device pointers)
@@ -862,9 +827,7 @@ int msgpu_ext_add_dev(msgpu_ctx* h, uint64_t* dst, const uint64_t* src, uint64_t
     return guard([&] {
         Ctx& c = h->c;
         if (n == 0) return;
-        KLaunch kl(c, "k_ext_add");
-        k_ext_add<<<(unsigned)((2 * n + 255) / 256), 256, 0, c.stream>>>((u64*)dst, (const u64*)src, n);
-        MSG_CUDA(cudaGetLastError());
+        launch(c, "k_ext_add", k_ext_add, (unsigned)((2 * n + 255) / 256), 256, 0, (u64*)dst, (const u64*)src, n);
     });
 }
 int msgpu_ext_add_scalar_dev(msgpu_ctx* h, uint64_t* v, uint64_t n, const uint64_t* c2) {
@@ -872,9 +835,7 @@ int msgpu_ext_add_scalar_dev(msgpu_ctx* h, uint64_t* v, uint64_t n, const uint64
         Ctx& c = h->c;
         MSG_REQUIRE(c2 && c2[0] < GLD_P && c2[1] < GLD_P, "ext_add_scalar: constant is not canonical");
         if (n == 0) return;
-        KLaunch kl(c, "k_ext_add_scalar");
-        k_ext_add_scalar<<<(unsigned)((2 * n + 255) / 256), 256, 0, c.stream>>>((u64*)v, n, gl::e2{c2[0], c2[1]});
-        MSG_CUDA(cudaGetLastError());
+        launch(c, "k_ext_add_scalar", k_ext_add_scalar, (unsigned)((2 * n + 255) / 256), 256, 0, (u64*)v, n, gl::e2{c2[0], c2[1]});
     });
 }
 
@@ -923,13 +884,11 @@ int msgpu_open_add_input(msgpu_open* op, uint64_t len, uint64_t** dev_ptr) {
         MSG_REQUIRE(dev_ptr && is_pow2(len), "open_add_input: bad argument");
         MSG_REQUIRE(op->layers.empty() && !op->cur_committed && op->next_input <= 1, "open_add_input: the commit phase has started");
         for (auto& in : op->inputs) MSG_REQUIRE(in.len != len, "open_add_input: this height already has an input (one height class per rank)");
-        u64* buf = (u64*)c.alloc(len * 16);
-        op->inputs.push_back(msgpu_open::Input{buf, len});
-        std::sort(op->inputs.begin(), op->inputs.end(), [](const msgpu_open::Input& a, const msgpu_open::Input& b) { return a.len > b.len; });
-        op->cur = op->inputs[0].ptr;
-        op->cur_len = op->inputs[0].len;
-        op->next_input = 1;
-        *dev_ptr = (uint64_t*)buf;
+        DevBuf buf(c, len * 16);
+        *dev_ptr = (uint64_t*)buf.p;
+        if (op->cur_own) op->inputs[0].own = std::move(op->cur_own);  // the commit phase starts over with the tallest input
+        op->inputs.push_back(msgpu_open::Input{buf.u(), len, std::move(buf)});
+        start_commit_phase(op);
     });
 }
 
@@ -946,23 +905,19 @@ int msgpu_fri_commit_round(msgpu_open* op, uint8_t* root32) {
         StageScope ss(c, "fri");
         MSG_REQUIRE(op->cur && !op->cur_committed, "fri_commit_round: nothing to commit");
         MSG_REQUIRE(op->cur_len >= 2, "fri_commit_round: vector too short to fold");
+        op->cur_committed = true;
         if (op->pending) {  // the fused fold has already hashed this vector: wait for its root
-            msgpu_pdata* pd = op->pending;
-            op->pending = nullptr;
-            op->cur_committed = true;
-            op->layers.push_back(pd);
+            op->layers.push_back(std::move(op->pending));
             c.sync();
-            memcpy(root32, pd->root, 32);
+            memcpy(root32, op->layers.back()->root, 32);
             return;
         }
-        msgpu_pdata* pd = new msgpu_pdata();
-        pd->ctx = &c;
+        auto pd = std::make_unique<msgpu_pdata>();
         // rows of 2 extension elements = 4 base columns (ExtensionMmcs flattening)
-        pd->mats.push_back(msgpu_pdata::Mat{op->cur, op->cur_len / 2, 4, true});
-        op->cur_committed = true;  // the layer owns the buffer from here on
-        op->layers.push_back(pd);
-        mmcs_build(c, pd);
-        memcpy(root32, pd->root, 32);
+        pd->mats.push_back(msgpu_pdata::Mat{op->cur, op->cur_len / 2, 4, std::move(op->cur_own)});
+        op->layers.push_back(std::move(pd));
+        mmcs_build(c, op->layers.back().get());
+        memcpy(root32, op->layers.back()->root, 32);
     });
 }
 
@@ -1002,27 +957,21 @@ int msgpu_fri_commit_phase(msgpu_open* op, const uint8_t* input_buffer, uint64_t
         MSG_CUDA(cudaMemcpyAsync(d_prefix, input_buffer, input_len, cudaMemcpyHostToDevice, c.stream));
         for (u64 k = 0; k < rounds; k++) {
             // commit the current vector (unless the fused fold of the previous round already did, transcript step included)
-            msgpu_pdata* pd;
             bool have_chal = false;
             if (op->pending) {
-                pd = op->pending;
-                op->pending = nullptr;
+                op->layers.push_back(std::move(op->pending));
                 have_chal = op->pending_has_chal;
                 op->pending_has_chal = false;
             } else {
-                pd = new msgpu_pdata();
-                pd->ctx = &c;
-                pd->mats.push_back(msgpu_pdata::Mat{op->cur, op->cur_len / 2, 4, true});  // ExtensionMmcs rows of 2 elements
+                op->layers.push_back(std::make_unique<msgpu_pdata>());  // ExtensionMmcs rows of 2 elements
+                op->layers.back()->mats.push_back(msgpu_pdata::Mat{op->cur, op->cur_len / 2, 4, std::move(op->cur_own)});
             }
             op->cur_committed = true;
-            op->layers.push_back(pd);
+            msgpu_pdata* pd = op->layers.back().get();
             if (!pd->digests) mmcs_build_async(c, pd);
-            if (!have_chal) {
-                KLaunch kl(c, "k_fri_challenge");
-                k_fri_challenge<<<1, 32, 0, c.stream>>>(k == 0 ? d_prefix : nullptr, (u32)input_len, d_state,
-                                                       (const u32*)(pd->digests + pd->layer_off.back() * 32), d_chal + k, d_roots + 8 * k);
-                MSG_CUDA(cudaGetLastError());
-            }
+            if (!have_chal)
+                launch(c, "k_fri_challenge", k_fri_challenge, 1, 32, 0, k == 0 ? d_prefix : nullptr, (u32)input_len, d_state,
+                       (const u32*)(pd->digests.bytes() + pd->layer_off.back() * 32), d_chal + k, d_roots + 8 * k);
             const bool last = k + 1 == rounds;
             fri_fold_impl(op, nullptr, d_chal + k, !last, last ? nullptr : d_state, last ? nullptr : d_chal + k + 1,
                           last ? nullptr : d_roots + 8 * (k + 1));
@@ -1051,13 +1000,8 @@ int msgpu_fri_read_current(msgpu_open* op, uint64_t* out) {
 
 uint64_t msgpu_fri_num_layers(const msgpu_open* op) { return op->layers.size(); }
 const msgpu_pdata* msgpu_fri_layer_pdata(const msgpu_open* op, uint64_t layer) {
-    return layer < op->layers.size() ? op->layers[layer] : nullptr;
+    return layer < op->layers.size() ? op->layers[layer].get() : nullptr;
 }
-void msgpu_open_free(msgpu_open* op) {
-    try {
-        open_destroy(op);
-    } catch (...) {
-    }
-}
+void msgpu_open_free(msgpu_open* op) { delete op; }
 
 }  // extern "C"

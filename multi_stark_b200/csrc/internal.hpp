@@ -5,6 +5,7 @@
 #include <cstdint>
 #include <cstddef>
 #include <map>
+#include <memory>
 #include <mutex>
 #include <set>
 #include <string>
@@ -37,11 +38,23 @@ struct Error : std::runtime_error {
         if (!(cond)) throw msg::Error(-1, std::string(msg_));    \
     } while (0)
 
+// Owner of a cudaMalloc'd table that lives as long as the context (Ctx caches, program uploads)
+struct CudaFree {
+    void operator()(void* p) const noexcept { cudaFree(p); }
+};
+template <class T>
+using CudaPtr = std::unique_ptr<T, CudaFree>;
+template <class T>
+CudaPtr<T> cuda_malloc(size_t n) {
+    void* p = nullptr;
+    MSG_CUDA(cudaMalloc(&p, n * sizeof(T)));
+    return CudaPtr<T>((T*)p);
+}
+
 struct DevPow {
-    u64* lo = nullptr;
-    u64* hi = nullptr;
+    CudaPtr<u64> lo, hi;
     u32 h1 = 0;
-    gl::PowTable view() const { gl::PowTable t; t.lo = lo; t.hi = hi; t.h1 = h1; return t; }
+    gl::PowTable view() const { gl::PowTable t; t.lo = lo.get(); t.hi = hi.get(); t.h1 = h1; return t; }
 };
 
 struct Ctx {
@@ -52,13 +65,12 @@ struct Ctx {
     unsigned long long launches = 0;  // kernels of this library launched so far
     bool canonicalize_inputs = false;  // MSGPU_OPT_CANONICALIZE_INPUTS: host matrices are reduced mod p on the device after upload
     int sm_count = 148;
-    u64* tw_full[2] = {nullptr, nullptr};  // w_1024^{i} / w_1024^{-i}, i < 1024
-    std::map<std::tuple<u32, u32, u32, u64>, u64*> ntt_tables;  // per-size inter-pass twiddles / coset scales (ntt.cu)
+    CudaPtr<u64> tw_full[2];  // w_1024^{i} / w_1024^{-i}, i < 1024
+    std::map<std::tuple<u32, u32, u32, u64>, CudaPtr<u64>> ntt_tables;  // per-size inter-pass twiddles / coset scales (ntt.cu)
     std::map<std::tuple<u64, u64, u32>, DevPow> pow_cache;
-    std::map<std::tuple<u32, u32, u64>, gl::PowTable*> coset_cache;  // (log_n, added_bits, shift) -> device array [B]
-    std::vector<void*> owned;  // table allocations freed with the context
+    std::map<std::tuple<u32, u32, u64>, CudaPtr<gl::PowTable>> coset_cache;  // (log_n, added_bits, shift) -> device array [B]
     struct SelCache {
-        u64 *first, *last, *inv_zh;
+        CudaPtr<u64> first, last, inv_zh, zh;
     };
     std::map<std::pair<u32, u32>, SelCache> sel_cache;  // selectors on the quotient coset per (log_n, log_q)
 
@@ -88,12 +100,14 @@ struct Ctx {
         std::vector<std::pair<char*, size_t>> segments;
         size_t reserved = 0, in_use = 0, peak_in_use = 0;
     } arena;
+    Ctx() = default;
+    ~Ctx();  // synchronises the stream, then frees the tables, the arena and the streams this context created
     void* alloc(size_t bytes);  // valid for work enqueued on `stream` after the call
     bool free(void* p) noexcept;  // the block may be reused by later work on `stream`; false = not a live block
     void arena_trim();          // give wholly free segments back to the driver
     void arena_destroy();
     void sync() { MSG_CUDA(cudaStreamSynchronize(stream)); }
-    DevPow pow_table(u64 g, u64 c, u32 bits);
+    const DevPow& pow_table(u64 g, u64 c, u32 bits);
     const gl::PowTable* coset_tables(u32 log_n, u32 added_bits, u64 shift);
     const gl::PowTable* lde_coeff_tables(u32 log_n, u32 added_bits);
 };
@@ -114,27 +128,76 @@ inline void ensure_max_smem(F* func, int bytes) {
     done.insert({dev, (const void*)func});
 }
 
+// Owner of one arena block of a context (Ctx::alloc). Empty when default-constructed, moved from or released.
+struct DevBuf {
+    Ctx* c = nullptr;
+    void* p = nullptr;
+    DevBuf() = default;
+    DevBuf(Ctx& c_, size_t bytes) : c(&c_), p(c_.alloc(bytes)) {}
+    DevBuf(Ctx& c_, void* adopted) : c(&c_), p(adopted) {}  // takes over a live block of c_ (msgpu_malloc)
+    DevBuf(DevBuf&& o) noexcept : c(o.c), p(o.release()) {}
+    DevBuf& operator=(DevBuf&& o) noexcept {
+        if (this != &o) {
+            reset();
+            c = o.c;
+            p = o.release();
+        }
+        return *this;
+    }
+    ~DevBuf() { reset(); }
+    void reset() noexcept {
+        if (p) c->free(p);
+        p = nullptr;
+    }
+    void* release() noexcept {
+        void* r = p;
+        p = nullptr;
+        return r;
+    }
+    explicit operator bool() const { return p != nullptr; }
+    u64* u() const { return (u64*)p; }
+    uint8_t* bytes() const { return (uint8_t*)p; }
+};
+
+// Owner of the event that marks the end of a copy into an arena block. It waits for the event before destroying it: a copy must
+// not outlive its block, so the owner is declared after the block's DevBuf (members are destroyed in reverse order).
+struct Event {
+    cudaEvent_t e = nullptr;
+    Event() = default;
+    Event(Event&& o) noexcept : e(o.e) { o.e = nullptr; }
+    Event& operator=(Event&&) = delete;
+    ~Event() {
+        if (e) {
+            cudaEventSynchronize(e);
+            cudaEventDestroy(e);
+        }
+    }
+    void record(cudaStream_t s) {
+        if (!e) MSG_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+        MSG_CUDA(cudaEventRecord(e, s));
+    }
+};
+
 inline double host_now_us() {
     return std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now().time_since_epoch()).count();
 }
-// Brackets one kernel launch: counts it and, when profiling, records events around it.
-struct KLaunch {
-    Ctx& c;
+// Every kernel of this library is launched here, on the context's stream: the launch is counted, timed under `name` when
+// profiling (bench.py looks kernels up by these names) and checked.
+template <class... P, class... A>
+void launch(Ctx& c, const char* name, void (*kernel)(P...), dim3 grid, dim3 block, size_t smem, A&&... args) {
     cudaEvent_t b = nullptr;
-    KLaunch(Ctx& c_, const char* kernel) : c(c_) {
-        if (c.profiling) {
-            cudaEvent_t a;
-            MSG_CUDA(cudaEventCreate(&a));
-            MSG_CUDA(cudaEventCreate(&b));
-            MSG_CUDA(cudaEventRecord(a, c.stream));
-            c.prof.push_back(Ctx::ProfRec{c.stage, kernel, a, b, host_now_us()});
-        }
+    if (c.profiling) {
+        cudaEvent_t a;
+        MSG_CUDA(cudaEventCreate(&a));
+        MSG_CUDA(cudaEventCreate(&b));
+        MSG_CUDA(cudaEventRecord(a, c.stream));
+        c.prof.push_back(Ctx::ProfRec{c.stage, name, a, b, host_now_us()});
     }
-    ~KLaunch() {
-        c.launches++;
-        if (b) cudaEventRecord(b, c.stream);
-    }
-};
+    kernel<<<grid, block, smem, c.stream>>>(std::forward<A>(args)...);
+    c.launches++;
+    if (b) cudaEventRecord(b, c.stream);
+    MSG_CUDA(cudaGetLastError());
+}
 // Names the stage of the launches inside it: the per-launch profile of bench.py groups by it, and it is an NVTX range named
 // after the reference's tracing spans (SURVEY 5: "stark/stage1_commit" ... are spans of src/prover.rs; the stages here are
 // the device-side pieces of those spans: lde, merkle, stage2, quotient, open, fri, transcript, exchange), so that

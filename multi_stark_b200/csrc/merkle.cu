@@ -412,27 +412,16 @@ __global__ void __launch_bounds__(128) k_b3_parent_level(const u32* in, u64 n_in
 void b3_hash_long(Ctx& c, const uint8_t* data_dev, u64 len, uint8_t* out_dev) {
     MSG_REQUIRE(len > 1024, "b3_hash_long: message fits one chunk");
     u64 nchunks = (len + 1023) / 1024;
-    u32* a = (u32*)c.alloc(nchunks * 32);
-    u32* b = (u32*)c.alloc((nchunks + 1) / 2 * 32);
-    {
-        KLaunch kl(c, "k_b3_chunk_cvs");
-        k_b3_chunk_cvs<<<(unsigned)((nchunks + 127) / 128), 128, 0, c.stream>>>((const uint4*)data_dev, len, nchunks, a);
-    }
-    MSG_CUDA(cudaGetLastError());
+    DevBuf a(c, nchunks * 32), b(c, (nchunks + 1) / 2 * 32);
+    launch(c, "k_b3_chunk_cvs", k_b3_chunk_cvs, (unsigned)((nchunks + 127) / 128), 128, 0, (const uint4*)data_dev, len, nchunks, (u32*)a.p);
     u64 n = nchunks;
     while (n > 1) {
         u64 n_out = (n + 1) / 2;
-        {
-            KLaunch kl(c, "k_b3_parent_level");
-            k_b3_parent_level<<<(unsigned)((n_out + 127) / 128), 128, 0, c.stream>>>(a, n, b);
-        }
-        MSG_CUDA(cudaGetLastError());
+        launch(c, "k_b3_parent_level", k_b3_parent_level, (unsigned)((n_out + 127) / 128), 128, 0, (const u32*)a.p, n, (u32*)b.p);
         std::swap(a, b);
         n = n_out;
     }
-    MSG_CUDA(cudaMemcpyAsync(out_dev, a, 32, cudaMemcpyDeviceToDevice, c.stream));
-    c.free(a);
-    c.free(b);
+    MSG_CUDA(cudaMemcpyAsync(out_dev, a.p, 32, cudaMemcpyDeviceToDevice, c.stream));
 }
 
 __global__ void __launch_bounds__(256) k_check_canonical(const u64* v, u64 n, u32* flag) {
@@ -452,19 +441,11 @@ __global__ void __launch_bounds__(256) k_canonicalize(u64* v, u64 n) {
 void canonicalize(Ctx& c, u64* v, u64 n) {
     if (n == 0) return;
     u64 blocks = std::min<u64>((n + 255) / 256, (u64)c.sm_count * 8);
-    {
-        KLaunch kl(c, "k_canonicalize");
-        k_canonicalize<<<(unsigned)std::max<u64>(blocks, 1), 256, 0, c.stream>>>(v, n);
-    }
-    MSG_CUDA(cudaGetLastError());
+    launch(c, "k_canonicalize", k_canonicalize, (unsigned)std::max<u64>(blocks, 1), 256, 0, v, n);
 }
 void check_canonical(Ctx& c, const u64* v, u64 n, u32* flag_dev) {
     u64 blocks = std::min<u64>((n + 255) / 256, (u64)c.sm_count * 8);
-    {
-        KLaunch kl(c, "k_check_canonical");
-        k_check_canonical<<<(unsigned)std::max<u64>(blocks, 1), 256, 0, c.stream>>>(v, n, flag_dev);
-    }
-    MSG_CUDA(cudaGetLastError());
+    launch(c, "k_check_canonical", k_check_canonical, (unsigned)std::max<u64>(blocks, 1), 256, 0, v, n, flag_dev);
 }
 
 // dst[r][col0_b + c] = blocks[b][r][c] (the fallback of the assembling leaf kernels)
@@ -518,9 +499,7 @@ void b3_hash_rows(Ctx& c, const std::vector<MatRef>& mats, uint8_t* digests, con
         gb.rows = height;
         gb.dst = t.dst;
         if (w == 0) return;
-        KLaunch kl(c, "k_gather_blocks");
-        k_gather_blocks<<<(unsigned)std::min<u64>((height * w + 255) / 256, (u64)c.sm_count * 16), 256, 0, c.stream>>>(gb);
-        MSG_CUDA(cudaGetLastError());
+        launch(c, "k_gather_blocks", k_gather_blocks, (unsigned)std::min<u64>((height * w + 255) / 256, (u64)c.sm_count * 16), 256, 0, gb);
     };
     u32 total_words = (u32)words;
     u32 pitch = total_words | 1u;
@@ -538,46 +517,37 @@ void b3_hash_rows(Ctx& c, const std::vector<MatRef>& mats, uint8_t* digests, con
         else gather(t);
     }
     LeafList d_mats{};
-    LeafMat* d_ext = nullptr;
+    DevBuf d_ext;
     if (lm.size() <= (size_t)kInlineMats) {
         for (size_t k = 0; k < lm.size(); k++) d_mats.inl[k] = lm[k];
     } else {
-        d_ext = (LeafMat*)c.alloc(lm.size() * sizeof(LeafMat));
-        MSG_CUDA(cudaMemcpyAsync(d_ext, lm.data(), lm.size() * sizeof(LeafMat), cudaMemcpyHostToDevice, c.stream));
-        d_mats.ext = d_ext;
+        d_ext = DevBuf(c, lm.size() * sizeof(LeafMat));
+        // the host vector `lm` is copied with a pageable-memory async copy, which is staged before return
+        MSG_CUDA(cudaMemcpyAsync(d_ext.p, lm.data(), lm.size() * sizeof(LeafMat), cudaMemcpyHostToDevice, c.stream));
+        d_mats.ext = (const LeafMat*)d_ext.p;
     }
     if (use_stream) {
         u64 blocks = (height + kLeafThreads - 1) / kLeafThreads;
-        KLaunch kl(c, "k_hash_rows_stream");
-        k_hash_rows_stream<<<(unsigned)blocks, kLeafThreads, 0, c.stream>>>(d_mats, (u32)lm.size(), height, total_words, (u32*)digests, asmb);
+        launch(c, "k_hash_rows_stream", k_hash_rows_stream, (unsigned)blocks, kLeafThreads, 0, d_mats, (u32)lm.size(), height, total_words,
+               (u32*)digests, asmb);
     } else if (use_staged) {
         if (rows > 32) rows = rows / 32 * 32;
         if (rows == 0) rows = 1;
         ensure_max_smem(k_hash_rows_staged, (int)budget);
         u64 blocks = (height + rows - 1) / rows;
-        KLaunch kl(c, "k_hash_rows_staged");
-        k_hash_rows_staged<<<(unsigned)blocks, kLeafThreads, (size_t)rows * pitch * 4, c.stream>>>(
-            d_mats, (u32)lm.size(), height, total_words, pitch, rows, (u32*)digests, asmb);
+        launch(c, "k_hash_rows_staged", k_hash_rows_staged, (unsigned)blocks, kLeafThreads, (size_t)rows * pitch * 4, d_mats, (u32)lm.size(),
+               height, total_words, pitch, rows, (u32*)digests, asmb);
     } else {
         u64 blocks = (height + kLeafThreads - 1) / kLeafThreads;
-        KLaunch kl(c, "k_hash_rows_direct");
-        k_hash_rows_direct<<<(unsigned)blocks, kLeafThreads, 0, c.stream>>>(d_mats, (u32)lm.size(), height, total_words,
-                                                                            (u32*)digests);
+        launch(c, "k_hash_rows_direct", k_hash_rows_direct, (unsigned)blocks, kLeafThreads, 0, d_mats, (u32)lm.size(), height, total_words,
+               (u32*)digests);
     }
-    MSG_CUDA(cudaGetLastError());
-    // the host vector `lm` was copied with a pageable-memory async copy, which is staged before return
-    if (d_ext) c.free(d_ext);
 }
 
 void b3_compress_layer(Ctx& c, const uint8_t* prev, const uint8_t* inject, uint8_t* next, u64 next_len) {
     if (next_len == 0) return;
     u64 blocks = (next_len + 255) / 256;
-    {
-        KLaunch kl(c, "k_compress_layer");
-        k_compress_layer<<<(unsigned)blocks, 256, 0, c.stream>>>((const uint4*)prev, (const uint4*)inject, (uint4*)next,
-                                                                 next_len);
-    }
-    MSG_CUDA(cudaGetLastError());
+    launch(c, "k_compress_layer", k_compress_layer, (unsigned)blocks, 256, 0, (const uint4*)prev, (const uint4*)inject, (uint4*)next, next_len);
 }
 
 // Reduces the layer `in` (len digests) by `levels` levels. out[l] / inject[l]: output layer l+1 and its injected digests.
@@ -593,19 +563,11 @@ void b3_merkle_subtrees(Ctx& c, const uint8_t* in, u64 len, u32 levels, uint8_t*
     size_t smem = ((size_t)1 << levels) * 24;  // chunk/2 + chunk/4 digests
     ensure_max_smem(k_merkle_subtree, 24 << kMaxFusedLevels);
     u32 threads = (u32)std::min<u64>(256, std::max<u64>(32, (1ull << levels) / 2));
-    {
-        KLaunch kl(c, "k_merkle_subtree");
-        k_merkle_subtree<<<(unsigned)(len >> levels), threads, smem, c.stream>>>(p);
-    }
-    MSG_CUDA(cudaGetLastError());
+    launch(c, "k_merkle_subtree", k_merkle_subtree, (unsigned)(len >> levels), threads, smem, p);
 }
 
 void b3_compress_raw_dev(Ctx& c, const u32* st, const u32* msg, u32* out) {
-    {
-        KLaunch kl(c, "k_compress_raw");
-        k_compress_raw<<<1, 1, 0, c.stream>>>(st, msg, out);
-    }
-    MSG_CUDA(cudaGetLastError());
+    launch(c, "k_compress_raw", k_compress_raw, 1, 1, 0, st, msg, out);
 }
 
 }  // namespace msg

@@ -17,8 +17,9 @@ struct OpenMat {
 
 // Stable sort of the matrices by height (descending) and the leaf digests of every height class:
 // digest[i] = BLAKE3(row i of the class's matrices, concatenated in commit order). `first_out`, when given, receives the
-// tallest class (layer 0 of a tree); the other classes get their own buffers. Returns (height, digests), tallest first.
-static std::vector<std::pair<u64, uint8_t*>> hash_classes(Ctx& c, msgpu_pdata* pd, uint8_t* first_out) {
+// tallest class (layer 0 of a tree); the other classes get their own buffers. Returns (height, digests), tallest first; the
+// first entry's buffer is empty when it went to `first_out`.
+static std::vector<std::pair<u64, DevBuf>> hash_classes(Ctx& c, msgpu_pdata* pd, uint8_t* first_out) {
     std::vector<size_t> order(pd->mats.size());
     std::iota(order.begin(), order.end(), 0);
     std::stable_sort(order.begin(), order.end(), [&](size_t a, size_t b) { return pd->mats[a].height > pd->mats[b].height; });
@@ -29,7 +30,7 @@ static std::vector<std::pair<u64, uint8_t*>> hash_classes(Ctx& c, msgpu_pdata* p
         pd->total_width += m.width;
         pd->max_height = std::max(pd->max_height, m.height);
     }
-    std::vector<std::pair<u64, uint8_t*>> classes;
+    std::vector<std::pair<u64, DevBuf>> classes;
     size_t pos = 0;
     while (pos < order.size()) {
         u64 h = pd->mats[order[pos]].height;
@@ -49,15 +50,10 @@ static std::vector<std::pair<u64, uint8_t*>> hash_classes(Ctx& c, msgpu_pdata* p
             }
             MSG_REQUIRE(w == m.width, "commit: the column blocks of a matrix do not add up to its width");
         }
-        uint8_t* out = (classes.empty() && first_out) ? first_out : (uint8_t*)c.alloc(h * 32);
-        classes.push_back({h, out});
-        try {
-            b3_hash_rows(c, group, out, assemble);
-        } catch (...) {
-            for (auto& cl : classes)
-                if (cl.second != first_out) c.free(cl.second);
-            throw;
-        }
+        DevBuf buf = (classes.empty() && first_out) ? DevBuf() : DevBuf(c, h * 32);
+        uint8_t* out = buf ? buf.bytes() : first_out;
+        classes.emplace_back(h, std::move(buf));
+        b3_hash_rows(c, group, out, assemble);
     }
     for (auto& m : pd->mats) m.blocks.clear();  // every matrix is materialised now
     return classes;
@@ -65,7 +61,7 @@ static std::vector<std::pair<u64, uint8_t*>> hash_classes(Ctx& c, msgpu_pdata* p
 
 void mmcs_layout_layers(Ctx& c, msgpu_pdata* pd, u64 max_h) {
     pd->max_height = max_h;
-    pd->digests = (uint8_t*)c.alloc((2 * max_h - 1) * 32);
+    pd->digests = DevBuf(c, (2 * max_h - 1) * 32);
     pd->layer_off.clear();
     pd->layer_len.clear();
     u64 off = 0;
@@ -93,17 +89,17 @@ static void build_nodes(Ctx& c, msgpu_pdata* pd, const std::vector<std::pair<u64
         uint8_t* outs[16];
         const uint8_t* injs[16];
         for (u32 k = 0; k < levels; k++) {
-            outs[k] = pd->digests + pd->layer_off[l + 1 + k] * 32;
+            outs[k] = pd->digests.bytes() + pd->layer_off[l + 1 + k] * 32;
             injs[k] = inj[l + 1 + k];
         }
-        b3_merkle_subtrees(c, pd->digests + pd->layer_off[l] * 32, len, levels, outs, injs);
+        b3_merkle_subtrees(c, pd->digests.bytes() + pd->layer_off[l] * 32, len, levels, outs, injs);
         l += levels;
     }
 }
 
 void mmcs_build(Ctx& c, msgpu_pdata* pd) {
     mmcs_build_async(c, pd);
-    MSG_CUDA(cudaMemcpyAsync(pd->root, pd->digests + pd->layer_off.back() * 32, 32, cudaMemcpyDeviceToHost, c.stream));
+    MSG_CUDA(cudaMemcpyAsync(pd->root, pd->digests.bytes() + pd->layer_off.back() * 32, 32, cudaMemcpyDeviceToHost, c.stream));
     c.sync();
 }
 
@@ -114,15 +110,10 @@ void mmcs_build_async(Ctx& c, msgpu_pdata* pd) {
     for (auto& m : pd->mats) max_h = std::max(max_h, m.height);
     MSG_REQUIRE(is_pow2(max_h), "commit: matrix heights must be powers of two");
     mmcs_layout_layers(c, pd, max_h);
-    std::vector<std::pair<u64, uint8_t*>> cls = hash_classes(c, pd, pd->digests);
-    std::vector<std::pair<u64, const uint8_t*>> view(cls.begin(), cls.end());
-    try {
-        build_nodes(c, pd, view);
-    } catch (...) {
-        for (size_t k = 1; k < cls.size(); k++) c.free(cls[k].second);
-        throw;
-    }
-    for (size_t k = 1; k < cls.size(); k++) c.free(cls[k].second);
+    std::vector<std::pair<u64, DevBuf>> cls = hash_classes(c, pd, pd->digests.bytes());
+    std::vector<std::pair<u64, const uint8_t*>> view;
+    for (auto& cl : cls) view.push_back({cl.first, cl.second ? cl.second.bytes() : pd->digests.bytes()});
+    build_nodes(c, pd, view);
 }
 
 void mmcs_build_local(Ctx& c, msgpu_pdata* pd) {
@@ -139,9 +130,9 @@ void mmcs_build_from_classes(Ctx& c, msgpu_pdata* pd, const std::vector<std::pai
     MSG_REQUIRE(!classes.empty() && is_pow2(classes[0].first), "tree: no leaf digests given");
     mmcs_layout_layers(c, pd, classes[0].first);
     pd->total_width = 0;
-    MSG_CUDA(cudaMemcpyAsync(pd->digests, classes[0].second, classes[0].first * 32, cudaMemcpyDeviceToDevice, c.stream));
+    MSG_CUDA(cudaMemcpyAsync(pd->digests.p, classes[0].second, classes[0].first * 32, cudaMemcpyDeviceToDevice, c.stream));
     build_nodes(c, pd, classes);
-    MSG_CUDA(cudaMemcpyAsync(pd->root, pd->digests + pd->layer_off.back() * 32, 32, cudaMemcpyDeviceToHost, c.stream));
+    MSG_CUDA(cudaMemcpyAsync(pd->root, pd->digests.bytes() + pd->layer_off.back() * 32, 32, cudaMemcpyDeviceToHost, c.stream));
     c.sync();
 }
 
@@ -190,7 +181,8 @@ void mmcs_open_multi(Ctx& c, const msgpu_pdata* const* pds, const u32* shifts, u
     }
     const size_t sz_t = n_trees * sizeof(MultiTree), sz_idx = n_idx * 8;
     std::vector<uint8_t> host(sz_t + sz_idx + desc_bytes);
-    uint8_t* d_in = (uint8_t*)c.alloc(host.size());
+    DevBuf in_buf(c, host.size());
+    uint8_t* d_in = in_buf.bytes();
     size_t off = sz_t + sz_idx;
     for (u64 k = 0; k < n_trees; k++) {
         const msgpu_pdata* pd = pds[k];
@@ -208,7 +200,7 @@ void mmcs_open_multi(Ctx& c, const msgpu_pdata* const* pds, const u32* shifts, u
         t.layer_off = (const u64*)(d_in + off);
         if (!pd->layer_off.empty()) memcpy(host.data() + off, pd->layer_off.data(), pd->layer_off.size() * 8);
         off += pd->layer_off.size() * 8;
-        t.digests = (const uint4*)pd->digests;
+        t.digests = (const uint4*)pd->digests.p;
         t.nmats = (u32)pd->mats.size();
         t.shift = shifts[k];
         t.depth = depth;
@@ -220,21 +212,13 @@ void mmcs_open_multi(Ctx& c, const msgpu_pdata* const* pds, const u32* shifts, u
     }
     memcpy(host.data(), mt.data(), sz_t);
     memcpy(host.data() + sz_t, indices_host, sz_idx);
-    u64* d_open = (u64*)c.alloc(std::max<u64>(opened_total * 8, 8));
-    uint4* d_proof = (uint4*)c.alloc(std::max<u64>(proof_total * 32, 32));
+    DevBuf d_open(c, std::max<u64>(opened_total * 8, 8)), d_proof(c, std::max<u64>(proof_total * 32, 32));
     MSG_CUDA(cudaMemcpyAsync(d_in, host.data(), host.size(), cudaMemcpyHostToDevice, c.stream));
-    {
-        KLaunch kl(c, "k_open_multi");
-        k_open_multi<<<dim3((unsigned)n_idx, (unsigned)n_trees), 128, 0, c.stream>>>((const MultiTree*)d_in, (const u64*)(d_in + sz_t), d_open,
-                                                                                      d_proof);
-    }
-    MSG_CUDA(cudaGetLastError());
-    if (opened_total) MSG_CUDA(cudaMemcpyAsync(opened_host, d_open, opened_total * 8, cudaMemcpyDeviceToHost, c.stream));
-    if (proof_total) MSG_CUDA(cudaMemcpyAsync(proof_host, d_proof, proof_total * 32, cudaMemcpyDeviceToHost, c.stream));
+    launch(c, "k_open_multi", k_open_multi, dim3((unsigned)n_idx, (unsigned)n_trees), 128, 0, (const MultiTree*)d_in, (const u64*)(d_in + sz_t),
+           d_open.u(), (uint4*)d_proof.p);
+    if (opened_total) MSG_CUDA(cudaMemcpyAsync(opened_host, d_open.p, opened_total * 8, cudaMemcpyDeviceToHost, c.stream));
+    if (proof_total) MSG_CUDA(cudaMemcpyAsync(proof_host, d_proof.p, proof_total * 32, cudaMemcpyDeviceToHost, c.stream));
     c.sync();
-    c.free(d_in);
-    c.free(d_open);
-    c.free(d_proof);
 }
 
 void mmcs_open_batch(Ctx& c, const msgpu_pdata* pd, const u64* indices_host, u64 n_idx, u64* opened_host,
@@ -300,9 +284,7 @@ void pack_column_blocks(Ctx& c, const u64* src, u64 rows, u64 width, const std::
     MSG_REQUIRE(c1.back() == width, "pack_column_blocks: blocks must cover every column");
     pp.col0[c0.size()] = (u32)width;
     if (rows * width == 0) return;
-    KLaunch kl(c, "k_pack_columns");
-    k_pack_columns<<<(unsigned)std::min<u64>((rows * width + 255) / 256, (u64)c.sm_count * 16), 256, 0, c.stream>>>(pp);
-    MSG_CUDA(cudaGetLastError());
+    launch(c, "k_pack_columns", k_pack_columns, (unsigned)std::min<u64>((rows * width + 255) / 256, (u64)c.sm_count * 16), 256, 0, pp);
 }
 void interleave_column_blocks(Ctx& c, const u64* src, u64 rows, const std::vector<u64>& widths, u64* dst) {
     MSG_REQUIRE(!widths.empty() && widths.size() <= (size_t)kMaxBlocks, "interleave_column_blocks: 1..16 blocks");
@@ -318,9 +300,7 @@ void interleave_column_blocks(Ctx& c, const u64* src, u64 rows, const std::vecto
     }
     ip.col0[widths.size()] = (u32)W;
     if (rows * W == 0) return;
-    KLaunch kl(c, "k_interleave_columns");
-    k_interleave_columns<<<(unsigned)std::min<u64>((rows * W + 255) / 256, (u64)c.sm_count * 16), 256, 0, c.stream>>>(ip);
-    MSG_CUDA(cudaGetLastError());
+    launch(c, "k_interleave_columns", k_interleave_columns, (unsigned)std::min<u64>((rows * W + 255) / 256, (u64)c.sm_count * 16), 256, 0, ip);
 }
 
 void mmcs_from_parts(Ctx& c, msgpu_pdata* pd, const std::vector<const u64*>& blocks, const std::vector<u64>& widths, u64 height,
@@ -339,16 +319,13 @@ void mmcs_from_parts(Ctx& c, msgpu_pdata* pd, const std::vector<const u64*>& blo
     ip.col0[blocks.size()] = (u32)W;
     ip.n_blocks = (u32)blocks.size();
     ip.rows = height;
-    u64* lde = (u64*)c.alloc(height * W * 8);
-    pd->mats.push_back(msgpu_pdata::Mat{lde, height, W, true});
+    pd->mats.push_back(msgpu_pdata::Mat::alloc(c, height, W));
     pd->total_width = W;
-    ip.out = lde;
+    ip.out = pd->mats.back().ptr;
     {
         StageScope ss(c, "lde");
-        KLaunch kl(c, "k_interleave_columns");
-        k_interleave_columns<<<(unsigned)std::min<u64>((height * W + 255) / 256, (u64)c.sm_count * 16), 256, 0, c.stream>>>(ip);
+        launch(c, "k_interleave_columns", k_interleave_columns, (unsigned)std::min<u64>((height * W + 255) / 256, (u64)c.sm_count * 16), 256, 0, ip);
     }
-    MSG_CUDA(cudaGetLastError());
     // digest layers: layer l of the tree is the concatenation of the parts' layer l while a part still has one
     StageScope ss(c, "merkle");
     mmcs_layout_layers(c, pd, height);
@@ -359,7 +336,7 @@ void mmcs_from_parts(Ctx& c, msgpu_pdata* pd, const std::vector<const u64*>& blo
         u64 off = 0;
         for (u32 l = 0; l < part_layers; l++) {
             const u64 len = shard >> l;
-            MSG_CUDA(cudaMemcpyAsync(pd->digests + (pd->layer_off[l] + p * len) * 32, part_digests[p] + off * 32, len * 32,
+            MSG_CUDA(cudaMemcpyAsync(pd->digests.bytes() + (pd->layer_off[l] + p * len) * 32, part_digests[p] + off * 32, len * 32,
                                      cudaMemcpyDeviceToDevice, c.stream));
             off += len;
         }
@@ -369,23 +346,13 @@ void mmcs_from_parts(Ctx& c, msgpu_pdata* pd, const std::vector<const u64*>& blo
         uint8_t* outs[16];
         const uint8_t* injs[16];
         for (u32 k = 0; k < levels; k++) {
-            outs[k] = pd->digests + pd->layer_off[l0 + 1 + k] * 32;
+            outs[k] = pd->digests.bytes() + pd->layer_off[l0 + 1 + k] * 32;
             injs[k] = nullptr;
         }
-        b3_merkle_subtrees(c, pd->digests + pd->layer_off[l0] * 32, n_parts, levels, outs, injs);
+        b3_merkle_subtrees(c, pd->digests.bytes() + pd->layer_off[l0] * 32, n_parts, levels, outs, injs);
     }
-    MSG_CUDA(cudaMemcpyAsync(pd->root, pd->digests + pd->layer_off.back() * 32, 32, cudaMemcpyDeviceToHost, c.stream));
+    MSG_CUDA(cudaMemcpyAsync(pd->root, pd->digests.bytes() + pd->layer_off.back() * 32, 32, cudaMemcpyDeviceToHost, c.stream));
     c.sync();
-}
-
-void pdata_destroy(msgpu_pdata* pd) {
-    if (!pd) return;
-    Ctx& c = *pd->ctx;
-    for (auto& m : pd->mats)
-        if (m.owned && m.ptr) c.free(m.ptr);
-    if (pd->digests) c.free(pd->digests);
-    for (auto& cl : pd->class_leaves) c.free(cl.second);
-    delete pd;
 }
 
 }  // namespace msg

@@ -7,14 +7,19 @@ struct msgpu_pdata {
     struct Mat {
         u64* ptr;
         u64 height, width;
-        bool owned;
+        msg::DevBuf own;  // holds `ptr` when this prover data owns the matrix; empty when it borrows it
         // not empty: `ptr` is still to be written -- the rows are read from these column blocks (pointer, width; dense
         // height x width_b, in column order, possibly in a peer GPU's memory) by the leaf-hash pass, which writes ptr as it goes
         std::vector<std::pair<const u64*, u64>> blocks;
+        // a new height x width matrix in an arena block of its own
+        static Mat alloc(msg::Ctx& c, u64 height, u64 width) {
+            msg::DevBuf b(c, height * width * 8);
+            u64* p = b.u();
+            return Mat{p, height, width, std::move(b), {}};
+        }
     };
-    msg::Ctx* ctx = nullptr;
     std::vector<Mat> mats;           // original (commit) order
-    uint8_t* digests = nullptr;      // all layers back to back
+    msg::DevBuf digests;             // all layers back to back
     std::vector<u64> layer_off;      // offset (in digests) of each layer
     std::vector<u64> layer_len;      // layer 0 = leaf digests of the tallest matrices
     u64 max_height = 0;
@@ -23,7 +28,7 @@ struct msgpu_pdata {
     // Sharded commitments (one proof over several GPUs): a LOCAL part holds this rank's matrices and, per LDE height
     // class, the leaf digests of its rows (no tree: digests == nullptr); the TREE part on the tree owner holds the digest
     // layers built from every rank's class digests (no matrices).
-    std::vector<std::pair<u64, uint8_t*>> class_leaves;  // (LDE height, 32 * height bytes), tallest first
+    std::vector<std::pair<u64, msg::DevBuf>> class_leaves;  // (LDE height, 32 * height bytes), tallest first
 };
 
 namespace msg {
@@ -49,5 +54,4 @@ void mmcs_from_parts(Ctx& c, msgpu_pdata* pd, const std::vector<const u64*>& blo
 // row block (rows x width) -> column blocks [c0[b], c1[b]) as contiguous matrices back to back in dst, and the inverse
 void pack_column_blocks(Ctx& c, const u64* src, u64 rows, u64 width, const std::vector<u64>& c0, const std::vector<u64>& c1, u64* dst);
 void interleave_column_blocks(Ctx& c, const u64* src, u64 rows, const std::vector<u64>& widths, u64* dst);
-void pdata_destroy(msgpu_pdata* pd);
 }  // namespace msg

@@ -474,26 +474,22 @@ static u32 tile_threads(u32 log_t) {
 }
 
 template <int TB>
-static void launch_strided_tb(const StridedParams& p, bool inverse, u64 blocks, cudaStream_t st) {
-    if (inverse) {
-        ensure_max_smem(k_ntt_strided<TB, true>, (int)tile_smem(kMaxLogT));
-        k_ntt_strided<TB, true><<<(unsigned)blocks, tile_threads(TB), tile_smem(TB), st>>>(p);
-    } else {
-        ensure_max_smem(k_ntt_strided<TB, false>, (int)tile_smem(kMaxLogT));
-        k_ntt_strided<TB, false><<<(unsigned)blocks, tile_threads(TB), tile_smem(TB), st>>>(p);
-    }
+static void launch_strided_tb(Ctx& c, const StridedParams& p, bool inverse, u64 blocks) {
+    auto* k = inverse ? k_ntt_strided<TB, true> : k_ntt_strided<TB, false>;
+    ensure_max_smem(k, (int)tile_smem(kMaxLogT));
+    launch(c, "k_ntt_strided", k, (unsigned)blocks, tile_threads(TB), tile_smem(TB), p);
 }
 template <int TB>
-static void launch_block_tb(const BlockParams& p, dim3 grid, cudaStream_t st) {
+static void launch_block_tb(Ctx& c, const BlockParams& p, dim3 grid) {
     ensure_max_smem(k_ntt_block<TB>, (int)tile_smem(kMaxLogT));
-    k_ntt_block<TB><<<grid, tile_threads(TB), tile_smem(TB), st>>>(p);
+    launch(c, "k_ntt_block", k_ntt_block<TB>, grid, tile_threads(TB), tile_smem(TB), p);
 }
 
 static size_t mid_smem(u32 log_t) { return (size_t)(1u << log_t) * kXt * sizeof(u64) * (log_t <= 4 ? 1 : 2); }
 template <int TB>
-static void launch_mid_tb(const MidParams& p, unsigned blocks, cudaStream_t st) {
+static void launch_mid_tb(Ctx& c, const MidParams& p, unsigned blocks) {
     ensure_max_smem(k_lde_mid<TB>, (int)mid_smem(kMaxLogT));
-    k_lde_mid<TB><<<blocks, tile_threads(TB), mid_smem(TB), st>>>(p);
+    launch(c, "k_lde_mid", k_lde_mid<TB>, blocks, tile_threads(TB), mid_smem(TB), p);
 }
 
 #define MSG_TB_SWITCH(tb, CALL)                               \
@@ -515,49 +511,37 @@ static void launch_mid_tb(const MidParams& p, unsigned blocks, cudaStream_t st) 
 static const u64* twp_table(Ctx& c, u32 log_big, u32 tb, bool inverse) {
     auto key = std::make_tuple(0u, log_big, tb, (u64)inverse);
     auto it = c.ntt_tables.find(key);
-    if (it != c.ntt_tables.end()) return it->second;
+    if (it != c.ntt_tables.end()) return it->second.get();
     msh::Fp g = msh::two_adic_generator(log_big);
     if (inverse) g = g.inverse();
     gl::PowTable tab = c.pow_table(g.v, 1, log_big).view();
     u64 total = 1ull << log_big;
-    u64* d;
-    MSG_CUDA(cudaMalloc(&d, total * 8));
-    c.owned.push_back(d);
-    k_fill_twp<<<(unsigned)std::min<u64>((total + 255) / 256, (u64)c.sm_count * 16), 256, 0, c.stream>>>(d, total, tb, tab);
-    MSG_CUDA(cudaGetLastError());
-    c.ntt_tables[key] = d;
-    return d;
+    CudaPtr<u64> d = cuda_malloc<u64>(total);
+    launch(c, "k_fill_twp", k_fill_twp, (unsigned)std::min<u64>((total + 255) / 256, (u64)c.sm_count * 16), 256, 0, d.get(), total, tb, tab);
+    return (c.ntt_tables[key] = std::move(d)).get();
 }
 // output twiddle table of the block pass: [b][s] = w_n^{b * s}
 static const u64* twb_table(Ctx& c, u32 log_n, u32 tb) {
     auto key = std::make_tuple(1u, log_n, tb, (u64)0);
     auto it = c.ntt_tables.find(key);
-    if (it != c.ntt_tables.end()) return it->second;
+    if (it != c.ntt_tables.end()) return it->second.get();
     gl::PowTable tab = c.pow_table(msh::two_adic_generator(log_n).v, 1, log_n).view();
     u64 total = 1ull << log_n;
-    u64* d;
-    MSG_CUDA(cudaMalloc(&d, total * 8));
-    c.owned.push_back(d);
-    k_fill_twb<<<(unsigned)std::min<u64>((total + 255) / 256, (u64)c.sm_count * 16), 256, 0, c.stream>>>(d, total, tb, tab);
-    MSG_CUDA(cudaGetLastError());
-    c.ntt_tables[key] = d;
-    return d;
+    CudaPtr<u64> d = cuda_malloc<u64>(total);
+    launch(c, "k_fill_twb", k_fill_twb, (unsigned)std::min<u64>((total + 255) / 256, (u64)c.sm_count * 16), 256, 0, d.get(), total, tb, tab);
+    return (c.ntt_tables[key] = std::move(d)).get();
 }
 // coset scales of the block pass: [beta][b][t] = (shift * w_{nB}^{rev(beta)})^{rev_tb(t) * S + b} / n
 static const u64* scale_table(Ctx& c, u32 log_n, u32 tb, u32 added_bits, u64 shift) {
     auto key = std::make_tuple(2u + (added_bits << 8), log_n, tb, shift);
     auto it = c.ntt_tables.find(key);
-    if (it != c.ntt_tables.end()) return it->second;
+    if (it != c.ntt_tables.end()) return it->second.get();
     const gl::PowTable* tabs = c.coset_tables(log_n, added_bits, shift);
     u64 n = 1ull << log_n, total = n << added_bits;
-    u64* d;
-    MSG_CUDA(cudaMalloc(&d, total * 8));
-    c.owned.push_back(d);
-    k_fill_scale<<<(unsigned)std::min<u64>((total + 255) / 256, (u64)c.sm_count * 16), 256, 0, c.stream>>>(d, n, tb, n >> tb, tabs,
-                                                                                                         1u << added_bits);
-    MSG_CUDA(cudaGetLastError());
-    c.ntt_tables[key] = d;
-    return d;
+    CudaPtr<u64> d = cuda_malloc<u64>(total);
+    launch(c, "k_fill_scale", k_fill_scale, (unsigned)std::min<u64>((total + 255) / 256, (u64)c.sm_count * 16), 256, 0, d.get(), n, tb, n >> tb,
+           tabs, 1u << added_bits);
+    return (c.ntt_tables[key] = std::move(d)).get();
 }
 
 // One DIF pass over bits [lo_bit, lo_bit + tb) of a size-2^log_m transform, for `count` transforms
@@ -566,7 +550,7 @@ static void launch_strided(Ctx& c, const u64* src, u64* dst, u32 log_m, u64 coun
     StridedParams p{};
     p.src = src;
     p.dst = dst;
-    p.tw = c.tw_full[inverse ? 1 : 0];
+    p.tw = c.tw_full[inverse ? 1 : 0].get();
     p.w = (u32)w;
     u64 S = 1ull << lo_bit;
     p.I = S * w;
@@ -574,11 +558,7 @@ static void launch_strided(Ctx& c, const u64* src, u64* dst, u32 log_m, u64 coun
     p.twp = lo_bit > 0 ? twp_table(c, lo_bit + tb, tb, inverse) : nullptr;
     u64 blocks = (p.a_total * p.I + kXt - 1) / kXt;
     MSG_REQUIRE(blocks < (1ull << 31), "ntt: grid too large");
-    {
-        KLaunch kl(c, "k_ntt_strided");
-        MSG_TB_SWITCH(tb, launch_strided_tb<TBV>(p, inverse, blocks, c.stream));
-    }
-    MSG_CUDA(cudaGetLastError());
+    MSG_TB_SWITCH(tb, launch_strided_tb<TBV>(c, p, inverse, blocks));
 }
 
 void ntt_dft_bitrev(Ctx& c, const u64* src, u64* dst, u64 n, u64 w, bool inverse, u64 batch) {
@@ -626,8 +606,8 @@ void ntt_coset_lde(Ctx& c, const u64* src, u64* dst, u64* tmp, u64 n, u64 w, u32
         MidParams p{};
         p.src = cur;
         p.dst = dst;
-        p.tw_inv = c.tw_full[1];
-        p.tw_fwd = c.tw_full[0];
+        p.tw_inv = c.tw_full[1].get();
+        p.tw_fwd = c.tw_full[0].get();
         p.scale = scale_table(c, log_n, tb, added_bits, shift);
         p.log_n = log_n;
         p.w = (u32)w;
@@ -637,11 +617,7 @@ void ntt_coset_lde(Ctx& c, const u64* src, u64* dst, u64* tmp, u64 n, u64 w, u32
         p.twb = p.S > 1 ? twb_table(c, log_n, tb) : nullptr;
         u64 blocks = (p.S * w + kXt - 1) / kXt;
         MSG_REQUIRE(blocks < (1ull << 31), "lde: grid too large");
-        {
-            KLaunch kl(c, "k_lde_mid");
-            MSG_TB_SWITCH(tb, launch_mid_tb<TBV>(p, (unsigned)blocks, c.stream));
-        }
-        MSG_CUDA(cudaGetLastError());
+        MSG_TB_SWITCH(tb, launch_mid_tb<TBV>(c, p, (unsigned)blocks));
     } else {
     // 1. inverse transform (unnormalised): coefficients in bit-reversed order
     ntt_dft_bitrev(c, src, tmp, n, w, true);
@@ -649,7 +625,7 @@ void ntt_coset_lde(Ctx& c, const u64* src, u64* dst, u64* tmp, u64 n, u64 w, u32
     BlockParams p{};
     p.src = tmp;
     p.dst = dst;
-    p.tw = c.tw_full[0];
+    p.tw = c.tw_full[0].get();
     p.scale = scale_table(c, log_n, tb, added_bits, shift);
     p.log_n = log_n;
     p.w = (u32)w;
@@ -659,11 +635,7 @@ void ntt_coset_lde(Ctx& c, const u64* src, u64* dst, u64* tmp, u64 n, u64 w, u32
     u64 blocks = (p.S * w + kXt - 1) / kXt;
     MSG_REQUIRE(blocks < (1ull << 31), "lde: grid too large");
     dim3 grid((unsigned)blocks, 1u << added_bits);
-    {
-        KLaunch kl(c, "k_ntt_block");
-        MSG_TB_SWITCH(tb, launch_block_tb<TBV>(p, grid, c.stream));
-    }
-    MSG_CUDA(cudaGetLastError());
+    MSG_TB_SWITCH(tb, launch_block_tb<TBV>(c, p, grid));
     }
     // 3. remaining forward passes: every block rev_T(k1) of S rows is an independent size-S DFT
     u32 log_s = log_n - tb;
@@ -686,11 +658,7 @@ void ntt_lde_from_coeffs(Ctx& c, const u64* src, u64* dst, u64 n, u64 w, u32 add
     const gl::PowTable* tabs = c.lde_coeff_tables(log_n, added_bits);
     u64 total = n * w;
     unsigned blocks = (unsigned)std::min<u64>((total + 255) / 256, (u64)c.sm_count * 16);
-    {
-        KLaunch kl(c, "k_scale_rows");
-        k_scale_rows<<<blocks, 256, 0, c.stream>>>(src, dst, n, w, tabs, 1u << added_bits);
-    }
-    MSG_CUDA(cudaGetLastError());
+    launch(c, "k_scale_rows", k_scale_rows, blocks, 256, 0, src, dst, n, w, tabs, 1u << added_bits);
     ntt_dft_bitrev(c, dst, dst, n, w, false, 1ull << added_bits);
 }
 
@@ -698,11 +666,7 @@ void ntt_bit_reverse_rows(Ctx& c, const u64* src, u64* dst, u64 n, u64 w) {
     if (n * w == 0) return;
     u64 total = n * w;
     unsigned blocks = (unsigned)std::min<u64>((total + 255) / 256, (u64)c.sm_count * 16);
-    {
-        KLaunch kl(c, "k_bitrev_rows_scale");
-        k_bitrev_rows_scale<<<blocks, 256, 0, c.stream>>>(src, dst, n, w, ilog2(n), 1);
-    }
-    MSG_CUDA(cudaGetLastError());
+    launch(c, "k_bitrev_rows_scale", k_bitrev_rows_scale, blocks, 256, 0, src, dst, n, w, ilog2(n), 1);
 }
 
 void ntt_idft_natural(Ctx& c, const u64* src, u64* dst, u64* tmp, u64 n, u64 w) {
@@ -710,17 +674,13 @@ void ntt_idft_natural(Ctx& c, const u64* src, u64* dst, u64* tmp, u64 n, u64 w) 
     ntt_dft_bitrev(c, src, tmp, n, w, true);
     u64 total = n * w;
     unsigned blocks = (unsigned)std::min<u64>((total + 255) / 256, (u64)c.sm_count * 16);
-    {
-        KLaunch kl(c, "k_bitrev_rows_scale");
-        k_bitrev_rows_scale<<<blocks, 256, 0, c.stream>>>(tmp, dst, n, w, ilog2(n), msh::Fp((msh::u64)n).inverse().v);
-    }
-    MSG_CUDA(cudaGetLastError());
+    launch(c, "k_bitrev_rows_scale", k_bitrev_rows_scale, blocks, 256, 0, tmp, dst, n, w, ilog2(n), msh::Fp((msh::u64)n).inverse().v);
 }
 
 // ------------------------------------------------------------------------------------------------
 // Tables
 // ------------------------------------------------------------------------------------------------
-DevPow Ctx::pow_table(u64 g, u64 cst, u32 bits) {
+const DevPow& Ctx::pow_table(u64 g, u64 cst, u32 bits) {
     auto key = std::make_tuple(g, cst, bits);
     auto it = pow_cache.find(key);
     if (it != pow_cache.end()) return it->second;
@@ -733,22 +693,17 @@ DevPow Ctx::pow_table(u64 g, u64 cst, u32 bits) {
     msh::Fp Gh = G.exp_power_of_2(t.h1);
     acc = msh::Fp::one();
     for (size_t i = 0; i < nhi; i++) { hi[i] = acc.v; acc *= Gh; }
-    MSG_CUDA(cudaMalloc(&t.lo, nlo * 8));
-    MSG_CUDA(cudaMalloc(&t.hi, nhi * 8));
-    owned.push_back(t.lo);
-    owned.push_back(t.hi);
-    MSG_CUDA(cudaMemcpyAsync(t.lo, lo.data(), nlo * 8, cudaMemcpyHostToDevice, stream));
-    MSG_CUDA(cudaMemcpyAsync(t.hi, hi.data(), nhi * 8, cudaMemcpyHostToDevice, stream));
+    t.lo = cuda_malloc<u64>(nlo);
+    t.hi = cuda_malloc<u64>(nhi);
+    MSG_CUDA(cudaMemcpyAsync(t.lo.get(), lo.data(), nlo * 8, cudaMemcpyHostToDevice, stream));
+    MSG_CUDA(cudaMemcpyAsync(t.hi.get(), hi.data(), nhi * 8, cudaMemcpyHostToDevice, stream));
     MSG_CUDA(cudaStreamSynchronize(stream));  // the host vectors die here
-    pow_cache[key] = t;
-    return t;
+    return pow_cache[key] = std::move(t);
 }
 
-static const gl::PowTable* upload_views(Ctx& c, const std::vector<gl::PowTable>& v) {
-    gl::PowTable* d;
-    MSG_CUDA(cudaMalloc(&d, v.size() * sizeof(gl::PowTable)));
-    c.owned.push_back(d);
-    MSG_CUDA(cudaMemcpyAsync(d, v.data(), v.size() * sizeof(gl::PowTable), cudaMemcpyHostToDevice, c.stream));
+static CudaPtr<gl::PowTable> upload_views(Ctx& c, const std::vector<gl::PowTable>& v) {
+    CudaPtr<gl::PowTable> d = cuda_malloc<gl::PowTable>(v.size());
+    MSG_CUDA(cudaMemcpyAsync(d.get(), v.data(), v.size() * sizeof(gl::PowTable), cudaMemcpyHostToDevice, c.stream));
     MSG_CUDA(cudaStreamSynchronize(c.stream));
     return d;
 }
@@ -757,7 +712,7 @@ static const gl::PowTable* upload_views(Ctx& c, const std::vector<gl::PowTable>&
 const gl::PowTable* Ctx::coset_tables(u32 log_n, u32 added_bits, u64 shift) {
     auto key = std::make_tuple(log_n, added_bits, shift);
     auto it = coset_cache.find(key);
-    if (it != coset_cache.end()) return it->second;
+    if (it != coset_cache.end()) return it->second.get();
     u32 B = 1u << added_bits;
     msh::Fp wN = msh::two_adic_generator(log_n + added_bits);
     msh::Fp ninv = msh::Fp((msh::u64)1 << log_n).inverse();
@@ -767,16 +722,15 @@ const gl::PowTable* Ctx::coset_tables(u32 log_n, u32 added_bits, u64 shift) {
         msh::Fp g = msh::Fp(shift) * wN.pow(s);
         views[beta] = pow_table(g.v, ninv.v, log_n).view();
     }
-    gl::PowTable* d = const_cast<gl::PowTable*>(upload_views(*this, views));
-    coset_cache[key] = d;
-    return d;
+    CudaPtr<gl::PowTable> d = upload_views(*this, views);
+    return (coset_cache[key] = std::move(d)).get();
 }
 
 // tab[beta](j) = w_{nB}^{rev_b(beta) * j}
 const gl::PowTable* Ctx::lde_coeff_tables(u32 log_n, u32 added_bits) {
     auto key = std::make_tuple(log_n, added_bits | 0x80000000u, (u64)0);
     auto it = coset_cache.find(key);
-    if (it != coset_cache.end()) return it->second;
+    if (it != coset_cache.end()) return it->second.get();
     u32 B = 1u << added_bits;
     msh::Fp wN = msh::two_adic_generator(log_n + added_bits);
     std::vector<gl::PowTable> views(B);
@@ -784,9 +738,8 @@ const gl::PowTable* Ctx::lde_coeff_tables(u32 log_n, u32 added_bits) {
         u32 s = (u32)msh::reverse_bits_len(beta, added_bits);
         views[beta] = pow_table(wN.pow(s).v, 1, log_n).view();
     }
-    gl::PowTable* d = const_cast<gl::PowTable*>(upload_views(*this, views));
-    coset_cache[key] = d;
-    return d;
+    CudaPtr<gl::PowTable> d = upload_views(*this, views);
+    return (coset_cache[key] = std::move(d)).get();
 }
 
 void ctx_init_tables(Ctx& c) {
@@ -801,12 +754,9 @@ void ctx_init_tables(Ctx& c) {
     msh::Fp w = msh::two_adic_generator(kTwLog), wi = w.inverse();
     msh::Fp a = msh::Fp::one(), b = msh::Fp::one();
     for (size_t i = 0; i < full; i++) { f[i] = a.v; inv[i] = b.v; a *= w; b *= wi; }
-    for (int d = 0; d < 2; d++) {
-        MSG_CUDA(cudaMalloc(&c.tw_full[d], full * 8));
-        c.owned.push_back(c.tw_full[d]);
-    }
-    MSG_CUDA(cudaMemcpyAsync(c.tw_full[0], f.data(), full * 8, cudaMemcpyHostToDevice, c.stream));
-    MSG_CUDA(cudaMemcpyAsync(c.tw_full[1], inv.data(), full * 8, cudaMemcpyHostToDevice, c.stream));
+    for (int d = 0; d < 2; d++) c.tw_full[d] = cuda_malloc<u64>(full);
+    MSG_CUDA(cudaMemcpyAsync(c.tw_full[0].get(), f.data(), full * 8, cudaMemcpyHostToDevice, c.stream));
+    MSG_CUDA(cudaMemcpyAsync(c.tw_full[1].get(), inv.data(), full * 8, cudaMemcpyHostToDevice, c.stream));
     MSG_CUDA(cudaStreamSynchronize(c.stream));
 }
 

@@ -43,11 +43,11 @@ static double run_peak(Ctx& c, u32* d_out) {
     cudaEvent_t a, b;
     MSG_CUDA(cudaEventCreate(&a));
     MSG_CUDA(cudaEventCreate(&b));
-    k_int_peak<MODE><<<blocks, 256, 0, c.stream>>>(d_out, 1u);  // warm-up
+    launch(c, "k_int_peak", k_int_peak<MODE>, blocks, 256, 0, d_out, 1u);  // warm-up
     float best = 1e30f;
     for (int rep = 0; rep < 5; rep++) {
         MSG_CUDA(cudaEventRecord(a, c.stream));
-        k_int_peak<MODE><<<blocks, 256, 0, c.stream>>>(d_out, 2u + rep);
+        launch(c, "k_int_peak", k_int_peak<MODE>, blocks, 256, 0, d_out, 2u + rep);
         MSG_CUDA(cudaEventRecord(b, c.stream));
         MSG_CUDA(cudaEventSynchronize(b));
         float ms = 0;
@@ -56,7 +56,6 @@ static double run_peak(Ctx& c, u32* d_out) {
     }
     cudaEventDestroy(a);
     cudaEventDestroy(b);
-    MSG_CUDA(cudaGetLastError());
     return per_thread * blocks * 256.0 / (best * 1e-3) / 1e9;
 }
 

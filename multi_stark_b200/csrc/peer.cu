@@ -247,9 +247,7 @@ int msgpu_peers_barrier(msgpu_peers* p) {
         Ctx& c = *p->c;
         p->epoch++;
         StageScope ss(c, "exchange");
-        KLaunch kl(c, "k_peer_barrier");
-        k_peer_barrier<<<1, 32, 0, c.stream>>>(p->flag_bases(), p->rank, p->world, p->epoch);
-        MSG_CUDA(cudaGetLastError());
+        launch(c, "k_peer_barrier", k_peer_barrier, 1, 32, 0, p->flag_bases(), p->rank, p->world, p->epoch);
     });
 }
 
@@ -265,10 +263,8 @@ int msgpu_peers_put(msgpu_peers* p, const void* src_dev, uint32_t seg, uint64_t 
         for (int e = 0; e < p->world; e++) b.p[e] = p->segs[seg].base[e];
         const u64 words = bytes / 8, total = words * (u64)p->world;
         StageScope ss(c, "exchange");
-        KLaunch kl(c, "k_peer_put");
-        k_peer_put<<<(unsigned)std::min<u64>((total + 255) / 256, (u64)c.sm_count * 8), 256, 0, c.stream>>>(b, (size_t)off, (const u64*)src_dev, words,
-                                                                                                        p->rank, p->world);
-        MSG_CUDA(cudaGetLastError());
+        launch(c, "k_peer_put", k_peer_put, (unsigned)std::min<u64>((total + 255) / 256, (u64)c.sm_count * 8), 256, 0, b, (size_t)off,
+               (const u64*)src_dev, words, p->rank, p->world);
     });
 }
 
@@ -281,9 +277,7 @@ int msgpu_peers_put_root(msgpu_peers* p, const uint8_t* root_dev, uint8_t** gath
         Ctx& c = *p->c;
         const size_t off = kRingOff + (size_t)(p->ring++ & 1u) * kMaxPeers * 32;
         StageScope ss(c, "exchange");
-        KLaunch kl(c, "k_peer_put");
-        k_peer_put<<<1, 64, 0, c.stream>>>(p->flag_bases(), off, (const u64*)root_dev, 4, p->rank, p->world);
-        MSG_CUDA(cudaGetLastError());
+        launch(c, "k_peer_put", k_peer_put, 1, 64, 0, p->flag_bases(), off, (const u64*)root_dev, 4, p->rank, p->world);
         *gathered_dev = (uint8_t*)(p->segs[0].base[p->rank] + off);
     });
 }
@@ -323,9 +317,7 @@ int msgpu_peers_pack_push(msgpu_peers* p, const uint64_t* src_dev, uint64_t rows
         }
         pp.col0[N] = (u32)width;
         StageScope ss(c, "exchange");
-        KLaunch kl(c, "k_peer_pack_push");
-        k_peer_pack_push<<<(unsigned)std::min<u64>((rows * width + 255) / 256, (u64)c.sm_count * 16), 256, 0, c.stream>>>(pp);
-        MSG_CUDA(cudaGetLastError());
+        launch(c, "k_peer_pack_push", k_peer_pack_push, (unsigned)std::min<u64>((rows * width + 255) / 256, (u64)c.sm_count * 16), 256, 0, pp);
     });
 }
 
@@ -353,9 +345,8 @@ int msgpu_peers_pull_interleave(msgpu_peers* p, uint32_t seg, uint64_t off, uint
         }
         pp.col0[N] = (u32)width;
         StageScope ss(c, "exchange");
-        KLaunch kl(c, "k_peer_pull_interleave");
-        k_peer_pull_interleave<<<(unsigned)std::min<u64>((rows * width + 255) / 256, (u64)c.sm_count * 16), 256, 0, c.stream>>>(pp);
-        MSG_CUDA(cudaGetLastError());
+        launch(c, "k_peer_pull_interleave", k_peer_pull_interleave, (unsigned)std::min<u64>((rows * width + 255) / 256, (u64)c.sm_count * 16), 256,
+               0, pp);
     });
 }
 

@@ -31,16 +31,14 @@ namespace msg {
 
 struct msgpu_program {
     msg::Ctx* ctx = nullptr;
-    msg::Instr* d_full = nullptr;
-    msg::Instr* d_prefix = nullptr;
+    msg::CudaPtr<msg::Instr> d_full, d_prefix;
     u32 n_full = 0, n_prefix = 0, slots_full = 0, slots_prefix = 0;
     u32 n_zeros = 0, n_lookups = 0, n_args = 0;
-    u32* d_zero_slots = nullptr;                       // full program
-    u32 *d_mult_full = nullptr, *d_args_full = nullptr;    // slots in the full program
-    u32 *d_mult_prefix = nullptr, *d_args_prefix = nullptr;  // slots in the prefix program
-    u32* d_arg_off = nullptr;
+    msg::CudaPtr<u32> d_zero_slots;                  // full program
+    msg::CudaPtr<u32> d_mult_full, d_args_full;      // slots in the full program
+    msg::CudaPtr<u32> d_mult_prefix, d_args_prefix;  // slots in the prefix program
+    msg::CudaPtr<u32> d_arg_off;
     u32 pre_width = 0, main_width = 0, stage2_width = 0;
-    std::vector<void*> owned;
 };
 
 namespace msg {
@@ -491,15 +489,13 @@ __global__ void __launch_bounds__(kScanThreads) k_claims(const u64* claims, u64 
 // host side
 // ------------------------------------------------------------------------------------------------
 template <class T>
-static T* upload_vec(Ctx& c, msgpu_program* prog, const std::vector<T>& v) {
-    T* d = nullptr;
-    MSG_CUDA(cudaMalloc(&d, std::max<size_t>(v.size(), 1) * sizeof(T)));
-    prog->owned.push_back(d);
-    if (!v.empty()) MSG_CUDA(cudaMemcpyAsync(d, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice, c.stream));
+static CudaPtr<T> upload_vec(Ctx& c, const std::vector<T>& v) {
+    CudaPtr<T> d = cuda_malloc<T>(std::max<size_t>(v.size(), 1));
+    if (!v.empty()) MSG_CUDA(cudaMemcpyAsync(d.get(), v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice, c.stream));
     return d;
 }
 
-static msgpu_program* program_create(Ctx& c, const msgpu_graph_desc& g) {
+static std::unique_ptr<msgpu_program> program_create(Ctx& c, const msgpu_graph_desc& g) {
     MSG_REQUIRE(g.lookup_prefix_len <= g.n_nodes, "program: lookup prefix longer than the node vector");
     MSG_REQUIRE(g.stage2_width == 2 * std::max<u32>(g.n_lookups, 1), "program: stage-2 width must be 2 * max(lookups, 1)");
     // k_lookup_messages has no stage-2 rows and no publics: lookup values are computed before either exists
@@ -525,38 +521,32 @@ static msgpu_program* program_create(Ctx& c, const msgpu_graph_desc& g) {
     if (getenv("MSGPU_TIMELINE"))
         fprintf(stderr, "[program] %u nodes, %u roots, %u lookups: full program %zu instructions / %u slots, lookup prefix %zu / %u\n", g.n_nodes,
                 g.n_zeros, g.n_lookups, full.code.size(), full.n_slots, prefix.code.size(), prefix.n_slots);
-    auto* prog = new msgpu_program();
+    auto prog = std::make_unique<msgpu_program>();
     prog->ctx = &c;
-    try {
-        prog->n_full = (u32)full.code.size();
-        prog->n_prefix = (u32)prefix.code.size();
-        prog->slots_full = full.n_slots;
-        prog->slots_prefix = prefix.n_slots;
-        prog->n_zeros = g.n_zeros;
-        prog->n_lookups = g.n_lookups;
-        prog->n_args = n_args;
-        prog->pre_width = g.pre_width;
-        prog->main_width = g.main_width;
-        prog->stage2_width = g.stage2_width;
-        prog->d_full = upload_vec(c, prog, full.code);
-        prog->d_prefix = upload_vec(c, prog, prefix.code);
-        std::vector<u32> zs, mf, af, mp, ap, off;
-        zs.assign(std::max<u32>(g.n_zeros, 1), 0);  // (the roots are folded by OP_ROOT instructions; kept for the layout)
-        for (u32 j = 0; j < g.n_lookups; j++) { mf.push_back(full.slot_of[g.lookup_mult[j]]); mp.push_back(prefix.slot_of[g.lookup_mult[j]]); }
-        for (u32 k = 0; k < n_args; k++) { af.push_back(full.slot_of[g.lookup_args[k]]); ap.push_back(prefix.slot_of[g.lookup_args[k]]); }
-        for (u32 j = 0; j <= g.n_lookups; j++) off.push_back(g.n_lookups ? g.lookup_arg_off[j] : 0);
-        prog->d_zero_slots = upload_vec(c, prog, zs);
-        prog->d_mult_full = upload_vec(c, prog, mf);
-        prog->d_args_full = upload_vec(c, prog, af);
-        prog->d_mult_prefix = upload_vec(c, prog, mp);
-        prog->d_args_prefix = upload_vec(c, prog, ap);
-        prog->d_arg_off = upload_vec(c, prog, off);
-        c.sync();
-    } catch (...) {
-        for (void* p : prog->owned) cudaFree(p);
-        delete prog;
-        throw;
-    }
+    prog->n_full = (u32)full.code.size();
+    prog->n_prefix = (u32)prefix.code.size();
+    prog->slots_full = full.n_slots;
+    prog->slots_prefix = prefix.n_slots;
+    prog->n_zeros = g.n_zeros;
+    prog->n_lookups = g.n_lookups;
+    prog->n_args = n_args;
+    prog->pre_width = g.pre_width;
+    prog->main_width = g.main_width;
+    prog->stage2_width = g.stage2_width;
+    prog->d_full = upload_vec(c, full.code);
+    prog->d_prefix = upload_vec(c, prefix.code);
+    std::vector<u32> zs, mf, af, mp, ap, off;
+    zs.assign(std::max<u32>(g.n_zeros, 1), 0);  // (the roots are folded by OP_ROOT instructions; kept for the layout)
+    for (u32 j = 0; j < g.n_lookups; j++) { mf.push_back(full.slot_of[g.lookup_mult[j]]); mp.push_back(prefix.slot_of[g.lookup_mult[j]]); }
+    for (u32 k = 0; k < n_args; k++) { af.push_back(full.slot_of[g.lookup_args[k]]); ap.push_back(prefix.slot_of[g.lookup_args[k]]); }
+    for (u32 j = 0; j <= g.n_lookups; j++) off.push_back(g.n_lookups ? g.lookup_arg_off[j] : 0);
+    prog->d_zero_slots = upload_vec(c, zs);
+    prog->d_mult_full = upload_vec(c, mf);
+    prog->d_args_full = upload_vec(c, af);
+    prog->d_mult_prefix = upload_vec(c, mp);
+    prog->d_args_prefix = upload_vec(c, ap);
+    prog->d_arg_off = upload_vec(c, off);
+    c.sync();
     return prog;
 }
 
@@ -566,7 +556,7 @@ static gl::PowTable coset_x_table(Ctx& c, u32 log_nq) {
     return c.pow_table(msh::two_adic_generator(log_nq).v, msh::GL_GENERATOR, log_nq).view();
 }
 
-static SelCache selectors(Ctx& c, u32 log_n, u32 log_q) {
+static const SelCache& selectors(Ctx& c, u32 log_n, u32 log_q) {
     auto& cache = c.sel_cache;
     auto key = std::make_pair(log_n, log_q);
     auto it = cache.find(key);
@@ -581,33 +571,24 @@ static SelCache selectors(Ctx& c, u32 log_n, u32 log_q) {
         izh[i] = z.inverse().v;
         acc *= wq;
     }
-    SelCache sc{};
-    u64* d_zh = nullptr;
-    MSG_CUDA(cudaMalloc(&sc.first, nq * 8));
-    MSG_CUDA(cudaMalloc(&sc.last, nq * 8));
-    MSG_CUDA(cudaMalloc(&sc.inv_zh, q * 8));
-    MSG_CUDA(cudaMalloc(&d_zh, q * 8));
-    for (void* p : {(void*)sc.first, (void*)sc.last, (void*)sc.inv_zh, (void*)d_zh}) c.owned.push_back(p);
-    MSG_CUDA(cudaMemcpyAsync(d_zh, zh.data(), q * 8, cudaMemcpyHostToDevice, c.stream));
-    MSG_CUDA(cudaMemcpyAsync(sc.inv_zh, izh.data(), q * 8, cudaMemcpyHostToDevice, c.stream));
+    SelCache sc{cuda_malloc<u64>(nq), cuda_malloc<u64>(nq), cuda_malloc<u64>(q), cuda_malloc<u64>(q)};
+    MSG_CUDA(cudaMemcpyAsync(sc.zh.get(), zh.data(), q * 8, cudaMemcpyHostToDevice, c.stream));
+    MSG_CUDA(cudaMemcpyAsync(sc.inv_zh.get(), izh.data(), q * 8, cudaMemcpyHostToDevice, c.stream));
     SelParams sp{};
     sp.xtab = coset_x_table(c, log_nq);
-    sp.zh = d_zh;
+    sp.zh = sc.zh.get();
     sp.g_inv = msh::two_adic_generator(log_n).inverse().v;
-    sp.first = sc.first;
-    sp.last = sc.last;
+    sp.first = sc.first.get();
+    sp.last = sc.last.get();
     sp.log_nq = log_nq;
     sp.log_q = log_q;
     u64 threads = (nq + kSelPerThread - 1) / kSelPerThread;
     {
         StageScope ss(c, "quotient");
-        KLaunch kl(c, "k_selectors");
-        k_selectors<<<(unsigned)((threads + 255) / 256), 256, 0, c.stream>>>(sp);
+        launch(c, "k_selectors", k_selectors, (unsigned)((threads + 255) / 256), 256, 0, sp);
     }
-    MSG_CUDA(cudaGetLastError());
     c.sync();  // zh / izh host vectors die here
-    cache[key] = sc;
-    return sc;
+    return cache[key] = std::move(sc);
 }
 
 template <class K>
@@ -628,11 +609,7 @@ static void quotient_slices(Ctx& c, const u64* S, u64* out, u32 log_big, u32 log
     for (u64 k = 0; k < q; k++) { w[k] = (acc * ninv).v; acc *= step; }
     DevBuf dw(c, q * 8);
     MSG_CUDA(cudaMemcpyAsync(dw.p, w.data(), q * 8, cudaMemcpyHostToDevice, c.stream));
-    {
-        KLaunch kl(c, "k_quotient_slices");
-        k_quotient_slices<<<(unsigned)((big + 255) / 256), 256, 0, c.stream>>>(S, out, log_big, log_n, d, dw.u());
-    }
-    MSG_CUDA(cudaGetLastError());
+    launch(c, "k_quotient_slices", k_quotient_slices, (unsigned)((big + 255) / 256), 256, 0, S, out, log_big, log_n, d, (const u64*)dw.u());
     c.sync();  // `w` dies here (pageable source of an async copy)
 }
 
@@ -650,9 +627,9 @@ using namespace msg;
 
 struct msgpu_claims {
     Ctx* ctx;
-    u64* d;
+    DevBuf d;
     u64 n, len;
-    cudaEvent_t ready = nullptr;  // prefetched claims: the copy on the context's copy stream has finished
+    Event ready;  // prefetched claims: the copy on the context's copy stream has finished
 };
 
 namespace msg {
@@ -677,12 +654,8 @@ static void claims_sum(Ctx& c, const u64* d_claims, u64 n_claims, u64 claim_len,
     u64 nblocks = (n_claims + kScanPerBlock - 1) / kScanPerBlock;
     DevBuf part(c, nblocks * 16 + 8);  // the block partials, then the zero-message flag
     MSG_CUDA(cudaMemsetAsync(part.u() + 2 * nblocks, 0, 8, c.stream));
-    {
-        KLaunch kl(c, "k_claims");
-        k_claims<<<(unsigned)nblocks, kScanThreads, 0, c.stream>>>(d_claims, n_claims, (u32)claim_len, gl::e2{beta2[0], beta2[1]},
-                                                                   gl::e2{gamma2[0], gamma2[1]}, part.u(), part.u() + 2 * nblocks);
-    }
-    MSG_CUDA(cudaGetLastError());
+    launch(c, "k_claims", k_claims, (unsigned)nblocks, kScanThreads, 0, d_claims, n_claims, (u32)claim_len, gl::e2{beta2[0], beta2[1]},
+           gl::e2{gamma2[0], gamma2[1]}, part.u(), part.u() + 2 * nblocks);
     std::vector<u64> hp(nblocks * 2 + 1);
     MSG_CUDA(cudaMemcpyAsync(hp.data(), part.p, nblocks * 16 + 8, cudaMemcpyDeviceToHost, c.stream));
     c.sync();
@@ -698,13 +671,12 @@ extern "C" {
 int msgpu_program_create(msgpu_ctx* h, const msgpu_graph_desc* desc, msgpu_program** out) {
     return guard([&] {
         MSG_REQUIRE(desc && out, "program_create: null argument");
-        *out = program_create(h->c, *desc);
+        *out = program_create(h->c, *desc).release();
     });
 }
 void msgpu_program_free(msgpu_program* prog) {
     if (!prog) return;
     cudaStreamSynchronize(prog->ctx->stream);
-    for (void* p : prog->owned) cudaFree(p);
     delete prog;
 }
 
@@ -731,11 +703,11 @@ int msgpu_stage2_trace(msgpu_ctx* h, const msgpu_program* prog, const uint64_t* 
         u64* zero_msg = bsums.u() + 2 * (nblocks + 1);
         MSG_CUDA(cudaMemsetAsync(zero_msg, 0, 8, c.stream));
         MsgParams mp{};
-        mp.prog = prog->d_prefix;
+        mp.prog = prog->d_prefix.get();
         mp.n_instr = prog->n_prefix;
-        mp.lk_mult = prog->d_mult_prefix;
-        mp.lk_argoff = prog->d_arg_off;
-        mp.lk_args = prog->d_args_prefix;
+        mp.lk_mult = prog->d_mult_prefix.get();
+        mp.lk_argoff = prog->d_arg_off.get();
+        mp.lk_args = prog->d_args_prefix.get();
         mp.pre = (const u64*)pre_dev;
         mp.main = (const u64*)main_dev;
         mp.msgs = msgs.u();
@@ -747,28 +719,15 @@ int msgpu_stage2_trace(msgpu_ctx* h, const msgpu_program* prog, const uint64_t* 
         mp.wpre = prog->pre_width;
         mp.wmain = prog->main_width;
         launch_by_slots(prog->slots_prefix, [&](auto ns) {
-            KLaunch kl(c, "k_lookup_messages");
             constexpr int NS = decltype(ns)::value;
             constexpr size_t smem = slots_smem_bytes<NS>();
             if (smem > 48 * 1024) ensure_max_smem(k_lookup_messages<NS>, (int)smem);
-            k_lookup_messages<NS><<<(unsigned)((rows + 127) / 128), kInterpThreads, smem, c.stream>>>(mp);
+            launch(c, "k_lookup_messages", k_lookup_messages<NS>, (unsigned)((rows + 127) / 128), kInterpThreads, smem, mp);
         });
-        MSG_CUDA(cudaGetLastError());
-        {
-            KLaunch kl(c, "k_terms_and_block_sums");
-            k_terms_and_block_sums<<<(unsigned)nblocks, kScanThreads, 0, c.stream>>>(msgs.u(), mults.u(), total, bsums.u(), zero_msg);
-        }
-        MSG_CUDA(cudaGetLastError());
-        {
-            KLaunch kl(c, "k_scan_block_sums");
-            k_scan_block_sums<<<1, 1024, 0, c.stream>>>(bsums.u(), nblocks);
-        }
-        MSG_CUDA(cudaGetLastError());
-        {
-            KLaunch kl(c, "k_scan_write");
-            k_scan_write<<<(unsigned)nblocks, kScanThreads, 0, c.stream>>>(msgs.u(), total, bsums.u(), (u64*)stage2_out_dev);
-        }
-        MSG_CUDA(cudaGetLastError());
+        launch(c, "k_terms_and_block_sums", k_terms_and_block_sums, (unsigned)nblocks, kScanThreads, 0, msgs.u(), mults.u(), total, bsums.u(),
+               zero_msg);
+        launch(c, "k_scan_block_sums", k_scan_block_sums, 1, 1024, 0, bsums.u(), nblocks);
+        launch(c, "k_scan_write", k_scan_write, (unsigned)nblocks, kScanThreads, 0, msgs.u(), total, bsums.u(), (u64*)stage2_out_dev);
         u64 tail[3];  // total, zero-message flag
         MSG_CUDA(cudaMemcpyAsync(tail, bsums.u() + 2 * nblocks, 24, cudaMemcpyDeviceToHost, c.stream));
         c.sync();
@@ -802,7 +761,7 @@ int msgpu_claims_upload(msgpu_ctx* h, const uint64_t* claims, uint64_t n_claims,
         DevBuf d(c, n_vals * 8);
         MSG_CUDA(cudaMemcpyAsync(d.p, claims, n_vals * 8, cudaMemcpyHostToDevice, c.stream));
         claims_digest(c, d.u(), n_claims, claim_len, prefix, prefix_len, digest32);
-        *out = new msgpu_claims{&c, (u64*)d.release(), n_claims, claim_len};
+        *out = new msgpu_claims{&c, std::move(d), n_claims, claim_len, Event()};
     });
 }
 
@@ -816,17 +775,15 @@ int msgpu_claims_prefetch(msgpu_ctx* h, const uint64_t* claims, uint64_t n_claim
         DevBuf d(c, n_vals * 8);
         // the copy starts behind everything already enqueued on the main stream (the block may have just been freed by it,
         // and the trace upload should have the link to itself) and runs under whatever the main stream does next
-        cudaEvent_t e0, ready;
+        auto cl = std::unique_ptr<msgpu_claims>(new msgpu_claims{&c, std::move(d), n_claims, claim_len, Event()});
+        cudaEvent_t e0;
         MSG_CUDA(cudaEventCreateWithFlags(&e0, cudaEventDisableTiming));
-        MSG_CUDA(cudaEventCreateWithFlags(&ready, cudaEventDisableTiming));
         MSG_CUDA(cudaEventRecord(e0, c.stream));
         MSG_CUDA(cudaStreamWaitEvent(c.copy_stream, e0, 0));
-        MSG_CUDA(cudaMemcpyAsync(d.p, claims, n_vals * 8, cudaMemcpyHostToDevice, c.copy_stream));
-        MSG_CUDA(cudaEventRecord(ready, c.copy_stream));
         cudaEventDestroy(e0);
-        msgpu_claims* cl = new msgpu_claims{&c, (u64*)d.release(), n_claims, claim_len};
-        cl->ready = ready;
-        *out = cl;
+        MSG_CUDA(cudaMemcpyAsync(cl->d.p, claims, n_vals * 8, cudaMemcpyHostToDevice, c.copy_stream));
+        cl->ready.record(c.copy_stream);
+        *out = cl.release();
     });
 }
 
@@ -834,8 +791,8 @@ int msgpu_claims_digest(msgpu_claims* cl, const uint8_t* prefix, uint64_t prefix
     return guard([&] {
         MSG_REQUIRE(cl && digest32, "claims_digest: null argument");
         Ctx& c = *cl->ctx;
-        if (cl->ready) MSG_CUDA(cudaStreamWaitEvent(c.stream, cl->ready, 0));
-        claims_digest(c, cl->d, cl->n, cl->len, prefix, prefix_len, digest32);
+        if (cl->ready.e) MSG_CUDA(cudaStreamWaitEvent(c.stream, cl->ready.e, 0));
+        claims_digest(c, cl->d.u(), cl->n, cl->len, prefix, prefix_len, digest32);
     });
 }
 
@@ -848,12 +805,8 @@ static void claims_digest(Ctx& c, const u64* d_claims, u64 n_claims, u64 claim_l
         MSG_CUDA(cudaMemsetAsync(flag.p, 0, 4, c.stream));
         check_canonical(c, d.u(), n_vals, (u32*)flag.p);
         if (prefix_len) MSG_CUDA(cudaMemcpyAsync(msg.p, prefix, prefix_len, cudaMemcpyHostToDevice, c.stream));
-        {
-            KLaunch kl(c, "k_encode_claims");
-            k_encode_claims<<<(unsigned)((n_words + 255) / 256), 256, 0, c.stream>>>(d.u(), n_words, (u32)claim_len,
-                                                                                     (uint8_t*)msg.p + prefix_len);
-        }
-        MSG_CUDA(cudaGetLastError());
+        launch(c, "k_encode_claims", k_encode_claims, (unsigned)((n_words + 255) / 256), 256, 0, d.u(), n_words, (u32)claim_len,
+               msg.bytes() + prefix_len);
         u32 bad = 0;
         if (msg_len > 1024) {
             uint8_t* out_dev = (uint8_t*)msg.p + ((msg_len + 15) / 16) * 16;
@@ -875,22 +828,11 @@ static void claims_digest(Ctx& c, const u64* d_claims, u64 n_claims, u64 claim_l
 int msgpu_claims_accumulate(msgpu_claims* cl, const uint64_t* beta2, const uint64_t* gamma2, uint64_t* out2) {
     return guard([&] {
         MSG_REQUIRE(cl && beta2 && gamma2 && out2, "claims_accumulate: null argument");
-        if (cl->ready) MSG_CUDA(cudaStreamWaitEvent(cl->ctx->stream, cl->ready, 0));
-        claims_sum(*cl->ctx, cl->d, cl->n, cl->len, beta2, gamma2, out2);
+        if (cl->ready.e) MSG_CUDA(cudaStreamWaitEvent(cl->ctx->stream, cl->ready.e, 0));
+        claims_sum(*cl->ctx, cl->d.u(), cl->n, cl->len, beta2, gamma2, out2);
     });
 }
-void msgpu_claims_free(msgpu_claims* cl) {
-    if (!cl) return;
-    if (cl->ready) {
-        cudaEventSynchronize(cl->ready);  // the copy must not outlive the block
-        cudaEventDestroy(cl->ready);
-    }
-    try {
-        cl->ctx->free(cl->d);
-    } catch (...) {
-    }
-    delete cl;
-}
+void msgpu_claims_free(msgpu_claims* cl) { delete cl; }
 
 }  // extern "C"
 
@@ -912,7 +854,7 @@ static void quotient_eval(Ctx& c, const msgpu_program* prog, const u64* const cu
         qp.wn[k] = next_widths3 ? next_widths3[k] : full_w[k];
         qp.cn[k] = next_col0_3 ? next_col0_3[k] : 0;
     }
-    SelCache sel = selectors(c, log_n, log_q);
+    const SelCache& sel = selectors(c, log_n, log_q);
     // alpha powers reversed (src/prover.rs:798-808): constraint j of k weighted by alpha^{k-1-j}
     u32 k = prog->n_zeros + 2 * std::max<u32>(prog->n_lookups, 1);
     std::vector<u64> apow(2 * (size_t)k);
@@ -925,21 +867,21 @@ static void quotient_eval(Ctx& c, const msgpu_program* prog, const u64* const cu
     DevBuf d_apow(c, apow.size() * 8);
     MSG_CUDA(cudaMemcpyAsync(d_apow.p, apow.data(), apow.size() * 8, cudaMemcpyHostToDevice, c.stream));
     msh::Fp inj_norm = (msh::Fp((msh::u64)n) * msh::two_adic_generator(log_n)).inverse();
-    qp.prog = prog->d_full;
+    qp.prog = prog->d_full.get();
     qp.n_instr = prog->n_full;
-    qp.zero_slots = prog->d_zero_slots;
+    qp.zero_slots = prog->d_zero_slots.get();
     qp.n_zeros = prog->n_zeros;
     qp.n_lookups = prog->n_lookups;
-    qp.lk_mult = prog->d_mult_full;
-    qp.lk_argoff = prog->d_arg_off;
-    qp.lk_args = prog->d_args_full;
+    qp.lk_mult = prog->d_mult_full.get();
+    qp.lk_argoff = prog->d_arg_off.get();
+    qp.lk_args = prog->d_args_full.get();
     qp.wpre = prog->pre_width;
     qp.w1 = prog->main_width;
     qp.w2 = prog->stage2_width;
     qp.apow = d_apow.u();
-    qp.sel_first = sel.first;
-    qp.sel_last = sel.last;
-    qp.inv_zh = sel.inv_zh;
+    qp.sel_first = sel.first.get();
+    qp.sel_last = sel.last.get();
+    qp.inv_zh = sel.inv_zh.get();
     qp.out = out;
     qp.xtab = coset_x_table(c, log_nq);
     for (int i = 0; i < 8; i++) qp.publics[i] = publics8[i];
@@ -950,10 +892,8 @@ static void quotient_eval(Ctx& c, const msgpu_program* prog, const u64* const cu
     qp.log_q = log_q;
     if (n_local) {
         launch_by_slots(prog->slots_full, [&](auto ns) {
-            KLaunch kl(c, "k_quotient_eval");
-            k_quotient_eval<decltype(ns)::value><<<(unsigned)((n_local + 127) / 128), kInterpThreads, 0, c.stream>>>(qp);
+            launch(c, "k_quotient_eval", k_quotient_eval<decltype(ns)::value>, (unsigned)((n_local + 127) / 128), kInterpThreads, 0, qp);
         });
-        MSG_CUDA(cudaGetLastError());
     }
     c.sync();  // apow (pageable) must outlive the copy; also surfaces kernel faults here
 }
@@ -966,15 +906,10 @@ static u64* quotient_finish(Ctx& c, u64* qv, u32 log_n, u32 log_q, u32 log_blowu
     ntt_dft_bitrev(c, qv, qv, nq, 2, false);
     DevBuf sl(c, n * q * 16);
     quotient_slices(c, qv, sl.u(), log_nq, log_n, 2);
-    u64* lde = (u64*)c.alloc((n << log_blowup) * q * 16);
-    try {
-        ntt_lde_from_coeffs(c, sl.u(), lde, n, 2 * q, log_blowup);
-        c.sync();
-    } catch (...) {
-        c.free(lde);
-        throw;
-    }
-    return lde;
+    DevBuf lde(c, (n << log_blowup) * q * 16);
+    ntt_lde_from_coeffs(c, sl.u(), lde.u(), n, 2 * q, log_blowup);
+    c.sync();
+    return (u64*)lde.release();
 }
 }  // namespace msg
 
@@ -1042,10 +977,8 @@ int msgpu_extract_columns_dev(msgpu_ctx* h, const uint64_t* src, uint64_t rows, 
         MSG_REQUIRE(src && dst && c0 < c1 && c1 <= width, "extract_columns: bad column range");
         if (rows == 0) return;
         StageScope ss(c, "exchange");
-        KLaunch kl(c, "k_extract_columns");
-        k_extract_columns<<<(unsigned)std::min<u64>((rows * (c1 - c0) + 255) / 256, (u64)c.sm_count * 16), 256, 0, c.stream>>>(
-            (const u64*)src, rows, (u32)width, (u32)c0, (u32)(c1 - c0), (u64*)dst);
-        MSG_CUDA(cudaGetLastError());
+        launch(c, "k_extract_columns", k_extract_columns, (unsigned)std::min<u64>((rows * (c1 - c0) + 255) / 256, (u64)c.sm_count * 16), 256, 0,
+               (const u64*)src, rows, (u32)width, (u32)c0, (u32)(c1 - c0), (u64*)dst);
     });
 }
 // values_stored_dev: ALL nq x 2 quotient evaluations in stored (bit-reversed) order, gathered from the shards (device, not
@@ -1083,13 +1016,13 @@ int msgpu_selectors_on_coset(msgpu_ctx* h, uint32_t log_n, uint32_t log_q, uint6
     return guard([&] {
         Ctx& c = h->c;
         MSG_REQUIRE(log_n + log_q <= msh::GL_TWO_ADICITY && is_first_row && is_last_row && inv_vanishing, "selectors: bad argument");
-        SelCache sc = selectors(c, log_n, log_q);
+        const SelCache& sc = selectors(c, log_n, log_q);
         const u32 log_nq = log_n + log_q;
         const u64 nq = 1ull << log_nq, q = 1ull << log_q;
         std::vector<u64> first(nq), last(nq), izh(q);
-        MSG_CUDA(cudaMemcpyAsync(first.data(), sc.first, nq * 8, cudaMemcpyDeviceToHost, c.stream));
-        MSG_CUDA(cudaMemcpyAsync(last.data(), sc.last, nq * 8, cudaMemcpyDeviceToHost, c.stream));
-        MSG_CUDA(cudaMemcpyAsync(izh.data(), sc.inv_zh, q * 8, cudaMemcpyDeviceToHost, c.stream));
+        MSG_CUDA(cudaMemcpyAsync(first.data(), sc.first.get(), nq * 8, cudaMemcpyDeviceToHost, c.stream));
+        MSG_CUDA(cudaMemcpyAsync(last.data(), sc.last.get(), nq * 8, cudaMemcpyDeviceToHost, c.stream));
+        MSG_CUDA(cudaMemcpyAsync(izh.data(), sc.inv_zh.get(), q * 8, cudaMemcpyDeviceToHost, c.stream));
         c.sync();
         for (u64 i = 0; i < nq; i++) {  // the tables are kept in stored (bit-reversed) order
             u64 sidx = msh::reverse_bits_len(i, log_nq);
