@@ -341,15 +341,20 @@ void mmcs_from_parts(Ctx& c, msgpu_pdata* pd, const std::vector<const u64*>& blo
             off += len;
         }
     }
-    if (n_parts > 1) {  // the top log2(n_parts) levels over the parts' roots
-        const u32 l0 = part_layers - 1, levels = ilog2(n_parts);
+    // the top log2(n_parts) levels over the parts' roots, in launches of at most 10 levels while the layer is longer than
+    // 4096 (as build_nodes: one launch reduces at most kMaxFusedLevels = 12)
+    const u32 top = part_layers - 1 + ilog2(n_parts);
+    for (u32 l = part_layers - 1; l < top;) {
+        const u64 len = pd->layer_len[l];
+        const u32 levels = len > 4096 ? 10 : top - l;
         uint8_t* outs[16];
         const uint8_t* injs[16];
         for (u32 k = 0; k < levels; k++) {
-            outs[k] = pd->digests.bytes() + pd->layer_off[l0 + 1 + k] * 32;
+            outs[k] = pd->digests.bytes() + pd->layer_off[l + 1 + k] * 32;
             injs[k] = nullptr;
         }
-        b3_merkle_subtrees(c, pd->digests.bytes() + pd->layer_off[l0] * 32, n_parts, levels, outs, injs);
+        b3_merkle_subtrees(c, pd->digests.bytes() + pd->layer_off[l] * 32, len, levels, outs, injs);
+        l += levels;
     }
     MSG_CUDA(cudaMemcpyAsync(pd->root, pd->digests.bytes() + pd->layer_off.back() * 32, 32, cudaMemcpyDeviceToHost, c.stream));
     c.sync();
