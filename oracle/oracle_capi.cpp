@@ -51,6 +51,46 @@ void orc_fp2_inv(const u64* a, u64* out) {
     Fp2 r = Fp2(Fp(a[0]), Fp(a[1])).inverse();
     out[0] = r.c[0].v; out[1] = r.c[1].v;
 }
+// Element-wise host field operations over arrays, for tests/test_host_field.py. Operands of the Fp ops go through Fp(u64),
+// so non-canonical inputs are reduced first; the simd:: ops and gl_reduce128 take the raw u64 words.
+void orc_fp_op(int op, const u64* a, const u64* b, u64* out, u64 n) {
+    for (u64 i = 0; i < n; i++) {
+        const Fp x(a[i]), y(b[i]);
+        switch (op) {
+            case 0: out[i] = x.v; break;
+            case 1: out[i] = (x + y).v; break;
+            case 2: out[i] = (x - y).v; break;
+            case 3: out[i] = (-x).v; break;
+            case 4: out[i] = (x * y).v; break;
+            case 5: out[i] = x.pow(b[i]).v; break;
+            case 6: out[i] = x.inverse().v; break;  // x != 0
+            case 7: out[i] = x.halve().v; break;
+            case 8: out[i] = simd::gl_mul(a[i], b[i]); break;
+            case 9: out[i] = simd::gl_add(a[i], b[i]); break;
+            case 10: out[i] = simd::gl_sub(a[i], b[i]); break;
+            case 11: out[i] = msh::gl_reduce128(((msh::u128)b[i] << 64) | a[i]); break;  // lo = a, hi = b
+            default: out[i] = 0; break;
+        }
+    }
+}
+// Fp2 operations over arrays of (c0, c1) pairs: 0 = a * b, 1 = a.inverse() (a != 0), 2 = a.halve()
+void orc_fp2_op(int op, const u64* a, const u64* b, u64* out, u64 n) {
+    for (u64 i = 0; i < n; i++) {
+        const Fp2 x(Fp(a[2 * i]), Fp(a[2 * i + 1])), y(Fp(b[2 * i]), Fp(b[2 * i + 1]));
+        const Fp2 r = op == 0 ? x * y : op == 1 ? x.inverse() : x.halve();
+        out[2 * i] = r.c[0].v;
+        out[2 * i + 1] = r.c[1].v;
+    }
+}
+void orc_fp_batch_inverse(const u64* in, u64* out, u64 n) {
+    std::vector<Fp> x(n), r(n);
+    for (u64 i = 0; i < n; i++) x[i] = Fp(in[i]);
+    batch_inverse(x.data(), r.data(), n);
+    for (u64 i = 0; i < n; i++) out[i] = r[i].v;
+}
+// the oracle's vectorised row kernels (AVX-512 with masked tails, or the auto-vectorised clones under ORC_NO_AVX512)
+void orc_dif_butterfly_row(u64* a, u64* b, u64 t, u64 w) { simd::dif_butterfly_row(a, b, t, w); }
+void orc_scale_row(u64* dst, const u64* src, u64 s, u64 w) { simd::scale_row(dst, src, s, w); }
 
 // ---- DFT / LDE (p3-dft semantics) ----------------------------------------------------------
 void orc_dft_batch(const u64* in, u64 rows, u64 cols, u64* out) { from_matrix(dft_batch(to_matrix(in, rows, cols)), out); }
