@@ -151,20 +151,8 @@ int msgpu_tree_from_digests(msgpu_ctx* ctx, uint64_t n_classes, const uint64_t* 
                             msgpu_pdata** out, uint8_t* root32);
 uint64_t msgpu_pdata_max_height(const msgpu_pdata* pd);
 int msgpu_pdata_root(const msgpu_pdata* pd, uint8_t* root32);
-/* ---- one WIDE matrix over several GPUs (SURVEY 8e, partitioning B: column blocks) -----------------------------------
- * Each rank extends its column block (msgpu_coset_lde_batch_bitrev_dev), an all-to-all turns blocks into row shards, every
- * rank commits its shard (msgpu_commit_ldes_dev over the received chunks: leaf = hash of the whole row) and the subtree roots
- * are combined with msgpu_tree_from_digests (multi_stark_b200/dist.py: commit_wide_sharded). To PROVE on one rank afterwards,
- * that rank gathers the column blocks and the shards' digest layers and assembles ordinary prover data:
- * pdata_digests: DEVICE pointer to all digest layers of a tree, back to back from the leaves up (2 * max_height - 1 digests);
- * pdata_from_parts: blocks[b] = DEVICE pointer to column block b of the LDE (lde_height x widths[b]), part_digests[p] = the
- * digest layers of row shard p's subtree (lde_height / n_parts leaves). The blocks are interleaved into one row-major matrix
- * owned by the result (the inputs are not modified), the layers are laid out as msgpu_commit would have and the top
- * log2(n_parts) levels rebuilt: root, rows and paths are those of a single-GPU commit of the whole matrix. */
+/* DEVICE pointer to all digest layers of a tree, back to back from the leaves up (2 * max_height - 1 digests) */
 int msgpu_pdata_digests(const msgpu_pdata* pd, uint8_t** dev_ptr, uint64_t* n_digests);
-int msgpu_pdata_from_parts(msgpu_ctx* ctx, uint64_t n_blocks, const uint64_t* const* blocks, const uint64_t* widths,
-                           uint64_t lde_height, uint64_t n_parts, const uint8_t* const* part_digests, msgpu_pdata** out,
-                           uint8_t* root32);
 /* Mmcs::commit on HOST matrices as they are (no LDE): used for the FRI layers' ExtensionMmcs rows
  * and by the parity tests of the tree shape (cases of src/types.rs:246-282). */
 int msgpu_mmcs_commit(msgpu_ctx* ctx, const uint64_t* const* mats, const uint64_t* heights, const uint64_t* widths,

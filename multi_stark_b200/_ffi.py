@@ -54,7 +54,6 @@ SIGNATURES = {
     "msgpu_pdata_max_height": (C.c_uint64, [C.c_void_p]),
     "msgpu_pdata_root": (C.c_int, [C.c_void_p, C.c_void_p]),
     "msgpu_pdata_digests": (C.c_int, [C.c_void_p, c_vpp, c_u64p]),
-    "msgpu_pdata_from_parts": (C.c_int, [C.c_void_p, C.c_uint64, c_vpp, c_u64p, C.c_uint64, C.c_uint64, c_vpp, c_vpp, C.c_void_p]),
     "msgpu_mmcs_commit": (C.c_int, [C.c_void_p, c_vpp, c_u64p, c_u64p, C.c_uint64, c_vpp, C.c_void_p]),
     "msgpu_pdata_free": (None, [C.c_void_p]),
     "msgpu_pdata_num_matrices": (C.c_uint64, [C.c_void_p]),
@@ -198,10 +197,8 @@ HOST_SIGNATURES = {
     "msh_dist_prover_create": (C.c_void_p, [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_int32)]),
     "msh_fib_trace": (None, [C.c_uint64, C.c_void_p]),
     "msh_wide_trace": (None, [C.c_uint64, C.c_uint64, C.c_uint64, C.c_void_p]),
-    "msh_wide_trace_block": (None, [C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint64, C.c_void_p]),
     "msh_prover_create": (C.c_void_p, [C.c_void_p, C.c_void_p]),
     "msh_prover_free": (None, [C.c_void_p]),
-    "msh_prover_inject_stage1": (C.c_int, [C.c_void_p, C.c_void_p]),
     "msh_prover_preprocessed_commit": (C.c_int, [C.c_void_p, C.c_void_p]),
     "msh_prove": (C.c_int, [C.c_void_p, c_vpp, c_u64p, c_u64p, c_u64p, C.c_uint64, C.c_uint64, c_vpp, c_u64p, C.POINTER(C.c_double)]),
     "msh_bytes_free": (None, [C.c_void_p]),

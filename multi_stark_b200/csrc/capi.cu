@@ -597,21 +597,6 @@ int msgpu_interleave_column_blocks_dev(msgpu_ctx* h, const uint64_t* src, uint64
         interleave_column_blocks(h->c, (const u64*)src, rows, std::vector<u64>(widths, widths + n_blocks), (u64*)dst);
     });
 }
-int msgpu_pdata_from_parts(msgpu_ctx* h, uint64_t n_blocks, const uint64_t* const* blocks, const uint64_t* widths, uint64_t lde_height,
-                           uint64_t n_parts, const uint8_t* const* part_digests, msgpu_pdata** out, uint8_t* root32) {
-    return guard([&] {
-        Ctx& c = h->c;
-        MSG_REQUIRE(blocks && widths && part_digests && out && root32 && n_blocks > 0 && n_parts > 0, "pdata_from_parts: null or empty argument");
-        std::vector<const u64*> bl;
-        std::vector<u64> ws;
-        for (u64 b = 0; b < n_blocks; b++) { bl.push_back((const u64*)blocks[b]); ws.push_back(widths[b]); }
-        std::vector<const uint8_t*> parts(part_digests, part_digests + n_parts);
-        auto pd = std::make_unique<msgpu_pdata>();
-        mmcs_from_parts(c, pd.get(), bl, ws, lde_height, parts);
-        memcpy(root32, pd->root, 32);
-        *out = pd.release();
-    });
-}
 
 int msgpu_mmcs_commit(msgpu_ctx* h, const uint64_t* const* mats, const uint64_t* heights, const uint64_t* widths,
                       uint64_t n_mats, msgpu_pdata** out, uint8_t* root32) {

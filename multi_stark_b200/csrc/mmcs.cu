@@ -303,61 +303,4 @@ void interleave_column_blocks(Ctx& c, const u64* src, u64 rows, const std::vecto
     launch(c, "k_interleave_columns", k_interleave_columns, (unsigned)std::min<u64>((rows * W + 255) / 256, (u64)c.sm_count * 16), 256, 0, ip);
 }
 
-void mmcs_from_parts(Ctx& c, msgpu_pdata* pd, const std::vector<const u64*>& blocks, const std::vector<u64>& widths, u64 height,
-                     const std::vector<const uint8_t*>& part_digests) {
-    const u64 n_parts = part_digests.size();
-    MSG_REQUIRE(!blocks.empty() && blocks.size() <= (size_t)kMaxBlocks && blocks.size() == widths.size(), "from_parts: 1..16 column blocks expected");
-    MSG_REQUIRE(is_pow2(height) && is_pow2(n_parts) && n_parts <= height, "from_parts: heights and part counts must be powers of two");
-    u64 W = 0;
-    InterleaveParams ip{};
-    for (size_t b = 0; b < blocks.size(); b++) {
-        MSG_REQUIRE(blocks[b] && widths[b] > 0 && W + widths[b] < (1ull << 31), "from_parts: bad column block");
-        ip.blocks[b] = blocks[b];
-        ip.col0[b] = (u32)W;
-        W += widths[b];
-    }
-    ip.col0[blocks.size()] = (u32)W;
-    ip.n_blocks = (u32)blocks.size();
-    ip.rows = height;
-    pd->mats.push_back(msgpu_pdata::Mat::alloc(c, height, W));
-    pd->total_width = W;
-    ip.out = pd->mats.back().ptr;
-    {
-        StageScope ss(c, "lde");
-        launch(c, "k_interleave_columns", k_interleave_columns, (unsigned)std::min<u64>((height * W + 255) / 256, (u64)c.sm_count * 16), 256, 0, ip);
-    }
-    // digest layers: layer l of the tree is the concatenation of the parts' layer l while a part still has one
-    StageScope ss(c, "merkle");
-    mmcs_layout_layers(c, pd, height);
-    const u64 shard = height / n_parts;
-    const u32 part_layers = ilog2(shard) + 1;
-    for (u64 p = 0; p < n_parts; p++) {
-        MSG_REQUIRE(part_digests[p], "from_parts: null digest part");
-        u64 off = 0;
-        for (u32 l = 0; l < part_layers; l++) {
-            const u64 len = shard >> l;
-            MSG_CUDA(cudaMemcpyAsync(pd->digests.bytes() + (pd->layer_off[l] + p * len) * 32, part_digests[p] + off * 32, len * 32,
-                                     cudaMemcpyDeviceToDevice, c.stream));
-            off += len;
-        }
-    }
-    // the top log2(n_parts) levels over the parts' roots, in launches of at most 10 levels while the layer is longer than
-    // 4096 (as build_nodes: one launch reduces at most kMaxFusedLevels = 12)
-    const u32 top = part_layers - 1 + ilog2(n_parts);
-    for (u32 l = part_layers - 1; l < top;) {
-        const u64 len = pd->layer_len[l];
-        const u32 levels = len > 4096 ? 10 : top - l;
-        uint8_t* outs[16];
-        const uint8_t* injs[16];
-        for (u32 k = 0; k < levels; k++) {
-            outs[k] = pd->digests.bytes() + pd->layer_off[l + 1 + k] * 32;
-            injs[k] = nullptr;
-        }
-        b3_merkle_subtrees(c, pd->digests.bytes() + pd->layer_off[l] * 32, len, levels, outs, injs);
-        l += levels;
-    }
-    MSG_CUDA(cudaMemcpyAsync(pd->root, pd->digests.bytes() + pd->layer_off.back() * 32, 32, cudaMemcpyDeviceToHost, c.stream));
-    c.sync();
-}
-
 }  // namespace msg

@@ -48,9 +48,6 @@ void mmcs_build_local(Ctx& c, msgpu_pdata* pd);
 void mmcs_build_from_classes(Ctx& c, msgpu_pdata* pd, const std::vector<std::pair<u64, const uint8_t*>>& classes);
 // allocates pd->digests for a tree over max_h leaves and fills layer_off / layer_len (layer 0 = leaf digests)
 void mmcs_layout_layers(Ctx& c, msgpu_pdata* pd, u64 max_h);
-// One matrix from its column blocks (interleaved into a new row-major matrix) + the digest layers of its row-shard subtrees.
-void mmcs_from_parts(Ctx& c, msgpu_pdata* pd, const std::vector<const u64*>& blocks, const std::vector<u64>& widths, u64 height,
-                     const std::vector<const uint8_t*>& part_digests);
 // row block (rows x width) -> column blocks [c0[b], c1[b]) as contiguous matrices back to back in dst, and the inverse
 void pack_column_blocks(Ctx& c, const u64* src, u64 rows, u64 width, const std::vector<u64>& c0, const std::vector<u64>& c1, u64* dst);
 void interleave_column_blocks(Ctx& c, const u64* src, u64 rows, const std::vector<u64>& widths, u64* dst);

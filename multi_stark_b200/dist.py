@@ -16,7 +16,6 @@ import torch
 import torch.distributed as dist
 
 from ._ffi import check, host_error, host_lib
-from .pcs import ProverData
 from .system import ProverBase
 
 
@@ -463,193 +462,3 @@ class RowShardProver(_ShardedProver):
                 raise ValueError("a trace given as a row block must hold exactly the rows this rank reads")
             ptrs.append(m.ctypes.data - row0 * m.shape[1] * 8 if m.size else None)  # the library touches [row0, row0 + rows) only
         return self._prove(ptrs, heights, claims)
-
-
-# ------------------------------------------------------------------------------------------------------------------
-# Pcs::commit of ONE wide matrix over the ranks (SURVEY 8e partitioning B, BASELINE configs[2]): column blocks.
-# ------------------------------------------------------------------------------------------------------------------
-def column_blocks(width, world_size):
-    """Contiguous balanced column blocks [c0, c1) per rank (the first width % world ranks get one more column)."""
-    base, rem = divmod(width, world_size)
-    out, c = [], 0
-    for r in range(world_size):
-        n = base + (1 if r < rem else 0)
-        out.append((c, c + n))
-        c += n
-    return out
-
-
-class WideCommit:
-    """Prover data of a column-block sharded commitment: this rank's ROW shard of the LDE (every column, rows
-    [rank * H / N, (rank + 1) * H / N) of the bit-reversed storage) with its Merkle subtree, and the top of the tree."""
-
-    def __init__(self, ctx, comm, local, top, root, lde_height, widths, recv_buf):
-        self.ctx, self.comm, self.local, self.top, self.root = ctx, comm, local, top, root
-        self.lde_height, self.widths, self._recv = lde_height, widths, recv_buf
-
-    def open_batch(self, indices):
-        """Mmcs::open_batch: (rows [n, width], sibling paths [n, log2(H), 32]) -- the same on every rank. The row and the
-        lower log2(H / N) siblings come from the rank that holds the row, the top log2(N) siblings from the top tree
-        (which every rank holds)."""
-        n, world = len(indices), self.comm.world
-        shard = self.lde_height // world
-        lo_depth, top_depth, width = shard.bit_length() - 1, world.bit_length() - 1, sum(self.widths)
-        owner = [int(i) // shard for i in indices]
-        rows = np.zeros((n, width), dtype=np.uint64)
-        low = np.zeros((n, lo_depth, 32), dtype=np.uint8)
-        mine = [k for k in range(n) if owner[k] == self.comm.rank]
-        if mine:
-            o, p = self.local.open_batch([int(indices[k]) % shard for k in mine])
-            rows[mine] = o
-            low[mine] = p
-        if world == 1:
-            return rows, low
-        # every rank contributes the openings of the rows it holds (zeros elsewhere); pick each index from its owner
-        blob = np.concatenate([rows.view(np.uint8).ravel(), low.ravel()])
-        gathered = np.zeros(blob.size * world, dtype=np.uint8)
-        self.comm.allgather_host(blob.ctypes.data, gathered.ctypes.data, blob.size)
-        gathered = gathered.reshape(world, -1)
-        all_rows = gathered[:, :rows.nbytes].copy().view(np.uint64).reshape(world, n, width)
-        all_low = gathered[:, rows.nbytes:].reshape(world, n, lo_depth, 32)
-        paths = np.zeros((n, lo_depth + top_depth, 32), dtype=np.uint8)
-        for k in range(n):
-            rows[k] = all_rows[owner[k], k]
-            paths[k, :lo_depth] = all_low[owner[k], k]
-        # the top tree has no matrices: sibling paths only
-        tidx = np.array(owner, dtype=np.uint64)
-        tp = np.zeros((n, top_depth, 32), dtype=np.uint8)
-        dummy = np.zeros(1, dtype=np.uint64)
-        check(self.ctx.L.msgpu_open_batch(self.ctx.h, self.top.h, tidx.ctypes.data_as(_C.c_void_p), n,
-                                          dummy.ctypes.data_as(_C.c_void_p), tp.ctypes.data_as(_C.c_void_p)))
-        paths[:, lo_depth:] = tp
-        return rows, paths
-
-    def free(self):
-        for h in (self.local, self.top):
-            if h is not None:
-                h.free()
-        if self._recv:
-            self.ctx.free(self._recv)
-            self._recv = None
-
-
-def commit_wide_sharded(ctx, comm, block, width, log_blowup, timings=None, keep_block=False):
-    """`Pcs::commit` (src/prover.rs:350) of one n x `width` matrix whose COLUMN block `column_blocks(width, N)[rank]` is
-    `block` (host array n x w_r, canonical values) on this rank. Per rank: upload + coset LDE of the block (the NTT is
-    column-local), ONE all-to-all that turns column blocks into row shards (the block's rows [d * H / N, (d+1) * H / N) are
-    contiguous and go to rank d), leaf hashing of the shard's full rows + its Merkle subtree, then the N subtree roots are
-    all-gathered and the top log2(N) levels built on every rank. Root and openings are bit-identical to a single-GPU commit."""
-    L = ctx.L
-    world, rank = comm.world, comm.rank
-    if world & (world - 1):
-        raise ValueError("column-block sharding needs a power-of-two number of ranks")
-    blocks = column_blocks(width, world)
-    widths = [c1 - c0 for c0, c1 in blocks]
-    a = np.ascontiguousarray(block, dtype=np.uint64)
-    n, w = a.shape
-    if w != widths[rank] or min(widths) == 0:
-        raise ValueError("this rank's block must have %d columns (and every rank at least one)" % widths[rank])
-    H = n << log_blowup
-    if H % world or H // world < 1:
-        raise ValueError("LDE height must be a multiple of the number of ranks")
-    shard = H // world
-    t = [time.perf_counter()]
-    d_in = ctx.upload_canonical(a)
-    t.append(time.perf_counter())
-    d_lde = ctx.malloc(H * w * 8)
-    check(L.msgpu_coset_lde_batch_bitrev_dev(ctx.h, _C.c_void_p(d_in), n, w, log_blowup, 7, _C.c_void_p(d_lde)))
-    ctx.free(d_in)
-    ctx.sync()
-    t.append(time.perf_counter())
-    # all-to-all: chunk d of my LDE (rows of shard d, my columns) -> rank d; I receive shard `rank` of every block
-    recv = ctx.malloc(shard * width * 8)
-    send_counts = [shard * w * 8] * world
-    recv_counts = [shard * ws * 8 for ws in widths]
-    comm.all_to_all_dev(d_lde, send_counts, recv, recv_counts)
-    if not keep_block:
-        ctx.free(d_lde)
-        d_lde = None
-    ctx.sync()
-    t.append(time.perf_counter())
-    # the shard as N matrices of one height: their rows concatenate in column order inside the leaf hash
-    ptrs, off = [], 0
-    for ws in widths:
-        ptrs.append(recv + off)
-        off += shard * ws * 8
-    pa = (_C.c_void_p * world)(*ptrs)
-    hs = (_C.c_uint64 * world)(*([shard] * world))
-    wa = (_C.c_uint64 * world)(*widths)
-    h = _C.c_void_p()
-    sub_root = np.zeros(32, dtype=np.uint8)
-    check(L.msgpu_commit_ldes_dev(ctx.h, pa, hs, wa, world, 0, _C.byref(h), sub_root.ctypes.data_as(_C.c_void_p)))
-    local = ProverData(ctx, h, bytes(sub_root))
-    t.append(time.perf_counter())
-    top, root = None, bytes(sub_root)
-    if world > 1:
-        roots = np.zeros(32 * world, dtype=np.uint8)
-        comm.allgather_host(sub_root.ctypes.data, roots.ctypes.data, 32)
-        d_roots = ctx.upload(roots)
-        th = _C.c_void_p()
-        r32 = np.zeros(32, dtype=np.uint8)
-        hh = (_C.c_uint64 * 1)(world)
-        pp = (_C.c_void_p * 1)(d_roots)
-        check(L.msgpu_tree_from_digests(ctx.h, 1, hh, pp, _C.byref(th), r32.ctypes.data_as(_C.c_void_p)))
-        ctx.free(d_roots)
-        top, root = ProverData(ctx, th, bytes(r32)), bytes(r32)
-    t.append(time.perf_counter())
-    if timings is not None:
-        for k, name in enumerate(["upload", "lde", "all_to_all", "leaf_hash_subtree", "top"]):
-            timings[name] = timings.get(name, 0.0) + (t[k + 1] - t[k]) * 1e3
-    wc = WideCommit(ctx, comm, local, top, root, H, widths, recv)
-    wc.lde_block = d_lde  # this rank's column block of the LDE (H x w), kept for prove_wide_sharded
-    return root, wc
-
-
-def prove_wide_sharded(ctx, comm, prover, block, width, log_blowup, claims=None, timings=None):
-    """`prove()` of a system with ONE wide, lookup-free circuit (BASELINE configs[2]) whose trace arrives as column blocks, one
-    per rank. The stage-1 commitment -- upload, LDE and leaf hashing of 256 columns, 83 % of the single-GPU proof -- is made
-    by all ranks (commit_wide_sharded); rank 0 then gathers the LDE blocks and the shards' digest layers over NVLink,
-    assembles ordinary prover data (msgpu_pdata_from_parts) and runs the remaining stages alone. Returns the proof bytes on
-    rank 0 (None elsewhere); they equal the single-GPU proof byte for byte. `prover` is a `Prover` on rank 0, None elsewhere."""
-    L = ctx.L
-    t = [time.perf_counter()]
-    root, wc = commit_wide_sharded(ctx, comm, block, width, log_blowup, timings=timings, keep_block=True)
-    t.append(time.perf_counter())
-    world, rank = comm.world, comm.rank
-    H, widths = wc.lde_height, wc.widths
-    dg, nd = _C.c_void_p(), _C.c_uint64()
-    check(L.msgpu_pdata_digests(wc.local.h, _C.byref(dg), _C.byref(nd)))
-    nd = int(nd.value)
-    if rank == 0:
-        blocks = [wc.lde_block] + [ctx.malloc(H * widths[r] * 8) for r in range(1, world)]
-        parts = [dg.value] + [ctx.malloc(nd * 32) for r in range(1, world)]
-        gathers = [(r, blocks[r], parts[r]) for r in range(1, world)]
-    else:
-        gathers = [(rank, wc.lde_block, dg.value)]
-    for r, block_ptr, part_ptr in gathers:  # rank r's LDE block and digest layer -> rank 0
-        comm.sendrecv_dev(block_ptr, H * widths[r] * 8, r, 0)
-        comm.sendrecv_dev(part_ptr, nd * 32, r, 0)
-    t.append(time.perf_counter())
-    if rank == 0:
-        pd, r32 = _C.c_void_p(), np.zeros(32, dtype=np.uint8)
-        ba = (_C.c_void_p * world)(*blocks)
-        wa = (_C.c_uint64 * world)(*widths)
-        pa = (_C.c_void_p * world)(*parts)
-        check(L.msgpu_pdata_from_parts(ctx.h, world, ba, wa, H, world, pa, _C.byref(pd), r32.ctypes.data_as(_C.c_void_p)))
-        for r in range(1, world):
-            ctx.free(blocks[r])
-            ctx.free(parts[r])
-        if bytes(r32) != root:
-            L.msgpu_pdata_free(pd)
-            raise RuntimeError("assembled commitment differs from the sharded one")
-    ctx.free(wc.lde_block)
-    wc.lde_block = None
-    wc.free()  # the row shard and its subtree are not needed any more: on rank 0 the assembled prover data serves the openings
-    t.append(time.perf_counter())
-    proof = prover.prove_precommitted(pd, [H >> log_blowup], claims) if rank == 0 else None
-    t.append(time.perf_counter())
-    if timings is not None:
-        names = ["commit_sharded", "gather"] + (["assemble", "prove_rest"] if rank == 0 else [])
-        for k, name in enumerate(names):
-            timings[name] = (t[k + 1] - t[k]) * 1e3
-    return proof

@@ -118,9 +118,6 @@ void msh_u32add_workload_seeded(uint64_t num_adds, uint32_t seed_a, uint32_t see
             for (int k = 0; k < 4; k++) claims_out[4 * i + k] = w.claims[i][k].v;
 }
 void msh_wide_trace(uint64_t row0, uint64_t rows, uint64_t width, uint64_t* out) { circuits::wide_cubic_fill(out, row0, rows, width); }
-void msh_wide_trace_block(uint64_t row0, uint64_t rows, uint64_t width, uint64_t c0, uint64_t c1, uint64_t* out) {
-    circuits::wide_cubic_fill_block(out, row0, rows, width, c0, c1);
-}
 void msh_fib_trace(uint64_t rows, uint64_t* out) {
     Matrix m = circuits::fib_cubic_trace(rows);
     for (size_t i = 0; i < m.values.size(); i++) out[i] = m.values[i].v;
@@ -216,17 +213,6 @@ int msh_rowshard_commit(msh_prover* p, const uint64_t* const* mats, const uint64
         Digest root{};
         auto h = be->commit_blocks(blocks, root);
         memcpy(root32, root.data(), 32);
-        return 0;
-    } catch (const std::exception& e) {
-        g_err = e.what();
-        return -1;
-    }
-}
-// The next msh_prove on this prover adopts `pd` (from msgpu_pdata_from_parts) as its stage-1 commitment instead of committing
-// the traces; pass NULL trace pointers with the true heights. The prover owns `pd` from here on.
-int msh_prover_inject_stage1(msh_prover* p, msgpu_pdata* pd) {
-    try {
-        p->backend->inject_stage1(pd);
         return 0;
     } catch (const std::exception& e) {
         g_err = e.what();

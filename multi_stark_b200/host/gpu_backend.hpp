@@ -308,29 +308,9 @@ class GpuBackend : public ProverBackend {
         return std::make_shared<GpuPcsHandle>(PdataPtr(pd));
     }
 
-    // The next proof's stage-1 commitment was made elsewhere (one wide matrix committed by column blocks over several GPUs and
-    // assembled with msgpu_pdata_from_parts): adopt it instead of uploading and committing the traces. Only for systems whose
-    // stage-2 construction does not read the main traces (no lookups): they are not on this device.
-    void inject_stage1(msgpu_pdata* pd) { injected_.reset(pd); }
-
     PcsHandlePtr commit_stage1(const std::vector<size_t>& circuits, const std::vector<MatrixView>& traces, Digest& root) override {
         end_proof();
         active_ = circuits;
-        if (injected_) {
-            auto h = std::make_shared<GpuPcsHandle>(std::move(injected_));
-            if (h->num_matrices() != traces.size()) throw GpuError("injected stage-1 commitment: matrix count does not match the active circuits");
-            for (size_t i = 0; i < traces.size(); i++) {
-                if (h->matrix_height(i) != (traces[i].height() << shape_.log_blowup()) || h->matrix_width(i) != traces[i].width)
-                    throw GpuError("injected stage-1 commitment: matrix shape does not match the trace");
-                if (shape_.circuits[circuits[i]].num_lookups != 0)
-                    throw GpuError("injected stage-1 commitment: a circuit with lookups needs its main trace on the device");
-                trace_rows_.push_back(traces[i].height());
-            }
-            trace_dev_.resize(traces.size());
-            announced_ = ClaimsView();
-            gpu_check(msgpu_pdata_root(h->pd, root.data()));
-            return h;
-        }
         std::vector<const uint64_t*> ptrs;
         std::vector<uint64_t> hs, ws;
         for (auto& m : traces) {
@@ -502,7 +482,6 @@ class GpuBackend : public ProverBackend {
         prefetched_n_ = cl.size();
         prefetched_len_ = len;
     }
-    PdataPtr injected_;
     ClaimsView announced_;
     const void* prefetched_from_ = nullptr;
     size_t prefetched_n_ = 0, prefetched_len_ = 0;

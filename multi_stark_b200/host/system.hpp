@@ -253,16 +253,6 @@ inline void wide_cubic_fill(u64* out, size_t row0, size_t rows, size_t width) {
         }
 }
 
-// columns [c0, c1) of the same trace as a dense rows x (c1 - c0) matrix (one rank's block of a column-sharded commit)
-inline void wide_cubic_fill_block(u64* out, size_t row0, size_t rows, size_t width, size_t c0, size_t c1) {
-    const size_t wb = c1 - c0;
-    for (size_t r = 0; r < rows; r++)
-        for (size_t c = c0; c < c1; c++) {
-            Fp a(splitmix64((u64)(row0 + r) * width + (c & ~(size_t)1)) % GL_P);
-            out[r * wb + (c - c0)] = (c & 1) ? (a * a * a).v : a.v;
-        }
-}
-
 }  // namespace circuits
 
 // Named systems used by bench.py and the tests (circuit order = matrix order inside every commitment).

@@ -168,16 +168,9 @@ def fib_trace(rows):
     return out
 
 
-def wide_trace(rows, width, row0=0, out=None, cols=None):
-    """Trace of the "wide:W" system (BASELINE configs[2]): column 2k = splitmix64(row * W + 2k) mod p, column 2k+1 its cube.
-    cols = (c0, c1): only that column block, as a dense rows x (c1 - c0) matrix (one rank's share of a column-sharded commit)."""
+def wide_trace(rows, width, row0=0, out=None):
+    """Trace of the "wide:W" system (BASELINE configs[2]): column 2k = splitmix64(row * W + 2k) mod p, column 2k+1 its cube."""
     H = _ffi.host_lib()
-    if cols is not None:
-        c0, c1 = cols
-        if out is None:
-            out = np.zeros((rows, c1 - c0), dtype=np.uint64)
-        H.msh_wide_trace_block(row0, rows, width, c0, c1, out.ctypes.data_as(C.c_void_p))
-        return out
     if out is None:
         out = np.zeros((rows, width), dtype=np.uint64)
     H.msh_wide_trace(row0, rows, width, out.ctypes.data_as(C.c_void_p))
@@ -346,16 +339,6 @@ class Prover(ProverBase):
         n = int(self.H.msh_last_transcript(ch.ctypes.data_as(C.c_void_p), 128, idx.ctypes.data_as(C.c_void_p), 4096,
                                            nidx.ctypes.data_as(C.c_void_p)))
         return [(int(ch[2 * i]), int(ch[2 * i + 1])) for i in range(n)], [int(v) for v in idx[:int(nidx[0])]]
-
-    def prove_precommitted(self, stage1_pdata, heights, claims=None):
-        """prove() whose stage-1 commitment was made elsewhere (`msgpu_pdata_from_parts`: one wide matrix committed by column
-        blocks over several GPUs). `stage1_pdata`: raw msgpu_pdata handle, adopted; heights[i]: trace rows of circuit i. Only
-        for lookup-free circuits (the stage-2 construction of a circuit with lookups reads its main trace)."""
-        if len(heights) != self.system.num_circuits:
-            raise _ffi.MsgpuError(-1, "expected one height per circuit")
-        if self.H.msh_prover_inject_stage1(self.h, stage1_pdata) != 0:
-            raise self._error(-1)
-        return self._prove([None] * len(heights), heights, claims)
 
     def __del__(self):
         try:

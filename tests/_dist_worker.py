@@ -1,7 +1,8 @@
 """One rank of a sharded proof (tests/test_gpu_dist_prove.py, tools/dist_prove.py). Launched with RANK / WORLD_SIZE /
 MASTER_ADDR / MASTER_PORT in the environment. backend gloo: every rank uses cuda:0 (single-GPU box), device buffers are staged
 through the host; backend nccl: rank r uses cuda:r and device buffers travel over NVLink.
-argv: backend kind log_heights(comma separated; first = byte table is implicit) owners(comma separated or "auto") out_prefix [params json]"""
+argv: backend kind log_heights(comma separated; first = byte table is implicit) owners(comma separated or "auto") out_prefix [params json]
+kind "commit:W" commits one 2^log_height x W matrix over the row shards instead of proving: the result files then hold roots."""
 import json
 import os
 import sys
@@ -31,6 +32,11 @@ def main():
     stream = torch.cuda.Stream()
     torch.cuda.set_stream(stream)
     ctx = ms.GpuContext(dev, stream=stream.cuda_stream)
+    if kind.startswith("commit:"):
+        commit_rows(ctx, int(kind[7:]), int(lhs), params, out_prefix, rank)
+        ctx.close()
+        dist.destroy_process_group()
+        return
     system = ms.System(kind, **params)
     log_heights = [int(x) for x in lhs.split(",")]
     if kind.startswith("multi:"):
@@ -100,6 +106,27 @@ def main():
     prover.close()
     ctx.close()
     dist.destroy_process_group()
+
+
+def commit_rows(ctx, width, log_rows, params, out_prefix, rank):
+    """`Pcs::commit` of one matrix of any width by RowShardProver.commit, each rank handing over only the rows it reads; rank 0
+    also commits the whole matrix on one GPU (GpuPcs) for reference."""
+    h = 1 << log_rows
+    whole = np.random.default_rng(h * width).integers(0, ms.P, size=(h, width), dtype=np.uint64)
+    prover = msd.RowShardProver(ctx, ms.System("fib", **params))  # the commitment reads only the system's log_blowup
+    row0, rows = prover.block_rows(h, width)
+    root = prover.commit([whole[row0:row0 + rows]], [h], [width], host=True)
+    with open("%s.rank%d.proof" % (out_prefix, rank), "wb") as f:
+        f.write(root)
+    with open("%s.rank%d.json" % (out_prefix, rank), "w") as f:
+        json.dump({"rank": rank, "rows": rows, "bytes_dev": prover.bytes_dev, "launches": ctx.launches}, f)
+    if rank == 0:
+        want, pd = ms.GpuPcs(ctx, params["log_blowup"]).commit([whole])
+        pd.free()
+        with open("%s.single.proof" % out_prefix, "wb") as f:
+            f.write(bytes(want))
+    dist.barrier()
+    prover.close()
 
 
 if __name__ == "__main__":

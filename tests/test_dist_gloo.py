@@ -140,14 +140,3 @@ def test_assign_owners_keeps_height_classes_together():
         if w >= 2:
             assert own[1] == own[3] and own[1] != own[2]  # the two 2^20 circuits together, the 2^19 one elsewhere
     assert msd.assign_owners(heights, 2) == msd.assign_owners(heights, 2)
-
-
-def test_column_blocks_cover_the_width():
-    from multi_stark_b200 import dist as msd
-    for width in (1, 7, 8, 200, 256):
-        for w in (1, 2, 4, 8):
-            blocks = msd.column_blocks(width, w)
-            assert blocks[0][0] == 0 and blocks[-1][1] == width and len(blocks) == w
-            assert all(a[1] == b[0] for a, b in zip(blocks, blocks[1:]))
-            sizes = [c1 - c0 for c0, c1 in blocks]
-            assert max(sizes) - min(sizes) <= 1

@@ -533,49 +533,3 @@ def test_column_blocks_refusals(gpu):
         assert L.msgpu_interleave_column_blocks_dev(ctx.h, C.c_void_p(buf), 4, 0, _u64p(w17), C.c_void_p(buf)) != 0
     finally:
         ctx.free(buf)
-
-
-@pytest.mark.gpu
-def test_pdata_from_parts_every_part_count(gpu):
-    """msgpu_pdata_from_parts with 1 .. height parts (2^13, so the top levels over the parts' roots take more than one
-    k_merkle_subtree launch at 2^13 parts): root, every digest layer, rows and paths are those of one commitment of the
-    whole matrix."""
-    ms, ctx = gpu
-    L = ctx.L
-    log_h = 13
-    H = 1 << log_h
-    widths = [2, 1, 4]
-    rng = np.random.default_rng(13)
-    m = rng.integers(0, P, size=(H, sum(widths)), dtype=np.uint64)
-    layers = R.mmcs_commit([m])
-    cuts = np.cumsum([0] + widths)
-    blocks = [ctx.upload(np.ascontiguousarray(m[:, a:b])) for a, b in zip(cuts, cuts[1:])]
-    idx = np.array([0, 1, H - 1, 4097, 4097, 77], dtype=np.uint64)
-    want_rows = np.stack([R.open_rows([m], int(i)) for i in idx])
-    want_paths = np.stack([R.open_path(layers, int(i)) for i in idx])
-    try:
-        for lp in range(0, log_h + 1):
-            n_parts, shard = 1 << lp, H >> lp
-            # part p's digest layers: its slice of every layer of the whole tree, leaves first
-            parts = np.concatenate([np.concatenate([layers[l][(p * shard) >> l:((p + 1) * shard) >> l] for l in range(log_h - lp + 1)])
-                                    for p in range(n_parts)])
-            dp = ctx.upload(parts)
-            per = (2 * shard - 1) * 32
-            out, root = C.c_void_p(), np.zeros(32, dtype=np.uint8)
-            rc = L.msgpu_pdata_from_parts(ctx.h, len(blocks), (C.c_void_p * len(blocks))(*blocks),
-                                          (C.c_uint64 * len(widths))(*widths), H, n_parts,
-                                          (C.c_void_p * n_parts)(*[dp + p * per for p in range(n_parts)]), C.byref(out), _u64p(root))
-            ctx.free(dp)
-            assert rc == 0, n_parts
-            pd = ms.ProverData(ctx, out, root)
-            assert bytes(root) == layers[-1][0].tobytes(), n_parts
-            got = pd.layers()
-            for l, (g, e) in enumerate(zip(got, layers)):
-                assert np.array_equal(g, e), (n_parts, l)
-            assert np.array_equal(pd.read_rows(0), m)
-            rows, paths = pd.open_batch(idx)
-            assert np.array_equal(rows, want_rows) and np.array_equal(paths, want_paths), n_parts
-            pd.free()
-    finally:
-        for b in blocks:
-            ctx.free(b)

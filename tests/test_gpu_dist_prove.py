@@ -8,7 +8,6 @@ import socket
 import subprocess
 import sys
 
-import numpy as np
 import pytest
 
 from tests import _oracle as orc
@@ -83,57 +82,3 @@ def test_same_height_on_two_ranks_is_refused(tmp_path):
     with pytest.raises(AssertionError) as e:
         run_world(tmp_path, 2, "multi:2", [10, 10], "0,0,1", dict(log_blowup=1, num_queries=5))
     assert "must live on one rank" in str(e.value)
-
-
-def run_wide(tmp_path, world, log_rows, width, lb):
-    port = free_port()
-    prefix = str(tmp_path / "wide")
-    procs = []
-    for r in range(world):
-        env = dict(os.environ, RANK=str(r), WORLD_SIZE=str(world), LOCAL_RANK=str(r), MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
-        procs.append(subprocess.Popen([sys.executable, os.path.join(ROOT, "tests", "_wide_worker.py"), "gloo", str(log_rows), str(width),
-                                       str(lb), prefix], env=env, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True))
-    outs = [p.communicate(timeout=600)[0] for p in procs]
-    if any(p.returncode != 0 for p in procs):
-        raise AssertionError("\n".join("---- rank %d rc %s ----\n%s" % (r, p.returncode, outs[r][-2500:]) for r, p in enumerate(procs)))
-    infos = [json.load(open("%s.rank%d.json" % (prefix, r))) for r in range(world)]
-    opens = [np.load("%s.rank%d.npz" % (prefix, r)) for r in range(world)]
-    return infos, opens
-
-
-@pytest.mark.parametrize("world,log_rows,width,lb", [(2, 10, 256, 2), (4, 8, 200, 1), (2, 6, 7, 3), (4, 12, 130, 1)])
-def test_column_block_sharded_commit_matches_single_gpu(tmp_path, world, log_rows, width, lb):
-    """SURVEY 8e partitioning B (BASELINE configs[2]): one wide matrix, column blocks per rank, all-to-all to row shards.
-    Root, opened rows and sibling paths must equal the single-GPU `Pcs::commit` of the whole matrix."""
-    infos, opens = run_wide(tmp_path, world, log_rows, width, lb)
-    assert all(i["errors"] == [] for i in infos)
-    assert len({i["root"] for i in infos}) == 1
-    assert infos[0]["root"] == infos[0]["single_root"], "sharded root differs from the single-GPU commitment"
-    assert infos[0]["openings_identical"]
-    for o in opens[1:]:
-        assert np.array_equal(o["rows"], opens[0]["rows"]) and np.array_equal(o["paths"], opens[0]["paths"])
-    assert sum(i["bytes_dev"] for i in infos) > 0
-
-
-@pytest.mark.parametrize("world,log_rows,width,lb", [(2, 8, 16, 2), (4, 7, 8, 2), (2, 10, 64, 1)])
-def test_wide_air_proved_from_column_blocks(tmp_path, oracle, world, log_rows, width, lb):
-    """BASELINE configs[2]: the wide AIR's trace arrives as column blocks, the stage-1 commitment is made by all ranks, rank 0
-    assembles ordinary prover data from the gathered blocks + subtree digests and finishes the proof. Byte-identical to the
-    single-GPU proof, accepted by the restated verifier."""
-    port = free_port()
-    prefix = str(tmp_path / "widep")
-    procs = []
-    for r in range(world):
-        env = dict(os.environ, RANK=str(r), WORLD_SIZE=str(world), LOCAL_RANK=str(r), MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
-        procs.append(subprocess.Popen([sys.executable, os.path.join(ROOT, "tests", "_wide_prove_worker.py"), "gloo", str(log_rows),
-                                       str(width), str(lb), prefix, "1", "20"], env=env, stdout=subprocess.PIPE,
-                                      stderr=subprocess.STDOUT, text=True))
-    outs = [p.communicate(timeout=600)[0] for p in procs]
-    if any(p.returncode != 0 for p in procs):
-        raise AssertionError("\n".join("---- rank %d rc %s ----\n%s" % (r, p.returncode, outs[r][-2500:]) for r, p in enumerate(procs)))
-    info = json.load(open(prefix + ".rank0.json"))
-    assert info["errors"] == [] and info["identical"], "sharded proof differs from the single-GPU proof"
-    proof = open(prefix + ".sharded.proof", "rb").read()
-    S = orc.OracleSystem(oracle, "wide:%d" % width, log_blowup=lb, num_queries=20)
-    assert S.verify([], proof) == "Ok"
-    S.close()

@@ -24,6 +24,10 @@ CASES = [
     (2, "fib", [8], dict(log_blowup=2, num_queries=8)),                             # 3 columns >= 2 ranks: next-row constraints
     (2, "mixed", [9, 8], dict(log_blowup=2, num_queries=12)),
     (2, "u32_add", [10], dict(log_blowup=1, num_queries=10, commit_pow_bits=2, query_pow_bits=2)),  # host-loop FRI on the owner
+    (2, "wide:16", [8], dict(log_blowup=2, num_queries=20)),
+    (4, "wide:8", [8], dict(log_blowup=2, num_queries=20)),                         # the least height split over 4 ranks
+    (2, "wide:64", [10], dict(log_blowup=1, num_queries=20)),
+    (2, "wide:256", [10], dict(log_blowup=2, num_queries=20)),                      # BASELINE configs[2]'s width
 ]
 
 
@@ -34,4 +38,15 @@ def test_rowsharded_proof_is_byte_identical(tmp_path, oracle, world, kind, log_h
         assert proofs[r] == single, "rank %d's proof differs from the single-GPU proof" % r
     assert all(i["launches"] > 0 for i in infos)
     # exchanged device bytes stay a fraction of the committed data: nothing of the size of a matrix is gathered on one rank
+    assert all(i["bytes_dev"] > 0 for i in infos)
+
+
+@pytest.mark.parametrize("world,log_rows,width,lb", [(4, 8, 200, 1), (2, 7, 7, 3), (4, 12, 130, 1)])
+def test_rowsharded_commit_of_any_width(tmp_path, world, log_rows, width, lb):
+    """RowShardProver.commit of one matrix whose width need not be a wide:W circuit's: every rank's root equals the single-GPU
+    `Pcs::commit` of the whole matrix"""
+    roots, single, infos = run_world(tmp_path, world, "commit:%d" % width, [log_rows], "rowshard", dict(log_blowup=lb))
+    for r in range(world):
+        assert roots[r] == single, "rank %d's root differs from the single-GPU commitment" % r
+    assert all(i["rows"] == (1 << log_rows) // world for i in infos), "the matrix was not split by rows"
     assert all(i["bytes_dev"] > 0 for i in infos)
