@@ -55,7 +55,6 @@ int msgpu_malloc(msgpu_ctx* ctx, size_t bytes, void** dptr);
 int msgpu_free(msgpu_ctx* ctx, void* dptr);
 int msgpu_memcpy_h2d(msgpu_ctx* ctx, void* dst_dev, const void* src_host, size_t bytes);
 int msgpu_memcpy_d2h(msgpu_ctx* ctx, void* dst_host, const void* src_dev, size_t bytes);
-int msgpu_memcpy_d2d(msgpu_ctx* ctx, void* dst_dev, const void* src_dev, size_t bytes); /* stream-ordered, does not wait */
 int msgpu_host_alloc(size_t bytes, void** hptr); /* pinned host memory */
 int msgpu_host_free(void* hptr);
 /* Page-lock host memory the caller owns (the Vec behind a p3 `RowMajorMatrix<Goldilocks>`), so that the host-pointer entry points
@@ -150,7 +149,6 @@ int msgpu_pdata_class_digests(const msgpu_pdata* pd, uint64_t k, uint64_t* lde_h
 int msgpu_tree_from_digests(msgpu_ctx* ctx, uint64_t n_classes, const uint64_t* lde_heights, const uint8_t* const* digests_dev,
                             msgpu_pdata** out, uint8_t* root32);
 uint64_t msgpu_pdata_max_height(const msgpu_pdata* pd);
-int msgpu_pdata_root(const msgpu_pdata* pd, uint8_t* root32);
 /* DEVICE pointer to all digest layers of a tree, back to back from the leaves up (2 * max_height - 1 digests) */
 int msgpu_pdata_digests(const msgpu_pdata* pd, uint8_t** dev_ptr, uint64_t* n_digests);
 /* Mmcs::commit on HOST matrices as they are (no LDE): used for the FRI layers' ExtensionMmcs rows
@@ -313,8 +311,7 @@ void msgpu_open_free(msgpu_open* op);
  *   shard one trace step further) and the tail of the quotient stage on the rank that gathered the values.
  * msgpu_open_begin_shard .. msgpu_open_finish_values: Pcs::open where every rank evaluates / reduces the rows it holds; the
  *   barycentric sums are added over the ranks by the caller, the reduced-opening shards are added into the FRI owner's vectors
- *   (msgpu_open_input_dev + msgpu_ext_add_dev). modes[r]: 0 = round held here in full, 1 = row shard `shard` of `n_shards`
- *   (the prover data holds the shard), 2 = held elsewhere (msgpu_pdata_placeholder carries the global shapes). */
+ *   (msgpu_open_input_dev + msgpu_ext_add_dev). Every prover data holds row shard `shard` of `n_shards` of its matrices. */
 int msgpu_pack_column_blocks_dev(msgpu_ctx* ctx, const uint64_t* src, uint64_t rows, uint64_t width, uint64_t n_blocks,
                                  const uint64_t* c0, const uint64_t* c1, uint64_t* dst);
 int msgpu_interleave_column_blocks_dev(msgpu_ctx* ctx, const uint64_t* src, uint64_t rows, uint64_t n_blocks, const uint64_t* widths,
@@ -328,12 +325,11 @@ int msgpu_quotient_values_shard(msgpu_ctx* ctx, const msgpu_program* prog, const
 int msgpu_extract_columns_dev(msgpu_ctx* ctx, const uint64_t* src, uint64_t rows, uint64_t width, uint64_t c0, uint64_t c1, uint64_t* dst);
 int msgpu_quotient_finish(msgpu_ctx* ctx, const uint64_t* values_stored_dev, uint32_t log_n, uint32_t log_quotient_degree,
                           uint32_t log_blowup, uint64_t** lde_out_dev);
-int msgpu_open_begin_shard(msgpu_ctx* ctx, uint64_t n_rounds, const msgpu_pdata* const* pds, const uint32_t* modes, uint32_t shard,
-                           uint32_t n_shards, int fri_owner, const uint64_t* n_points, const uint64_t* points, uint32_t log_blowup,
+int msgpu_open_begin_shard(msgpu_ctx* ctx, uint64_t n_rounds, const msgpu_pdata* const* pds, uint32_t shard, uint32_t n_shards,
+                           int fri_owner, const uint64_t* n_points, const uint64_t* points, uint32_t log_blowup,
                            msgpu_open** out, uint64_t* n_values, uint64_t* n_sums);
 int msgpu_open_sums(msgpu_open* op, uint64_t* out);
 int msgpu_open_finish_values(msgpu_open* op, const uint64_t* total_sums);
-int msgpu_pdata_placeholder(msgpu_ctx* ctx, uint64_t n_mats, const uint64_t* heights, const uint64_t* widths, msgpu_pdata** out);
 int msgpu_ext_add_dev(msgpu_ctx* ctx, uint64_t* dst, const uint64_t* src, uint64_t n_ext);
 int msgpu_ext_add_scalar_dev(msgpu_ctx* ctx, uint64_t* v, uint64_t n_ext, const uint64_t* c2);
 
@@ -352,23 +348,20 @@ int msgpu_peers_segment_create(msgpu_peers* p, uint64_t bytes, uint8_t* handle64
 int msgpu_peers_segment_open(msgpu_peers* p, const uint8_t* handles);
 /* ranks inside ONE process (no IPC): bases[e] = rank e's window address (msgpu_peers_ptr of ITS object, offset 0) */
 int msgpu_peers_segment_open_local(msgpu_peers* p, void* const* bases);
-uint64_t msgpu_peers_num_segments(const msgpu_peers* p);
 int msgpu_peers_alloc(msgpu_peers* p, uint64_t bytes, uint32_t* segment, uint64_t* offset);
 int msgpu_peers_free_block(msgpu_peers* p, uint32_t segment, uint64_t offset);
 void* msgpu_peers_ptr(const msgpu_peers* p, uint32_t segment, uint64_t offset, int32_t peer);
 /* stream-ordered: work enqueued afterwards sees everything every peer wrote (and enqueued) before ITS call */
 int msgpu_peers_barrier(msgpu_peers* p);
-/* all-gather by remote stores: `bytes` from src_dev land at offset + rank * bytes of the block on every peer */
-int msgpu_peers_put(msgpu_peers* p, const void* src_dev, uint32_t segment, uint64_t offset, uint64_t bytes);
 /* the 32-byte subtree root of a row-sharded commitment -> slot `rank` on every peer; *gathered_dev = world x 32 bytes (local),
  * complete after the next msgpu_peers_barrier */
 int msgpu_peers_put_root(msgpu_peers* p, const uint8_t* root_dev, uint8_t** gathered_dev);
 /* after a stream synchronisation: MSGPU_ERR_CUDA if a barrier timed out */
 int msgpu_peers_check(msgpu_peers* p);
-/* The two exchanges of a row-sharded Pcs::commit (src/prover.rs:350,419 on N GPUs): row blocks -> the owners' column blocks
- * (remote stores) before the column-local LDE, column blocks of the LDE -> this rank's row shard (remote loads) after it. */
+/* The first exchange of a row-sharded Pcs::commit (src/prover.rs:350,419 on N GPUs): row blocks -> the owners' column blocks
+ * (remote stores) before the column-local LDE. The second, column blocks of the LDE -> this rank's row shard (remote loads), is
+ * the leaf-hash pass of msgpu_commit_ldes_blocks_dev over msgpu_peers_ptr addresses. */
 int msgpu_peers_pack_push(msgpu_peers* p, const uint64_t* src_dev, uint64_t rows, uint64_t width, uint32_t segment, uint64_t offset);
-int msgpu_peers_pull_interleave(msgpu_peers* p, uint32_t segment, uint64_t offset, uint64_t rows, uint64_t width, uint64_t* dst_dev);
 void msgpu_peers_destroy(msgpu_peers* p);
 
 /* ---- transcript helper ---------------------------------------------------------------------------

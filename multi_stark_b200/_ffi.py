@@ -52,7 +52,6 @@ SIGNATURES = {
     "msgpu_pdata_class_digests": (C.c_int, [C.c_void_p, C.c_uint64, c_u64p, c_vpp]),
     "msgpu_tree_from_digests": (C.c_int, [C.c_void_p, C.c_uint64, c_u64p, c_vpp, c_vpp, C.c_void_p]),
     "msgpu_pdata_max_height": (C.c_uint64, [C.c_void_p]),
-    "msgpu_pdata_root": (C.c_int, [C.c_void_p, C.c_void_p]),
     "msgpu_pdata_digests": (C.c_int, [C.c_void_p, c_vpp, c_u64p]),
     "msgpu_mmcs_commit": (C.c_int, [C.c_void_p, c_vpp, c_u64p, c_u64p, C.c_uint64, c_vpp, C.c_void_p]),
     "msgpu_pdata_free": (None, [C.c_void_p]),
@@ -100,11 +99,10 @@ SIGNATURES = {
                                               C.c_uint64, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "msgpu_extract_columns_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint64, C.c_void_p]),
     "msgpu_quotient_finish": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p]),
-    "msgpu_open_begin_shard": (C.c_int, [C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_int, C.c_void_p,
-                                         C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "msgpu_open_begin_shard": (C.c_int, [C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint32, C.c_uint32, C.c_int, C.c_void_p, C.c_void_p,
+                                         C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "msgpu_open_sums": (C.c_int, [C.c_void_p, C.c_void_p]),
     "msgpu_open_finish_values": (C.c_int, [C.c_void_p, C.c_void_p]),
-    "msgpu_pdata_placeholder": (C.c_int, [C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p]),
     "msgpu_ext_add_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64]),
     "msgpu_ext_add_scalar_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]),
     "msgpu_host_register": (C.c_int, [C.c_void_p, C.c_size_t]),
@@ -114,21 +112,17 @@ SIGNATURES = {
     "msgpu_selectors_on_coset": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "msgpu_commit_ldes_blocks_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p,
                                                C.c_int, C.c_void_p, C.c_void_p]),
-    "msgpu_memcpy_d2d": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t]),
     "msgpu_peers_create": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p]),
     "msgpu_peers_segment_create": (C.c_int, [C.c_void_p, C.c_uint64, C.c_void_p]),
     "msgpu_peers_segment_open": (C.c_int, [C.c_void_p, C.c_void_p]),
     "msgpu_peers_segment_open_local": (C.c_int, [C.c_void_p, C.c_void_p]),
-    "msgpu_peers_num_segments": (C.c_uint64, [C.c_void_p]),
     "msgpu_peers_alloc": (C.c_int, [C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]),
     "msgpu_peers_free_block": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint64]),
     "msgpu_peers_ptr": (C.c_void_p, [C.c_void_p, C.c_uint32, C.c_uint64, C.c_int32]),
     "msgpu_peers_barrier": (C.c_int, [C.c_void_p]),
-    "msgpu_peers_put": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint64, C.c_uint64]),
     "msgpu_peers_put_root": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "msgpu_peers_check": (C.c_int, [C.c_void_p]),
     "msgpu_peers_pack_push": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint64]),
-    "msgpu_peers_pull_interleave": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint64, C.c_uint64, C.c_uint64, C.c_void_p]),
     "msgpu_peers_destroy": (None, [C.c_void_p]),
 }
 

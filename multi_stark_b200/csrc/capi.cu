@@ -234,11 +234,6 @@ int msgpu_memcpy_d2h(msgpu_ctx* h, void* dst, const void* src, size_t bytes) {
         h->c.sync();
     });
 }
-int msgpu_memcpy_d2d(msgpu_ctx* h, void* dst, const void* src, size_t bytes) {
-    return guard([&] {
-        if (bytes) MSG_CUDA(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, h->c.stream));
-    });
-}
 int msgpu_host_alloc(size_t bytes, void** hptr) {
     return guard([&] { MSG_CUDA(cudaHostAlloc(hptr, bytes ? bytes : 8, cudaHostAllocDefault)); });
 }
@@ -568,12 +563,6 @@ int msgpu_tree_from_digests(msgpu_ctx* h, uint64_t n_classes, const uint64_t* ld
     });
 }
 uint64_t msgpu_pdata_max_height(const msgpu_pdata* pd) { return pd->max_height; }
-int msgpu_pdata_root(const msgpu_pdata* pd, uint8_t* root32) {
-    return guard([&] {
-        MSG_REQUIRE(pd && root32 && pd->digests, "pdata_root: prover data without a tree");
-        memcpy(root32, pd->root, 32);
-    });
-}
 int msgpu_pdata_digests(const msgpu_pdata* pd, uint8_t** dev_ptr, uint64_t* n_digests) {
     return guard([&] {
         MSG_REQUIRE(pd && pd->digests && dev_ptr && n_digests, "pdata_digests: prover data without a tree");
@@ -585,8 +574,10 @@ int msgpu_pack_column_blocks_dev(msgpu_ctx* h, const uint64_t* src, uint64_t row
                                  const uint64_t* c1, uint64_t* dst) {
     return guard([&] {
         MSG_REQUIRE(src && dst && c0 && c1, "pack_column_blocks: null argument");
+        std::vector<u64*> blocks;
+        for (u64 b = 0; b < n_blocks; b++) blocks.push_back((u64*)dst + rows * c0[b]);
         StageScope ss(h->c, "exchange");
-        pack_column_blocks(h->c, (const u64*)src, rows, width, std::vector<u64>(c0, c0 + n_blocks), std::vector<u64>(c1, c1 + n_blocks), (u64*)dst);
+        pack_column_blocks(h->c, (const u64*)src, rows, width, std::vector<u64>(c0, c0 + n_blocks), std::vector<u64>(c1, c1 + n_blocks), blocks);
     });
 }
 int msgpu_interleave_column_blocks_dev(msgpu_ctx* h, const uint64_t* src, uint64_t rows, uint64_t n_blocks, const uint64_t* widths,

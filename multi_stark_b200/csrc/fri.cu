@@ -420,9 +420,9 @@ struct msgpu_open {
         u32 log_h;
         std::vector<msh::Fp2> points;
         std::vector<std::vector<msh::Fp2>> values;  // [point][column]
-        // row shards (msgpu_open_begin_shard): this rank holds stored rows [row0, row0 + rows) of the matrix at `ptr`;
-        // rows = 0: the matrix lives elsewhere (shapes only). Unsharded: row0 = 0, rows = height.
-        u64 row0 = 0, rows = 0;
+        // row shards (msgpu_open_begin_shard): this rank holds stored rows [row0, row0 + rows) of the matrix at `ptr`.
+        // Unsharded: row0 = 0, rows = height.
+        u64 row0, rows;
     };
     msg::Ctx* ctx = nullptr;
     u32 log_blowup = 0;
@@ -517,7 +517,6 @@ static void evaluate_all(Ctx& c, msgpu_open* op) {
     //    (point, height, row range) of the rows this rank holds
     for (auto& round : op->rounds)
         for (auto& m : round) {
-            if (m.rows == 0) continue;
             for (auto& z : m.points) {
                 bool found = false;
                 for (auto& d : op->invdens) {
@@ -601,7 +600,7 @@ static void reduce_all(Ctx& c, msgpu_open* op, msh::Fp2 alpha) {
     // checked before anything is allocated or copied, so that a refused opening leaves nothing behind
     for (auto& round : op->rounds)
         for (auto& m : round)
-            MSG_REQUIRE(m.points.empty() || m.rows == 0 || reduce_smem(m.width) <= kRedMaxSmem,
+            MSG_REQUIRE(m.points.empty() || reduce_smem(m.width) <= kRedMaxSmem,
                         "open: matrix too wide for the reduced-openings kernel (more than 4266 columns)");
     size_t max_w = 1;
     for (auto& round : op->rounds)
@@ -621,19 +620,14 @@ static void reduce_all(Ctx& c, msgpu_open* op, msh::Fp2 alpha) {
         for (auto& m : round) {
             u32 lh = m.log_h;
             // the FRI owner keeps full-length vectors (the other ranks' shards are added into them); another rank only the
-            // rows it holds, and nothing for heights it has no rows of
+            // rows it holds
             const bool full = !op->sharded || op->fri_owner;
-            if (!ro[lh] && (full || m.rows)) {  // p3 creates the height's vector for every matrix of every round, opened or not
+            if (!ro[lh]) {  // p3 creates the height's vector for every matrix of every round, opened or not
                 ro_len[lh] = full ? m.height : m.rows;
                 ro[lh] = DevBuf(c, ro_len[lh] * 16);
                 MSG_CUDA(cudaMemsetAsync(ro[lh].p, 0, ro_len[lh] * 16, c.stream));
             }
             if (m.points.empty()) continue;
-            if (m.rows == 0) {  // lives elsewhere: only the alpha-power counter of its height advances
-                num_reduced[lh] += m.width * m.points.size();
-                continue;
-            }
-            MSG_REQUIRE(full || ro_len[lh] == m.rows, "open_reduce: shards of one height must cover the same rows");
             for (size_t p0 = 0; p0 < m.points.size(); p0 += kMaxPts) {
                 u32 npts = (u32)std::min<size_t>(kMaxPts, m.points.size() - p0);
                 ReduceParams rp{};
@@ -724,11 +718,9 @@ static void fri_fold_impl(msgpu_open* op, const msh::Fp2* beta, const FriChal* c
     op->cur_committed = false;
 }
 
-// shared by msgpu_open_begin / msgpu_open_begin_shard. modes[r] (sharded only): 0 = the round's matrices are here in full
-// (e.g. the quotient commitment on the rank that built it), 1 = this rank holds row shard `shard` of `n_shards` of every matrix
-// (the prover data holds the SHARDS: heights are 1 / n_shards of the matrices'), 2 = the round lives elsewhere (a placeholder
-// prover data carries the shapes).
-static void open_begin_impl(msgpu_ctx* h, uint64_t n_rounds, const msgpu_pdata* const* pds, const uint32_t* modes, uint32_t shard,
+// shared by msgpu_open_begin / msgpu_open_begin_shard. Sharded: this rank holds row shard `shard` of `n_shards` of every
+// matrix (the prover data holds the SHARDS: heights are 1 / n_shards of the matrices'). Unsharded: shard 0 of 1.
+static void open_begin_impl(msgpu_ctx* h, uint64_t n_rounds, const msgpu_pdata* const* pds, bool sharded, uint32_t shard,
                             uint32_t n_shards, int fri_owner, const uint64_t* n_points, const uint64_t* points, uint32_t log_blowup,
                             msgpu_open** out, uint64_t* n_values) {
     Ctx& c = h->c;
@@ -736,22 +728,18 @@ static void open_begin_impl(msgpu_ctx* h, uint64_t n_rounds, const msgpu_pdata* 
     auto op = std::make_unique<msgpu_open>();
     op->ctx = &c;
     op->log_blowup = log_blowup;
-    op->sharded = modes != nullptr;
+    op->sharded = sharded;
     op->fri_owner = fri_owner != 0;
     size_t mi = 0, pi = 0;
     u64 total = 0;
     const msh::Fp gen_inv = msh::Fp(msh::GL_GENERATOR).inverse();
     for (u64 r = 0; r < n_rounds; r++) {
         MSG_REQUIRE(pds[r], "open_begin: null prover data");
-        const u32 mode = modes ? modes[r] : 0;
-        MSG_REQUIRE(mode <= 2, "open_begin: bad round mode");
         std::vector<msgpu_open::Mat> round;
         for (auto& pm : pds[r]->mats) {
-            const u64 gh = mode == 1 ? pm.height * n_shards : pm.height;
-            msgpu_open::Mat m{pm.ptr, gh, pm.width, ilog2(gh), {}, {}};
-            m.rows = mode == 2 ? 0 : pm.height;
-            m.row0 = mode == 1 ? (u64)shard * pm.height : 0;
-            MSG_REQUIRE(mode == 2 || pm.ptr || pm.width == 0, "open_begin: prover data without matrices (a placeholder needs mode 2)");
+            const u64 gh = pm.height * n_shards;
+            msgpu_open::Mat m{pm.ptr, gh, pm.width, ilog2(gh), {}, {}, (u64)shard * pm.height, pm.height};
+            MSG_REQUIRE(pm.ptr || pm.width == 0, "open_begin: prover data holds a matrix without device memory");
             MSG_REQUIRE(m.log_h >= log_blowup, "open_begin: committed matrix shorter than the blowup");
             u64 np = n_points[mi++];
             for (u64 k = 0; k < np; k++, pi++) {
@@ -781,16 +769,16 @@ extern "C" {
 
 int msgpu_open_begin(msgpu_ctx* h, uint64_t n_rounds, const msgpu_pdata* const* pds, const uint64_t* n_points,
                      const uint64_t* points, uint32_t log_blowup, msgpu_open** out, uint64_t* n_values) {
-    return guard([&] { open_begin_impl(h, n_rounds, pds, nullptr, 0, 1, 1, n_points, points, log_blowup, out, n_values); });
+    return guard([&] { open_begin_impl(h, n_rounds, pds, false, 0, 1, 1, n_points, points, log_blowup, out, n_values); });
 }
 
 // ---- Pcs::open over ROW SHARDS (one proof over several GPUs) -----------------------------------------------------------------
-int msgpu_open_begin_shard(msgpu_ctx* h, uint64_t n_rounds, const msgpu_pdata* const* pds, const uint32_t* modes, uint32_t shard,
-                           uint32_t n_shards, int fri_owner, const uint64_t* n_points, const uint64_t* points, uint32_t log_blowup,
-                           msgpu_open** out, uint64_t* n_values, uint64_t* n_sums) {
+int msgpu_open_begin_shard(msgpu_ctx* h, uint64_t n_rounds, const msgpu_pdata* const* pds, uint32_t shard, uint32_t n_shards,
+                           int fri_owner, const uint64_t* n_points, const uint64_t* points, uint32_t log_blowup, msgpu_open** out,
+                           uint64_t* n_values, uint64_t* n_sums) {
     return guard([&] {
-        MSG_REQUIRE(modes && n_sums && n_shards >= 1 && shard < n_shards && is_pow2(n_shards), "open_begin_shard: bad argument");
-        open_begin_impl(h, n_rounds, pds, modes, shard, n_shards, fri_owner, n_points, points, log_blowup, out, n_values);
+        MSG_REQUIRE(n_sums && n_shards >= 1 && shard < n_shards && is_pow2(n_shards), "open_begin_shard: bad argument");
+        open_begin_impl(h, n_rounds, pds, true, shard, n_shards, fri_owner, n_points, points, log_blowup, out, n_values);
         *n_sums = (*out)->raw_sums.size();
     });
 }
@@ -805,21 +793,6 @@ int msgpu_open_finish_values(msgpu_open* op, const uint64_t* total_sums) {
         MSG_REQUIRE(op && op->sharded && !op->pending_sums.empty() && (total_sums || op->raw_sums.empty()), "open_finish_values: nothing pending");
         for (size_t i = 0; i < op->raw_sums.size(); i++) MSG_REQUIRE(total_sums[i] < GLD_P, "open_finish_values: sum is not canonical");
         finish_values(op, (const u64*)total_sums);
-    });
-}
-// prover data that carries shapes only (a round whose matrices live on other ranks)
-int msgpu_pdata_placeholder(msgpu_ctx* h, uint64_t n_mats, const uint64_t* heights, const uint64_t* widths, msgpu_pdata** out) {
-    return guard([&] {
-        MSG_REQUIRE(out && n_mats > 0 && heights && widths, "pdata_placeholder: bad argument");
-        auto pd = std::make_unique<msgpu_pdata>();
-        for (u64 i = 0; i < n_mats; i++) {
-            MSG_REQUIRE(is_pow2(heights[i]), "pdata_placeholder: heights must be powers of two");
-            pd->mats.push_back(msgpu_pdata::Mat{nullptr, heights[i], widths[i]});
-            pd->total_width += widths[i];
-            pd->max_height = std::max<u64>(pd->max_height, heights[i]);
-        }
-        memset(pd->root, 0, 32);
-        *out = pd.release();
     });
 }
 // dst[i] += src[i] / v[i] += c over n extension elements (device pointers)

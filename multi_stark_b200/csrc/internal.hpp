@@ -241,8 +241,6 @@ struct AsmTarget {
 };
 // digests[i] = BLAKE3(le_bytes(row i of mats[0]) || le_bytes(row i of mats[1]) ...), all mats same height
 void b3_hash_rows(Ctx& c, const std::vector<MatRef>& mats, uint8_t* digests, const std::vector<AsmTarget>& assemble = {});
-// next[i] = H(prev[2i] || prev[2i+1]), optionally followed by H(that || inject[i])
-void b3_compress_layer(Ctx& c, const uint8_t* prev, const uint8_t* inject, uint8_t* next, u64 next_len);
 
 // `levels` node layers in one launch (each CTA reduces 2^levels adjacent digests through shared memory)
 void b3_merkle_subtrees(Ctx& c, const uint8_t* in, u64 len, u32 levels, uint8_t* const* out, const uint8_t* const* inject);

@@ -269,26 +269,6 @@ __global__ void __launch_bounds__(kLeafThreads) k_hash_rows_direct(const __grid_
     o[1] = make_uint4(dg[4], dg[5], dg[6], dg[7]);
 }
 
-__global__ void __launch_bounds__(256) k_compress_layer(const uint4* prev, const uint4* inject, uint4* next, u64 next_len) {
-    u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= next_len) return;
-    uint4 a0 = prev[4 * i], a1 = prev[4 * i + 1], b0 = prev[4 * i + 2], b1 = prev[4 * i + 3];
-    u32 l[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
-    u32 r[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
-    u32 d[8];
-    b3::hash_pair(l, r, d);
-    if (inject) {
-        uint4 c0 = inject[2 * i], c1 = inject[2 * i + 1];
-        u32 x[8] = {c0.x, c0.y, c0.z, c0.w, c1.x, c1.y, c1.z, c1.w};
-        u32 d2[8];
-        b3::hash_pair(d, x, d2);
-#pragma unroll
-        for (int k = 0; k < 8; k++) d[k] = d2[k];
-    }
-    next[2 * i] = make_uint4(d[0], d[1], d[2], d[3]);
-    next[2 * i + 1] = make_uint4(d[4], d[5], d[6], d[7]);
-}
-
 // Several node layers per launch: a CTA owns `chunk` adjacent digests of the input layer and reduces them to one,
 // level by level through shared memory, writing every intermediate layer to its place in the tree (the prover data
 // keeps all layers for the opening proofs). Level l output i = H(in[2i] || in[2i+1]), then H(that || inject_l[i]) when
@@ -542,12 +522,6 @@ void b3_hash_rows(Ctx& c, const std::vector<MatRef>& mats, uint8_t* digests, con
         launch(c, "k_hash_rows_direct", k_hash_rows_direct, (unsigned)blocks, kLeafThreads, 0, d_mats, (u32)lm.size(), height, total_words,
                (u32*)digests);
     }
-}
-
-void b3_compress_layer(Ctx& c, const uint8_t* prev, const uint8_t* inject, uint8_t* next, u64 next_len) {
-    if (next_len == 0) return;
-    u64 blocks = (next_len + 255) / 256;
-    launch(c, "k_compress_layer", k_compress_layer, (unsigned)blocks, 256, 0, (const uint4*)prev, (const uint4*)inject, (uint4*)next, next_len);
 }
 
 // Reduces the layer `in` (len digests) by `levels` levels. out[l] / inject[l]: output layer l+1 and its injected digests.

@@ -250,10 +250,11 @@ __global__ void __launch_bounds__(256) k_interleave_columns(const __grid_constan
     }
 }
 
-// blocks[b][r][c] = in[r][col0_b + c]: the inverse (row block -> per-destination column blocks, back to back in `out`)
+// out[b][r][c] = in[r][col0_b + c]: the inverse (row block -> per-destination column blocks). The row block is read once,
+// coalesced; consecutive threads write consecutive addresses of one destination block except at the block boundaries of a row.
 struct PackParams {
     const u64* in;
-    u64* out;
+    u64* out[kMaxBlocks];
     u32 col0[kMaxBlocks + 1];
     u32 n_blocks;
     u64 rows;
@@ -267,19 +268,21 @@ __global__ void __launch_bounds__(256) k_pack_columns(const __grid_constant__ Pa
         u32 b = 0;
         while (b + 1 < p.n_blocks && p.col0[b + 1] <= col) b++;
         const u32 wb = p.col0[b + 1] - p.col0[b];
-        p.out[p.rows * p.col0[b] + r * wb + (col - p.col0[b])] = p.in[e];
+        p.out[b][r * wb + (col - p.col0[b])] = p.in[e];
     }
 }
-void pack_column_blocks(Ctx& c, const u64* src, u64 rows, u64 width, const std::vector<u64>& c0, const std::vector<u64>& c1, u64* dst) {
-    MSG_REQUIRE(!c0.empty() && c0.size() == c1.size() && c0.size() <= (size_t)kMaxBlocks, "pack_column_blocks: 1..16 blocks");
+void pack_column_blocks(Ctx& c, const u64* src, u64 rows, u64 width, const std::vector<u64>& c0, const std::vector<u64>& c1,
+                        const std::vector<u64*>& dst) {
+    MSG_REQUIRE(!c0.empty() && c0.size() == c1.size() && c0.size() == dst.size() && c0.size() <= (size_t)kMaxBlocks,
+                "pack_column_blocks: 1..16 blocks");
     PackParams pp{};
     pp.in = src;
-    pp.out = dst;
     pp.n_blocks = (u32)c0.size();
     pp.rows = rows;
     for (size_t b = 0; b < c0.size(); b++) {
         MSG_REQUIRE(c0[b] == (b ? c1[b - 1] : 0) && c1[b] >= c0[b], "pack_column_blocks: blocks must tile the columns in order");
         pp.col0[b] = (u32)c0[b];
+        pp.out[b] = dst[b];
     }
     MSG_REQUIRE(c1.back() == width, "pack_column_blocks: blocks must cover every column");
     pp.col0[c0.size()] = (u32)width;

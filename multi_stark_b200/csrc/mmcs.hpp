@@ -48,7 +48,9 @@ void mmcs_build_local(Ctx& c, msgpu_pdata* pd);
 void mmcs_build_from_classes(Ctx& c, msgpu_pdata* pd, const std::vector<std::pair<u64, const uint8_t*>>& classes);
 // allocates pd->digests for a tree over max_h leaves and fills layer_off / layer_len (layer 0 = leaf digests)
 void mmcs_layout_layers(Ctx& c, msgpu_pdata* pd, u64 max_h);
-// row block (rows x width) -> column blocks [c0[b], c1[b]) as contiguous matrices back to back in dst, and the inverse
-void pack_column_blocks(Ctx& c, const u64* src, u64 rows, u64 width, const std::vector<u64>& c0, const std::vector<u64>& c1, u64* dst);
+// row block (rows x width) -> column blocks [c0[b], c1[b]), block b a dense rows x (c1[b] - c0[b]) matrix at dst[b] (back to back
+// in one buffer, or in the peers' windows); and the inverse, from blocks back to back in src
+void pack_column_blocks(Ctx& c, const u64* src, u64 rows, u64 width, const std::vector<u64>& c0, const std::vector<u64>& c1,
+                        const std::vector<u64*>& dst);
 void interleave_column_blocks(Ctx& c, const u64* src, u64 rows, const std::vector<u64>& widths, u64* dst);
 }  // namespace msg

@@ -1,16 +1,18 @@
 // Peer memory over NVLink / NVSwitch: symmetric device windows mapped into every rank of one node with CUDA IPC, so that the
 // kernels of the row-sharded prover (host/rowshard_backend.hpp) read their inputs from, and write their results into, the other
 // GPUs' HBM directly instead of going through pack -> NCCL all-to-all -> unpack:
-//   * k_peer_pack_push turns a rank's natural-order row block into column blocks written straight into the owners' windows,
-//   * k_peer_pull_interleave assembles a rank's row shard from the peers' column blocks of the LDE with remote loads,
-//     (both sides of the transfer are whole lines: an NTT pass that gathered / scattered its 8-56-byte row segments itself
-//     ran at 190 GB/s over NVLink, profiles/rowshard_step_r2.md)
-//   * 32-byte subtree roots and other small per-rank results are written into every peer's window (k_peer_put),
+//   * msgpu_peers_pack_push turns a rank's natural-order row block into column blocks written straight into the owners'
+//     windows; it launches the column-block pack of the collective path, k_pack_columns (mmcs.cu). The stores are whole lines:
+//     an NTT pass that scattered its 8-56-byte row segments itself ran at 190 GB/s over NVLink (profiles/rowshard_step_r2.md).
+//   * 32-byte subtree roots are written into every peer's window (k_peer_put),
 //   * ordering is a flag barrier in peer memory (k_peer_barrier): one store per peer, one spin per peer, no host round trip.
+// The leaf-hash pass of the commitment reads the peers' column blocks of the LDE through msgpu_peers_ptr
+// (msgpu_commit_ldes_blocks_dev).
 // One process per GPU; the 64-byte IPC handles travel once per window over the caller's host all-gather. The allocator inside a
 // window is deterministic (first fit, lowest offset): every rank performs the same sequence of calls with the same sizes, so a
 // block has the same (segment, offset) on every rank and no addresses are ever exchanged.
 #include "capi_common.hpp"
+#include "mmcs.hpp"
 #include "peer_heap.hpp"
 
 #include <cstring>
@@ -58,48 +60,6 @@ __global__ void k_peer_put(PeerBases b, size_t off_bytes, const u64* __restrict_
         const int e = (int)(t / words);
         const u64 i = t % words;
         ((u64*)(b.p[e] + off_bytes))[(u64)rank * words + i] = src[i];
-    }
-}
-
-// out_b[r][c] = in[r][col0_b + c]: the row block is read once, coalesced; consecutive threads write consecutive addresses of one
-// destination block except at the block boundaries of a row
-struct PushParams {
-    const u64* in;
-    u64* out[kMaxPeers];
-    u32 col0[kMaxPeers + 1];
-    u32 n_blocks;
-    u64 rows;
-};
-__global__ void __launch_bounds__(256) k_peer_pack_push(const __grid_constant__ PushParams p) {
-    const u32 W = p.col0[p.n_blocks];
-    const u64 total = p.rows * W;
-    for (u64 e = (u64)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (u64)gridDim.x * blockDim.x) {
-        const u64 r = e / W;
-        const u32 col = (u32)(e % W);
-        u32 b = 0;
-        while (b + 1 < p.n_blocks && p.col0[b + 1] <= col) b++;
-        const u32 wb = p.col0[b + 1] - p.col0[b];
-        p.out[b][r * wb + (col - p.col0[b])] = p.in[e];
-    }
-}
-// out[r][col0_b + c] = blocks[b][r][c]
-struct PullParams {
-    const u64* blocks[kMaxPeers];
-    u32 col0[kMaxPeers + 1];
-    u32 n_blocks;
-    u64 rows;
-    u64* out;
-};
-__global__ void __launch_bounds__(256) k_peer_pull_interleave(const __grid_constant__ PullParams p) {
-    const u32 W = p.col0[p.n_blocks];
-    const u64 total = p.rows * W;
-    for (u64 e = (u64)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (u64)gridDim.x * blockDim.x) {
-        const u64 r = e / W;
-        const u32 col = (u32)(e % W);
-        u32 b = 0;
-        while (b + 1 < p.n_blocks && p.col0[b + 1] <= col) b++;
-        const u32 wb = p.col0[b + 1] - p.col0[b];
-        p.out[e] = p.blocks[b][r * wb + (col - p.col0[b])];
     }
 }
 }  // namespace
@@ -207,8 +167,6 @@ int msgpu_peers_segment_open_local(msgpu_peers* p, void* const* bases) {
     });
 }
 
-uint64_t msgpu_peers_num_segments(const msgpu_peers* p) { return p->segs.size(); }
-
 // Deterministic first fit. Returns 1 (not an error: no last-error text) when no window has room: the caller grows collectively.
 int msgpu_peers_alloc(msgpu_peers* p, uint64_t bytes, uint32_t* seg, uint64_t* off) {
     int rc = 1;
@@ -251,23 +209,6 @@ int msgpu_peers_barrier(msgpu_peers* p) {
     });
 }
 
-// All-gather by remote stores: every peer's block (seg, off) receives `bytes` (a multiple of 8) from this rank at
-// off + rank * bytes. Not ordered against the peers: follow with msgpu_peers_barrier.
-int msgpu_peers_put(msgpu_peers* p, const void* src_dev, uint32_t seg, uint64_t off, uint64_t bytes) {
-    return guard([&] {
-        MSG_REQUIRE(p && src_dev && seg < p->segs.size() && p->segs[seg].opened && bytes % 8 == 0, "peers: bad put");
-        MSG_REQUIRE(off + bytes * (uint64_t)p->world <= p->segs[seg].bytes, "peers: put outside the segment");
-        if (bytes == 0) return;
-        Ctx& c = *p->c;
-        PeerBases b{};
-        for (int e = 0; e < p->world; e++) b.p[e] = p->segs[seg].base[e];
-        const u64 words = bytes / 8, total = words * (u64)p->world;
-        StageScope ss(c, "exchange");
-        launch(c, "k_peer_put", k_peer_put, (unsigned)std::min<u64>((total + 255) / 256, (u64)c.sm_count * 8), 256, 0, b, (size_t)off,
-               (const u64*)src_dev, words, p->rank, p->world);
-    });
-}
-
 // The 32-byte subtree roots of a row-sharded commitment: this rank's root goes into slot `rank` of the current ring entry on
 // every peer; returns the local address of the entry (world x 32 bytes, complete after the next msgpu_peers_barrier). Two ring
 // entries: a peer can run at most one commitment ahead of the slowest rank (it needs that rank's barrier flag to go further).
@@ -301,52 +242,19 @@ int msgpu_peers_pack_push(msgpu_peers* p, const uint64_t* src_dev, uint64_t rows
     return guard([&] {
         MSG_REQUIRE(p && src_dev && seg < p->segs.size() && p->segs[seg].opened && width >= 1, "peers: bad pack_push");
         if (rows == 0) return;
-        Ctx& c = *p->c;
         const u64 N = (u64)p->world, base = width / N, rem = width % N;
-        PushParams pp{};
-        pp.in = (const u64*)src_dev;
-        pp.rows = rows;
-        pp.n_blocks = (u32)N;
+        std::vector<u64> c0(N), c1(N);
+        std::vector<u64*> dst(N);
         u64 col = 0;
         for (u64 e = 0; e < N; e++) {
             const u64 wd = base + (e < rem ? 1 : 0);
             MSG_REQUIRE(off + rows * N * wd * 8 <= p->segs[seg].bytes, "peers: pack_push outside the segment");
-            pp.col0[e] = (u32)col;
-            pp.out[e] = (u64*)(p->segs[seg].base[e] + off) + (u64)p->rank * rows * wd;
-            col += wd;
+            c0[e] = col;
+            c1[e] = col += wd;
+            dst[e] = (u64*)(p->segs[seg].base[e] + off) + (u64)p->rank * rows * wd;
         }
-        pp.col0[N] = (u32)width;
-        StageScope ss(c, "exchange");
-        launch(c, "k_peer_pack_push", k_peer_pack_push, (unsigned)std::min<u64>((rows * width + 255) / 256, (u64)c.sm_count * 16), 256, 0, pp);
-    });
-}
-
-// Column blocks -> row shard by remote loads. Block (seg, off) of rank e's window is e's dense column block of the LDE
-// (rows * world x wd_e); this rank reads rows [rank * rows, (rank + 1) * rows) of every peer's block (contiguous: full-line NVLink
-// loads) and writes its shard dst (rows x width, local, row-major over all columns). Needs a barrier before (the peers' LDEs are
-// complete) and one after, before the peers release their blocks.
-int msgpu_peers_pull_interleave(msgpu_peers* p, uint32_t seg, uint64_t off, uint64_t rows, uint64_t width, uint64_t* dst_dev) {
-    return guard([&] {
-        MSG_REQUIRE(p && dst_dev && seg < p->segs.size() && p->segs[seg].opened && width >= 1, "peers: bad pull_interleave");
-        if (rows == 0) return;
-        Ctx& c = *p->c;
-        const u64 N = (u64)p->world, base = width / N, rem = width % N;
-        PullParams pp{};
-        pp.out = (u64*)dst_dev;
-        pp.rows = rows;
-        pp.n_blocks = (u32)N;
-        u64 col = 0;
-        for (u64 e = 0; e < N; e++) {
-            const u64 wd = base + (e < rem ? 1 : 0);
-            MSG_REQUIRE(off + rows * N * wd * 8 <= p->segs[seg].bytes, "peers: pull_interleave outside the segment");
-            pp.col0[e] = (u32)col;
-            pp.blocks[e] = (const u64*)(p->segs[seg].base[e] + off) + (u64)p->rank * rows * wd;
-            col += wd;
-        }
-        pp.col0[N] = (u32)width;
-        StageScope ss(c, "exchange");
-        launch(c, "k_peer_pull_interleave", k_peer_pull_interleave, (unsigned)std::min<u64>((rows * width + 255) / 256, (u64)c.sm_count * 16), 256,
-               0, pp);
+        StageScope ss(*p->c, "exchange");
+        pack_column_blocks(*p->c, (const u64*)src_dev, rows, width, c0, c1, dst);
     });
 }
 

@@ -562,7 +562,6 @@ class RowShardOpenDevice : public ShardedOpenDevice {
     RowShardOpenDevice(RowShardBackend& be, const std::vector<OpenRound>& rounds, uint32_t log_blowup) : ShardedOpenDevice(be.ctx(), be.comm(), rounds) {
         const int N = comm_.world(), d = comm_.rank();
         std::vector<const msgpu_pdata*> pds;
-        std::vector<uint32_t> modes;
         std::vector<uint64_t> npts, pts;
         size_t max_h = 0;
         for (auto& r : rounds) {
@@ -571,7 +570,6 @@ class RowShardOpenDevice : public ShardedOpenDevice {
             if (r.points.size() != h->shapes.size()) throw DistError("open: one point list per committed matrix expected");
             handles_.push_back(h);
             pds.push_back(h->local.get());
-            modes.push_back(1);
             for (size_t m = 0; m < h->shapes.size(); m++) {
                 max_h = std::max(max_h, h->shapes[m].first);
                 npts.push_back(r.points[m].size());
@@ -581,7 +579,7 @@ class RowShardOpenDevice : public ShardedOpenDevice {
         log_max_height_ = log2_strict(max_h);
         if (pts.empty()) pts.push_back(0);
         uint64_t n_sums = 0;
-        gpu_check(msgpu_open_begin_shard(ctx_, pds.size(), pds.data(), modes.data(), (uint32_t)d, (uint32_t)N, d == fri_owner_ ? 1 : 0, npts.data(),
+        gpu_check(msgpu_open_begin_shard(ctx_, pds.size(), pds.data(), (uint32_t)d, (uint32_t)N, d == fri_owner_ ? 1 : 0, npts.data(),
                                          pts.data(), log_blowup, &op_, &n_values_, &n_sums));
         rs_trace(d, "open_begin done", n_sums);
         // barycentric sums of all ranks, added in the field

@@ -210,10 +210,9 @@ class Opening:
             check(self.L.msgpu_open_begin(ctx.h, len(pds), arr, _u64p(npts), _u64p(pts), log_blowup, C.byref(self.h), C.byref(nv)))
         else:
             index, n_shards, owner = shard
-            modes = np.ones(len(pds), dtype=np.uint32)
             ns = C.c_uint64()
-            check(self.L.msgpu_open_begin_shard(ctx.h, len(pds), arr, _ptr(modes), index, n_shards, owner, _ptr(npts), _ptr(pts),
-                                                log_blowup, C.byref(self.h), C.byref(nv), C.byref(ns)))
+            check(self.L.msgpu_open_begin_shard(ctx.h, len(pds), arr, index, n_shards, owner, _ptr(npts), _ptr(pts), log_blowup,
+                                                C.byref(self.h), C.byref(nv), C.byref(ns)))
             self.n_sums = int(ns.value)
         self.n_values = int(nv.value)
         assert self.n_values == sum(len(m.points) * m.w for r in rounds for m in r)
@@ -602,7 +601,7 @@ def test_device_transcript_zero_rounds_and_refusals(gpu):
 
 # ---- a row-sharded opening on one GPU ----------------------------------------------------------------------------------
 @pytest.mark.gpu
-def test_sharded_opening_matches_unsharded(gpu):
+def test_row_shard_opening_matches_unsharded(gpu):
     """Two row shards of a 19-column matrix (msgpu_open_begin_shard): the summed barycentric sums give the unsharded values,
     and the non-owner's reduced rows added into the owner's give the unsharded input."""
     ms, ctx = gpu

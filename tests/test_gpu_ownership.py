@@ -41,35 +41,6 @@ def arena_unchanged(ctx):
 
 
 # ---- refused calls ----------------------------------------------------------------------------------------------------------
-def test_reduce_refusing_mixed_shard_rows_frees_its_vectors(gpu):
-    """fri_owner = 0 with a whole (mode 0) and a row-sharded (mode 1) round of one global height: the reduced-openings vector
-    of that height is allocated for the first matrix, then the second is refused."""
-    ms, ctx = gpu
-    from multi_stark_b200._ffi import check
-    rnd = random.Random(41)
-    lb = 1
-    whole = Mat(rand_coeffs(rnd, 8, 3), 3, lb, [rand_ext(rnd)])   # LDE height 16, all rows here
-    shard = Mat(rand_coeffs(rnd, 4, 2), 2, lb, [rand_ext(rnd)])   # 8 rows: shard 0 of 2 of a height-16 matrix
-    start = in_use(ctx)
-    pds = commit_rounds(ms, ctx, [[whole], [shard]], lb)
-    npts = np.array([1, 1], dtype=np.uint64)
-    pts = np.array([v for m in (whole, shard) for z in m.points for v in (z.a, z.b)], dtype=np.uint64)
-    modes = np.array([0, 1], dtype=np.uint32)
-    arr = (C.c_void_p * 2)(*[pd.h for pd in pds])
-    op, nv, ns = C.c_void_p(), C.c_uint64(), C.c_uint64()
-    check(ctx.L.msgpu_open_begin_shard(ctx.h, 2, arr, _ptr(modes), 0, 2, 0, _ptr(npts), _ptr(pts), lb, C.byref(op), C.byref(nv),
-                                       C.byref(ns)))
-    alpha = np.array([5, 7], dtype=np.uint64)
-    n, lmh = C.c_uint64(), C.c_uint32()
-    with arena_unchanged(ctx):
-        assert ctx.L.msgpu_open_reduce(op, _ptr(alpha), C.byref(n), C.byref(lmh)) != 0
-        assert b"cover the same rows" in ctx.L.msgpu_last_error()
-    ctx.L.msgpu_open_free(op)
-    for pd in pds:
-        pd.free()
-    assert in_use(ctx) == start
-
-
 def test_reduce_refusing_4267_columns(gpu):
     ms, ctx = gpu
     from multi_stark_b200._ffi import MsgpuError
@@ -182,6 +153,27 @@ def test_commit_open_reduce_commit_phase_then_free(gpu):
         rc, roots, _ = op.commit_phase(b"y" * 40, 1, 16)
         assert rc == 0 and len(roots) == 10
         free_all(op, pds)
+
+
+def test_sharded_open_reduce_then_free(gpu):
+    """A rank that does not run the FRI commit phase (fri_owner = 0) holds shard 0 of 2 of two heights: its reduced-openings
+    vectors cover only the rows it holds, and freeing the opening and the prover data returns every byte."""
+    ms, ctx = gpu
+    from multi_stark_b200._ffi import check
+    rnd = random.Random(41)
+    lb = 1
+    tall = Mat(rand_coeffs(rnd, 8, 3), 3, lb, [rand_ext(rnd)])    # 16 rows: shard 0 of 2 of a height-32 matrix
+    short = Mat(rand_coeffs(rnd, 4, 2), 2, lb, [rand_ext(rnd)])   # 8 rows: shard 0 of 2 of a height-16 matrix
+    start = in_use(ctx)
+    pds = commit_rounds(ms, ctx, [[tall], [short]], lb)
+    op = Opening(ctx, pds, [[tall], [short]], lb, shard=(0, 2, 0))
+    sums = np.zeros(max(op.n_sums, 1), dtype=np.uint64)
+    check(ctx.L.msgpu_open_sums(op.h, _ptr(sums)))
+    check(ctx.L.msgpu_open_finish_values(op.h, _ptr(sums)))
+    assert op.reduce(E(5, 7)) == (2, 4)
+    assert [len(op.read_input(k)) // 2 for k in range(2)] == [16, 8]
+    free_all(op, pds)
+    assert in_use(ctx) == start
 
 
 def test_program_create_and_free(gpu):

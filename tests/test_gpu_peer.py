@@ -64,7 +64,7 @@ def _col_split(w, n):
 
 
 @pytest.mark.parametrize("world,log_n,w,lb", [(2, 12, 14, 1), (4, 12, 26, 1), (8, 12, 14, 1), (4, 11, 2, 2), (8, 13, 3, 1)])
-def test_peer_abi_in_process_ranks(world, log_n, w, lb):
+def test_peer_push_and_root_ring_in_process_ranks(world, log_n, w, lb):
     import multi_stark_b200 as ms
     from multi_stark_b200._ffi import check
     from tests import _oracle as orc
@@ -99,12 +99,10 @@ def test_peer_abi_in_process_ranks(world, log_n, w, lb):
         check(L.msgpu_coset_lde_batch_bitrev_dev(ctxs[r].h, C.c_void_p(a), n, wd, lb, 7, C.c_void_p(b)))
         sh = ctxs[r].upload(np.ascontiguousarray(want_lde[:Ls]))
         sh2 = ctxs[r].malloc(Ls * w * 8)
-        sh3 = ctxs[r].malloc(Ls * w * 8)
-        tg = ctxs[r].malloc(16)
         rr = ctxs[r].upload(np.ascontiguousarray(m[:nb]))
         _, pdw = ms.GpuPcs(ctxs[r], lb).commit_ldes([(sh, Ls, w)])
         pdw.free()
-        for q in (a, b, sh, sh2, sh3, tg, rr):
+        for q in (a, b, sh, sh2, rr):
             ctxs[r].free(q)
         ctxs[r].sync()
     bases = (C.c_void_p * N)(*[L.msgpu_peers_ptr(peers[r], 0, 0, r) for r in range(N)])
@@ -118,11 +116,9 @@ def test_peer_abi_in_process_ranks(world, log_n, w, lb):
             check(L.msgpu_peers_alloc(peers[r], n * wmax * 8, C.byref(seg), C.byref(off)))
             col = (seg.value, off.value)
             check(L.msgpu_peers_alloc(peers[r], H * wmax * 8, C.byref(seg), C.byref(off)))
-            lde = (seg.value, off.value)
-            check(L.msgpu_peers_alloc(peers[r], 16 * N, C.byref(seg), C.byref(off)))
-            blocks.append((col, lde, (seg.value, off.value)))
+            blocks.append((col, (seg.value, off.value)))
         assert all(b == blocks[0] for b in blocks)
-        (cseg, coff), (lseg, loff), (pseg, poff) = blocks[0]
+        (cseg, coff), (lseg, loff) = blocks[0]
         # phase 1: upload the row block, push it into every owner's column block, barrier
         row_dev = []
         for r in range(N):
@@ -138,15 +134,8 @@ def test_peer_abi_in_process_ranks(world, log_n, w, lb):
                                                          C.c_void_p(L.msgpu_peers_ptr(peers[r], lseg, loff, r))))
             check(L.msgpu_peers_barrier(peers[r]))
         # phase 3: the leaf pass assembles rank r's row shard from every rank's LDE column block; subtree root -> ring; barrier
-        pds, shards, gathered, pulled, tags = [], [], [], [], []
+        pds, shards, gathered = [], [], []
         for r in range(N):
-            # the unfused form of the exchange (remote loads by a pass of its own) and the generic all-gather by remote stores
-            pull = ctxs[r].malloc(Ls * w * 8)
-            pulled.append(pull)
-            check(L.msgpu_peers_pull_interleave(peers[r], lseg, loff, Ls, w, C.c_void_p(pull)))
-            tag = ctxs[r].upload(np.array([r, 1000 + r * r], dtype=np.uint64))
-            tags.append(tag)
-            check(L.msgpu_peers_put(peers[r], C.c_void_p(tag), pseg, poff, 16))
             shard = ctxs[r].malloc(Ls * w * 8)
             shards.append(shard)
             blks = [(L.msgpu_peers_ptr(peers[r], lseg, loff, e) + r * Ls * split[e][1] * 8, split[e][1]) for e in range(N)]
@@ -177,16 +166,10 @@ def test_peer_abi_in_process_ranks(world, log_n, w, lb):
             assert roots[r] == bytes(want_root), "rank %d: root differs from the single-GPU commitment" % r
             got = ctxs[r].download(shards[r], (Ls, w))
             assert np.array_equal(got, want_lde[r * Ls:(r + 1) * Ls]), "rank %d: row shard differs from the single-GPU LDE" % r
-            assert np.array_equal(ctxs[r].download(pulled[r], (Ls, w)), got), "rank %d: pull_interleave differs" % r
-            allg = ctxs[r].download(L.msgpu_peers_ptr(peers[r], pseg, poff, r), (N, 2))
-            assert allg.tolist() == [[e, 1000 + e * e] for e in range(N)], "rank %d: all-gather by remote stores" % r
         for r in range(N):
             pds[r].free()
             ctxs[r].free(shards[r])
-            ctxs[r].free(pulled[r])
-            ctxs[r].free(tags[r])
             ctxs[r].free(row_dev[r])
-            check(L.msgpu_peers_free_block(peers[r], pseg, poff))
             check(L.msgpu_peers_free_block(peers[r], cseg, coff))
             check(L.msgpu_peers_free_block(peers[r], lseg, loff))
     finally:
